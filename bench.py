@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — frames/s of MOPED's recognition core (MATCH..FILTER2) on the BASELINE.json workload.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json metric): synthetic 1000-object database (~1M 128-d descriptors), 640x480 frames of
@@ -280,6 +280,36 @@ def resolve_auto(args, world):
 # ------------------------------------------------------------------------------------------------
 # our arm
 # ------------------------------------------------------------------------------------------------
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_frame_results(path, frames, max_objects, seed=0):
+    """--dump-outputs: the per-frame results of one step (list of dict(model, pose, score, info) in frame order, as
+    mc_process_frames_dev returns them) as .npy files under `path`, one row per frame, objects in the order the call returned them:
+    frame_index [F] (frame of the batch), frame_info [F,4] {objects, status, accepted matches, clusters after CLUSTER},
+    obj_model [F,MO] (-1 = empty slot), obj_pose [F,MO,7] (qx qy qz qw tx ty tz; 0 in empty slots), obj_score [F,MO].
+    A batch larger than DUMP_LIMIT_BYTES keeps a fixed, seeded sample of its frames, so two runs write the same frames."""
+    per_frame = 8 * (1 + 4 + max_objects) + 4 * 8 * max_objects
+    idx = np.arange(len(frames))
+    keep = (DUMP_LIMIT_BYTES - 4096) // per_frame             # 4096: the five .npy headers
+    if len(frames) > keep:
+        idx = np.sort(np.random.default_rng(seed).choice(len(frames), keep, replace=False))
+    info = np.zeros((len(idx), 4), np.float64)
+    model = np.full((len(idx), max_objects), -1.0, np.float64)
+    pose = np.zeros((len(idx), max_objects, 7), np.float32)
+    score = np.zeros((len(idx), max_objects), np.float32)
+    for j, f in enumerate(idx):
+        fr = frames[f]
+        k = len(fr["model"])
+        info[j] = fr["info"]
+        model[j, :k] = fr["model"]
+        pose[j, :k] = fr["pose"]
+        score[j, :k] = fr["score"]
+    os.makedirs(path, exist_ok=True)
+    for name, a in (("frame_index", idx.astype(np.float64)), ("frame_info", info), ("obj_model", model), ("obj_pose", pose), ("obj_score", score)):
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def run_ours(args, rank, world, local_rank):
     os.environ.setdefault("CUDA_DEVICE_MAX_CONNECTIONS", "32")   # the frame lanes are concurrent streams
     os.environ.setdefault("NCCL_DEBUG_FILE", "/dev/stderr")      # NCCL's banner ("NCCL version ...") must not land on stdout beside the JSON line
@@ -486,10 +516,13 @@ def run_ours(args, rank, world, local_rank):
                 dist.all_reduce(t, op=dist.ReduceOp.MAX)
             return float(t.item()), ctx.launches - l0, n_obj, n_match
 
+    last_out = []                                     # per-frame results of the latest single-GPU step_dev (--dump-outputs)
+
     def step_dev(i):
         k = i % n_pool
         if world == 1:
             out = ctx.process_frames_dev(d_q[k].data_ptr(), d_xy[k].data_ptr(), d_img[k].data_ptr(), fo, params, MO)
+            last_out[:] = out
             return sum(len(o["model"]) for o in out), sum(int(o["info"][2]) for o in out)
         return sharded_step(d_q[k], d_xy[k], d_img[k])
 
@@ -549,6 +582,8 @@ def run_ours(args, rank, world, local_rank):
     if args.pipeline:
         total_ms, launches, n_obj, n_match = timed_pipe(False, args.steps, args.warmup)
         clocks = sampler.stop()
+        # the last timed step is step warmup + steps - 1; its all-gathered results are still in its host buffer
+        dumped = pblk.unpack(p_reshost[(args.warmup + args.steps - 1) % P].numpy()) if args.dump_outputs else None
         e2e_ms, _, n_obj_e, _ = timed_pipe(True, args.steps, args.warmup)
         kms = []                                      # dominant-kernel time: a separate short pass, reading the library's event pair
         for i in range(min(args.steps, 8)):           # after every step would put the host in lock-step with the match stream
@@ -561,6 +596,9 @@ def run_ours(args, rank, world, local_rank):
     else:
         total_ms, kms, launches, n_obj, n_match = timed(step_dev, args.steps, args.warmup, collect_kernel=True)
         clocks = sampler.stop()
+        dumped = None
+        if args.dump_outputs:                          # before the e2e leg reuses the result buffers
+            dumped = list(last_out) if world == 1 else blk.unpack(res_host.numpy())
         match_stats = np.array(mstats, np.int64) if mstats else np.zeros((1, 4), np.int64)
         tier_rows = list(mtiers)                      # (the e2e leg below reuses the lists)
         e2e_ms, _, _, n_obj_e, _ = timed(step_e2e, args.steps, args.warmup)
@@ -647,6 +685,9 @@ def run_ours(args, rank, world, local_rank):
                 out["cpu_baseline"] = {"value": None, "unit": UNIT, "cores": 0, "kind": "reference", "sample": f"failed: {e}"}
         if world == 1 and args.other_configs and default_metric_config(args):
             out["other_configs"] = other_config_lines()
+        if args.dump_outputs:
+            dump_frame_results(args.dump_outputs, dumped, MO)
+            log(f"[bench] outputs of the last timed step ({len(dumped)} frames) written to {args.dump_outputs}")
         print(json.dumps(out))
     if world > 1:
         dist.destroy_process_group()
@@ -1511,11 +1552,19 @@ def main():
                     help="ransac workload: 1 = persistent phase-synchronous thread-per-hypothesis kernel (default), 0 = the one-launch kernel; same results")
     ap.add_argument("--clusters", type=int, default=64)
     ap.add_argument("--hyp", type=int, default=2048, help="hypotheses per cluster (ransac workload)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="frames workload: after the timed steps, write the per-frame results of the last timed step as DIR/<name>.npy "
+                         "(see dump_frame_results); the inputs are seeded, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     resolve_auto(args, world)
+    cluster_partition_run = args.partition == "cluster" or (args.partition == "auto" and world > 1 and args.frames < world)
+    if args.dump_outputs and (args.workload != "frames" or args.impl != "ours" or cluster_partition_run):
+        ap.error("--dump-outputs covers the frames workload of --impl ours with the frames partitioned by GPU")
     if args.workload == "ransac":
         if args.impl == "reference":
             run_ransac_reference(args, rank, world)
@@ -1543,7 +1592,7 @@ def main():
             run_sift_ours(args, rank, world, local_rank)
     elif args.impl == "reference":
         run_reference(args, rank, world)
-    elif args.partition == "cluster" or (args.partition == "auto" and world > 1 and args.frames < world):
+    elif cluster_partition_run:
         args.warmup = max(args.warmup, 3)
         run_ours_cluster_partition(args, rank, world, local_rank)
     else:
