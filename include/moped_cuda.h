@@ -372,6 +372,54 @@ mc_status mc_cluster_linkage(mc_ctx *ctx, const float *match_xy, const float *ma
 mc_status mc_linkage_agglomerate(mc_ctx *ctx, const float *similarity, int n, float cutoff, int min_pts, int linkage_type,
                                  int32_t *n_clusters, int32_t *cluster_offsets, int32_t *members);
 
+/* ---- moped3d frames on the device: CLUSTER -> POSE -> FILTER -> POSE2 -> FILTER2 of moped3d's shipped pipeline
+ *      (moped3d/libmoped/src/config.hpp:45-49) in one call, from FrameData as DEPTHPROP leaves it ------------------------------- */
+typedef struct {
+	int32_t variant;              /* 0 = POSE_RANSAC_LM_DIFF_BACKPROJECTION_DEPTH (shipped), 1 = ..._REPROJECTION_DEPTH; the Cauchy
+	                               * scale of the fill distance follows (0.100 / 25.0) */
+	float cluster_cutoff; int32_t cluster_min_pts, cluster_use_3d_filter, cluster_linkage_type;   /* CLUSTER_LINKAGE, as mc_cluster_linkage */
+	float cluster_sigma_2d, cluster_sigma_3d;
+	mc_pose_params pose;  float pose_alpha;                                                      /* POSE (+ Alpha) */
+	int32_t filter_min_points;  float filter_feature_distance,  filter_min_score;                /* FILTER (FILTER_PROJECTION) */
+	mc_pose_params pose2; float pose2_alpha;                                                     /* POSE2 */
+	int32_t filter2_min_points; float filter2_feature_distance, filter2_min_score;               /* FILTER2 */
+} mc_depth_pipeline_params;
+
+/* the parameters addCudaRecognition3d registers (stages/pipeline3d_cuda.hpp; moped3d config.hpp:45-49); RANSAC seeds 1 and 2 */
+void mc_depth_pipeline_default_params(mc_depth_pipeline_params *p);
+
+/* A batch of n_frames frames (n_frames = 1: one frame). Per frame, the matches of every model as DEPTHPROP leaves them:
+ *   match_offsets  host, n_frames x (n_models + 1): row f is frame f's model-major CSR, global indices into the per-match arrays
+ *                  (ascending within a row; rows need not be contiguous)
+ *   per match      match_image (imageIdx), match_xy (coord2D, 2), match_xyz (coord3D, 3), match_world (depthData.coord3D, 3),
+ *                  match_fill (depthData.fillDistance), in FrameData::matches[model] order
+ *   depth / fill_distance  n_frames x height x width: the depth map and its ".distance" map of each frame
+ * Cameras come from mc_set_cameras (MC_ERR_STATE without them); no database is needed.
+ * Outputs as mc_process_frames: n_objects[f], obj_model / obj_score [f * max_objects + i], obj_pose [(f * max_objects + i) * 7],
+ * frame_info (optional) [4f..4f+3] = {objects, status (1 = a match outside the depth map), matches, clusters after CLUSTER}.
+ * stage_ms (optional, 5 floats): device time of CLUSTER, POSE, FILTER, POSE2, FILTER2 summed over the frames; with it the
+ * frames run one after another on one lane, without it they are dealt to the frame lanes (mc_set_tuning).
+ * Every frame gives exactly the result of the stage-by-stage calls (mc_cluster_linkage per model, mc_pose_depth_ransac with the
+ * match index as tie id, mc_filter_projection, ...). The models of a frame are clustered together: one launch per linkage kernel.
+ * Errors: MC_ERR_ARG for a model with more than 2048 matches in a frame, cluster_cutoff <= -1, n_pts_align outside 1..8,
+ * variant outside 0..1, offsets that do not ascend, or a match outside its frame's depth map (checked before any launch);
+ * MC_ERR_CAPACITY when a frame has more than max_objects objects (n_objects[f] holds the true count) or when the sum over a
+ * frame's models of n^2 exceeds 2^24 (the similarity matrices and merge lists would take more than 400 MB per lane). */
+mc_status mc_process_depth_frames(mc_ctx *ctx, const int32_t *match_offsets, int n_frames, int n_models,
+                                  const int32_t *match_image, const float *match_xy, const float *match_xyz, const float *match_world,
+                                  const float *match_fill, const float *depth, const float *fill_distance, int width, int height,
+                                  const mc_depth_pipeline_params *params, int max_objects,
+                                  int32_t *n_objects, int32_t *obj_model, float *obj_pose, float *obj_score, int32_t *frame_info, float *stage_ms);
+/* The same with the per-match arrays and the maps resident on the device (match_offsets and the outputs stay on the host).
+ * A match outside the depth map is found on the device: its frame reads nothing out of range, reports status 1 and no
+ * objects, and the call returns MC_ERR_ARG naming the first such frame. */
+mc_status mc_process_depth_frames_dev(mc_ctx *ctx, const int32_t *match_offsets, int n_frames, int n_models,
+                                      const int32_t *match_image_dev, const float *match_xy_dev, const float *match_xyz_dev,
+                                      const float *match_world_dev, const float *match_fill_dev, const float *depth_dev,
+                                      const float *fill_distance_dev, int width, int height, const mc_depth_pipeline_params *params,
+                                      int max_objects, int32_t *n_objects, int32_t *obj_model, float *obj_pose, float *obj_score,
+                                      int32_t *frame_info, float *stage_ms);
+
 /* Named integer options (scheduling / kernel-shape choices; unknown keys are an error):
  *   "pose_fit_thread_min"  mc_pose_hypotheses* calls with at least this many hypotheses and no inlier masks run one
  *                          THREAD per hypothesis instead of one 8-lane group (default 16384; 1 = always)
@@ -381,7 +429,7 @@ mc_status mc_linkage_agglomerate(mc_ctx *ctx, const float *similarity, int n, fl
  *                          Same arithmetic per hypothesis.
  *   "depth_team_lanes"     32 (default) or 8: lanes that share one explicit hypothesis in mc_pose_depth_hypotheses* (8 = four hypotheses
  *                          per warp). Results do not depend on it (the LM keeps levmar's summation order for any team width).
- *   "linkage_cached"       != 0: mc_cluster_linkage / mc_linkage_agglomerate with average linkage keep a cached maximum per row
+ *   "linkage_cached"       != 0: mc_cluster_linkage / mc_linkage_agglomerate / mc_process_depth_frames* with average linkage keep a cached maximum per row
  *                          (same merge sequence and clusters; O(n) per merge instead of an O(n^2) scan). Default 1 (2.7x at 600 matches
  *                          on B200); 0 = the O(n^2)-scan kernel.
  *   "pose_exact_order"     != 0: mc_pose_hypotheses / mc_pose_ransac (host entries) run the order-preserving LM of the depth stages

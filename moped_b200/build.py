@@ -15,7 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "libmoped_cuda.so")
-SOURCES = ["api.cu", "match.cu", "adaptive.cu", "cluster.cu", "pose.cu", "pose_exact.cu", "pose_depth.cu", "filter.cu", "pipeline.cu", "sift.cu", "linkage.cu", "sm_partition.cu", "model_db.cpp"]
+SOURCES = ["api.cu", "match.cu", "adaptive.cu", "cluster.cu", "pose.cu", "pose_exact.cu", "pose_depth.cu", "filter.cu", "pipeline.cu", "depth_frames.cu", "sift.cu", "linkage.cu", "sm_partition.cu", "model_db.cpp"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 COMMON = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC", "-Xcompiler", "-Wall"] + os.environ.get("MOPED_NVCC_FLAGS", "").split()
 LIB = os.environ.get("MOPED_LIB", LIB)

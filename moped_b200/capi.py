@@ -38,6 +38,17 @@ class PipelineParams(C.Structure):
                 ("pose2", PoseParams), ("filter2_min_points", C.c_int32), ("filter2_feature_distance", C.c_float), ("filter2_min_score", C.c_float)]
 
 
+class DepthPipelineParams(C.Structure):
+    """mc_depth_pipeline_params: moped3d's CLUSTER_LINKAGE -> POSE -> FILTER -> POSE2 -> FILTER2."""
+    _fields_ = [("variant", C.c_int32),
+                ("cluster_cutoff", C.c_float), ("cluster_min_pts", C.c_int32), ("cluster_use_3d_filter", C.c_int32), ("cluster_linkage_type", C.c_int32),
+                ("cluster_sigma_2d", C.c_float), ("cluster_sigma_3d", C.c_float),
+                ("pose", PoseParams), ("pose_alpha", C.c_float),
+                ("filter_min_points", C.c_int32), ("filter_feature_distance", C.c_float), ("filter_min_score", C.c_float),
+                ("pose2", PoseParams), ("pose2_alpha", C.c_float),
+                ("filter2_min_points", C.c_int32), ("filter2_feature_distance", C.c_float), ("filter2_min_score", C.c_float)]
+
+
 # every symbol include/moped_cuda.h declares: name -> (restype, argtypes)
 SIGNATURES = {
     "mc_create": (C.c_int, [C.POINTER(C.c_void_p), C.c_int]),
@@ -88,6 +99,11 @@ SIGNATURES = {
     "mc_cluster_linkage": (C.c_int, [C.c_void_p, _f32p, _f32p, _f32p, C.c_int, _f32p, _f32p, C.c_int, C.c_int, C.c_float, C.c_int, C.c_int, C.c_int,
                                      C.c_float, C.c_float, C.POINTER(C.c_int32), _i32p, _i32p, C.c_void_p]),
     "mc_linkage_agglomerate": (C.c_int, [C.c_void_p, _f32p, C.c_int, C.c_float, C.c_int, C.c_int, C.POINTER(C.c_int32), _i32p, _i32p]),
+    "mc_depth_pipeline_default_params": (None, [C.POINTER(DepthPipelineParams)]),
+    "mc_process_depth_frames": (C.c_int, [C.c_void_p, _i32p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, _f32p, _f32p,
+                                          C.c_int, C.c_int, C.POINTER(DepthPipelineParams), C.c_int, _i32p, _i32p, _f32p, _f32p, _i32p, C.c_void_p]),
+    "mc_process_depth_frames_dev": (C.c_int, [C.c_void_p, _i32p, C.c_int, C.c_int] + [C.c_void_p] * 7 + [C.c_int, C.c_int, C.POINTER(DepthPipelineParams),
+                                              C.c_int, _i32p, _i32p, _f32p, _f32p, _i32p, C.c_void_p]),
     "mc_sift_extract": (C.c_int, [C.c_void_p, _u8p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _i32p, _f32p, C.c_void_p, _f32p]),
     "mc_sift_extract_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "mc_process_images": (C.c_int, [C.c_void_p, _u8p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(PipelineParams), C.c_int, _i32p, _i32p,
@@ -580,6 +596,46 @@ class Context:
                                                  os_.reshape(-1), info.ctypes.data, times.ctypes.data if times is not None else None),
                     "mc_process_frames_dev")
         return self._unpack_frames(nf, max_objects, n_obj, om, op, os_, info)
+
+    # ---- moped3d frames
+    def default_depth_params(self) -> DepthPipelineParams:
+        p = DepthPipelineParams()
+        self.L.mc_depth_pipeline_default_params(C.byref(p))
+        return p
+
+    def _depth_frames(self, fn, what, match_offsets, n_models, arrays, params, max_objects, times):
+        p = params or self.default_depth_params()
+        mo = _i32(match_offsets).reshape(-1)
+        nf = len(mo) // (int(n_models) + 1)
+        n_obj = np.zeros(nf, np.int32)
+        om = np.zeros((nf, max_objects), np.int32)
+        op = np.zeros((nf, max_objects, 7), np.float32)
+        os_ = np.zeros((nf, max_objects), np.float32)
+        info = np.zeros((nf, 4), np.int32)
+        st = fn(self.h, mo, nf, int(n_models), *arrays, C.byref(p), int(max_objects), n_obj, om.reshape(-1), op.reshape(-1), os_.reshape(-1),
+                info.reshape(-1), times.ctypes.data if times is not None else None)
+        self._check(st, what)
+        return self._unpack_frames(nf, max_objects, n_obj, om, op, os_, info)
+
+    def process_depth_frames(self, match_offsets, n_models, match_image, match_xy, match_xyz, match_world, match_fill, depth, fill_distance,
+                             params=None, max_objects=64, times=None):
+        """moped3d CLUSTER..FILTER2 on host arrays. match_offsets: [n_frames, n_models + 1] global CSR rows; depth / fill_distance:
+        [n_frames, H, W] (or [H, W] for one frame). `times` (optional float32[5]) receives the per-step device time.
+        Returns a list of per-frame dict(model, pose, score, info)."""
+        d, fd = _f32(depth), _f32(fill_distance)
+        H, W = d.shape[-2], d.shape[-1]
+        keep = [_i32(match_image).reshape(-1), _f32(match_xy).reshape(-1), _f32(match_xyz).reshape(-1), _f32(match_world).reshape(-1),
+                _f32(match_fill).reshape(-1)]
+        arrays = [a.ctypes.data if a.size else None for a in keep] + [d.reshape(-1), fd.reshape(-1), W, H]
+        return self._depth_frames(self.L.mc_process_depth_frames, "mc_process_depth_frames", match_offsets, n_models, arrays, params, max_objects,
+                                  times)
+
+    def process_depth_frames_dev(self, match_offsets, n_models, image_ptr, xy_ptr, xyz_ptr, world_ptr, fill_ptr, depth_ptr, fill_distance_ptr,
+                                 width, height, params=None, max_objects=64, times=None):
+        """The same with the per-match arrays and maps on the device (pointers); match_offsets stays a host array."""
+        arrays = [image_ptr, xy_ptr, xyz_ptr, world_ptr, fill_ptr, depth_ptr, fill_distance_ptr, int(width), int(height)]
+        return self._depth_frames(self.L.mc_process_depth_frames_dev, "mc_process_depth_frames_dev", match_offsets, n_models, arrays, params,
+                                  max_objects, times)
 
     def process_frames_matched_dev(self, nn_row_ptr, acc_ptr, xy_ptr, img_ptr, frame_offsets, frame_begin, frame_end, params, max_objects,
                                    info_ptr, model_ptr, pose_ptr, score_ptr):

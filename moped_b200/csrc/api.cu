@@ -34,7 +34,8 @@ mc_status pose_depth_hypotheses_device(mc_ctx *ctx, int variant, const int32_t *
                                        float *d_lm_err, uint8_t *d_mask);
 mc_status pose_depth_ransac_device(mc_ctx *ctx, int variant, const int32_t *d_cluster_offsets, int n_clusters, int n_max, const float *d_xy,
                                    const float *d_xyz, const float *d_world, const float *d_cauchy, const int32_t *d_image, const int32_t *d_tie,
-                                   const mc_pose_params *pp, float alpha, uint8_t *d_found, float *d_pose, int32_t *d_n_tests);
+                                   const mc_pose_params *pp, float alpha, uint8_t *d_found, float *d_pose, int32_t *d_n_tests,
+                                   const int32_t *d_n_clusters);
 mc_status filter_device(mc_ctx *ctx, const int32_t *d_match_offsets, const int32_t *d_match_image, const float *d_match_xy,
                         const float *d_match_xyz, int n_models, int max_matches, const int32_t *d_obj_model, const float *d_obj_pose,
                         const int32_t *d_n_obj, int n_obj_cap, int min_points, float feat_dist, float min_score,
@@ -626,7 +627,7 @@ mc_status mc_pose_depth_ransac(mc_ctx *ctx, int variant, const int32_t *cluster_
 	MC_TRY(pose_depth_ransac_device(ctx, variant, (int32_t *)(b + o_co), n_clusters, largest_cluster(cluster_offsets, n_clusters), (float *)(b + o_xy),
 	                                (float *)(b + o_xyz), (float *)(b + o_w), (float *)(b + o_cw), (int32_t *)(b + o_im),
 	                                pt_tie ? (int32_t *)(b + o_tie) : nullptr, params, alpha, (uint8_t *)(b + o_f), (float *)(b + o_p),
-	                                (int32_t *)(b + o_nt)));
+	                                (int32_t *)(b + o_nt), nullptr));
 	MC_TRY(d2h(ctx, found, (const uint8_t *)(b + o_f), (size_t)n_tasks));
 	MC_TRY(d2h(ctx, pose, (const float *)(b + o_p), 7 * (size_t)n_tasks));
 	MC_TRY(d2h(ctx, n_tests, (const int32_t *)(b + o_nt), (size_t)n_tasks));

@@ -199,6 +199,35 @@ mc_status process_frame_sharded_device(mc_ctx *ctx, int phase, const int32_t *d_
                                        int max_objects, int32_t *d_out_info, int32_t *d_out_model, float *d_out_pose, float *d_out_score);
 mc_status match_device(mc_ctx *ctx, const float *d_q, int Q, float ratio, int mode,
                        int32_t *d_nn_row, float *d_nn_dist, uint8_t *d_accepted);
+
+// ---- frame lanes and chain pieces shared by the moped2 and moped3d frame chains (pipeline.cu) ----
+mc_status ensure_lanes(mc_ctx *ctx, int n);
+mc_status join_lanes(mc_ctx *ctx);
+mc_status gather_depth_points_device(mc_ctx *ctx, const int32_t *d_n, const int32_t *d_cluster_model, const int32_t *d_cluster_offsets,
+                                     const int32_t *d_members, const int32_t *d_match_offsets, const int32_t *d_match_image, const float *d_match_xy,
+                                     const float *d_match_xyz, const float *d_match_world, const float *d_match_fill, float cauchy_scale, float *d_pt_xy,
+                                     float *d_pt_xyz, float *d_pt_world, float *d_pt_cauchy, int32_t *d_pt_image, int32_t *d_pt_tie);
+mc_status copy_objects_device(mc_ctx *ctx, const int32_t *d_n, const int32_t *d_src_model, const float *d_src_pose, int32_t *d_dst_n,
+                              int32_t *d_dst_model, float *d_dst_pose);
+
+// ---- moped3d linkage clustering of all models of a frame at once (linkage.cu) ----
+struct LinkSlice {         // one model of a frame: matches lo .. lo+n of the frame, n x n matrix block at element sq of the arena
+	int64_t sq;
+	int32_t lo, n, model, pad;
+};
+struct LinkFrame {         // device pointers unless noted
+	const LinkSlice *slices; int n_slices, n_max;      // models with matches, ascending; n_slices / n_max (largest n) on the host
+	const float *xy, *xyz, *world;                     // the frame's per-match arrays
+	const float *depth, *distance; int W, H;           // depth map and its fill-distance map
+	int32_t *status;                                   // nullable: set to 1 when a match lies outside the maps (the frame is then skipped)
+	float *K2D, *K3D, *K3F, *K, *D, *tmp, *scal;       // arena (link_carve)
+	int32_t *valid, *lists, *sz, *ints3, *out_count, *out_offsets, *out_members, *compact;
+};
+size_t link_arena_bytes(int64_t sq_total, int M, int S);
+void link_carve(void *arena, int64_t sq_total, int M, int S, LinkFrame &F);
+mc_status link_frame_device(mc_ctx *ctx, const LinkFrame &F, float cutoff, int min_pts, int use3DFilter, int linkage, float sigma2D, float sigma3D);
+mc_status link_compact_device(mc_ctx *ctx, const LinkFrame &F, int32_t *d_out_n, int32_t *d_cluster_model, int32_t *d_cluster_offsets,
+                              int32_t *d_members, int32_t *d_n_obj);
 mc_status match_merge_device(mc_ctx *ctx, const int32_t *rows_all, const float *dist_all, size_t stride, int n_shards, int Q, float ratio,
                              int32_t *d_nn_row, float *d_nn_dist, uint8_t *d_accepted);
 

@@ -1,0 +1,380 @@
+// depth_frames.cu — moped3d's recognition steps chained on the device (mc_process_depth_frames*): the FrameData of a frame after
+// DEPTHPROP goes CLUSTER (CLUSTER_LINKAGE) -> POSE -> FILTER -> POSE2 -> FILTER2 (moped3d/libmoped/src/config.hpp:45-49) with the
+// per-match arrays and depth maps copied to the device once and the objects copied back once.
+//
+// Every step is the kernel of its stage-by-stage entry, so a frame gives exactly what mc_cluster_linkage (per model),
+// mc_pose_depth_ransac (tie = match index inside the model, as pose_depth_cuda_base.hpp passes it) and mc_filter_projection give:
+//   CLUSTER  the linkage kernels of linkage.cu over all models of the frame at once (one launch per kernel, one agglomeration CTA
+//            per model), then the clusters model-major (k_link_compact)
+//   POSE     k_gather_points with depthData.coord3D and the Cauchy weight of depthData.fillDistance, k_depth_ransac reading the
+//            cluster count from the device (grid and LM scratch sized by host upper bounds), k_pose_append
+//   FILTER   filter_device (moped3d's FILTER_PROJECTION_CPU is moped2's)
+//   POSE2    the survivors stay in the object list (k_copy_objects), new objects from their rebuilt clusters are appended
+// No host synchronisation between the steps: counts stay on the device. The frames of a batch are dealt to the context's frame
+// lanes (pipeline.cu), each of which owns its buffers.
+#include "common.cuh"
+
+#include <algorithm>
+#include <cstring>
+
+namespace mc {
+
+mc_status pose_depth_ransac_device(mc_ctx *ctx, int variant, const int32_t *d_cluster_offsets, int n_clusters, int n_max, const float *d_xy,
+                                   const float *d_xyz, const float *d_world, const float *d_cauchy, const int32_t *d_image, const int32_t *d_tie,
+                                   const mc_pose_params *pp, float alpha, uint8_t *d_found, float *d_pose, int32_t *d_n_tests,
+                                   const int32_t *d_n_clusters);
+mc_status pose_append_device(mc_ctx *ctx, const int32_t *d_cluster_model, const int32_t *d_n_clusters, int n_clusters_cap, int max_obj,
+                             const uint8_t *d_found, const float *d_pose, int32_t *d_n_obj, int obj_cap, int32_t *d_obj_model, float *d_obj_pose);
+mc_status filter_device(mc_ctx *ctx, const int32_t *d_match_offsets, const int32_t *d_match_image, const float *d_match_xy,
+                        const float *d_match_xyz, int n_models, int max_matches, const int32_t *d_obj_model, const float *d_obj_pose,
+                        const int32_t *d_n_obj, int n_obj_cap, int min_points, float feat_dist, float min_score,
+                        uint8_t *d_keep, float *d_score, int32_t *d_out_n, int32_t *d_cluster_model, int32_t *d_cluster_offsets,
+                        int32_t *d_members, int32_t *d_surv_model, float *d_surv_pose, float *d_surv_score);
+
+// sum over a frame's models of n^2: the five similarity matrices and the merge lists of the linkage take 24 bytes per element,
+// so 2^24 elements are ~400 MB per lane (several models of the 2048-match limit of mc_cluster_linkage)
+constexpr int64_t kLinkArenaMax = (int64_t)1 << 24;
+constexpr int kMaxModelMatches = 2048;
+
+__global__ void k_depth_export(const int32_t *__restrict__ st /* {status, n_obj, cl_n[2], f_n[2]} */, int n_matches,
+                               const int32_t *__restrict__ surv_model, const float *__restrict__ surv_pose, const float *__restrict__ surv_score,
+                               int max_objects, int32_t *__restrict__ out_info, int32_t *__restrict__ out_model, float *__restrict__ out_pose,
+                               float *__restrict__ out_score) {
+	const int n = st[4];
+	const int m = n < max_objects ? n : max_objects;
+	for (int i = threadIdx.x; i < m; i += blockDim.x) { out_model[i] = surv_model[i]; out_score[i] = surv_score[i]; }
+	for (int i = threadIdx.x; i < 7 * m; i += blockDim.x) out_pose[i] = surv_pose[i];
+	if (threadIdx.x == 0) { out_info[0] = n; out_info[1] = st[0]; out_info[2] = n_matches; out_info[3] = st[2]; }
+}
+
+// host view of one frame of a batch
+struct DepthPlan {
+	int base, M;                 // global index of the frame's first match, its match count
+	int n_slices, n_max;         // models with matches, the largest
+	int64_t sq;                  // sum of n^2 over its models
+	int cl_cap;                  // clusters <= sum over models of n / (min_pts + 1)
+	size_t meta;                 // offset of its local offsets (n_models + 1) and LinkSlices in the metadata buffer
+};
+
+struct DepthInputs { const int32_t *image; const float *xy, *xyz, *world, *fill, *depth, *distance; };     // device, whole batch
+
+struct DepthCaps { int cl_cap, cl2_cap, obj_cap, task_cap; };
+
+static DepthCaps depth_caps(const DepthPlan &p, const mc_depth_pipeline_params *P) {
+	const int mo1 = std::max(P->pose.max_objects_per_cluster, 0), mo2 = std::max(P->pose2.max_objects_per_cluster, 0);
+	DepthCaps c;
+	c.cl_cap = p.cl_cap;
+	c.cl2_cap = p.cl_cap * mo1;                      // FILTER keeps at most the objects of POSE, one cluster each
+	c.obj_cap = c.cl2_cap + c.cl2_cap * mo2;         // POSE2 appends to the survivors
+	c.task_cap = std::max(c.cl_cap * mo1, c.cl2_cap * mo2);
+	return c;
+}
+
+struct DepthBufs {
+	int32_t *st;                 // {status, n_obj, cl_n[2], f_n[2]}
+	int32_t *cl_model, *cl_offsets, *cl_members;
+	float *pt_xy, *pt_xyz, *pt_world, *pt_cauchy; int32_t *pt_image, *pt_tie;
+	uint8_t *found; float *task_pose; int32_t *n_tests;
+	int32_t *obj_model; float *obj_pose, *obj_score; uint8_t *keep;
+	int32_t *f_model, *f_offsets, *f_members, *surv_model; float *surv_pose, *surv_score;
+};
+
+static mc_status depth_carve(mc_ctx *lane, int M, const DepthCaps &c, DepthBufs &B) {
+	size_t off = 0;
+	auto take = [&](size_t bytes) { size_t o = off; off += (bytes + 255) & ~(size_t)255; return o; };
+	const size_t m1 = (size_t)M + 2, c2 = (size_t)c.cl_cap + 2, o2 = (size_t)c.obj_cap + 2, t1 = (size_t)c.task_cap + 1;
+	const size_t o_st = take(64), o_clm = take(4 * c2), o_clo = take(4 * c2), o_clmem = take(4 * m1);
+	const size_t o_pxy = take(8 * m1), o_pxyz = take(12 * m1), o_pw = take(12 * m1), o_pc = take(4 * m1), o_pim = take(4 * m1), o_ptie = take(4 * m1);
+	const size_t o_found = take(t1), o_tpose = take(28 * t1), o_nt = take(4 * t1);
+	const size_t o_om = take(4 * o2), o_op = take(28 * o2), o_os = take(4 * o2), o_keep = take(o2);
+	const size_t o_fm = take(4 * o2), o_fo = take(4 * o2), o_fmem = take(4 * m1), o_sm = take(4 * o2), o_sp = take(28 * o2), o_ss = take(4 * o2);
+	MC_TRY(reserve(lane, lane->scratch[9], off));
+	char *b = (char *)lane->scratch[9].p;
+	B.st = (int32_t *)(b + o_st); B.cl_model = (int32_t *)(b + o_clm); B.cl_offsets = (int32_t *)(b + o_clo); B.cl_members = (int32_t *)(b + o_clmem);
+	B.pt_xy = (float *)(b + o_pxy); B.pt_xyz = (float *)(b + o_pxyz); B.pt_world = (float *)(b + o_pw); B.pt_cauchy = (float *)(b + o_pc);
+	B.pt_image = (int32_t *)(b + o_pim); B.pt_tie = (int32_t *)(b + o_ptie);
+	B.found = (uint8_t *)(b + o_found); B.task_pose = (float *)(b + o_tpose); B.n_tests = (int32_t *)(b + o_nt);
+	B.obj_model = (int32_t *)(b + o_om); B.obj_pose = (float *)(b + o_op); B.obj_score = (float *)(b + o_os); B.keep = (uint8_t *)(b + o_keep);
+	B.f_model = (int32_t *)(b + o_fm); B.f_offsets = (int32_t *)(b + o_fo); B.f_members = (int32_t *)(b + o_fmem);
+	B.surv_model = (int32_t *)(b + o_sm); B.surv_pose = (float *)(b + o_sp); B.surv_score = (float *)(b + o_ss);
+	return MC_OK;
+}
+
+// Enqueue one frame on lane->stream; its objects go to the frame's output slots. `ev` (nullable, 6 events) brackets the five steps.
+static mc_status depth_frame_enqueue(mc_ctx *lane, const DepthPlan &p, const char *d_meta, const DepthInputs &in, int f, int n_models, int W, int H,
+                                     const mc_depth_pipeline_params *P, int max_objects, int32_t *d_info, int32_t *d_model, float *d_pose,
+                                     float *d_score, cudaEvent_t *ev) {
+	mc_ctx *ctx = lane;
+	cudaStream_t s = lane->stream;
+	int32_t *o_info = d_info + 4 * (size_t)f;
+	if (p.M == 0) {                                     // nothing to cluster: no objects
+		MC_CUDA(cudaMemsetAsync(o_info, 0, 16, s));
+		if (ev) for (int i = 0; i < 6; i++) MC_CUDA(cudaEventRecord(ev[i], s));
+		return MC_OK;
+	}
+	const DepthCaps c = depth_caps(p, P);
+	DepthBufs B;
+	MC_TRY(depth_carve(lane, p.M, c, B));
+	MC_TRY(reserve(lane, lane->link_buf, link_arena_bytes(p.sq, p.M, p.n_slices)));
+	const int32_t *d_off = (const int32_t *)(d_meta + p.meta);                 // the frame's model CSR, from 0
+	const size_t slice_at = (((size_t)n_models + 1) * 4 + 15) & ~(size_t)15;
+	const int32_t *image = in.image + p.base;
+	const float *xy = in.xy + 2 * (size_t)p.base, *xyz = in.xyz + 3 * (size_t)p.base, *world = in.world + 3 * (size_t)p.base, *fill = in.fill + p.base;
+	const size_t px = (size_t)W * H;
+	LinkFrame F;
+	F.slices = (const LinkSlice *)(d_meta + p.meta + slice_at); F.n_slices = p.n_slices; F.n_max = p.n_max;
+	F.xy = xy; F.xyz = xyz; F.world = world; F.depth = in.depth + (size_t)f * px; F.distance = in.distance + (size_t)f * px; F.W = W; F.H = H;
+	F.status = B.st;
+	link_carve(lane->link_buf.p, p.sq, p.M, p.n_slices, F);
+	const float scale = P->variant == 1 ? (float)25.0 : (float)0.100;
+	auto mark = [&](int i) { if (ev) cudaEventRecord(ev[i], s); };
+	MC_CUDA(cudaMemsetAsync(B.st, 0, 64, s));
+	mark(0);
+	// CLUSTER
+	MC_TRY(link_frame_device(lane, F, P->cluster_cutoff, P->cluster_min_pts, P->cluster_use_3d_filter, P->cluster_linkage_type, P->cluster_sigma_2d,
+	                         P->cluster_sigma_3d));
+	MC_TRY(link_compact_device(lane, F, B.st + 2, B.cl_model, B.cl_offsets, B.cl_members, B.st + 1));
+	mark(1);
+	// POSE
+	MC_TRY(gather_depth_points_device(lane, B.st + 2, B.cl_model, B.cl_offsets, B.cl_members, d_off, image, xy, xyz, world, fill, scale, B.pt_xy,
+	                                  B.pt_xyz, B.pt_world, B.pt_cauchy, B.pt_image, B.pt_tie));
+	MC_TRY(pose_depth_ransac_device(lane, P->variant, B.cl_offsets, c.cl_cap, p.n_max, B.pt_xy, B.pt_xyz, B.pt_world, B.pt_cauchy, B.pt_image, B.pt_tie,
+	                                &P->pose, P->pose_alpha, B.found, B.task_pose, B.n_tests, B.st + 2));
+	MC_TRY(pose_append_device(lane, B.cl_model, B.st + 2, c.cl_cap, P->pose.max_objects_per_cluster, B.found, B.task_pose, B.st + 1, c.obj_cap,
+	                          B.obj_model, B.obj_pose));
+	mark(2);
+	// FILTER
+	MC_TRY(filter_device(lane, d_off, image, xy, xyz, n_models, p.M, B.obj_model, B.obj_pose, B.st + 1, c.obj_cap, P->filter_min_points,
+	                     P->filter_feature_distance, P->filter_min_score, B.keep, B.obj_score, B.st + 4, B.f_model, B.f_offsets, B.f_members,
+	                     B.surv_model, B.surv_pose, B.surv_score));
+	mark(3);
+	// POSE2: the surviving objects stay in the list, the objects found on their rebuilt clusters are appended
+	MC_TRY(copy_objects_device(lane, B.st + 4, B.surv_model, B.surv_pose, B.st + 1, B.obj_model, B.obj_pose));
+	MC_TRY(gather_depth_points_device(lane, B.st + 4, B.f_model, B.f_offsets, B.f_members, d_off, image, xy, xyz, world, fill, scale, B.pt_xy,
+	                                  B.pt_xyz, B.pt_world, B.pt_cauchy, B.pt_image, B.pt_tie));
+	MC_TRY(pose_depth_ransac_device(lane, P->variant, B.f_offsets, c.cl2_cap, p.n_max, B.pt_xy, B.pt_xyz, B.pt_world, B.pt_cauchy, B.pt_image, B.pt_tie,
+	                                &P->pose2, P->pose2_alpha, B.found, B.task_pose, B.n_tests, B.st + 4));
+	MC_TRY(pose_append_device(lane, B.f_model, B.st + 4, c.cl2_cap, P->pose2.max_objects_per_cluster, B.found, B.task_pose, B.st + 1, c.obj_cap,
+	                          B.obj_model, B.obj_pose));
+	mark(4);
+	// FILTER2
+	MC_TRY(filter_device(lane, d_off, image, xy, xyz, n_models, p.M, B.obj_model, B.obj_pose, B.st + 1, c.obj_cap, P->filter2_min_points,
+	                     P->filter2_feature_distance, P->filter2_min_score, B.keep, B.obj_score, B.st + 4, B.f_model, B.f_offsets, B.f_members,
+	                     B.surv_model, B.surv_pose, B.surv_score));
+	mark(5);
+	k_depth_export<<<1, 128, 0, s>>>(B.st, p.M, B.surv_model, B.surv_pose, B.surv_score, max_objects, o_info, d_model + (size_t)f * max_objects,
+	                                 d_pose + 7 * (size_t)f * max_objects, d_score + (size_t)f * max_objects);
+	MC_LAUNCH_CHECK();
+	return MC_OK;
+}
+
+// Checks on the host, then plans every frame and lays out the metadata (per frame: local CSR, LinkSlices). Returns the number of
+// matches the per-match arrays must hold.
+static mc_status depth_plan(mc_ctx *ctx, const char *who, const int32_t *match_offsets, int n_frames, int n_models, int width, int height,
+                            const mc_depth_pipeline_params *P, int max_objects, std::vector<DepthPlan> &plans, std::vector<char> &meta, int *m_total) {
+	auto fail = [&](mc_status st, const std::string &msg) { ctx->err = std::string(who) + ": " + msg; return st; };
+	if (!match_offsets || n_frames < 1 || n_models < 1 || width < 1 || height < 1 || max_objects <= 0) return fail(MC_ERR_ARG, "bad argument");
+	if (P->variant < 0 || P->variant > 1) return fail(MC_ERR_ARG, "variant must be 0 (back-projection) or 1 (reprojection)");
+	// with cutoff <= -1 the merge loop has no stopping point once a single cluster is left (the reference then spins on the host)
+	if (!(P->cluster_cutoff > -1.f)) return fail(MC_ERR_ARG, "cluster_cutoff must be > -1");
+	if (P->pose.n_pts_align < 1 || P->pose.n_pts_align > 8 || P->pose2.n_pts_align < 1 || P->pose2.n_pts_align > 8)
+		return fail(MC_ERR_ARG, "n_pts_align must be in 1..8");
+	const int per_cl = P->cluster_min_pts + 1 > 1 ? P->cluster_min_pts + 1 : 1;     // a cluster has more than min_pts members
+	plans.assign((size_t)n_frames, DepthPlan());
+	meta.clear();
+	int mt = 0;
+	for (int f = 0; f < n_frames; f++) {
+		const int32_t *row = match_offsets + (size_t)f * (n_models + 1);
+		DepthPlan &p = plans[(size_t)f];
+		if (row[0] < 0) return fail(MC_ERR_ARG, "match_offsets must be >= 0 (frame " + std::to_string(f) + ")");
+		p.base = row[0]; p.M = 0; p.n_slices = 0; p.n_max = 0; p.sq = 0; p.cl_cap = 0;
+		std::vector<LinkSlice> sl;
+		for (int m = 0; m < n_models; m++) {
+			const int n = row[m + 1] - row[m];
+			if (n < 0) return fail(MC_ERR_ARG, "match_offsets must ascend (frame " + std::to_string(f) + ")");
+			if (n > kMaxModelMatches) return fail(MC_ERR_ARG, "a model has more than 2048 matches (frame " + std::to_string(f) + ")");
+			if (n == 0) continue;
+			sl.push_back(LinkSlice{ p.sq, row[m] - row[0], n, m, 0 });
+			p.sq += (int64_t)n * n;
+			p.n_max = std::max(p.n_max, n);
+			p.cl_cap += n / per_cl;
+		}
+		if (p.sq > kLinkArenaMax) return fail(MC_ERR_CAPACITY, "the models of frame " + std::to_string(f) + " need more than 2^24 similarity entries");
+		p.M = row[n_models] - row[0];
+		p.n_slices = (int)sl.size();
+		mt = std::max(mt, (int)row[n_models]);
+		p.meta = meta.size();
+		const size_t slice_at = (((size_t)n_models + 1) * 4 + 15) & ~(size_t)15;
+		meta.resize(p.meta + ((slice_at + sizeof(LinkSlice) * sl.size() + 255) & ~(size_t)255));
+		int32_t *loc = (int32_t *)(meta.data() + p.meta);
+		for (int m = 0; m <= n_models; m++) loc[m] = row[m] - row[0];
+		if (!sl.empty()) memcpy(meta.data() + p.meta + slice_at, sl.data(), sizeof(LinkSlice) * sl.size());
+	}
+	if (!ctx->d_cams) return fail(MC_ERR_STATE, "cameras not set (mc_set_cameras)");
+	*m_total = mt;
+	return MC_OK;
+}
+
+static mc_status depth_frames_run(mc_ctx *ctx, const char *who, const std::vector<DepthPlan> &plans, const std::vector<char> &meta,
+                                  const DepthInputs &in, int n_models, int W, int H, const mc_depth_pipeline_params *P, int max_objects,
+                                  int32_t *n_objects, int32_t *obj_model, float *obj_pose, float *obj_score, int32_t *frame_info, float *stage_ms) {
+	const int nf = (int)plans.size();
+	MC_TRY(reserve(ctx, ctx->scratch[23], meta.size() + 256));
+	char *d_meta = (char *)ctx->scratch[23].p;
+	MC_CUDA(cudaMemcpyAsync(d_meta, meta.data(), meta.size(), cudaMemcpyHostToDevice, ctx->stream));
+	const size_t per = 16 + (size_t)max_objects * 36;
+	const size_t bytes = per * (size_t)nf;
+	MC_TRY(reserve(ctx, ctx->batch_out, bytes + 256));
+	MC_TRY(pinned(ctx, bytes + 256));
+	char *d = (char *)ctx->batch_out.p;
+	int32_t *d_info = (int32_t *)d;
+	int32_t *d_model = (int32_t *)(d + 16ull * nf);
+	float *d_pose = (float *)(d + (16ull + 4ull * max_objects) * nf);
+	float *d_score = (float *)(d + (16ull + 32ull * max_objects) * nf);
+	int n_lanes = stage_ms ? 1 : std::min(std::max(ctx->n_lanes_wanted, 1), nf);
+	MC_TRY(ensure_lanes(ctx, n_lanes));
+	for (int l = 0; l < n_lanes; l++) { ctx->lanes[(size_t)l]->linkage_cached = ctx->linkage_cached; ctx->lanes[(size_t)l]->lm_finite_check = ctx->lm_finite_check; }
+	std::vector<cudaEvent_t> ev;
+	if (stage_ms) {
+		ev.resize(6 * (size_t)nf);
+		for (auto &e : ev) MC_CUDA(cudaEventCreate(&e));
+	}
+	MC_CUDA(cudaEventRecord(ctx->ev_fork, ctx->stream));
+	for (int l = 0; l < n_lanes; l++) MC_CUDA(cudaStreamWaitEvent(ctx->lanes[(size_t)l]->stream, ctx->ev_fork, 0));
+	if (n_lanes > ctx->lanes_pending) ctx->lanes_pending = n_lanes;
+	mc_status st = MC_OK;
+	for (int f = 0; f < nf && st == MC_OK; f++) {
+		mc_ctx *lane = ctx->lanes[(size_t)(f % n_lanes)];
+		st = depth_frame_enqueue(lane, plans[(size_t)f], d_meta, in, f, n_models, W, H, P, max_objects, d_info, d_model, d_pose, d_score,
+		                         stage_ms ? &ev[6 * (size_t)f] : nullptr);
+		if (st != MC_OK) ctx->err = lane->err;
+	}
+	const mc_status sj = join_lanes(ctx);
+	if (st == MC_OK) st = sj;
+	char *h = (char *)ctx->h_pinned;
+	if (st == MC_OK) {
+		MC_CUDA(cudaMemcpyAsync(h, d, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+		MC_CUDA(cudaStreamSynchronize(ctx->stream));
+	}
+	if (stage_ms) {
+		if (st == MC_OK) {
+			for (int i = 0; i < 5; i++) stage_ms[i] = 0.f;
+			for (int f = 0; f < nf; f++)
+				for (int i = 0; i < 5; i++) { float ms = 0.f; cudaEventElapsedTime(&ms, ev[6 * (size_t)f + i], ev[6 * (size_t)f + i + 1]); stage_ms[i] += ms; }
+		}
+		for (auto &e : ev) cudaEventDestroy(e);
+	}
+	if (st != MC_OK) return st;
+	const int32_t *h_info = (const int32_t *)h;
+	const int32_t *h_model = (const int32_t *)(h + 16ull * nf);
+	const float *h_pose = (const float *)(h + (16ull + 4ull * max_objects) * nf);
+	const float *h_score = (const float *)(h + (16ull + 32ull * max_objects) * nf);
+	int bad_frame = -1, over_frame = -1;
+	for (int f = 0; f < nf; f++) {
+		const int n = h_info[4 * f];
+		if (frame_info) memcpy(frame_info + 4 * f, h_info + 4 * f, 16);
+		n_objects[f] = n;
+		if (h_info[4 * f + 1]) { if (bad_frame < 0) bad_frame = f; continue; }
+		if (n > max_objects) { if (over_frame < 0) over_frame = f; continue; }
+		memcpy(obj_model + (size_t)f * max_objects, h_model + (size_t)f * max_objects, 4ull * n);
+		memcpy(obj_pose + 7 * (size_t)f * max_objects, h_pose + 7 * (size_t)f * max_objects, 28ull * n);
+		memcpy(obj_score + (size_t)f * max_objects, h_score + (size_t)f * max_objects, 4ull * n);
+	}
+	if (bad_frame >= 0) { ctx->err = std::string(who) + ": a match of frame " + std::to_string(bad_frame) + " lies outside the depth map"; return MC_ERR_ARG; }
+	if (over_frame >= 0) { ctx->err = std::string(who) + ": frame " + std::to_string(over_frame) + " has more than max_objects objects"; return MC_ERR_CAPACITY; }
+	return MC_OK;
+}
+
+} // namespace mc
+
+using namespace mc;
+
+extern "C" {
+
+void mc_depth_pipeline_default_params(mc_depth_pipeline_params *p) {
+	if (!p) return;
+	memset(p, 0, sizeof *p);
+	p->variant = 0;
+	p->cluster_cutoff = 0.1f; p->cluster_min_pts = 7; p->cluster_use_3d_filter = 2; p->cluster_linkage_type = 1;   // CLUSTER_LINKAGE(0.1, 7, 2, 1, 0.0, 1, -1, -1)
+	p->cluster_sigma_2d = -1.f; p->cluster_sigma_3d = -1.f;
+	p->pose = mc_pose_params{ 192, 100, 4, 5, 6, 8.f, 1 }; p->pose_alpha = 0.5f;          // POSE(192, 100, 4, 5, 6, 8, 0.5)
+	p->filter_min_points = 6; p->filter_feature_distance = 4096.f; p->filter_min_score = 2.f;     // FILTER(6, 4096, 2)
+	p->pose2 = mc_pose_params{ 64, 250, 4, 6, 8, 5.f, 2 }; p->pose2_alpha = 0.5f;          // POSE2(64, 250, 4, 6, 8, 5, 0.5)
+	p->filter2_min_points = 8; p->filter2_feature_distance = 8192.f; p->filter2_min_score = 1e-4f;  // FILTER2(8, 8192, 1e-4)
+}
+
+mc_status mc_process_depth_frames(mc_ctx *ctx, const int32_t *match_offsets, int n_frames, int n_models, const int32_t *match_image,
+                                  const float *match_xy, const float *match_xyz, const float *match_world, const float *match_fill,
+                                  const float *depth, const float *fill_distance, int width, int height, const mc_depth_pipeline_params *params,
+                                  int max_objects, int32_t *n_objects, int32_t *obj_model, float *obj_pose, float *obj_score, int32_t *frame_info,
+                                  float *stage_ms) {
+	const char *who = "mc_process_depth_frames";
+	if (!ctx) return MC_ERR_ARG;
+	if (!params || !n_objects || !obj_model || !obj_pose || !obj_score || !depth || !fill_distance) { ctx->err = std::string(who) + ": bad argument"; return MC_ERR_ARG; }
+	std::vector<DepthPlan> plans;
+	std::vector<char> meta;
+	int M = 0;
+	MC_TRY(depth_plan(ctx, who, match_offsets, n_frames, n_models, width, height, params, max_objects, plans, meta, &M));
+	if (M > 0 && (!match_image || !match_xy || !match_xyz || !match_world || !match_fill)) { ctx->err = std::string(who) + ": null match array"; return MC_ERR_ARG; }
+	// the blend kernel reads the fill-distance map at every match's pixel unchecked (like the reference, CLUSTER_LINKAGE_CPU.hpp:324-365):
+	// a coordinate outside the map is an argument error, found before anything is copied
+	for (int f = 0; f < n_frames; f++) {
+		const DepthPlan &p = plans[(size_t)f];
+		for (int i = p.base; i < p.base + p.M; i++) {
+			const float x = match_xy[2 * (size_t)i], y = match_xy[2 * (size_t)i + 1];
+			if (!(x >= 0.f && y >= 0.f && (int)x < width && (int)y < height)) {
+				ctx->err = std::string(who) + ": a match of frame " + std::to_string(f) + " lies outside the depth map";
+				return MC_ERR_ARG;
+			}
+		}
+	}
+	MC_CUDA(cudaSetDevice(ctx->device));
+	const size_t px = (size_t)width * height, Ms = (size_t)M + 1;
+	size_t off = 0;
+	auto take = [&](size_t b) { size_t o = off; off += (b + 255) & ~(size_t)255; return o; };
+	const size_t o_im = take(4 * Ms), o_xy = take(8 * Ms), o_xyz = take(12 * Ms), o_w = take(12 * Ms), o_f = take(4 * Ms);
+	const size_t o_d = take(4 * px * n_frames), o_fd = take(4 * px * n_frames);
+	MC_TRY(reserve(ctx, ctx->scratch[15], off));
+	char *b = (char *)ctx->scratch[15].p;
+	cudaStream_t s = ctx->stream;
+	if (M > 0) {
+		MC_CUDA(cudaMemcpyAsync(b + o_im, match_image, 4ull * M, cudaMemcpyHostToDevice, s));
+		MC_CUDA(cudaMemcpyAsync(b + o_xy, match_xy, 8ull * M, cudaMemcpyHostToDevice, s));
+		MC_CUDA(cudaMemcpyAsync(b + o_xyz, match_xyz, 12ull * M, cudaMemcpyHostToDevice, s));
+		MC_CUDA(cudaMemcpyAsync(b + o_w, match_world, 12ull * M, cudaMemcpyHostToDevice, s));
+		MC_CUDA(cudaMemcpyAsync(b + o_f, match_fill, 4ull * M, cudaMemcpyHostToDevice, s));
+	}
+	MC_CUDA(cudaMemcpyAsync(b + o_d, depth, 4 * px * n_frames, cudaMemcpyHostToDevice, s));
+	MC_CUDA(cudaMemcpyAsync(b + o_fd, fill_distance, 4 * px * n_frames, cudaMemcpyHostToDevice, s));
+	DepthInputs in;
+	in.image = (const int32_t *)(b + o_im); in.xy = (const float *)(b + o_xy); in.xyz = (const float *)(b + o_xyz); in.world = (const float *)(b + o_w);
+	in.fill = (const float *)(b + o_f); in.depth = (const float *)(b + o_d); in.distance = (const float *)(b + o_fd);
+	return depth_frames_run(ctx, who, plans, meta, in, n_models, width, height, params, max_objects, n_objects, obj_model, obj_pose, obj_score,
+	                        frame_info, stage_ms);
+}
+
+mc_status mc_process_depth_frames_dev(mc_ctx *ctx, const int32_t *match_offsets, int n_frames, int n_models, const int32_t *match_image_dev,
+                                      const float *match_xy_dev, const float *match_xyz_dev, const float *match_world_dev, const float *match_fill_dev,
+                                      const float *depth_dev, const float *fill_distance_dev, int width, int height,
+                                      const mc_depth_pipeline_params *params, int max_objects, int32_t *n_objects, int32_t *obj_model, float *obj_pose,
+                                      float *obj_score, int32_t *frame_info, float *stage_ms) {
+	const char *who = "mc_process_depth_frames_dev";
+	if (!ctx) return MC_ERR_ARG;
+	if (!params || !n_objects || !obj_model || !obj_pose || !obj_score || !depth_dev || !fill_distance_dev) { ctx->err = std::string(who) + ": bad argument"; return MC_ERR_ARG; }
+	std::vector<DepthPlan> plans;
+	std::vector<char> meta;
+	int M = 0;
+	MC_TRY(depth_plan(ctx, who, match_offsets, n_frames, n_models, width, height, params, max_objects, plans, meta, &M));
+	if (M > 0 && (!match_image_dev || !match_xy_dev || !match_xyz_dev || !match_world_dev || !match_fill_dev)) {
+		ctx->err = std::string(who) + ": null match array";
+		return MC_ERR_ARG;
+	}
+	MC_CUDA(cudaSetDevice(ctx->device));
+	DepthInputs in;
+	in.image = match_image_dev; in.xy = match_xy_dev; in.xyz = match_xyz_dev; in.world = match_world_dev; in.fill = match_fill_dev;
+	in.depth = depth_dev; in.distance = fill_distance_dev;
+	return depth_frames_run(ctx, who, plans, meta, in, n_models, width, height, params, max_objects, n_objects, obj_model, obj_pose, obj_score,
+	                        frame_info, stage_ms);
+}
+
+} // extern "C"

@@ -8,6 +8,9 @@
 // live pairs: one CTA, the argmax and the row update parallel over the CTA, the chain itself serial (latency-bound, like
 // mean-shift in cluster.cu).
 //
+// mc_process_depth_frames* runs the same kernels over all models of a frame at once (a model dimension in every grid, one
+// agglomeration CTA per model: the serial merge chains of different models run side by side); mc_cluster_linkage is the case of one model.
+//
 // Arithmetic: compiled with -fmad=false; every expression in the reference's order and types (the stage is built without
 // -fsingle-precision-constant: literals are double where the reference's are). expf/atan2f/sqrtf: CUDA's vs glibc's differ by
 // an ulp, so similarity values agree with the oracle to ~1e-6 and the agglomeration — which only compares them — is checked
@@ -41,10 +44,28 @@ __device__ __forceinline__ float sq_dist3(const float *a, const float *b) {
 	return r;
 }
 
+// Every kernel below works on the models of one frame at once (LinkSlice, common.cuh): model a of the launch owns matches
+// lo .. lo+n of the frame's per-match arrays, n x n floats at element sq of each matrix arena, and n-element slices at lo of the
+// per-match state (3n at 3 lo for the triples). Scalars: scal[4a .. 4a+3] = sigma2D, sigma3D, first and second maximum.
+// mc_cluster_linkage runs them with one model at 0.
+
 // getAverageNNDistances (:98-123): nearest-neighbour distance of every match in the image and in model space; the two averages
-// are summed by one thread in match order (float sums are order-dependent)
-__global__ void __launch_bounds__(kLinkThreads) k_link_sigma(int n, const float *__restrict__ xy, const float *__restrict__ xyz,
-                                                            float sigma2D, float sigma3D, float *__restrict__ nn_scratch, float *__restrict__ sigmas) {
+// are summed by one thread in match order (float sums are order-dependent). One CTA per model. With `status` given, a match
+// outside the W x H maps sets it to 1 (the blend and agglomeration kernels then skip the frame).
+__global__ void __launch_bounds__(kLinkThreads, 1) k_link_sigma(const LinkSlice *__restrict__ slices, const float *__restrict__ xy_all,
+                                                            const float *__restrict__ xyz_all, float sigma2D, float sigma3D, float *__restrict__ tmp,
+                                                            float *__restrict__ scal, int W, int H, int32_t *__restrict__ status) {
+	const int n = slices[blockIdx.x].n, lo = slices[blockIdx.x].lo;
+	const float *xy = xy_all + 2 * (size_t)lo, *xyz = xyz_all + 3 * (size_t)lo;
+	float *nn_scratch = tmp + 3 * (size_t)lo, *sigmas = scal + 4 * (size_t)blockIdx.x;
+	if (status) {
+		int bad = 0;
+		for (int i = threadIdx.x; i < n; i += blockDim.x) {
+			const float x = xy[2 * i], y = xy[2 * i + 1];
+			bad |= !(x >= 0.f && y >= 0.f && x < (float)W && y < (float)H);
+		}
+		if (__syncthreads_or(bad) && threadIdx.x == 0) atomicOr(status, 1);
+	}
 	if (sigma2D == -1 || sigma3D == -1) {
 		for (int i = threadIdx.x; i < n; i += blockDim.x) {
 			float b2 = (float)DBL_MAX, b3 = (float)DBL_MAX;
@@ -115,13 +136,19 @@ __device__ float discontinuity(const float *xy_i, const float *xy_j, int W, int 
 }
 
 // One thread per pair (i <= j): K2D, K3D + BK (getGaussK :133-150, getSum :295-301) and K3F (get3DFilterK :152-172)
-__global__ void __launch_bounds__(kLinkThreads) k_link_pairs(int n, const float *__restrict__ xy, const float *__restrict__ xyz,
-                                                            const float *__restrict__ world, int W, int H, const float *__restrict__ depth,
-                                                            const float *__restrict__ sigmas, int use3DFilter,
-                                                            float *__restrict__ K2D, float *__restrict__ K3D, float *__restrict__ K3F) {
+// grid (columns / kLinkThreads, rows, models)
+__global__ void __launch_bounds__(kLinkThreads) k_link_pairs(const LinkSlice *__restrict__ slices, int n_slices, const float *__restrict__ xy_all,
+                                                            const float *__restrict__ xyz_all, const float *__restrict__ world_all, int W, int H,
+                                                            const float *__restrict__ depth, const float *__restrict__ scal, int use3DFilter,
+                                                            float *__restrict__ K2D_all, float *__restrict__ K3D_all, float *__restrict__ K3F_all) {
+	for (int m = blockIdx.z; m < n_slices; m += gridDim.z) {
+	const LinkSlice sl = slices[m];
+	const int n = sl.n;
 	const int j = blockIdx.x * blockDim.x + threadIdx.x, i = blockIdx.y;
-	if (j >= n || j < i) return;
-	const float s2 = sigmas[0], s3 = sigmas[1];
+	if (j >= n || j < i) continue;
+	const float *xy = xy_all + 2 * (size_t)sl.lo, *xyz = xyz_all + 3 * (size_t)sl.lo, *world = world_all + 3 * (size_t)sl.lo;
+	float *K2D = K2D_all + sl.sq, *K3D = K3D_all + sl.sq, *K3F = K3F_all + sl.sq;
+	const float s2 = scal[4 * (size_t)m], s3 = scal[4 * (size_t)m + 1];
 	const float two2 = 2 * s2 * s2, two3 = 2 * s3 * s3;
 	const float k2 = expf(-1 * sq_dist2(xy + 2 * i, xy + 2 * j) / two2);
 	float k3 = expf(-1 * sq_dist3(world + 3 * i, world + 3 * j) / two3);
@@ -141,12 +168,20 @@ __global__ void __launch_bounds__(kLinkThreads) k_link_pairs(int n, const float 
 		}
 		K3F[a] = f; K3F[b] = f;
 	}
+	}
 }
 
 // normalizeSimilarityMatrix (:303-322) in two kernels: the maximum (order-independent), then the division. `combine`: 0 = plain,
 // 1 = K += F first, 2 = K *= F first (getSum / getProduct before the second normalisation, :636-642)
-__global__ void __launch_bounds__(kLinkThreads) k_link_max(size_t nn, float *__restrict__ K, const float *__restrict__ F, int combine, float *__restrict__ out_max) {
+// grid (blocks per model, models); `slot` = 2 (first maximum) or 3 (second)
+__global__ void __launch_bounds__(kLinkThreads) k_link_max(const LinkSlice *__restrict__ slices, float *__restrict__ K_all, const float *__restrict__ F_all,
+                                                          int combine, float *__restrict__ scal, int slot) {
 	__shared__ float s_m[kLinkThreads / 32];
+	const LinkSlice sl = slices[blockIdx.y];
+	const size_t nn = (size_t)sl.n * sl.n;
+	float *K = K_all + sl.sq;
+	const float *F = F_all + sl.sq;
+	float *out_max = scal + 4 * (size_t)blockIdx.y + slot;
 	float m = -1;
 	for (size_t k = (size_t)blockIdx.x * blockDim.x + threadIdx.x; k < nn; k += (size_t)gridDim.x * blockDim.x) {
 		float v = K[k];
@@ -164,16 +199,30 @@ __global__ void __launch_bounds__(kLinkThreads) k_link_max(size_t nn, float *__r
 		atomicMax((int *)out_max, __float_as_int(m));
 	}
 }
-__global__ void __launch_bounds__(kLinkThreads) k_link_scale(size_t nn, float *__restrict__ K, const float *__restrict__ mx) {
-	const float m = *mx;
+__global__ void __launch_bounds__(kLinkThreads) k_link_scale(const LinkSlice *__restrict__ slices, float *__restrict__ K_all, const float *__restrict__ scal,
+                                                            int slot) {
+	const LinkSlice sl = slices[blockIdx.y];
+	const size_t nn = (size_t)sl.n * sl.n;
+	float *K = K_all + sl.sq;
+	const float m = scal[4 * (size_t)blockIdx.y + slot];
 	for (size_t k = (size_t)blockIdx.x * blockDim.x + threadIdx.x; k < nn; k += (size_t)gridDim.x * blockDim.x) K[k] = K[k] / m;
 }
 
 // adaptiveWeightSum (:324-365) with alpha = 0.5, gamma = 25 (:651)
-__global__ void __launch_bounds__(kLinkThreads) k_link_blend(int n, const float *__restrict__ xy, int W, const float *__restrict__ distance,
-                                                            const float *__restrict__ K2D, const float *__restrict__ K3D, float *__restrict__ K) {
+// grid as k_link_pairs. Reads the fill-distance map at every match's pixel unclamped, like the reference: a frame whose `status`
+// was set by k_link_sigma is skipped
+__global__ void __launch_bounds__(kLinkThreads) k_link_blend(const LinkSlice *__restrict__ slices, int n_slices, const float *__restrict__ xy_all, int W,
+                                                            const float *__restrict__ distance, const float *__restrict__ K2D_all,
+                                                            const float *__restrict__ K3D_all, float *__restrict__ K_all, const int32_t *__restrict__ status) {
+	if (status && *status) return;
+	for (int m = blockIdx.z; m < n_slices; m += gridDim.z) {
+	const LinkSlice sl = slices[m];
+	const int n = sl.n;
 	const int j = blockIdx.x * blockDim.x + threadIdx.x, i = blockIdx.y;
-	if (j >= n || j < i) return;
+	if (j >= n || j < i) continue;
+	const float *xy = xy_all + 2 * (size_t)sl.lo;
+	const float *K2D = K2D_all + sl.sq, *K3D = K3D_all + sl.sq;
+	float *K = K_all + sl.sq;
 	const float alpha = (float)0.5, gamma = 25;
 	const float gammaSq = gamma * gamma;
 	const float di = distance[(size_t)((int)xy[2 * i + 1]) * W + (int)xy[2 * i]], dj = distance[(size_t)((int)xy[2 * j + 1]) * W + (int)xy[2 * j]];
@@ -184,18 +233,30 @@ __global__ void __launch_bounds__(kLinkThreads) k_link_blend(int n, const float 
 	const float w2D = (float)(alpha + alphaBar * (1.0 - joint)), w3D = alphaBar * joint;
 	const float val = w2D * k2 + w3D * k3;
 	K[(size_t)j * n + i] = val; K[(size_t)i * n + j] = val;
+	}
 }
 
 // hierarchicalCluster (:414-531): one CTA. D = working similarity matrix (n x n, global), members = n lists in a pool of n*n
 // ints is avoided: cluster c's members live in `pool` as a linked structure would cost pointer chasing, so each cluster owns a
 // slice of `lists` that is rebuilt on merge by thread 0 (total copies are O(n^2) in the worst case, n is a few hundred).
-__global__ void __launch_bounds__(kLinkThreads) k_link_agglomerate(int n, const float *__restrict__ K, float *__restrict__ D, float cutoff, int min_pts, int linkage,
-                                                                  int *__restrict__ valid, int *__restrict__ lists, int *__restrict__ sz, float *__restrict__ tmp,
-                                                                  int *__restrict__ out_count, int *__restrict__ out_offsets, int *__restrict__ out_members) {
+// One CTA per model (the merge chains of a frame's models run side by side). Model a's result: out_count[a] clusters, their
+// offsets at out_offsets[lo + a ..], members (match indices inside the model) at out_members[lo ..].
+__global__ void __launch_bounds__(kLinkThreads, 1) k_link_agglomerate(const LinkSlice *__restrict__ slices, const float *__restrict__ K_all, float *__restrict__ D_all,
+                                                                  float cutoff, int min_pts, int linkage, int *__restrict__ valid_all, int *__restrict__ lists_all,
+                                                                  int *__restrict__ sz_all, float *__restrict__ tmp_all, int *__restrict__ out_count_all,
+                                                                  int *__restrict__ out_offsets_all, int *__restrict__ out_members_all,
+                                                                  const int32_t *__restrict__ status) {
 	__shared__ float s_val[kLinkThreads];
 	__shared__ int s_a[kLinkThreads], s_b[kLinkThreads];
 	__shared__ int s_nv, s_r, s_p1, s_p2, s_stop, s_sU, s_sR;
 	const int tid = threadIdx.x;
+	const int n = slices[blockIdx.x].n, lo = slices[blockIdx.x].lo;
+	const int64_t sq = slices[blockIdx.x].sq;
+	int *out_count = out_count_all + blockIdx.x, *out_offsets = out_offsets_all + lo + blockIdx.x, *out_members = out_members_all + lo;
+	if (status && *status) { if (tid == 0) { *out_count = 0; out_offsets[0] = 0; } return; }
+	const float *K = K_all + sq;
+	float *D = D_all + sq, *tmp = tmp_all + 3 * (size_t)lo;
+	int *valid = valid_all + lo, *lists = lists_all + sq, *sz = sz_all + lo;
 	for (size_t k = tid; k < (size_t)n * n; k += blockDim.x) D[k] = K[k];       // distances[i][j] = K->getProb(i, j) (:434-439)
 	for (int i = tid; i < n; i += blockDim.x) { valid[i] = i; lists[(size_t)i * n] = i; sz[i] = 1; }
 	if (tid == 0) { s_nv = n; s_r = -1; s_stop = 0; }
@@ -283,84 +344,166 @@ __global__ void __launch_bounds__(kLinkThreads) k_link_agglomerate(int n, const 
 
 // The same agglomeration with a cached maximum per row (linkage_cached.cuh; average linkage only): O(n) per merge plus repairs
 // instead of an O(n^2) scan. mc_set_option("linkage_cached", 1).
-__global__ void __launch_bounds__(kLinkThreads) k_link_agglomerate_cached(int n, const float *__restrict__ K, float *__restrict__ D, float cutoff, int min_pts,
-                                                                         int *__restrict__ L, int *__restrict__ lists, int *__restrict__ sz,
-                                                                         float *__restrict__ tmp3, int *__restrict__ ints3,
-                                                                         int *__restrict__ out_count, int *__restrict__ out_offsets,
-                                                                         int *__restrict__ out_members) {
+__global__ void __launch_bounds__(kLinkThreads) k_link_agglomerate_cached(const LinkSlice *__restrict__ slices, const float *__restrict__ K_all,
+                                                                         float *__restrict__ D_all, float cutoff, int min_pts, int *__restrict__ L_all,
+                                                                         int *__restrict__ lists_all, int *__restrict__ sz_all, float *__restrict__ tmp3_all,
+                                                                         int *__restrict__ ints3_all, int *__restrict__ out_count_all,
+                                                                         int *__restrict__ out_offsets_all, int *__restrict__ out_members_all,
+                                                                         const int32_t *__restrict__ status) {
 	__shared__ float s_val[kLinkThreads];
 	__shared__ int s_idx[kLinkThreads], s_ctl[16];
+	const LinkSlice sl = slices[blockIdx.x];
+	const int n = sl.n;
+	int *out_count = out_count_all + blockIdx.x, *out_offsets = out_offsets_all + sl.lo + blockIdx.x, *out_members = out_members_all + sl.lo;
+	if (status && *status) { if (threadIdx.x == 0) { *out_count = 0; out_offsets[0] = 0; } return; }
+	float *tmp3 = tmp3_all + 3 * (size_t)sl.lo;
+	int *ints3 = ints3_all + 3 * (size_t)sl.lo;
 	lkx::State s;
-	s.n = n; s.D = D; s.L = L; s.lists = lists; s.sz = sz;
+	s.n = n; s.D = D_all + sl.sq; s.L = L_all + sl.lo; s.lists = lists_all + sl.sq; s.sz = sz_all + sl.lo;
 	s.tmp = tmp3; s.oldcol = tmp3 + n; s.best = tmp3 + 2 * (size_t)n;
 	s.posOf = ints3; s.arg = ints3 + n; s.tmpi = ints3 + 2 * (size_t)n;
 	s.s_val = s_val; s.s_idx = s_idx; s.ctl = s_ctl;
 	lkx::Block<kLinkThreads> blk;
 	blk.tid = threadIdx.x;
-	lkx::agglomerate_average(blk, s, K, cutoff, min_pts, out_count, out_offsets, out_members);
+	lkx::agglomerate_average(blk, s, K_all + sl.sq, cutoff, min_pts, out_count, out_offsets, out_members);
+}
+
+// The clusters of every model of a frame, model-major (what CLUSTER_LINKAGE leaves in frameData.clusters[model]): cluster_model,
+// cluster_offsets (into members), members = match indices inside the model in the agglomeration's list order. One CTA.
+// out_n = {clusters, members}. Also zeroes the frame's object count for the POSE step that follows.
+__global__ void __launch_bounds__(kLinkThreads) k_link_compact(const LinkSlice *__restrict__ slices, int n_slices, const int *__restrict__ out_count,
+                                                              const int *__restrict__ out_offsets, const int *__restrict__ out_members,
+                                                              int *__restrict__ base, int32_t *__restrict__ out_n, int32_t *__restrict__ cluster_model,
+                                                              int32_t *__restrict__ cluster_offsets, int32_t *__restrict__ members,
+                                                              int32_t *__restrict__ n_obj) {
+	if (threadIdx.x == 0) {                     // cluster and member base of every model
+		int c = 0, k = 0;
+		for (int a = 0; a < n_slices; a++) {
+			base[2 * a] = c; base[2 * a + 1] = k;
+			const int nc = out_count[a];
+			c += nc; k += out_offsets[slices[a].lo + a + nc];
+		}
+		out_n[0] = c; out_n[1] = k;
+		cluster_offsets[c] = k;
+		*n_obj = 0;
+	}
+	__syncthreads();
+	for (int a = 0; a < n_slices; a++) {
+		const LinkSlice sl = slices[a];
+		const int nc = out_count[a], c0 = base[2 * a], k0 = base[2 * a + 1];
+		const int *off = out_offsets + sl.lo + a, *mem = out_members + sl.lo;
+		for (int c = threadIdx.x; c < nc; c += blockDim.x) { cluster_model[c0 + c] = sl.model; cluster_offsets[c0 + c] = k0 + off[c]; }
+		for (int t = threadIdx.x; t < off[nc]; t += blockDim.x) members[k0 + t] = mem[t];
+	}
 }
 
 // ---- host side -------------------------------------------------------------------------------------------------------------
 
-struct LinkBufs { float *xy, *xyz, *world, *depth, *distance, *K2D, *K3D, *K3F, *K, *D, *tmp, *scal; int *valid, *lists, *sz, *ints3, *out; };
+// Arena of one frame's linkage (sq_total = sum of n^2 over its models, M = its matches, S = its models): five n x n matrices and the
+// merge lists per model, per-match state, and the per-model outputs. Laid out by link_carve.
+size_t link_arena_bytes(int64_t sq_total, int M, int S) {
+	const size_t floats = 5 * (size_t)sq_total + 3 * (size_t)M + 4 * (size_t)S;
+	const size_t ints = (size_t)sq_total + 5 * (size_t)M + (size_t)S + ((size_t)M + S + 1) + (size_t)M + 2 * (size_t)S + 2;
+	return (floats + ints) * 4 + 64;
+}
 
-static mc_status link_alloc(mc_ctx *ctx, int n, size_t px, LinkBufs &B) {
+void link_carve(void *arena, int64_t sq_total, int M, int S, LinkFrame &F) {
+	const size_t sq = (size_t)sq_total;
+	float *f = (float *)arena;
+	F.K2D = f; f += sq; F.K3D = f; f += sq; F.K3F = f; f += sq; F.K = f; f += sq; F.D = f; f += sq;
+	F.tmp = f; f += 3 * (size_t)M; F.scal = f; f += 4 * (size_t)S;
+	int *i = (int *)f;
+	F.valid = i; i += M; F.lists = i; i += sq; F.sz = i; i += M; F.ints3 = i; i += 3 * (size_t)M;
+	F.out_count = i; i += S; F.out_offsets = i; i += (size_t)M + S + 1; F.out_members = i; i += M; F.compact = i;
+}
+
+static mc_status link_agglomerate_only(mc_ctx *ctx, const LinkFrame &F, float cutoff, int min_pts, int linkage);
+
+// sigma -> pairs -> max/scale (x2 with the 3-D filter) -> blend -> agglomeration for every model of F, one launch each
+mc_status link_frame_device(mc_ctx *ctx, const LinkFrame &F, float cutoff, int min_pts, int use3DFilter, int linkage, float sigma2D, float sigma3D) {
+	cudaStream_t st = ctx->stream;
+	const int S = F.n_slices, nmax = F.n_max;
+	if (S <= 0) return MC_OK;
+	MC_CUDA(cudaMemsetAsync(F.scal, 0, 4 * (size_t)S * sizeof(float), st));
+	k_link_sigma<<<S, kLinkThreads, 0, st>>>(F.slices, F.xy, F.xyz, sigma2D, sigma3D, F.tmp, F.scal, F.W, F.H, F.status);
+	MC_LAUNCH_CHECK();
+	const dim3 g((nmax + kLinkThreads - 1) / kLinkThreads, nmax, S < 65535 ? S : 65535);
+	k_link_pairs<<<g, kLinkThreads, 0, st>>>(F.slices, S, F.xy, F.xyz, F.world, F.W, F.H, F.depth, F.scal, use3DFilter, F.K2D, F.K3D, F.K3F);
+	MC_LAUNCH_CHECK();
+	// the maximum is order-independent and the scaling elementwise: any number of blocks per model gives the same bits
+	const int64_t want = ((int64_t)nmax * nmax + kLinkThreads - 1) / kLinkThreads, per = (4 * ctx->num_sms + S - 1) / S;
+	const dim3 gr((unsigned)(want < per ? want : per), S);
+	k_link_max<<<gr, kLinkThreads, 0, st>>>(F.slices, F.K3D, nullptr, 0, F.scal, 2);
+	MC_LAUNCH_CHECK();
+	k_link_scale<<<gr, kLinkThreads, 0, st>>>(F.slices, F.K3D, F.scal, 2);
+	MC_LAUNCH_CHECK();
+	if (use3DFilter) {
+		k_link_max<<<gr, kLinkThreads, 0, st>>>(F.slices, F.K3D, F.K3F, use3DFilter == 1 ? 1 : 2, F.scal, 3);
+		MC_LAUNCH_CHECK();
+		k_link_scale<<<gr, kLinkThreads, 0, st>>>(F.slices, F.K3D, F.scal, 3);
+		MC_LAUNCH_CHECK();
+	}
+	k_link_blend<<<g, kLinkThreads, 0, st>>>(F.slices, S, F.xy, F.W, F.distance, F.K2D, F.K3D, F.K, F.status);
+	MC_LAUNCH_CHECK();
+	return link_agglomerate_only(ctx, F, cutoff, min_pts, linkage);
+}
+
+static mc_status link_agglomerate_only(mc_ctx *ctx, const LinkFrame &F, float cutoff, int min_pts, int linkage) {
+	cudaStream_t st = ctx->stream;
+	const int S = F.n_slices;
+	if (ctx->linkage_cached && linkage == 1)
+		k_link_agglomerate_cached<<<S, kLinkThreads, 0, st>>>(F.slices, F.K, F.D, cutoff, min_pts, F.valid, F.lists, F.sz, F.tmp, F.ints3, F.out_count,
+		                                                      F.out_offsets, F.out_members, F.status);
+	else
+		k_link_agglomerate<<<S, kLinkThreads, 0, st>>>(F.slices, F.K, F.D, cutoff, min_pts, linkage, F.valid, F.lists, F.sz, F.tmp, F.out_count,
+		                                               F.out_offsets, F.out_members, F.status);
+	MC_LAUNCH_CHECK();
+	return MC_OK;
+}
+
+mc_status link_compact_device(mc_ctx *ctx, const LinkFrame &F, int32_t *d_out_n, int32_t *d_cluster_model, int32_t *d_cluster_offsets,
+                              int32_t *d_members, int32_t *d_n_obj) {
+	k_link_compact<<<1, kLinkThreads, 0, ctx->stream>>>(F.slices, F.n_slices, F.out_count, F.out_offsets, F.out_members, F.compact, d_out_n,
+	                                                    d_cluster_model, d_cluster_offsets, d_members, d_n_obj);
+	MC_LAUNCH_CHECK();
+	return MC_OK;
+}
+
+// One model on ctx->stream (mc_cluster_linkage, mc_linkage_agglomerate): its inputs and slice descriptor ahead of the arena in
+// ctx->link_buf
+struct LinkOne { float *xy, *xyz, *world, *depth, *distance; LinkFrame F; };
+
+static mc_status link_one_alloc(mc_ctx *ctx, int n, size_t px, LinkOne &B) {
 	const size_t nn = (size_t)n * n;
-	size_t floats = (size_t)n * 8 + 2 * px + 5 * nn + (size_t)n * 3 + 16;
-	size_t ints = (size_t)n + nn + (size_t)n + (size_t)3 * n + (size_t)2 * n + 8;
-	MC_TRY(reserve(ctx, ctx->link_buf, floats * sizeof(float) + ints * sizeof(int) + 1024));
+	const size_t in_floats = 8 * (size_t)n + 2 * px + 8;
+	MC_TRY(reserve(ctx, ctx->link_buf, in_floats * sizeof(float) + sizeof(LinkSlice) + link_arena_bytes((int64_t)nn, n, 1) + 256));
 	float *f = (float *)ctx->link_buf.p;
 	B.xy = f; f += 2 * (size_t)n; B.xyz = f; f += 3 * (size_t)n; B.world = f; f += 3 * (size_t)n;
 	B.depth = f; f += px; B.distance = f; f += px;
-	B.K2D = f; f += nn; B.K3D = f; f += nn; B.K3F = f; f += nn; B.K = f; f += nn; B.D = f; f += nn;
-	B.tmp = f; f += 3 * (size_t)n; B.scal = f; f += 16;
-	int *i = (int *)f;
-	B.valid = i; i += n; B.lists = i; i += nn; B.sz = i; i += n; B.ints3 = i; i += 3 * (size_t)n; B.out = i;
+	LinkSlice *slice = (LinkSlice *)(((uintptr_t)f + 63) & ~(uintptr_t)63);
+	const LinkSlice one = { 0, 0, n, 0, 0 };
+	MC_CUDA(cudaMemcpyAsync(slice, &one, sizeof one, cudaMemcpyHostToDevice, ctx->stream));
+	LinkFrame &F = B.F;
+	F.slices = slice; F.n_slices = 1; F.n_max = n;
+	F.xy = B.xy; F.xyz = B.xyz; F.world = B.world; F.depth = B.depth; F.distance = B.distance; F.W = 0; F.H = 0;
+	F.status = nullptr;
+	link_carve(slice + 1, (int64_t)nn, n, 1, F);
 	return MC_OK;
 }
 
-static mc_status link_similarity_device(mc_ctx *ctx, const LinkBufs &B, int n, int W, int H, int use3DFilter, float sigma2D, float sigma3D) {
+// the model's clusters -> host (CSR as mc_cluster_linkage returns it)
+static mc_status link_one_download(mc_ctx *ctx, const LinkOne &B, int n, int32_t *n_clusters, int32_t *cluster_offsets, int32_t *members) {
 	cudaStream_t st = ctx->stream;
-	const size_t nn = (size_t)n * n;
-	MC_CUDA(cudaMemsetAsync(B.scal, 0, 16 * sizeof(float), st));
-	k_link_sigma<<<1, kLinkThreads, 0, st>>>(n, B.xy, B.xyz, sigma2D, sigma3D, B.tmp, B.scal);
-	MC_LAUNCH_CHECK();
-	dim3 g((n + kLinkThreads - 1) / kLinkThreads, n);
-	k_link_pairs<<<g, kLinkThreads, 0, st>>>(n, B.xy, B.xyz, B.world, W, H, B.depth, B.scal, use3DFilter, B.K2D, B.K3D, B.K3F);
-	MC_LAUNCH_CHECK();
-	const int rb = (int)((nn + kLinkThreads - 1) / kLinkThreads) < 4 * ctx->num_sms ? (int)((nn + kLinkThreads - 1) / kLinkThreads) : 4 * ctx->num_sms;
-	k_link_max<<<rb, kLinkThreads, 0, st>>>(nn, B.K3D, nullptr, 0, B.scal + 2);
-	MC_LAUNCH_CHECK();
-	k_link_scale<<<rb, kLinkThreads, 0, st>>>(nn, B.K3D, B.scal + 2);
-	MC_LAUNCH_CHECK();
-	if (use3DFilter) {
-		k_link_max<<<rb, kLinkThreads, 0, st>>>(nn, B.K3D, B.K3F, use3DFilter == 1 ? 1 : 2, B.scal + 3);
-		MC_LAUNCH_CHECK();
-		k_link_scale<<<rb, kLinkThreads, 0, st>>>(nn, B.K3D, B.scal + 3);
-		MC_LAUNCH_CHECK();
-	}
-	k_link_blend<<<g, kLinkThreads, 0, st>>>(n, B.xy, W, B.distance, B.K2D, B.K3D, B.K);
-	MC_LAUNCH_CHECK();
-	return MC_OK;
-}
-
-static mc_status link_agglomerate_device(mc_ctx *ctx, const LinkBufs &B, int n, float cutoff, int min_pts, int linkage,
-                                         int32_t *n_clusters, int32_t *cluster_offsets, int32_t *members) {
-	cudaStream_t st = ctx->stream;
-	int *d_count = B.out, *d_off = B.out + 1, *d_mem = B.out + 2 + n;
-	if (ctx->linkage_cached && linkage == 1)
-		k_link_agglomerate_cached<<<1, kLinkThreads, 0, st>>>(n, B.K, B.D, cutoff, min_pts, B.valid, B.lists, B.sz, B.tmp, B.ints3, d_count, d_off, d_mem);
-	else
-	k_link_agglomerate<<<1, kLinkThreads, 0, st>>>(n, B.K, B.D, cutoff, min_pts, linkage, B.valid, B.lists, B.sz, B.tmp, d_count, d_off, d_mem);
-	MC_LAUNCH_CHECK();
-	MC_TRY(pinned(ctx, (size_t)(2 * n + 4) * sizeof(int)));
+	// out_count, out_offsets (n + 2) and out_members are contiguous in the arena
+	const size_t words = 1 + (size_t)(n + 2) + (size_t)n;
+	MC_TRY(pinned(ctx, words * sizeof(int)));
 	int *h = (int *)ctx->h_pinned;
-	MC_CUDA(cudaMemcpyAsync(h, B.out, (size_t)(2 * n + 3) * sizeof(int), cudaMemcpyDeviceToHost, st));
+	MC_CUDA(cudaMemcpyAsync(h, B.F.out_count, words * sizeof(int), cudaMemcpyDeviceToHost, st));
 	MC_CUDA(cudaStreamSynchronize(st));
 	const int nc = h[0];
 	*n_clusters = nc;
 	for (int c = 0; c <= nc; c++) cluster_offsets[c] = h[1 + c];
-	for (int k = 0; k < h[1 + nc]; k++) members[k] = h[2 + n + k];
+	for (int k = 0; k < h[1 + nc]; k++) members[k] = h[1 + (n + 2) + k];
 	return MC_OK;
 }
 
@@ -394,17 +537,18 @@ extern "C" mc_status mc_cluster_linkage(mc_ctx *ctx, const float *match_xy, cons
 	MC_CUDA(cudaSetDevice(ctx->device));
 	const int n = n_matches;
 	const size_t px = (size_t)width * height;
-	LinkBufs B;
-	MC_TRY(link_alloc(ctx, n, px, B));
+	LinkOne B;
+	MC_TRY(link_one_alloc(ctx, n, px, B));
 	cudaStream_t st = ctx->stream;
 	MC_CUDA(cudaMemcpyAsync(B.xy, match_xy, sizeof(float) * 2 * n, cudaMemcpyHostToDevice, st));
 	MC_CUDA(cudaMemcpyAsync(B.xyz, match_xyz, sizeof(float) * 3 * n, cudaMemcpyHostToDevice, st));
 	MC_CUDA(cudaMemcpyAsync(B.world, match_world, sizeof(float) * 3 * n, cudaMemcpyHostToDevice, st));
 	MC_CUDA(cudaMemcpyAsync(B.depth, depth, sizeof(float) * px, cudaMemcpyHostToDevice, st));
 	MC_CUDA(cudaMemcpyAsync(B.distance, fill_distance, sizeof(float) * px, cudaMemcpyHostToDevice, st));
-	MC_TRY(link_similarity_device(ctx, B, n, width, height, use_3d_filter, sigma_2d, sigma_3d));
-	if (similarity_out) MC_CUDA(cudaMemcpyAsync(similarity_out, B.K, sizeof(float) * (size_t)n * n, cudaMemcpyDeviceToHost, st));
-	return link_agglomerate_device(ctx, B, n, cutoff, min_pts, linkage_type, n_clusters, cluster_offsets, members);
+	B.F.W = width; B.F.H = height;
+	MC_TRY(link_frame_device(ctx, B.F, cutoff, min_pts, use_3d_filter, linkage_type, sigma_2d, sigma_3d));
+	if (similarity_out) MC_CUDA(cudaMemcpyAsync(similarity_out, B.F.K, sizeof(float) * (size_t)n * n, cudaMemcpyDeviceToHost, st));
+	return link_one_download(ctx, B, n, n_clusters, cluster_offsets, members);
 }
 
 extern "C" mc_status mc_linkage_agglomerate(mc_ctx *ctx, const float *similarity, int n, float cutoff, int min_pts, int linkage_type,
@@ -415,8 +559,9 @@ extern "C" mc_status mc_linkage_agglomerate(mc_ctx *ctx, const float *similarity
 	MC_TRY(link_check(ctx, n, "mc_linkage_agglomerate"));
 	if (!(cutoff > -1.f)) { ctx->err = "mc_linkage_agglomerate: cutoff must be > -1"; return MC_ERR_ARG; }
 	MC_CUDA(cudaSetDevice(ctx->device));
-	LinkBufs B;
-	MC_TRY(link_alloc(ctx, n, 1, B));
-	MC_CUDA(cudaMemcpyAsync(B.K, similarity, sizeof(float) * (size_t)n * n, cudaMemcpyHostToDevice, ctx->stream));
-	return link_agglomerate_device(ctx, B, n, cutoff, min_pts, linkage_type, n_clusters, cluster_offsets, members);
+	LinkOne B;
+	MC_TRY(link_one_alloc(ctx, n, 1, B));
+	MC_CUDA(cudaMemcpyAsync(B.F.K, similarity, sizeof(float) * (size_t)n * n, cudaMemcpyHostToDevice, ctx->stream));
+	MC_TRY(link_agglomerate_only(ctx, B.F, cutoff, min_pts, linkage_type));
+	return link_one_download(ctx, B, n, n_clusters, cluster_offsets, members);
 }

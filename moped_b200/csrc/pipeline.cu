@@ -102,11 +102,15 @@ k_match_compact(const FrameDesc *__restrict__ fd, int64_t row_base,
 
 // cluster members -> contiguous per-cluster point arrays (what preprocessAllMatches + `cl` build,
 // POSE_..._CPU.hpp:213-237,288-290). tie = match index inside the model (the reference's pointer order).
+// moped3d's depth pose stages also take depthData.coord3D (pt_world, nullable) and the Cauchy weight of depthData.fillDistance
+// (pt_cauchy, nullable): getCauchyWeight, (float)(1.0 / (1 + f*f)) with f = fill / scale, every operation rounded on its own.
 __global__ void k_gather_points(const int32_t *__restrict__ n_p /* {#clusters, #members} */, const int32_t *__restrict__ cluster_model,
                                 const int32_t *__restrict__ cluster_offsets, const int32_t *__restrict__ members,
                                 const int32_t *__restrict__ match_offsets, const int32_t *__restrict__ match_image,
                                 const float *__restrict__ match_xy, const float *__restrict__ match_xyz,
-                                float *__restrict__ pt_xy, float *__restrict__ pt_xyz, int32_t *__restrict__ pt_image, int32_t *__restrict__ pt_tie) {
+                                float *__restrict__ pt_xy, float *__restrict__ pt_xyz, int32_t *__restrict__ pt_image, int32_t *__restrict__ pt_tie,
+                                const float *__restrict__ match_world = nullptr, const float *__restrict__ match_fill = nullptr,
+                                float cauchy_scale = 1.f, float *__restrict__ pt_world = nullptr, float *__restrict__ pt_cauchy = nullptr) {
 	const int n_clusters = n_p[0];
 	for (int c = blockIdx.x; c < n_clusters; c += gridDim.x) {
 		const int lo = match_offsets[cluster_model[c]];
@@ -116,6 +120,11 @@ __global__ void k_gather_points(const int32_t *__restrict__ n_p /* {#clusters, #
 			pt_xyz[3 * t] = match_xyz[3 * j]; pt_xyz[3 * t + 1] = match_xyz[3 * j + 1]; pt_xyz[3 * t + 2] = match_xyz[3 * j + 2];
 			pt_image[t] = match_image[j];
 			pt_tie[t] = mi;
+			if (pt_world) { pt_world[3 * t] = match_world[3 * j]; pt_world[3 * t + 1] = match_world[3 * j + 1]; pt_world[3 * t + 2] = match_world[3 * j + 2]; }
+			if (pt_cauchy) {
+				const float f = __fdiv_rn(match_fill[j], cauchy_scale);
+				pt_cauchy[t] = __double2float_rn(__ddiv_rn(1.0, (double)__fadd_rn(1.f, __fmul_rn(f, f))));
+			}
 		}
 	}
 }
@@ -250,6 +259,25 @@ static mc_status frame_enqueue(mc_ctx *ctx, const float *d_q, int Q, const mc_pi
 		k_export_objects<<<1, 128, 0, ctx->stream>>>(fd, B.f_n, B.status, B.match_offsets, ctx->n_models, B.cl_n, B.surv_model, B.surv_pose, B.surv_score);
 		MC_LAUNCH_CHECK();
 	}
+	return MC_OK;
+}
+
+// for the moped3d frame chain (depth_frames.cu)
+mc_status gather_depth_points_device(mc_ctx *ctx, const int32_t *d_n, const int32_t *d_cluster_model, const int32_t *d_cluster_offsets,
+                                     const int32_t *d_members, const int32_t *d_match_offsets, const int32_t *d_match_image, const float *d_match_xy,
+                                     const float *d_match_xyz, const float *d_match_world, const float *d_match_fill, float cauchy_scale, float *d_pt_xy,
+                                     float *d_pt_xyz, float *d_pt_world, float *d_pt_cauchy, int32_t *d_pt_image, int32_t *d_pt_tie) {
+	k_gather_points<<<ctx->num_sms, 128, 0, ctx->stream>>>(d_n, d_cluster_model, d_cluster_offsets, d_members, d_match_offsets, d_match_image, d_match_xy,
+	                                                     d_match_xyz, d_pt_xy, d_pt_xyz, d_pt_image, d_pt_tie, d_match_world, d_match_fill, cauchy_scale,
+	                                                     d_pt_world, d_pt_cauchy);
+	MC_LAUNCH_CHECK();
+	return MC_OK;
+}
+
+mc_status copy_objects_device(mc_ctx *ctx, const int32_t *d_n, const int32_t *d_src_model, const float *d_src_pose, int32_t *d_dst_n,
+                              int32_t *d_dst_model, float *d_dst_pose) {
+	k_copy_objects<<<1, 256, 0, ctx->stream>>>(d_n, d_src_model, d_src_pose, d_dst_n, d_dst_model, d_dst_pose);
+	MC_LAUNCH_CHECK();
 	return MC_OK;
 }
 
@@ -515,7 +543,7 @@ static void lane_borrow(mc_ctx *ctx, mc_ctx *lane) {
 	lane->pose_exact_order = ctx->pose_exact_order;
 }
 
-static mc_status ensure_lanes(mc_ctx *ctx, int n) {
+mc_status ensure_lanes(mc_ctx *ctx, int n) {
 	if (!ctx->ev_fork) MC_CUDA(cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming));
 	while ((int)ctx->lanes.size() < n) {
 		mc_ctx *lane = new mc_ctx;

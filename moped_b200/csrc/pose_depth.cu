@@ -79,9 +79,10 @@ k_depth_hypotheses(const int32_t *__restrict__ cluster_offsets, const float *__r
 // ---- RANSAC: one CTA per (cluster, try) task, one warp per test, rounds of kDepthWarps consecutive tests ----
 // Reference semantics (RANSAC(), …BACKPROJECTION_DEPTH_CPU.hpp:278-314): sequential tests, return at the FIRST one whose
 // consistent set exceeds MinNPtsObject, refitted on that set. The lowest successful index of a round is that test.
-template <int V>
+// kDevCount: the cluster count is read from the device (*n_clusters_p, at most n_clusters_cap); tasks past it find nothing
+template <int V, bool kDevCount>
 __global__ void __launch_bounds__(32 * kDepthWarps)
-k_depth_ransac(const int32_t *__restrict__ cluster_offsets, int n_clusters, const float *__restrict__ xy, const float *__restrict__ xyz,
+k_depth_ransac(const int32_t *__restrict__ cluster_offsets, int n_clusters_cap, const int32_t *__restrict__ n_clusters_p, const float *__restrict__ xy, const float *__restrict__ xyz,
                const float *__restrict__ world, const float *__restrict__ cauchy, const int32_t *__restrict__ image,
                const int32_t *__restrict__ tie, const Camera *__restrict__ cams, float alpha, int max_obj, int max_ransac, int max_lm, int n_align,
                int min_npts, float thr, uint64_t seed, int finite_check, float *__restrict__ scratch, size_t slice, int n_max,
@@ -95,6 +96,7 @@ k_depth_ransac(const int32_t *__restrict__ cluster_offsets, int n_clusters, cons
 	uint8_t *my_mask = reinterpret_cast<uint8_t *>(my + lmx::hypothesis_scratch_floats(n_max, R));
 	lmx::Team<32> team;
 	team.init(lane);
+	const int n_clusters = kDevCount ? min(*n_clusters_p, n_clusters_cap) : n_clusters_cap;
 	for (int task = blockIdx.x; task < n_tasks; task += gridDim.x) {
 	const int cidx = task / max_obj;
 	if (cidx >= n_clusters) { if (threadIdx.x == 0) { found[task] = 0; n_tests[task] = 0; } continue; }
@@ -181,9 +183,12 @@ mc_status pose_depth_hypotheses_device(mc_ctx *ctx, int variant, const int32_t *
 	return MC_OK;
 }
 
+// d_n_clusters (nullable): the cluster count on the device (the moped3d frame chain); n_clusters and n_max are then upper bounds
+// that size the grid and the LM scratch
 mc_status pose_depth_ransac_device(mc_ctx *ctx, int variant, const int32_t *d_cluster_offsets, int n_clusters, int n_max, const float *d_xy,
                                    const float *d_xyz, const float *d_world, const float *d_cauchy, const int32_t *d_image, const int32_t *d_tie,
-                                   const mc_pose_params *pp, float alpha, uint8_t *d_found, float *d_pose, int32_t *d_n_tests) {
+                                   const mc_pose_params *pp, float alpha, uint8_t *d_found, float *d_pose, int32_t *d_n_tests,
+                                   const int32_t *d_n_clusters) {
 	if (!ctx->d_cams) { ctx->err = "pose (depth): cameras not set (mc_set_cameras)"; return MC_ERR_STATE; }
 	if (variant < 0 || variant > 2) { ctx->err = "pose (exact order): variant must be 0 (back-projection + depth), 1 (reprojection + depth) or 2 (moped2 reprojection)"; return MC_ERR_ARG; }
 	if (variant != 2 && (!d_world || !d_cauchy)) { ctx->err = "pose (depth): world3D and Cauchy weights are required"; return MC_ERR_ARG; }
@@ -193,20 +198,24 @@ mc_status pose_depth_ransac_device(mc_ctx *ctx, int variant, const int32_t *d_cl
 	const int R = variant == 1 ? 3 : 2;
 	const size_t slice = depth_slice_floats(n_max, R);
 	int per_sm = 0;
-	const void *fn = variant == 0 ? (const void *)k_depth_ransac<0> : variant == 1 ? (const void *)k_depth_ransac<1> : (const void *)k_depth_ransac<2>;
+	if (d_n_clusters && variant == 2) { ctx->err = "pose (exact order): no device cluster count for variant 2"; return MC_ERR_ARG; }
+	const void *fn = d_n_clusters ? (variant == 0 ? (const void *)k_depth_ransac<0, true> : (const void *)k_depth_ransac<1, true>)
+	                              : (variant == 0 ? (const void *)k_depth_ransac<0, false> : variant == 1 ? (const void *)k_depth_ransac<1, false>
+	                                                                                                   : (const void *)k_depth_ransac<2, false>);
 	MC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, 32 * kDepthWarps, 0));
 	int grid = ctx->num_sms * (per_sm > 0 ? per_sm : 1);
 	if (grid > n_tasks) grid = n_tasks;
 	while (grid > 1 && (size_t)grid * kDepthWarps * slice * sizeof(float) > ((size_t)1 << 30)) grid = (grid + 1) / 2;
 	float *scratch = nullptr;
 	MC_TRY(depth_scratch(ctx, (size_t)grid * kDepthWarps, slice, &scratch));
-#define MC_DEPTH_RANSAC(V)                                                                                                                      \
-	k_depth_ransac<V><<<grid, 32 * kDepthWarps, 0, ctx->stream>>>(d_cluster_offsets, n_clusters, d_xy, d_xyz, d_world, d_cauchy, d_image, d_tie, \
+#define MC_DEPTH_RANSAC(V, DC)                                                                                                                  \
+	k_depth_ransac<V, DC><<<grid, 32 * kDepthWarps, 0, ctx->stream>>>(d_cluster_offsets, n_clusters, d_n_clusters, d_xy, d_xyz, d_world, d_cauchy, d_image, d_tie, \
 	                                                                ctx->d_cams, alpha, pp->max_objects_per_cluster, pp->max_ransac_tests,     \
 	                                                                pp->max_lm_tests, pp->n_pts_align, pp->min_npts_object, pp->error_threshold, \
 	                                                                pp->seed, ctx->lm_finite_check ? 1 : 0, scratch, slice, n_max, n_tasks,    \
 	                                                                d_found, d_pose, d_n_tests)
-	if (variant == 0) MC_DEPTH_RANSAC(0); else if (variant == 1) MC_DEPTH_RANSAC(1); else MC_DEPTH_RANSAC(2);
+	if (d_n_clusters) { if (variant == 0) MC_DEPTH_RANSAC(0, true); else MC_DEPTH_RANSAC(1, true); }
+	else if (variant == 0) MC_DEPTH_RANSAC(0, false); else if (variant == 1) MC_DEPTH_RANSAC(1, false); else MC_DEPTH_RANSAC(2, false);
 #undef MC_DEPTH_RANSAC
 	MC_LAUNCH_CHECK();
 	return MC_OK;

@@ -281,3 +281,85 @@ def make_filter_depth_scene(seed: int = 1, n_models: int = 3, pts_per_model: int
                 match_offsets=np.array(m_off, np.int32), match_xy=np.concatenate(m_xy).astype(np.float32),
                 match_xyz=np.concatenate(m_xyz).astype(np.float32), match_image=np.zeros(m_off[-1], np.int32),
                 obj_model=np.array(obj_model, np.int32)[order], obj_pose=np.stack(obj_pose).astype(np.float32)[order])
+
+
+def make_depth_frame(seed: int = 1, n_models: int = 12, W: int = 640, H: int = 480, pts_per_model: int = 160, outlier_frac: float = 0.15):
+    """One 640x480 RGB-D frame of moped3d's recognition steps in the C-ABI layout of mc_process_depth_frames (FrameData after DEPTHPROP,
+    identity camera, Kinect-like K): about a third of the `n_models` models are seen once or twice at planted poses (40-70 matched
+    keypoints each, `outlier_frac` of them at random pixels with wrong depth), a few models get a handful of junk matches (3-6, too few
+    to form a cluster) and the rest none. The depth map shows every instance as a patch at its depth over a slanted background; the
+    fill-distance map has holes (> 0 = hallucinated depth). A model's matches come in random (query) order, instances interleaved.
+    Returns dict(match_offsets[n_models+1], match_image, match_xy, match_xyz, match_world, match_fill, depth[H,W], fill_distance[H,W],
+    K, cam_pose, gt_model[V], gt_pose[V,7], junk_models)."""
+    rng = np.random.default_rng(BASE_SEED + 6151 * seed)
+    K = K_DEPTH
+    depth = (2.2 + 0.0006 * np.arange(W)[None, :] + 0.0004 * np.arange(H)[:, None]).astype(np.float32)
+    fill_map = np.zeros((H, W), np.float32)
+    holes = rng.random((H, W)) < 0.15
+    fill_map[holes] = rng.uniform(1, 40, int(holes.sum())).astype(np.float32)
+    model_pts = [np.random.default_rng(BASE_SEED + 31 * m).uniform(-0.06, 0.06, (pts_per_model, 3)) for m in range(n_models)]
+    order = rng.permutation(n_models)
+    n_seen = max(1, n_models // 3)
+    seen, junk = order[:n_seen], order[n_seen:n_seen + max(1, n_models // 4)]
+    cells = [(c, r) for r in range(3) for c in range(4)]                      # 160 x 160 cells: instances never overlap
+    free = list(rng.permutation(len(cells)))
+    per_model = {m: [] for m in range(n_models)}
+    gt_model, gt_pose = [], []
+    for m in seen:
+        for _ in range(1 if rng.random() < 0.6 or len(free) < 2 else 2):
+            if not free:
+                break
+            c, r = cells[free.pop()]
+            cx, cy = 80 + 160 * c + rng.uniform(-15, 15), 80 + 160 * r + rng.uniform(-15, 15)
+            z = rng.uniform(0.7, 1.1)
+            t = np.array([(cx - K[2]) / K[0] * z, (cy - K[3]) / K[1] * z, z])
+            q = rng.normal(size=4)
+            q /= np.linalg.norm(q)
+            n = int(rng.integers(40, 71))
+            X = model_pts[m][rng.choice(pts_per_model, n, replace=False)]
+            cam3 = X @ quat_to_R(q).T + t
+            uv = np.stack([cam3[:, 0] / cam3[:, 2] * K[0] + K[2], cam3[:, 1] / cam3[:, 2] * K[1] + K[3]], 1) + rng.normal(0, 0.4, (n, 2))
+            w = cam3 * (1 + rng.normal(0, 0.0035, (n, 1)) * cam3[:, 2:3])
+            bad = rng.random(n) < outlier_frac
+            uv[bad] = rng.uniform([0, 0], [W - 1, H - 1], (int(bad.sum()), 2))
+            uv = np.clip(uv, 0.5, [W - 1.5, H - 1.5])
+            w[bad] = w[bad] + rng.normal(0, 0.2, (int(bad.sum()), 3))
+            half = 45
+            depth[max(0, int(cy) - half):int(cy) + half, max(0, int(cx) - half):int(cx) + half] = np.float32(z)
+            per_model[m].append((uv, X, w))
+            gt_model.append(int(m)); gt_pose.append(np.concatenate([q, t]).astype(np.float32))
+    for m in junk:
+        n = int(rng.integers(3, 7))
+        uv = rng.uniform([0, 0], [W - 1, H - 1], (n, 2))
+        X = model_pts[m][rng.choice(pts_per_model, n, replace=False)]
+        zz = depth[uv[:, 1].astype(int), uv[:, 0].astype(int)][:, None]
+        w = np.concatenate([(uv - K[2:4]) / K[0:2] * zz, zz], 1)
+        per_model[m].append((uv, X, w))
+    offs, xy, xyz, world = [0], [], [], []
+    for m in range(n_models):
+        if per_model[m]:
+            uv = np.concatenate([a[0] for a in per_model[m]]); X = np.concatenate([a[1] for a in per_model[m]])
+            w = np.concatenate([a[2] for a in per_model[m]])
+            perm = rng.permutation(len(uv))
+            xy.append(uv[perm]); xyz.append(X[perm]); world.append(w[perm])
+        offs.append(offs[-1] + (len(xy[-1]) if per_model[m] else 0))
+    M = offs[-1]
+    cat = lambda a, k: (np.concatenate(a) if a else np.zeros((0, k))).astype(np.float32)
+    fill = np.where(rng.random(M) < 0.7, 0.0, rng.uniform(0, 0.3, M)).astype(np.float32)
+    return dict(match_offsets=np.array(offs, np.int32), match_image=np.zeros(M, np.int32), match_xy=cat(xy, 2), match_xyz=cat(xyz, 3),
+                match_world=cat(world, 3), match_fill=fill, depth=depth, fill_distance=fill_map, K=K.copy(), cam_pose=CAM_IDENTITY.copy(),
+                gt_model=np.array(gt_model, np.int32), gt_pose=np.stack(gt_pose) if gt_pose else np.zeros((0, 7), np.float32),
+                junk_models=np.sort(junk).astype(np.int32))
+
+
+def stack_depth_frames(frames):
+    """Frames of make_depth_frame -> the batch layout of mc_process_depth_frames: match_offsets [n_frames, n_models+1] as global
+    indices into the concatenated per-match arrays, depth / fill_distance [n_frames, H, W]."""
+    base, rows = 0, []
+    for fr in frames:
+        rows.append(fr["match_offsets"] + base)
+        base += int(fr["match_offsets"][-1])
+    cat = lambda k: np.concatenate([fr[k] for fr in frames])
+    return dict(match_offsets=np.stack(rows).astype(np.int32), match_image=cat("match_image"), match_xy=cat("match_xy"), match_xyz=cat("match_xyz"),
+                match_world=cat("match_world"), match_fill=cat("match_fill"), depth=np.stack([fr["depth"] for fr in frames]),
+                fill_distance=np.stack([fr["fill_distance"] for fr in frames]))
