@@ -19,6 +19,7 @@
 #include "common.cuh"
 
 #include <math_constants.h>
+#include <type_traits>
 
 // MC_COARSE_DBG (experiments only, never in the shipped library): 1 = the epilogue hands the accumulator stage back without
 // reading it (MMA + TMA pace alone), 2 = the epilogue reads TMEM but skips the top-k scan (adds the TMEM-read pace),
@@ -47,18 +48,20 @@ __device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
 __device__ __forceinline__ void mbar_arrive(uint32_t bar) {
 	asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
 }
+// the retry loop branches on the try_wait predicate itself (labels are local to the braces, so every inlined copy has its own)
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-	uint32_t ok;
-	do {
-		asm volatile(
-		    "{\n\t.reg .pred p;\n\t"
-		    "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-		    "selp.u32 %0, 1, 0, p;\n\t}"
-		    : "=r"(ok)
-		    : "r"(bar), "r"(parity)
-		    : "memory");
-	} while (!ok);
+	asm volatile(
+	    "{\n\t.reg .pred p;\n"
+	    "MC_WAIT:\n\t"
+	    "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
+	    "@!p bra MC_WAIT;\n\t}"
+	    ::"r"(bar), "r"(parity)
+	    : "memory");
 }
+// warpgroup-wide register budget (all 128 threads of the warpgroup execute it, before any divergence): the warpgroup's threads
+// give registers back to the CTA's pool / take them from it
+template <uint32_t R> __device__ __forceinline__ void regs_dec() { asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(R)); }
+template <uint32_t R> __device__ __forceinline__ void regs_inc() { asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(R)); }
 __device__ __forceinline__ void fence_barrier_init() {
 	asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
 	asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
@@ -285,6 +288,17 @@ template <> struct CoarseKind<1> {
 	static constexpr int kTile = kTile8Bytes, kStages = 8, kABuf = 2, kK = kTopK8 / kCG, kSteps = 4;
 };
 constexpr int kCoarseThreads = 128 + 256 * kCG;   // warp 0 TMA, warp 1 MMA, warp 2 TMEM alloc, warp 3 second MMA issuer, then 8 epilogue warps per column group
+// Register budgets (setmaxnreg): the CTA is launched with what __launch_bounds__(kCoarseThreads, 1) allows every thread (96 for
+// kCG = 2); warpgroup 0 runs single-lane control code and gives half of it back, the epilogue warpgroups take it:
+// 128 x 48 + 512 x 104 <= 640 x 96. (At 32 / 40 the MMA issuers spill, and the epilogue cannot use more than 104 either way.)
+constexpr uint32_t kRegsLaunch = (65536 / kCoarseThreads) & ~7u;
+constexpr uint32_t kRegsControl = 48;
+constexpr uint32_t kRegsEpilogue = ((kRegsLaunch * kCoarseThreads - 128 * kRegsControl) / (256 * kCG)) & ~7u;
+static_assert(kRegsEpilogue <= 256 && 128 * kRegsControl + 256 * kCG * kRegsEpilogue <= kRegsLaunch * kCoarseThreads, "register pool");
+// the CTA-wide barrier before TMEM is freed, reached from both warpgroup branches: barrier.sync without .aligned (code reachable
+// from the epilogue that needs a warp-collective call, as the .aligned forms in divergent code do, pins its registers to the
+// launch budget)
+__device__ __forceinline__ void teardown_sync() { asm volatile("barrier.sync 1, %0;" ::"n"(kCoarseThreads) : "memory"); }
 constexpr uint32_t kSmemA = 0;          // A operand: kABuf x (2 halves x kTile) = 64 KiB for both kinds
 constexpr uint32_t kSmemB = 65536;      // B ring: kStages x kTile = 128 KiB for both kinds
 constexpr uint32_t kSmemBar = kSmemB + 131072;
@@ -439,7 +453,9 @@ k_match_coarse(const CoarseArgs a) {
 		t0 = (int64_t)split * a.tiles_per_split;
 		const int64_t t1 = (t0 + a.tiles_per_split < a.n_tiles) ? t0 + a.tiles_per_split : a.n_tiles;
 		ntiles = (int)(t1 > t0 ? t1 - t0 : 0);
-		first = a.stagger ? (int)((int64_t)ntiles * blockIdx.x / gridDim.x) : 0;
+		// 32-bit on purpose: a 64-bit division is a called subroutine, and a call in the epilogue pins its registers to the launch
+		// budget. The product wraps only beyond 2^32 / gridDim.x tiles in a split, and the quotient stays below ntiles even then.
+		first = a.stagger ? (int)((uint32_t)ntiles * blockIdx.x / gridDim.x) : 0;
 	};
 	auto tile_at = [](int i, int first, int ntiles) { const int t = i + first; return t >= ntiles ? t - ntiles : t; };
 	// consumers of the item ring: the it-th item of this CTA, or -1 when the counter has run out
@@ -452,175 +468,181 @@ k_match_coarse(const CoarseArgs a) {
 		return item;
 	};
 
-	if (warp == 0) {
-		// ===== TMA producer =====
-		if (lane == 0) {
-			uint32_t tc = 0;
-			for (uint32_t it = 0;; it++) {
-				const uint32_t sl = it & 1;
-				mbar_wait(bar_iempty(sl), ((it >> 1) & 1) ^ 1);
-				int item = (int)atomicAdd(a.item_counter, 1u);
-				if (item >= n_items) item = -1;
-				item_ring[sl] = item;
-				mbar_arrive(bar_ifull(sl));            // release: the consumers' wait acquires the slot
-				if (item < 0) break;
-				int mtile, split, ntiles, first; int64_t t0;
-				item_range(item, mtile, split, t0, ntiles, first);
-				const uint32_t ab = it % C::kABuf;
-				mbar_wait(bar_aempty(ab), ((it / C::kABuf) & 1) ^ 1);
-				mbar_expect_tx(bar_afull(ab), 2 * C::kTile);
-				bulk_g2s(smem_base + kSmemA + ab * 2 * C::kTile, a.q_img + (size_t)mtile * 2 * C::kTile, 2 * C::kTile, bar_afull(ab));
-				for (int i = 0; i < ntiles; i++, tc++) {
-					const uint32_t b = tc % C::kStages;
-					mbar_wait(bar_empty(b), ((tc / C::kStages) & 1) ^ 1);
+	if (warp < 4) {
+		// warpgroup 0 (TMA producer, MMA issuers, TMEM allocator) runs single-lane code: it gives registers to the epilogue
+		regs_dec<kRegsControl>();
+		if (warp == 0) {
+			// ===== TMA producer =====
+			if (lane == 0) {
+				uint32_t tc = 0;
+				for (uint32_t it = 0;; it++) {
+					const uint32_t sl = it & 1;
+					mbar_wait(bar_iempty(sl), ((it >> 1) & 1) ^ 1);
+					int item = (int)atomicAdd(a.item_counter, 1u);
+					if (item >= n_items) item = -1;
+					item_ring[sl] = item;
+					mbar_arrive(bar_ifull(sl));            // release: the consumers' wait acquires the slot
+					if (item < 0) break;
+					int mtile, split, ntiles, first; int64_t t0;
+					item_range(item, mtile, split, t0, ntiles, first);
+					const uint32_t ab = it % C::kABuf;
+					mbar_wait(bar_aempty(ab), ((it / C::kABuf) & 1) ^ 1);
+					mbar_expect_tx(bar_afull(ab), 2 * C::kTile);
+					bulk_g2s(smem_base + kSmemA + ab * 2 * C::kTile, a.q_img + (size_t)mtile * 2 * C::kTile, 2 * C::kTile, bar_afull(ab));
+					for (int i = 0; i < ntiles; i++, tc++) {
+						const uint32_t b = tc % C::kStages;
+						mbar_wait(bar_empty(b), ((tc / C::kStages) & 1) ^ 1);
 #if MC_COARSE_DBG == 6
-					mbar_arrive(bar_full(b));
+						mbar_arrive(bar_full(b));
 #else
-					mbar_expect_tx(bar_full(b), C::kTile);
-					bulk_g2s(smem_base + kSmemB + b * C::kTile, a.db_img + (size_t)(t0 + tile_at(i, first, ntiles)) * C::kTile, C::kTile, bar_full(b));
-#endif
-				}
-			}
-		}
-		__syncwarp();
-	} else if (warp == 1 || (warp == 3 && MC_MMA_THREADS == 2)) {
-		// ===== MMA issuer(s): one thread, or two that take alternate tiles (thread p owns accumulator stage p) =====
-		// ONE tcgen05.commit per DB tile: every commit costs the issuing thread about 190 cycles in which it issues nothing
-		// (measured: tile time = MMA floor + 190 x commits), so the shared-memory stage is handed back to the TMA producer by
-		// an epilogue thread once it has seen this commit, and a second issuer fills the gap of the first.
-		const int p = warp == 3 ? 1 : 0;
-		if (lane == 0) {
-			uint32_t tc = 0;
-			for (uint32_t it = 0;; it++) {
-				const int item = next_item(it, false);
-				if (item < 0) break;
-				int mtile, split, ntiles, first; int64_t t0;
-				item_range(item, mtile, split, t0, ntiles, first);
-				const uint32_t ab = it % C::kABuf;
-				uint32_t idesc[2] = { kIdescF16, kIdescF16 };
-				if (KIND == 1)
-					for (int h = 0; h < 2; h++) idesc[h] = kIdescI8 | ((uint32_t)a.a_signed[2 * mtile + h] << 7) | (a.b_signed << 10);
-				mbar_wait(bar_afull(ab), (it / C::kABuf) & 1);
-				for (int i = 0; i < ntiles; i++, tc++) {
-					if (MC_MMA_THREADS == 2 && (int)(tc & 1) != p) continue;
-					const uint32_t s = tc & 1, b = tc % C::kStages;
-					mbar_wait(bar_full(b), (tc / C::kStages) & 1);
-#pragma unroll
-					for (int h = 0; h < 2; h++) {
-						mbar_wait(bar_tempty(s, h), ((tc >> 1) & 1) ^ 1);
-						tc_fence_after();
-#if MC_COARSE_DBG != 5
-						const uint32_t d_tmem = tmem_base + (uint32_t)(s * 256 + h * 128);
-#pragma unroll
-						for (int k = 0; k < C::kSteps; k++) {
-							const uint32_t koff = KIND == 0 ? (uint32_t)((k >> 2) * 16384 + (k & 3) * 32) : (uint32_t)(k * 32);
-							const uint64_t a_desc = make_desc(smem_base + kSmemA + (ab * 2 + h) * C::kTile + koff);
-							const uint64_t b_desc = make_desc(smem_base + kSmemB + b * C::kTile + koff);
-							if (KIND == 0) umma_f16(d_tmem, a_desc, b_desc, idesc[h], k > 0 ? 1u : 0u);
-							else umma_i8(d_tmem, a_desc, b_desc, idesc[h], k > 0 ? 1u : 0u);
-						}
+						mbar_expect_tx(bar_full(b), C::kTile);
+						bulk_g2s(smem_base + kSmemB + b * C::kTile, a.db_img + (size_t)(t0 + tile_at(i, first, ntiles)) * C::kTile, C::kTile, bar_full(b));
 #endif
 					}
-#if MC_COARSE_DBG == 5
-					(void)idesc;
-					mbar_arrive(bar_tfull(s));
-#else
-					umma_commit(bar_tfull(s));         // both halves of the accumulator stage complete, shared-memory stage b read
-#endif
 				}
-				umma_commit(bar_aempty(ab));           // query image reusable once the item's MMAs (of this issuer) have read it
 			}
+			__syncwarp();
+		} else if (warp == 1 || (warp == 3 && MC_MMA_THREADS == 2)) {
+			// ===== MMA issuer(s): one thread, or two that take alternate tiles (thread p owns accumulator stage p) =====
+			// ONE tcgen05.commit per DB tile: every commit costs the issuing thread about 190 cycles in which it issues nothing
+			// (measured: tile time = MMA floor + 190 x commits), so the shared-memory stage is handed back to the TMA producer by
+			// an epilogue thread once it has seen this commit, and a second issuer fills the gap of the first.
+			const int p = warp == 3 ? 1 : 0;
+			if (lane == 0) {
+				uint32_t tc = 0;
+				for (uint32_t it = 0;; it++) {
+					const int item = next_item(it, false);
+					if (item < 0) break;
+					int mtile, split, ntiles, first; int64_t t0;
+					item_range(item, mtile, split, t0, ntiles, first);
+					const uint32_t ab = it % C::kABuf;
+					uint32_t idesc[2] = { kIdescF16, kIdescF16 };
+					if (KIND == 1)
+						for (int h = 0; h < 2; h++) idesc[h] = kIdescI8 | ((uint32_t)a.a_signed[2 * mtile + h] << 7) | (a.b_signed << 10);
+					mbar_wait(bar_afull(ab), (it / C::kABuf) & 1);
+					for (int i = 0; i < ntiles; i++, tc++) {
+						if (MC_MMA_THREADS == 2 && (int)(tc & 1) != p) continue;
+						const uint32_t s = tc & 1, b = tc % C::kStages;
+						mbar_wait(bar_full(b), (tc / C::kStages) & 1);
+#pragma unroll
+						for (int h = 0; h < 2; h++) {
+							mbar_wait(bar_tempty(s, h), ((tc >> 1) & 1) ^ 1);
+							tc_fence_after();
+#if MC_COARSE_DBG != 5
+							const uint32_t d_tmem = tmem_base + (uint32_t)(s * 256 + h * 128);
+#pragma unroll
+							for (int k = 0; k < C::kSteps; k++) {
+								const uint32_t koff = KIND == 0 ? (uint32_t)((k >> 2) * 16384 + (k & 3) * 32) : (uint32_t)(k * 32);
+								const uint64_t a_desc = make_desc(smem_base + kSmemA + (ab * 2 + h) * C::kTile + koff);
+								const uint64_t b_desc = make_desc(smem_base + kSmemB + b * C::kTile + koff);
+								if (KIND == 0) umma_f16(d_tmem, a_desc, b_desc, idesc[h], k > 0 ? 1u : 0u);
+								else umma_i8(d_tmem, a_desc, b_desc, idesc[h], k > 0 ? 1u : 0u);
+							}
+#endif
+						}
+#if MC_COARSE_DBG == 5
+						(void)idesc;
+						mbar_arrive(bar_tfull(s));
+#else
+						umma_commit(bar_tfull(s));         // both halves of the accumulator stage complete, shared-memory stage b read
+#endif
+					}
+					umma_commit(bar_aempty(ab));           // query image reusable once the item's MMAs (of this issuer) have read it
+				}
+			}
+			__syncwarp();
 		}
-		__syncwarp();
-	} else if (warp >= 4) {
+		tc_fence_before();
+		teardown_sync();
+		if (warp == 2) { tc_fence_after(); tmem_dealloc(tmem_base, 512); }
+	} else {
+		regs_inc<kRegsEpilogue>();
 		// ===== epilogue: one (query, column group) per thread =====
 		// kCG = 2: 16 warps, four per SM sub-partition; a thread scans 64 of the tile's 128 columns for its query and keeps its
 		// own top-k — the chain "wait for the stage, tcgen05.ld, max tree, compare" is latency-bound (about 7 cycles per
 		// instruction with two warps per sub-partition), four warps hide twice as much of it.
-		const int e = warp - 4;
+		const int e = __shfl_sync(0xffffffffu, warp, 0) - 4;     // known to be warp-uniform: per-warp values stay in uniform registers
 		const int quarter = e & 3, half = (e >> 2) & 1, cg = e >> 3;          // TMEM lane quarter == warp % 4
+		constexpr int kCols = 128 / kCG;                   // accumulator columns (DB rows of a tile) per thread
+		// accumulator stage s = tc & 1 adds 256 columns to the TMEM address and 8 s / 16 s bytes to its full / empty barrier
+		const uint32_t taddr0 = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(half * 128 + cg * kCols);
+		const uint32_t tfull0 = bar_tfull(0), tempty0 = bar_tempty(0, half);
+		const bool returns_stage = e == 0 && lane == 0;   // hands the shared-memory stage of a tile back to the TMA producer
 		uint32_t tc = 0;
 		T ra[32], rb[32];
 		uint32_t (&ua)[32] = reinterpret_cast<uint32_t (&)[32]>(ra);
 		uint32_t (&ub)[32] = reinterpret_cast<uint32_t (&)[32]>(rb);
-		constexpr int kCols = 128 / kCG;                   // accumulator columns (DB rows of a tile) per thread
 		for (uint32_t it = 0;; it++) {
 			const int item = next_item(it, true);
 			if (item < 0) break;
 			int mtile, split, ntiles, first; int64_t t0;
 			item_range(item, mtile, split, t0, ntiles, first);
 			const int qid = mtile * kMTile + half * 128 + quarter * 32 + lane;
+			uint32_t *const gtau = a.g_tau + qid;
 			T ts[K]; int ti[K];
 #pragma unroll
 			for (int j = 0; j < K; j++) { ts[j] = S::none(); ti[j] = -1; }
 			T tau = KIND == 1 ? (T)0 : S::none(), published = tau;
 			uint32_t og = 0;
-			const int last_tile = (int)(a.n_tiles - 1 - t0);                     // index (within the split) of the database's ragged last tile
-			for (int i = 0; i < ntiles; i++, tc++) {
-				const uint32_t s = tc & 1;
-				// other items' threshold: fetched every 8th tile and consumed 7 tiles later (a load the next tile already waits
-				// for would put an L2 round trip into every tile); this thread's k-th best is published at the same pace
-				if ((i & 7) == 7) {
+			// first DB row of this thread's columns: runs through the split from tile `first` and wraps to the split's first tile
+			const int row_lo = (int)t0 * kTileRows + cg * kCols, row_end = row_lo + ntiles * kTileRows;
+			int row0 = row_lo + first * kTileRows;
+			// the tile loop; only the items whose split holds the database's ragged last tile run the instance that masks it
+			auto tiles = [&](auto ragged) {
+				for (int i0 = 0; i0 < ntiles; i0 += 8) {
+					// other items' threshold: fetched once per 8 tiles and consumed 8 tiles later (a load the next tile already waits
+					// for would put an L2 round trip into every tile); this thread's k-th best is published at the same pace. Both
+					// are no-ops in the first block: og = 0 decodes to -inf and the list is still empty.
 					tau = S::vmax(tau, S::dec(og));
-					if (ts[K - 1] > published) { published = ts[K - 1]; atomicMax(&a.g_tau[qid], S::enc(published)); }
-				}
-				if ((i & 7) == 0) og = __ldcg(&a.g_tau[qid]);
-				const int tl = tile_at(i, first, ntiles);
-				const int row0 = (int)(t0 + tl) * kTileRows + cg * kCols;
-				const bool tail = tl == last_tile;
-				const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(s * 256 + half * 128 + cg * kCols);
-				mbar_wait(bar_tfull(s), (tc >> 1) & 1);
-				tc_fence_after();
-				if (e == 0 && lane == 0) mbar_arrive(bar_empty(tc % C::kStages));   // the tile's MMAs have read their shared-memory stage
+					if (ts[K - 1] > published) { published = ts[K - 1]; atomicMax(gtau, S::enc(published)); }
+					og = __ldcg(gtau);
+					const int n = ntiles - i0 < 8 ? ntiles - i0 : 8;
+					for (int j = 0; j < n; j++, tc++) {
+						const uint32_t s = tc & 1;
+						const uint32_t taddr = taddr0 + (s << 8);
+						mbar_wait(tfull0 + 8 * s, (tc >> 1) & 1);
+						tc_fence_after();
+						if (returns_stage) mbar_arrive(bar_empty(tc % C::kStages));   // the tile's MMAs have read their shared-memory stage
 #if MC_COARSE_DBG == 1 || MC_COARSE_DBG == 5 || MC_COARSE_DBG == 6
-				tc_fence_before();
-				__syncwarp();
-				if (lane == 0) mbar_arrive(bar_tempty(s, half));
-				(void)taddr; (void)tail; (void)ua; (void)ub; (void)row0;
+						tc_fence_before();
+						__syncwarp();
+						if (lane == 0) mbar_arrive(tempty0 + 16 * s);
+						(void)taddr; (void)ua; (void)ub; (void)ragged;
 #elif MC_COARSE_DBG == 2
-				for (int c = 0; c < kCols; c += 64) {
-					tmem_ld32(taddr + c, ua); tmem_ld32(taddr + c + 32, ub); tmem_ld_wait();
-					tau = S::vmax(tau, S::vmax(ra[0], rb[31]));
-				}
-				tc_fence_before();
-				__syncwarp();
-				if (lane == 0) mbar_arrive(bar_tempty(s, half));
-				(void)tail; (void)row0;
+						for (int c = 0; c < kCols; c += 64) {
+							tmem_ld32(taddr + c, ua); tmem_ld32(taddr + c + 32, ub); tmem_ld_wait();
+							tau = S::vmax(tau, S::vmax(ra[0], rb[31]));
+						}
+						tc_fence_before();
+						__syncwarp();
+						if (lane == 0) mbar_arrive(tempty0 + 16 * s);
+						(void)ragged;
 #else
-				if (kCG == 2) {
-					tmem_ld32(taddr, ua);
-					tmem_ld32(taddr + 32, ub);
-					tmem_ld_wait();
-					// all TMEM reads of this thread's part of the half stage are done: hand it back to the MMA thread
-					tc_fence_before();
-					__syncwarp();
-					if (lane == 0) mbar_arrive(bar_tempty(s, half));
-					if (tail) { mask_tail<T>(ra, row0, a.n_rows); mask_tail<T>(rb, row0 + 32, a.n_rows); }
-					scan_chunk<T, K>(ra, row0, tau, ts, ti);
-					scan_chunk<T, K>(rb, row0 + 32, tau, ts, ti);
-				} else {
-					tmem_ld32(taddr, ua);
-					tmem_ld_wait();
-					tmem_ld32(taddr + 32, ub);
-					if (tail) mask_tail<T>(ra, row0, a.n_rows);
-					scan_chunk<T, K>(ra, row0, tau, ts, ti);
-					tmem_ld_wait();
-					tmem_ld32(taddr + 64, ua);
-					if (tail) mask_tail<T>(rb, row0 + 32, a.n_rows);
-					scan_chunk<T, K>(rb, row0 + 32, tau, ts, ti);
-					tmem_ld_wait();
-					tmem_ld32(taddr + 96, ub);
-					if (tail) mask_tail<T>(ra, row0 + 64, a.n_rows);
-					scan_chunk<T, K>(ra, row0 + 64, tau, ts, ti);
-					tmem_ld_wait();
-					tc_fence_before();
-					__syncwarp();
-					if (lane == 0) mbar_arrive(bar_tempty(s, half));
-					if (tail) mask_tail<T>(rb, row0 + 96, a.n_rows);
-					scan_chunk<T, K>(rb, row0 + 96, tau, ts, ti);
-				}
+#pragma unroll
+						for (int c = 0; c < kCols; c += 64) {
+							tmem_ld32(taddr + c, ua);
+							tmem_ld32(taddr + c + 32, ub);
+							tmem_ld_wait();
+							if (c + 64 == kCols) {
+								// all TMEM reads of this thread's part of the half stage are done: hand it back to the MMA thread
+								tc_fence_before();
+								__syncwarp();
+								if (lane == 0) mbar_arrive(tempty0 + 16 * s);
+							}
+							if constexpr (decltype(ragged)::value) {
+								if (row0 + c + 64 > a.n_rows) { mask_tail<T>(ra, row0 + c, a.n_rows); mask_tail<T>(rb, row0 + c + 32, a.n_rows); }
+							}
+							scan_chunk<T, K>(ra, row0 + c, tau, ts, ti);
+							scan_chunk<T, K>(rb, row0 + c + 32, tau, ts, ti);
+						}
 #endif
-			}
+						row0 += kTileRows;
+						if (row0 == row_end) row0 = row_lo;
+					}
+				}
+			};
+			if (a.n_rows % kTileRows != 0 && t0 + ntiles == a.n_tiles) tiles(std::true_type());
+			else tiles(std::false_type());
 			if (ts[K - 1] > published) atomicMax(&a.g_tau[qid], S::enc(ts[K - 1]));   // what the certificate reads: every list's final k-th best
 			const size_t o = (((size_t)qid * a.n_splits + split) * kCG + cg) * K;
 #pragma unroll
@@ -629,11 +651,9 @@ k_match_coarse(const CoarseArgs a) {
 				a.cand_row[o + j] = ti[j];
 			}
 		}
+		tc_fence_before();
+		teardown_sync();
 	}
-
-	tc_fence_before();
-	__syncthreads();
-	if (warp == 2) { tc_fence_after(); tmem_dealloc(tmem_base, 512); }
 }
 
 // =============================================================================================

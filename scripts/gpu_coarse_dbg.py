@@ -1,7 +1,8 @@
 """Timing of the coarse matching kernels on the bench's MATCH pass (1 M rows x 128 000 queries of the synthetic workload), run on the
 GPU box:  python scripts/gpu_coarse_dbg.py [label]   — per coarse kind (8-bit cascade / fp16 only) and reserved-SM count: device
 time of the dominant kernel (events inside the library), of the whole mc_match_dev pass, and the cascade's tier counts.
-MOPED_LIB selects another build of the library (e.g. one compiled with -DMC_COARSE_DBG=1)."""
+MOPED_LIB selects another build of the library (e.g. one compiled with -DMC_COARSE_DBG=1). DBG_SAVE=DIR writes every configuration's
+nn_row / nn_dist / accepted to DIR as .npy files, so that the results of two builds can be compared array by array."""
 import json
 import os
 import sys
@@ -63,6 +64,10 @@ for kind, reserve, stagger, splits in [(c[0], c[1], c[2], sp) for c in configs f
     res = (nn_row.cpu().numpy().copy(), nn_dist.cpu().numpy().copy(), acc.cpu().numpy().copy())
     same = True if ref is None else all(np.array_equal(a, b) for a, b in zip(ref, res))
     ref = ref or res
+    if os.environ.get("DBG_SAVE"):
+        os.makedirs(os.environ["DBG_SAVE"], exist_ok=True)
+        for name, arr in zip(("nn_row", "nn_dist", "accepted"), res):
+            np.save(os.path.join(os.environ["DBG_SAVE"], f"k{kind}_r{reserve}_s{stagger}_p{splits}_{name}.npy"), arr)
     km = float(np.median(ms[2:]))
     print(json.dumps({"label": label, "coarse_kind": kind, "reserve_sms": reserve, "stagger": stagger, "splits": splits, "rows": len(dbn), "queries": QT, "coarse_ms": km, "match_ms": float(np.median(tot[2:])),
                       "tera_ops": 2.0 * len(dbn) * QT * 128 / (km * 1e-3) / 1e12,
