@@ -112,6 +112,42 @@ void mc_adaptive_model_init(mc_adaptive_model *out, const float *bbox_min, const
 mc_status mc_match_adaptive(mc_ctx *ctx, const float *q_desc, const float *q_xy, int n_queries, const float *depth, const float *fill_distance,
                             int width, int height, const mc_adaptive_model *models, int n_models, float maximum_depth, float default_depth,
                             float cauchy_scale, int32_t *nn_row, float *nn_dist, uint8_t *accepted);
+/* moped3d's MATCH step for a batch of n_frames independent frames: what MATCH_ADAPTIVE_CUDA::process does per frame, with ONE
+ * matching pass over the queries of all frames.
+ *   q_desc Q x D normalised, q_xy Q x 2 (coord2D), q_image Q (imageIdx; NULL = 0), Q = frame_offsets[n_frames]
+ *   frame_offsets  host, n_frames + 1 ascending ints from 0: frame f owns features [frame_offsets[f], frame_offsets[f+1])
+ *   depth / fill_distance  n_frames x height x width: each frame's depth map and its ".distance" map (one map per frame applies
+ *                  to all of its features, as in the single-frame entry)
+ *   models / n_models / maximum_depth / default_depth / cauchy_scale  as mc_match_adaptive (models stays a host array)
+ * Outputs:
+ *   match_offsets  host, n_frames x (n_models + 1): row f = frame f's model-major CSR, GLOBAL indices into the per-match arrays.
+ *                  Frame f's matches start at frame_offsets[f], so frames leave gaps (allowed by mc_process_depth_frames*); what the
+ *                  per-match arrays hold inside a gap is unspecified.
+ *   per match (capacity Q): match_feature (global feature index), match_image, match_xy, match_xyz (coord3D of the nearest row).
+ *                  Accepted features of a model appear in feature order (FrameData::matches after MATCH).
+ *   optional, per feature: nn_row Q x 2, nn_dist Q x 2, accepted Q (exactly what mc_match_adaptive returns for that frame)
+ *   optional frame_info n_frames x 3: {features, accepted matches, status (1 = more than 8192 accepted matches)}
+ * Every frame's results are bit for bit those of mc_match_adaptive on that frame's features followed by MATCH_ADAPTIVE_CUDA::emit,
+ * whatever the batch. Kernel launches per call do not depend on n_frames.
+ * Errors (the context stays usable): MC_ERR_STATE without a database or with an object-sharded one (row_base != 0, or global tables
+ * larger than the shard); MC_ERR_ARG for a NULL required pointer, n_frames outside 1..65535, frame_offsets that do not start at 0 or do
+ * not ascend, width / height < 1, fewer curves than database models; MC_ERR_CAPACITY when a frame has more than 8192 accepted matches:
+ * that frame's row is empty and its frame_info status is 1, every other frame's results are complete. */
+mc_status mc_match_adaptive_frames(mc_ctx *ctx, const float *q_desc, const float *q_xy, const int32_t *q_image,
+                                   const int32_t *frame_offsets, int n_frames, const float *depth, const float *fill_distance,
+                                   int width, int height, const mc_adaptive_model *models, int n_models,
+                                   float maximum_depth, float default_depth, float cauchy_scale,
+                                   int32_t *match_offsets, int32_t *match_feature, int32_t *match_image, float *match_xy, float *match_xyz,
+                                   int32_t *nn_row, float *nn_dist, uint8_t *accepted, int32_t *frame_info);
+/* The same with the queries, the planes and the per-match / per-feature outputs on the device. frame_offsets, models, match_offsets
+ * and frame_info stay on the host: the call synchronises once, to return the offsets mc_process_depth_frames_dev takes. */
+mc_status mc_match_adaptive_frames_dev(mc_ctx *ctx, const float *q_desc_dev, const float *q_xy_dev, const int32_t *q_image_dev,
+                                       const int32_t *frame_offsets, int n_frames, const float *depth_dev, const float *fill_distance_dev,
+                                       int width, int height, const mc_adaptive_model *models, int n_models,
+                                       float maximum_depth, float default_depth, float cauchy_scale,
+                                       int32_t *match_offsets, int32_t *match_feature_dev, int32_t *match_image_dev, float *match_xy_dev,
+                                       float *match_xyz_dev, int32_t *nn_row_dev, float *nn_dist_dev, uint8_t *accepted_dev,
+                                       int32_t *frame_info);
 
 /* The same for shards gathered as ONE packed block each — [nn_row Q x 2 int32 | nn_dist Q x 2 fp32], 16 Q bytes per shard, n_shards
  * blocks back to back: mc_match_dev can write both halves of a rank's block directly (nn_row_dev = block, nn_dist_dev = block + 8 Q

@@ -139,7 +139,35 @@ SIGNATURES = {
     "mc_adaptive_model_init": (None, [C.c_void_p, _f32p, _f32p, _f32p, C.c_int, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float]),
     "mc_match_adaptive": (C.c_int, [C.c_void_p, _f32p, _f32p, C.c_int, _f32p, _f32p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_float, C.c_float,
                                     C.c_float, _i32p, _f32p, _u8p]),
+    "mc_match_adaptive_frames": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, _i32p, C.c_int, _f32p, _f32p, C.c_int, C.c_int, C.c_void_p,
+                                           C.c_int, C.c_float, C.c_float, C.c_float, _i32p] + [C.c_void_p] * 8),
+    "mc_match_adaptive_frames_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, _i32p, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
+                                               C.c_void_p, C.c_int, C.c_float, C.c_float, C.c_float, _i32p] + [C.c_void_p] * 8),
 }
+
+MC_ERR_CAPACITY = -4
+
+# mc_adaptive_model: one moped3d ratio curve per database model
+ADAPTIVE_MODEL = np.dtype([("depth_peak", np.float32), ("depth_fade", np.float32), ("ratio_low", np.float32), ("ratio_high", np.float32)])
+# MATCH_ADAPTIVE_FLANN_CPU's constructor values in moped3d's pipeline (MinRatioMin .. MaxRatioMax, DimensionPeak, DimensionFade)
+ADAPTIVE_DEFAULTS = (0.6, 0.75, 0.65, 0.8, 150.0, 50.0)
+# MaximumDepth, DefaultDepth, CauchyScale as the stage sets them
+ADAPTIVE_DEPTHS = (4.0, 1.0, 0.1)
+
+
+def adaptive_model_init(bbox_min, bbox_max, K, n_features, params=ADAPTIVE_DEFAULTS):
+    """mc_adaptive_model_init per model: bbox_min / bbox_max [n_models, 3], K = (fx, fy, cx, cy), n_features [n_models] (database rows
+    of each model), params = (MinRatioMin, MinRatioMax, MaxRatioMin, MaxRatioMax, DimensionPeak, DimensionFade).
+    Returns a structured array of ADAPTIVE_MODEL records (host computation; no device needed)."""
+    lo, hi = _f32(bbox_min).reshape(-1, 3), _f32(bbox_max).reshape(-1, 3)
+    nf = np.asarray(n_features, np.int64).reshape(-1)
+    Kf = _f32(K).reshape(4)
+    lib = load()
+    out = np.zeros(len(lo), ADAPTIVE_MODEL)
+    for m in range(len(lo)):
+        lib.mc_adaptive_model_init(out[m:m + 1].ctypes.data, np.ascontiguousarray(lo[m]), np.ascontiguousarray(hi[m]), Kf, int(nf[m]),
+                                   *[float(p) for p in params])
+    return out
 
 _lib = None
 
@@ -282,6 +310,80 @@ class Context:
 
     def join_lanes(self):
         self._check(self.L.mc_join_lanes(self.h), "mc_join_lanes")
+
+    # ---- MATCH, moped3d's depth-adaptive variant
+    @staticmethod
+    def _curves(models):
+        return np.ascontiguousarray(models, dtype=ADAPTIVE_MODEL)
+
+    def match_adaptive(self, q_desc, q_xy, depth, fill_distance, models, depths=ADAPTIVE_DEPTHS):
+        """One frame: q_desc [Q, D] normalised, q_xy [Q, 2], depth / fill_distance [H, W], models = ADAPTIVE_MODEL records (one per database
+        model), depths = (maximum_depth, default_depth, cauchy_scale). Returns (nn_row [Q, 2], nn_dist [Q, 2], accepted [Q] bool)."""
+        q, xy = _f32(q_desc).reshape(-1, self.D), _f32(q_xy).reshape(-1, 2)
+        d, fd = _f32(depth), _f32(fill_distance)
+        cv = self._curves(models)
+        Q = len(q)
+        nn_row = np.full((Q, 2), -1, np.int32)
+        nn_dist = np.zeros((Q, 2), np.float32)
+        acc = np.zeros(Q, np.uint8)
+        if Q == 0:
+            q, xy = np.zeros((1, self.D), np.float32), np.zeros((1, 2), np.float32)
+        self._check(self.L.mc_match_adaptive(self.h, q, xy, Q, d.reshape(-1), fd.reshape(-1), d.shape[1], d.shape[0], cv.ctypes.data, len(cv),
+                                             *[float(v) for v in depths], nn_row.reshape(-1) if Q else np.zeros(2, np.int32),
+                                             nn_dist.reshape(-1) if Q else np.zeros(2, np.float32), acc if Q else np.zeros(1, np.uint8)),
+                    "mc_match_adaptive")
+        return nn_row, nn_dist, acc.astype(bool)
+
+    def _adaptive_frames_result(self, st, what, partial, out):
+        if st != 0 and not (partial and st == MC_ERR_CAPACITY):
+            self._check(st, what)
+        out["status"] = int(st)
+        if st != 0:
+            out["error"] = self.L.mc_last_error(self.h).decode()
+        return out
+
+    def match_adaptive_frames(self, q_desc, q_xy, q_image, frame_offsets, depth, fill_distance, models, depths=ADAPTIVE_DEPTHS, partial=False):
+        """A batch of frames in one matching pass (mc_match_adaptive_frames). q_desc [Q, D], q_xy [Q, 2], q_image [Q] or None,
+        frame_offsets [n_frames + 1], depth / fill_distance [n_frames, H, W]. Returns dict(match_offsets [n_frames, n_models + 1] global,
+        match_feature / match_image / match_xy / match_xyz with capacity Q (frame f's matches from frame_offsets[f] on), nn_row, nn_dist,
+        accepted, frame_info [n_frames, 3], status). partial=True returns a capacity error (a frame with more than 8192 accepted matches)
+        as status -4 with the results instead of raising."""
+        fo = _i32(frame_offsets).reshape(-1)
+        nf = len(fo) - 1
+        cv = self._curves(models)
+        d, fd = _f32(depth), _f32(fill_distance)
+        H, W = d.shape[-2], d.shape[-1]
+        q, xy = _f32(q_desc).reshape(-1, self.D), _f32(q_xy).reshape(-1, 2)
+        img = _i32(q_image).reshape(-1) if q_image is not None else None
+        Q = len(q)
+        n = max(Q, 1)
+        out = dict(match_offsets=np.zeros((nf, len(cv) + 1), np.int32), match_feature=np.zeros(n, np.int32), match_image=np.zeros(n, np.int32),
+                   match_xy=np.zeros((n, 2), np.float32), match_xyz=np.zeros((n, 3), np.float32), nn_row=np.full((n, 2), -1, np.int32),
+                   nn_dist=np.zeros((n, 2), np.float32), accepted=np.zeros(n, np.uint8), frame_info=np.zeros((nf, 3), np.int32))
+        p = lambda a: a.ctypes.data if a is not None and a.size else None
+        st = self.L.mc_match_adaptive_frames(self.h, p(q), p(xy), p(img), fo, nf, d.reshape(-1), fd.reshape(-1), W, H, cv.ctypes.data,
+                                             len(cv), *[float(v) for v in depths], out["match_offsets"].reshape(-1),
+                                             *[out[k].ctypes.data for k in ("match_feature", "match_image", "match_xy", "match_xyz", "nn_row", "nn_dist",
+                                                                            "accepted", "frame_info")])
+        out["accepted"] = out["accepted"].astype(bool)
+        for k in ("match_feature", "match_image", "match_xy", "match_xyz", "nn_row", "nn_dist", "accepted"):
+            out[k] = out[k][:Q]
+        return self._adaptive_frames_result(st, "mc_match_adaptive_frames", partial, out)
+
+    def match_adaptive_frames_dev(self, q_ptr, xy_ptr, img_ptr, frame_offsets, depth_ptr, fill_ptr, width, height, models, match_feature_ptr,
+                                  match_image_ptr, match_xy_ptr, match_xyz_ptr, nn_row_ptr=None, nn_dist_ptr=None, acc_ptr=None, depths=ADAPTIVE_DEPTHS,
+                                  partial=False):
+        """mc_match_adaptive_frames_dev: the same with device pointers for the queries, the planes and the per-match / per-feature outputs
+        (img_ptr, nn_row_ptr, nn_dist_ptr, acc_ptr may be None). Returns dict(match_offsets, frame_info, status) (host arrays)."""
+        fo = _i32(frame_offsets).reshape(-1)
+        nf = len(fo) - 1
+        cv = self._curves(models)
+        out = dict(match_offsets=np.zeros((nf, len(cv) + 1), np.int32), frame_info=np.zeros((nf, 3), np.int32))
+        st = self.L.mc_match_adaptive_frames_dev(self.h, q_ptr, xy_ptr, img_ptr, fo, nf, depth_ptr, fill_ptr, int(width), int(height), cv.ctypes.data,
+                                                 len(cv), *[float(v) for v in depths], out["match_offsets"].reshape(-1), match_feature_ptr,
+                                                 match_image_ptr, match_xy_ptr, match_xyz_ptr, nn_row_ptr, nn_dist_ptr, acc_ptr,
+                                                 out["frame_info"].ctypes.data)
+        return self._adaptive_frames_result(st, "mc_match_adaptive_frames_dev", partial, out)
 
     # ---- CLUSTER
     def cluster(self, matches, n_images=1, radius=200.0, merge=20.0, minpts=7, maxiter=100):

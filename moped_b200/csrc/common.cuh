@@ -209,6 +209,10 @@ mc_status gather_depth_points_device(mc_ctx *ctx, const int32_t *d_n, const int3
                                      float *d_pt_xyz, float *d_pt_world, float *d_pt_cauchy, int32_t *d_pt_image, int32_t *d_pt_tie);
 mc_status copy_objects_device(mc_ctx *ctx, const int32_t *d_n, const int32_t *d_src_model, const float *d_src_pose, int32_t *d_dst_n,
                               int32_t *d_dst_model, float *d_dst_pose);
+mc_status match_compact_frames_device(mc_ctx *ctx, const FrameDesc *d_fd, const int32_t *d_out_base, int n_frames, int n_models, int32_t *d_acc_list,
+                                      int32_t *d_match_offsets, int32_t *d_match_query, int32_t *d_match_row, int32_t *d_match_image,
+                                      float *d_match_xy, float *d_match_xyz, int32_t *d_status, int32_t *d_n_obj);
+constexpr int kCompactCap = 8192;    // accepted matches per frame handled by the compaction (k_match_compact)
 
 // ---- moped3d linkage clustering of all models of a frame at once (linkage.cu) ----
 struct LinkSlice {         // one model of a frame: matches lo .. lo+n of the frame, n x n matrix block at element sq of the arena

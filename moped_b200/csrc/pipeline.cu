@@ -24,24 +24,32 @@ mc_status filter_device(mc_ctx *ctx, const int32_t *d_match_offsets, const int32
                         uint8_t *d_keep, float *d_score, int32_t *d_out_n, int32_t *d_cluster_model, int32_t *d_cluster_offsets,
                         int32_t *d_members, int32_t *d_surv_model, float *d_surv_pose, float *d_surv_score);
 
-constexpr int kCompactCap = 8192;    // accepted matches per frame handled by the single-CTA compaction
-
 // Accepted queries -> matches bucketed by model, query order preserved inside a model
 // (`matches[correspModel[nx[0]]].push_back(...)` in query order, MATCH_ANN_CPU.hpp:165-176; the order matters:
-// mean-shift is order dependent). Single CTA: stable compaction of the accepted queries, then a bitonic sort
+// mean-shift is order dependent). One CTA per frame: stable compaction of the accepted queries, then a bitonic sort
 // of (model << 13 | rank) keys in shared memory.
+// Frame f = blockIdx.x reads fd[f]. out_base (nullable = every frame at 0) places its matches: the per-match arrays and
+// acc_list from element out_base[f] on, match_query = out_base[f] + query index in the frame (with out_base = the frames'
+// first query ids: the batch-global query id); match_offsets row f (n_models + 1 entries, frame-local: 0 .. matches),
+// status[f] and n_obj[f]. A frame cannot write past its own queries' range (matches <= queries), so a batch needs no packing.
 __global__ void k_set_desc(FrameDesc *dst, FrameDesc v) { *dst = v; }
 
 __global__ void __launch_bounds__(1024)
-k_match_compact(const FrameDesc *__restrict__ fd, int64_t row_base,
+k_match_compact(const FrameDesc *__restrict__ fd, const int32_t *__restrict__ out_base, int64_t row_base,
                 const int32_t *__restrict__ model_of_row, const float *__restrict__ db_xyz, int n_models, int32_t *__restrict__ acc_list,
                 int32_t *__restrict__ match_offsets, int32_t *__restrict__ match_query, int32_t *__restrict__ match_row,
                 int32_t *__restrict__ match_image, float *__restrict__ match_xy, float *__restrict__ match_xyz,
                 int32_t *__restrict__ status, int32_t *__restrict__ n_obj) {
+	const int f = blockIdx.x;
+	fd += f;
+	const int base = out_base ? out_base[f] : 0;
+	acc_list += base; match_query += base; match_row += base; match_image += base; match_xy += 2 * (size_t)base; match_xyz += 3 * (size_t)base;
+	match_offsets += (size_t)f * (n_models + 1);
+	status += f; n_obj += f;
 	const int32_t *__restrict__ nn_row = fd->nn_row;
 	const uint8_t *__restrict__ accepted = fd->accepted;
 	const float *__restrict__ q_xy = fd->q_xy;
-	const int32_t *__restrict__ q_image = fd->q_image;
+	const int32_t *__restrict__ q_image = fd->q_image;     // nullable: every query from image 0
 	const int Q = fd->Q;
 	__shared__ uint32_t keys[kCompactCap];
 	__shared__ int s_warp[32];
@@ -88,8 +96,8 @@ k_match_compact(const FrameDesc *__restrict__ fd, int64_t row_base,
 		const uint32_t key = keys[i];
 		const int m = (int)(key >> 13), q = acc_list[key & 8191u];
 		const int row = nn_row[2 * q];
-		match_query[i] = q; match_row[i] = row;
-		match_image[i] = q_image[q];
+		match_query[i] = base + q; match_row[i] = row;
+		match_image[i] = q_image ? q_image[q] : 0;
 		match_xy[2 * i] = q_xy[2 * q]; match_xy[2 * i + 1] = q_xy[2 * q + 1];
 		const int64_t lr = (int64_t)row - row_base;
 		match_xyz[3 * i] = db_xyz[3 * lr]; match_xyz[3 * i + 1] = db_xyz[3 * lr + 1]; match_xyz[3 * i + 2] = db_xyz[3 * lr + 2];
@@ -220,7 +228,7 @@ static mc_status frame_enqueue(mc_ctx *ctx, const float *d_q, int Q, const mc_pi
 	auto mark = [&](int i) { if (ev) cudaEventRecord(ev[i], ctx->stream); };
 	mark(0);                                             // (B.status / B.n_obj are zeroed by k_match_compact)
 	if (d_q) MC_TRY(match_device(ctx, d_q, Q, P->match_ratio, P->match_mode, B.nn_row, B.nn_dist, B.accepted));
-	k_match_compact<<<1, 1024, 0, ctx->stream>>>(fd, ctx->table_base, ctx->d_model_of_row, ctx->d_xyz, ctx->n_models,
+	k_match_compact<<<1, 1024, 0, ctx->stream>>>(fd, nullptr, ctx->table_base, ctx->d_model_of_row, ctx->d_xyz, ctx->n_models,
 	                                            B.acc_list, B.match_offsets, B.match_query, B.match_row, B.match_image, B.match_xy, B.match_xyz, B.status, B.n_obj);
 	MC_LAUNCH_CHECK();
 	mark(1);
@@ -270,6 +278,17 @@ mc_status gather_depth_points_device(mc_ctx *ctx, const int32_t *d_n, const int3
 	k_gather_points<<<ctx->num_sms, 128, 0, ctx->stream>>>(d_n, d_cluster_model, d_cluster_offsets, d_members, d_match_offsets, d_match_image, d_match_xy,
 	                                                     d_match_xyz, d_pt_xy, d_pt_xyz, d_pt_image, d_pt_tie, d_match_world, d_match_fill, cauchy_scale,
 	                                                     d_pt_world, d_pt_cauchy);
+	MC_LAUNCH_CHECK();
+	return MC_OK;
+}
+
+// for moped3d's batched MATCH (adaptive.cu): the compaction of n_frames frames in one launch
+mc_status match_compact_frames_device(mc_ctx *ctx, const FrameDesc *d_fd, const int32_t *d_out_base, int n_frames, int n_models, int32_t *d_acc_list,
+                                      int32_t *d_match_offsets, int32_t *d_match_query, int32_t *d_match_row, int32_t *d_match_image,
+                                      float *d_match_xy, float *d_match_xyz, int32_t *d_status, int32_t *d_n_obj) {
+	k_match_compact<<<n_frames, 1024, 0, ctx->stream>>>(d_fd, d_out_base, ctx->table_base, ctx->d_model_of_row, ctx->d_xyz, n_models, d_acc_list,
+	                                                   d_match_offsets, d_match_query, d_match_row, d_match_image, d_match_xy, d_match_xyz, d_status,
+	                                                   d_n_obj);
 	MC_LAUNCH_CHECK();
 	return MC_OK;
 }
@@ -485,7 +504,7 @@ mc_status process_frame_sharded_device(mc_ctx *ctx, int phase, const int32_t *d_
 		d.out_info = d_out_info; d.out_model = d_out_model; d.out_pose = d_out_pose; d.out_score = d_out_score;
 		MC_TRY(set_frame_desc(ctx, d));
 		fd = (const FrameDesc *)ctx->frame_desc.p;
-		k_match_compact<<<1, 1024, 0, ctx->stream>>>(fd, ctx->table_base, ctx->d_model_of_row, ctx->d_xyz, ctx->n_models,
+		k_match_compact<<<1, 1024, 0, ctx->stream>>>(fd, nullptr, ctx->table_base, ctx->d_model_of_row, ctx->d_xyz, ctx->n_models,
 		                                            B.acc_list, B.match_offsets, B.match_query, B.match_row, B.match_image, B.match_xy, B.match_xyz, B.status, B.n_obj);
 		MC_LAUNCH_CHECK();
 		MC_TRY(cluster_device(ctx, B.match_offsets, B.match_image, B.match_xy, ctx->n_models, ctx->n_images, Q, P->cluster_radius, P->cluster_merge,

@@ -10,7 +10,8 @@ configuration runs on seeded synthetic data:
   ``n_visible`` objects posed in front of the camera, ``pts_visible`` of their points projected with
   N(0, 0.5 px) noise and N(0, 0.02) descriptor noise; the rest of the Q features are distractors.
 
-Pure numpy; used by tests/ and bench.py (inputs only — no algorithm of the hot path lives here).
+Pure numpy (make_adaptive_frames also calls the library's host-side mc_adaptive_model_init); used by tests/ and bench.py (inputs
+only — no algorithm of the hot path lives here).
 """
 from __future__ import annotations
 
@@ -363,3 +364,79 @@ def stack_depth_frames(frames):
     return dict(match_offsets=np.stack(rows).astype(np.int32), match_image=cat("match_image"), match_xy=cat("match_xy"), match_xyz=cat("match_xyz"),
                 match_world=cat("match_world"), match_fill=cat("match_fill"), depth=np.stack([fr["depth"] for fr in frames]),
                 fill_distance=np.stack([fr["fill_distance"] for fr in frames]))
+
+
+# ---- moped3d's depth-adaptive MATCH step (MATCH_ADAPTIVE_FLANN_CPU) on frame batches -------------------------------------------------
+# DimensionPeak / DimensionFade of the generator's curves. The pipeline's 150 / 50 px put twice the fade depth of make_db's 0.2 m models
+# (4.2 m) beyond the 4 m depth cut, which would leave the curve's zero segment in front of the cut empty; 80 px puts it at ~2.6 m.
+ADAPTIVE_DIMENSIONS = (150.0, 80.0)
+
+
+def adaptive_segments(curves, maximum_depth: float = 4.0):
+    """Depth intervals (lo, hi) inside the segments of ALL curves: ramp, plateau, fade, zero (beyond twice the fade depth, within
+    maximum_depth) and beyond maximum_depth, each kept clear of every curve's breakpoints by a few per cent. Empty segments are left out."""
+    pk_lo, pk_hi = float(curves["depth_peak"].min()), float(curves["depth_peak"].max())
+    fd_lo, fd_hi = float(curves["depth_fade"].min()), float(curves["depth_fade"].max())
+    seg = dict(ramp=(0.05, 0.95 * pk_lo), plateau=(1.05 * pk_hi, 0.95 * fd_lo), fade=(1.05 * fd_hi, 1.95 * fd_lo),
+               zero=(2.05 * fd_hi, 0.98 * maximum_depth), beyond=(1.02 * maximum_depth, 2.0 * maximum_depth))
+    return {k: v for k, v in seg.items() if v[1] > v[0]}
+
+
+def make_adaptive_frames(db, n_frames: int, n_features=None, seed: int = BASE_SEED, empty=(1,), far=(2,), W: int = 640, H: int = 480,
+                         maximum_depth: float = 4.0, cauchy_scale: float = 0.1, dimensions=ADAPTIVE_DIMENSIONS):
+    """A batch of RGB-D frames for moped3d's MATCH step (mc_match_adaptive_frames), built on make_db / make_frame.
+    * features: make_frame's planted copies of database rows and distractors, pixel coordinates clipped into the W x H map; frame f has
+      `n_features` features (int, or per-frame counts; None = seeded counts in 300..2500, none a multiple of 256), frames listed in
+      `empty` have none;
+    * depth planes: 80 x 80 px cells, each at one depth drawn from a segment of the ratio curves (adaptive_segments: ramp, plateau,
+      fade, zero, beyond maximum_depth) plus a 1 mm ramp; frames listed in `far` lie entirely beyond maximum_depth;
+    * fill-distance planes: half the pixels 0 (measured depth), the rest log-uniform in 10^-2.5 .. 10^1.5 m, so the Cauchy weight of
+      the fill distance goes from 1 down to ~1e-5;
+    * curves: mc_adaptive_model_init over each model's bounding box with K_DEPTH, the moped3d ratio ranges and `dimensions`;
+    * world / fill per feature: the depth under the feature back-projected through K_DEPTH and the fill distance under it (what
+      DEPTHPROP gives moped3d's later steps).
+    Returns dict(desc[Q,d], xy[Q,2], image[Q], frame_offsets[n_frames+1], depth[F,H,W], fill_distance[F,H,W], world[Q,3], fill[Q],
+    curves (capi.ADAPTIVE_MODEL records), segments, maximum_depth, cauchy_scale)."""
+    from . import capi
+    rng = np.random.default_rng(seed + 15731)
+    starts = np.concatenate([[0], np.cumsum(db["n_pts"])]).astype(np.int64)
+    lo = np.minimum.reduceat(db["xyz"], starts[:-1], axis=0)
+    hi = np.maximum.reduceat(db["xyz"], starts[:-1], axis=0)
+    p = capi.ADAPTIVE_DEFAULTS
+    curves = capi.adaptive_model_init(lo, hi, K_DEPTH, db["n_pts"], (p[0], p[1], p[2], p[3], dimensions[0], dimensions[1]))
+    segs = adaptive_segments(curves, maximum_depth)
+    kinds = list(segs)
+    if n_features is None:
+        counts = rng.integers(300, 2501, size=n_frames)
+        counts[counts % 256 == 0] += 1
+    else:
+        counts = np.broadcast_to(np.asarray(n_features, np.int64), (n_frames,)).copy()
+    counts[[f for f in empty if f < n_frames]] = 0
+    desc, xy, depth, fill_map = [], [], np.empty((n_frames, H, W), np.float32), np.empty((n_frames, H, W), np.float32)
+    cy, cx = np.arange(H)[:, None] // 80, np.arange(W)[None, :] // 80
+    ramp = (0.001 * (np.arange(W)[None, :] % 80) / 80).astype(np.float32)
+    for f in range(n_frames):
+        cells = rng.integers(0, len(kinds), size=((H + 79) // 80, (W + 79) // 80))
+        if f in far:
+            cells[:] = kinds.index("beyond")
+        bounds = np.array([segs[k] for k in kinds])[cells]
+        zc = rng.uniform(bounds[..., 0], bounds[..., 1]).astype(np.float32)
+        depth[f] = zc[cy, cx] + ramp
+        measured = rng.random((H, W)) < 0.5
+        fill_map[f] = np.where(measured, 0.0, 10.0 ** rng.uniform(-2.5, 1.5, (H, W))).astype(np.float32)
+        n = int(counts[f])
+        if n:
+            fr = make_frame(db, n, n_visible=8, pts_visible=60, frame_id=f, seed=seed)
+            desc.append(fr["desc"])
+            xy.append(np.clip(fr["xy"], 0, [W - 1, H - 1]).astype(np.float32))
+    d = db["desc"].shape[1]
+    desc = np.concatenate(desc) if desc else np.zeros((0, d), np.float32)
+    xy = np.concatenate(xy) if xy else np.zeros((0, 2), np.float32)
+    offsets = np.concatenate([[0], np.cumsum(counts)]).astype(np.int32)
+    frame_of = np.repeat(np.arange(n_frames), counts)
+    px, py = xy[:, 0].astype(np.int64), xy[:, 1].astype(np.int64)
+    zf = depth[frame_of, py, px]
+    world = np.stack([(xy[:, 0] - K_DEPTH[2]) / K_DEPTH[0] * zf, (xy[:, 1] - K_DEPTH[3]) / K_DEPTH[1] * zf, zf], 1).astype(np.float32)
+    return dict(desc=np.ascontiguousarray(desc, np.float32), xy=xy, image=np.zeros(len(desc), np.int32), frame_offsets=offsets, depth=depth,
+                fill_distance=fill_map, world=world, fill=fill_map[frame_of, py, px].astype(np.float32), curves=curves, segments=segs,
+                maximum_depth=float(maximum_depth), cauchy_scale=float(cauchy_scale))
