@@ -148,6 +148,35 @@ mc_status mc_match_adaptive_frames_dev(mc_ctx *ctx, const float *q_desc_dev, con
                                        int32_t *match_offsets, int32_t *match_feature_dev, int32_t *match_image_dev, float *match_xy_dev,
                                        float *match_xyz_dev, int32_t *nn_row_dev, float *nn_dist_dev, uint8_t *accepted_dev,
                                        int32_t *frame_info);
+/* moped3d's MATCH step on an object-sharded database, for the frames [frame_begin, frame_end) of a batch of n_frames frames.
+ *   packed_all_dev  n_shards blocks back to back in the layout of mc_match_merge_packed_dev: [nn_row Q x 2 int32 | nn_dist Q x 2 fp32]
+ *                  per shard, Q = frame_offsets[n_frames]; each block is what mc_match_dev(ratio 1.0, MC_MATCH_TENSOR) writes for the whole
+ *                  batch on a context holding one shard (the all-gathered blocks of the ranks)
+ * The features of the range get the global two nearest rows (smaller distance, then smaller global row id, as mc_match_merge_dev), then
+ * the depth-adaptive test and the model-major lists of mc_match_adaptive_frames_dev. Index conventions:
+ *   q_xy_dev, q_image_dev (NULL = image 0), the per-feature and the per-match outputs: GLOBAL feature indices, capacity Q; only the
+ *                  slots of the range's features are written (frame f's matches from frame_offsets[f] on)
+ *   depth_dev / fill_distance_dev  (frame_end - frame_begin) x height x width: the planes of the range's frames only, starting with frame
+ *                  frame_begin (the same planes mc_process_depth_frames_dev takes for these frames)
+ *   match_offsets  host, (frame_end - frame_begin) x (n_models + 1): one row per frame of the range, global indices
+ *   frame_info     optional host, (frame_end - frame_begin) x 3: {features, accepted matches, status}; status 1 = more than 8192 accepted
+ *                  matches, 2 = a row id in the blocks that is neither -1 nor inside the context's tables
+ * The context needs coord3D and model tables covering every row id of the blocks: mc_db_set_global_tables on a shard context, or a context
+ * holding the whole database (then n_shards = 1 with that context's own mc_match_dev block reproduces mc_match_adaptive_frames_dev).
+ * Its descriptors are not read. Every frame of the range equals, bit for bit, what mc_match_adaptive_frames_dev returns for it on one
+ * context holding the whole database. Kernel launches per call depend neither on n_frames, nor on the range, nor on n_shards.
+ * Errors (the context stays usable): MC_ERR_STATE without tables; MC_ERR_ARG for a NULL required pointer, n_shards < 1, a range outside
+ * 0 <= frame_begin <= frame_end <= n_frames (an empty range returns MC_OK and writes nothing), and the cases of mc_match_adaptive_frames;
+ * MC_ERR_CAPACITY as mc_match_adaptive_frames (status 1). A row outside the tables is never used as an index: its feature is not accepted,
+ * its frame's status is 2 and its row is empty, every other frame is complete, and the call returns MC_ERR_ARG naming the first such
+ * frame (before a capacity error). */
+mc_status mc_match_adaptive_frames_merged_dev(mc_ctx *ctx, const void *packed_all_dev, int n_shards, const float *q_xy_dev,
+                                              const int32_t *q_image_dev, const int32_t *frame_offsets, int n_frames, int frame_begin,
+                                              int frame_end, const float *depth_dev, const float *fill_distance_dev, int width, int height,
+                                              const mc_adaptive_model *models, int n_models, float maximum_depth, float default_depth,
+                                              float cauchy_scale, int32_t *match_offsets, int32_t *match_feature_dev, int32_t *match_image_dev,
+                                              float *match_xy_dev, float *match_xyz_dev, int32_t *nn_row_dev, float *nn_dist_dev,
+                                              uint8_t *accepted_dev, int32_t *frame_info);
 
 /* The same for shards gathered as ONE packed block each — [nn_row Q x 2 int32 | nn_dist Q x 2 fp32], 16 Q bytes per shard, n_shards
  * blocks back to back: mc_match_dev can write both halves of a rank's block directly (nn_row_dev = block, nn_dist_dev = block + 8 Q

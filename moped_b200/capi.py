@@ -143,8 +143,12 @@ SIGNATURES = {
                                            C.c_int, C.c_float, C.c_float, C.c_float, _i32p] + [C.c_void_p] * 8),
     "mc_match_adaptive_frames_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, _i32p, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
                                                C.c_void_p, C.c_int, C.c_float, C.c_float, C.c_float, _i32p] + [C.c_void_p] * 8),
+    "mc_match_adaptive_frames_merged_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, _i32p, C.c_int, C.c_int, C.c_int,
+                                                      C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_float, C.c_float, C.c_float,
+                                                      _i32p] + [C.c_void_p] * 8),
 }
 
+MC_ERR_ARG = -2
 MC_ERR_CAPACITY = -4
 
 # mc_adaptive_model: one moped3d ratio curve per database model
@@ -334,8 +338,8 @@ class Context:
                     "mc_match_adaptive")
         return nn_row, nn_dist, acc.astype(bool)
 
-    def _adaptive_frames_result(self, st, what, partial, out):
-        if st != 0 and not (partial and st == MC_ERR_CAPACITY):
+    def _adaptive_frames_result(self, st, what, partial, out, partial_status=(MC_ERR_CAPACITY,)):
+        if st != 0 and not (partial and st in partial_status):
             self._check(st, what)
         out["status"] = int(st)
         if st != 0:
@@ -384,6 +388,25 @@ class Context:
                                                  match_image_ptr, match_xy_ptr, match_xyz_ptr, nn_row_ptr, nn_dist_ptr, acc_ptr,
                                                  out["frame_info"].ctypes.data)
         return self._adaptive_frames_result(st, "mc_match_adaptive_frames_dev", partial, out)
+
+    def match_adaptive_frames_merged_dev(self, packed_all_ptr, n_shards, xy_ptr, img_ptr, frame_offsets, frame_begin, frame_end, depth_ptr, fill_ptr,
+                                         width, height, models, match_feature_ptr, match_image_ptr, match_xy_ptr, match_xyz_ptr, nn_row_ptr=None,
+                                         nn_dist_ptr=None, acc_ptr=None, depths=ADAPTIVE_DEPTHS, partial=False):
+        """mc_match_adaptive_frames_merged_dev: frames [frame_begin, frame_end) of the batch from the n_shards gathered packed blocks at
+        packed_all_ptr (device, n_shards x 16 Q bytes). depth_ptr / fill_ptr hold the range's planes only; the per-feature and per-match
+        outputs use global feature indices (nn_row_ptr, nn_dist_ptr, acc_ptr may be None). Returns dict(match_offsets
+        [frame_end - frame_begin, n_models + 1], frame_info [frame_end - frame_begin, 3], status). partial=True returns a capacity error
+        (frame_info status 1) or a row outside the tables (status 2, MC_ERR_ARG) as status with the results instead of raising."""
+        fo = _i32(frame_offsets).reshape(-1)
+        nf, nr = len(fo) - 1, int(frame_end) - int(frame_begin)
+        cv = self._curves(models)
+        out = dict(match_offsets=np.zeros((max(nr, 1), len(cv) + 1), np.int32), frame_info=np.zeros((max(nr, 1), 3), np.int32))
+        st = self.L.mc_match_adaptive_frames_merged_dev(self.h, packed_all_ptr, int(n_shards), xy_ptr, img_ptr, fo, nf, int(frame_begin), int(frame_end),
+                                                        depth_ptr, fill_ptr, int(width), int(height), cv.ctypes.data, len(cv),
+                                                        *[float(v) for v in depths], out["match_offsets"].reshape(-1), match_feature_ptr, match_image_ptr,
+                                                        match_xy_ptr, match_xyz_ptr, nn_row_ptr, nn_dist_ptr, acc_ptr, out["frame_info"].ctypes.data)
+        out["match_offsets"], out["frame_info"] = out["match_offsets"][:max(nr, 0)], out["frame_info"][:max(nr, 0)]
+        return self._adaptive_frames_result(st, "mc_match_adaptive_frames_merged_dev", partial, out, (MC_ERR_CAPACITY, MC_ERR_ARG))
 
     # ---- CLUSTER
     def cluster(self, matches, n_images=1, radius=200.0, merge=20.0, minpts=7, maxiter=100):

@@ -17,6 +17,7 @@
 //   k_match_exact*    exhaustive exact scan (fallback for uncertified queries, and MC_MATCH_EXACT)
 //   k_match_finalize  ratio test
 #include "common.cuh"
+#include "top2.cuh"
 
 #include <math_constants.h>
 #include <type_traits>
@@ -658,30 +659,9 @@ k_match_coarse(const CoarseArgs a) {
 
 // =============================================================================================
 // exact arithmetic of the reference: dist = sum_d (q[d]-p[d])^2, sequential, product and sum each
-// rounded to fp32 (VMULSS + VADDSS in the compiled reference, libs.tgz!ann_1.1.1/kd_search.cpp:188-199)
+// rounded to fp32 (VMULSS + VADDSS in the compiled reference, libs.tgz!ann_1.1.1/kd_search.cpp:188-199);
+// the two nearest rows are kept by Top2 (top2.cuh)
 // =============================================================================================
-struct Top2 {
-	float d0, d1;
-	int32_t i0, i1;
-};
-__device__ __forceinline__ bool closer(float d, int32_t i, float e, int32_t j) { return d < e || (d == e && (uint32_t)i < (uint32_t)j); }
-__device__ __forceinline__ void top2_push(Top2 &t, float d, int32_t i) {
-	if (i < 0) return;
-	if (closer(d, i, t.d0, t.i0)) { t.d1 = t.d0; t.i1 = t.i0; t.d0 = d; t.i0 = i; }
-	else if (closer(d, i, t.d1, t.i1)) { t.d1 = d; t.i1 = i; }
-}
-__device__ __forceinline__ void top2_warp_reduce(Top2 &t) {
-#pragma unroll
-	for (int o = 16; o; o >>= 1) {
-		float d0 = __shfl_xor_sync(0xffffffffu, t.d0, o), d1 = __shfl_xor_sync(0xffffffffu, t.d1, o);
-		int32_t i0 = __shfl_xor_sync(0xffffffffu, t.i0, o), i1 = __shfl_xor_sync(0xffffffffu, t.i1, o);
-		top2_push(t, d0, i0);
-		top2_push(t, d1, i1);
-	}
-}
-__device__ __forceinline__ Top2 top2_empty() {
-	Top2 t; t.d0 = t.d1 = 3.402823466e+38f /* PQ_NULL_KEY = ANN_DIST_INF: a missing neighbour */; t.i0 = t.i1 = -1; return t;
-}
 
 // Exact re-rank of the coarse candidates; one warp per query.
 //
