@@ -485,6 +485,54 @@ mc_status mc_process_depth_frames_dev(mc_ctx *ctx, const int32_t *match_offsets,
                                       int max_objects, int32_t *n_objects, int32_t *obj_model, float *obj_pose, float *obj_score,
                                       int32_t *frame_info, float *stage_ms);
 
+/* moped3d's MATCH -> (DEPTHPROP's per-feature depth data, gathered per match) -> CLUSTER -> POSE -> FILTER -> POSE2 -> FILTER2 for a
+ * batch of n_frames independent frames, in one call: features in, objects out.
+ *   q_desc, q_xy, q_image, frame_offsets, depth / fill_distance, models .. cauchy_scale  as mc_match_adaptive_frames
+ *   q_world Q x 3, q_fill Q  DEPTHPROP's depthData.coord3D and depthData.fillDistance of every feature (required when Q > 0)
+ *   params, max_objects, outputs  as mc_process_depth_frames: n_objects[f], obj_model / obj_score [f * max_objects + i],
+ *                  obj_pose [(f * max_objects + i) * 7]
+ *   frame_info     optional, n_frames x 4: {objects, status, accepted matches, clusters after CLUSTER}
+ *   stage_ms       optional, 2 floats: device time of MATCH (cascade, finalize, compaction), then of CLUSTER..FILTER2 (events on the
+ *                  context's stream around the fork to the frame lanes and their join: the frames stay dealt to the lanes)
+ * Every frame's objects and frame_info equal mc_match_adaptive_frames_dev, a gather of q_world / q_fill through match_feature and
+ * mc_process_depth_frames_dev on the same batch, bit for bit. The per-match arrays stay in the context's memory; the call synchronises
+ * once between MATCH and CLUSTER (the chain's plan needs the per-model counts) and once for the objects. Kernel launches per call are
+ * those of mc_match_adaptive_frames_dev plus those of mc_process_depth_frames_dev on the same batch.
+ * A frame that fails gets status != 0 and no objects; every other frame is complete and the context stays usable:
+ *   1  an accepted match outside the frame's depth map (MATCH clamps pixels into the map, so a feature at x == width or x < 0 can be
+ *      accepted; nothing is read out of range)                                                         MC_ERR_ARG
+ *   2  a row id in the gathered blocks outside the tables (mc_process_depth_queries_merged_dev)        MC_ERR_ARG
+ *   3  more than 8192 accepted matches (accepted matches reported as 0: the lists are empty)          MC_ERR_CAPACITY
+ *   4  a model with more than 2048 matches, or more than 2^24 similarity entries over the frame's models MC_ERR_CAPACITY
+ *   0  with more than max_objects objects (n_objects[f] holds the true count)                          MC_ERR_CAPACITY
+ * The call returns the code of the first failed frame, MC_ERR_ARG before MC_ERR_CAPACITY.
+ * Other errors: MC_ERR_STATE without a database, with an object-sharded one, or without cameras; MC_ERR_ARG for a NULL required pointer
+ * (q_world / q_fill included) and the argument errors of mc_match_adaptive_frames and mc_process_depth_frames. */
+mc_status mc_process_depth_queries(mc_ctx *ctx, const float *q_desc, const float *q_xy, const int32_t *q_image, const float *q_world,
+                                   const float *q_fill, const int32_t *frame_offsets, int n_frames, const float *depth, const float *fill_distance,
+                                   int width, int height, const mc_adaptive_model *models, int n_models, float maximum_depth, float default_depth,
+                                   float cauchy_scale, const mc_depth_pipeline_params *params, int max_objects, int32_t *n_objects,
+                                   int32_t *obj_model, float *obj_pose, float *obj_score, int32_t *frame_info, float *stage_ms);
+/* The same with q_* and the planes on the device; frame_offsets, models and the outputs stay on the host. */
+mc_status mc_process_depth_queries_dev(mc_ctx *ctx, const float *q_desc_dev, const float *q_xy_dev, const int32_t *q_image_dev,
+                                       const float *q_world_dev, const float *q_fill_dev, const int32_t *frame_offsets, int n_frames,
+                                       const float *depth_dev, const float *fill_distance_dev, int width, int height,
+                                       const mc_adaptive_model *models, int n_models, float maximum_depth, float default_depth,
+                                       float cauchy_scale, const mc_depth_pipeline_params *params, int max_objects, int32_t *n_objects,
+                                       int32_t *obj_model, float *obj_pose, float *obj_score, int32_t *frame_info, float *stage_ms);
+/* One rank of an object-sharded database: the all-gathered mc_match_dev blocks take the place of the matching pass, for frames
+ * [frame_begin, frame_end) of the batch, with the conventions of mc_match_adaptive_frames_merged_dev: q_xy_dev, q_image_dev, q_world_dev,
+ * q_fill_dev hold the whole batch (global feature ids); depth_dev / fill_distance_dev hold the range's planes only; n_objects,
+ * frame_info and the obj_* rows are one per frame of the range. Every frame equals mc_process_depth_queries_dev on one context holding
+ * the whole database. An empty range returns MC_OK and writes nothing. */
+mc_status mc_process_depth_queries_merged_dev(mc_ctx *ctx, const void *packed_all_dev, int n_shards, const float *q_xy_dev,
+                                              const int32_t *q_image_dev, const float *q_world_dev, const float *q_fill_dev,
+                                              const int32_t *frame_offsets, int n_frames, int frame_begin, int frame_end, const float *depth_dev,
+                                              const float *fill_distance_dev, int width, int height, const mc_adaptive_model *models,
+                                              int n_models, float maximum_depth, float default_depth, float cauchy_scale,
+                                              const mc_depth_pipeline_params *params, int max_objects, int32_t *n_objects, int32_t *obj_model,
+                                              float *obj_pose, float *obj_score, int32_t *frame_info, float *stage_ms);
+
 /* Named integer options (scheduling / kernel-shape choices; unknown keys are an error):
  *   "pose_fit_thread_min"  mc_pose_hypotheses* calls with at least this many hypotheses and no inlier masks run one
  *                          THREAD per hypothesis instead of one 8-lane group (default 16384; 1 = always)

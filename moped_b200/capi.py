@@ -146,6 +146,14 @@ SIGNATURES = {
     "mc_match_adaptive_frames_merged_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, _i32p, C.c_int, C.c_int, C.c_int,
                                                       C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_float, C.c_float, C.c_float,
                                                       _i32p] + [C.c_void_p] * 8),
+    "mc_process_depth_queries": (C.c_int, [C.c_void_p] * 6 + [_i32p, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_float,
+                                           C.c_float, C.c_float, C.POINTER(DepthPipelineParams), C.c_int, _i32p, _i32p, _f32p, _f32p, _i32p, C.c_void_p]),
+    "mc_process_depth_queries_dev": (C.c_int, [C.c_void_p] * 6 + [_i32p, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int,
+                                               C.c_float, C.c_float, C.c_float, C.POINTER(DepthPipelineParams), C.c_int, _i32p, _i32p, _f32p, _f32p,
+                                               _i32p, C.c_void_p]),
+    "mc_process_depth_queries_merged_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int] + [C.c_void_p] * 4 + [_i32p, C.c_int, C.c_int, C.c_int,
+                                                      C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_float, C.c_float, C.c_float,
+                                                      C.POINTER(DepthPipelineParams), C.c_int, _i32p, _i32p, _f32p, _f32p, _i32p, C.c_void_p]),
 }
 
 MC_ERR_ARG = -2
@@ -761,6 +769,61 @@ class Context:
         arrays = [image_ptr, xy_ptr, xyz_ptr, world_ptr, fill_ptr, depth_ptr, fill_distance_ptr, int(width), int(height)]
         return self._depth_frames(self.L.mc_process_depth_frames_dev, "mc_process_depth_frames_dev", match_offsets, n_models, arrays, params,
                                   max_objects, times)
+
+    def _depth_queries(self, fn, what, n_frames, n_models, args, params, max_objects, times, partial):
+        p = params or self.default_depth_params()
+        n_obj = np.zeros(n_frames, np.int32)
+        om = np.zeros((max(n_frames, 1), max_objects), np.int32)
+        op = np.zeros((max(n_frames, 1), max_objects, 7), np.float32)
+        os_ = np.zeros((max(n_frames, 1), max_objects), np.float32)
+        info = np.zeros((max(n_frames, 1), 4), np.int32)
+        st = fn(self.h, *args, C.byref(p), int(max_objects), n_obj if n_frames else np.zeros(1, np.int32), om.reshape(-1), op.reshape(-1),
+                os_.reshape(-1), info.reshape(-1), times.ctypes.data if times is not None else None)
+        if st != 0 and not (partial and st in (MC_ERR_ARG, MC_ERR_CAPACITY)):
+            self._check(st, what)
+        n_obj = np.where((info[:n_frames, 1] != 0) | (n_obj > max_objects), 0, n_obj)   # a failed frame has no objects; info keeps its counts
+        frames = self._unpack_frames(n_frames, max_objects, n_obj, om, op, os_, info)
+        return (frames, int(st)) if partial else frames
+
+    def process_depth_queries(self, q_desc, q_xy, q_image, q_world, q_fill, frame_offsets, depth, fill_distance, models, depths=ADAPTIVE_DEPTHS,
+                              params=None, max_objects=64, times=None, partial=False):
+        """moped3d from features to objects on host arrays (mc_process_depth_queries): MATCH, the per-match gather of DEPTHPROP's q_world
+        [Q, 3] / q_fill [Q], CLUSTER..FILTER2. q_desc [Q, D], q_xy [Q, 2], q_image [Q] or None, frame_offsets [n_frames + 1],
+        depth / fill_distance [n_frames, H, W], models = ADAPTIVE_MODEL records. `times` (optional float32[2]) receives the device time
+        of MATCH and of CLUSTER..FILTER2. Returns the per-frame dict(model, pose, score, info) of process_depth_frames; info = {objects,
+        status, accepted matches, clusters}. partial=True returns (frames, status) and does not raise for a frame that failed (MC_ERR_ARG,
+        MC_ERR_CAPACITY)."""
+        fo = _i32(frame_offsets).reshape(-1)
+        cv = self._curves(models)
+        d, fd = _f32(depth), _f32(fill_distance)
+        keep = [_f32(q_desc).reshape(-1, self.D), _f32(q_xy).reshape(-1, 2), _i32(q_image).reshape(-1) if q_image is not None else None,
+                _f32(q_world).reshape(-1, 3) if q_world is not None else None, _f32(q_fill).reshape(-1) if q_fill is not None else None]
+        ptrs = [a.ctypes.data if a is not None and a.size else None for a in keep]
+        args = ptrs + [fo, len(fo) - 1, d.ctypes.data, fd.ctypes.data, d.shape[-1], d.shape[-2], cv.ctypes.data, len(cv), *[float(v) for v in depths]]
+        return self._depth_queries(self.L.mc_process_depth_queries, "mc_process_depth_queries", len(fo) - 1, len(cv), args, params, max_objects,
+                                   times, partial)
+
+    def process_depth_queries_dev(self, q_ptr, xy_ptr, img_ptr, world_ptr, fill_ptr, frame_offsets, depth_ptr, fill_distance_ptr, width, height,
+                                  models, depths=ADAPTIVE_DEPTHS, params=None, max_objects=64, times=None, partial=False):
+        """mc_process_depth_queries_dev: the same with the per-feature arrays and the planes on the device (pointers)."""
+        fo = _i32(frame_offsets).reshape(-1)
+        cv = self._curves(models)
+        args = [q_ptr, xy_ptr, img_ptr, world_ptr, fill_ptr, fo, len(fo) - 1, depth_ptr, fill_distance_ptr, int(width), int(height), cv.ctypes.data,
+                len(cv), *[float(v) for v in depths]]
+        return self._depth_queries(self.L.mc_process_depth_queries_dev, "mc_process_depth_queries_dev", len(fo) - 1, len(cv), args, params,
+                                   max_objects, times, partial)
+
+    def process_depth_queries_merged_dev(self, packed_all_ptr, n_shards, xy_ptr, img_ptr, world_ptr, fill_ptr, frame_offsets, frame_begin, frame_end,
+                                         depth_ptr, fill_distance_ptr, width, height, models, depths=ADAPTIVE_DEPTHS, params=None, max_objects=64,
+                                         times=None, partial=False):
+        """mc_process_depth_queries_merged_dev: frames [frame_begin, frame_end) from the n_shards gathered packed blocks; the per-feature
+        arrays hold the whole batch, depth_ptr / fill_distance_ptr the range's planes only. One dict per frame of the range."""
+        fo = _i32(frame_offsets).reshape(-1)
+        cv = self._curves(models)
+        args = [packed_all_ptr, int(n_shards), xy_ptr, img_ptr, world_ptr, fill_ptr, fo, len(fo) - 1, int(frame_begin), int(frame_end), depth_ptr,
+                fill_distance_ptr, int(width), int(height), cv.ctypes.data, len(cv), *[float(v) for v in depths]]
+        return self._depth_queries(self.L.mc_process_depth_queries_merged_dev, "mc_process_depth_queries_merged_dev",
+                                   max(int(frame_end) - int(frame_begin), 0), len(cv), args, params, max_objects, times, partial)
 
     def process_frames_matched_dev(self, nn_row_ptr, acc_ptr, xy_ptr, img_ptr, frame_offsets, frame_begin, frame_end, params, max_objects,
                                    info_ptr, model_ptr, pose_ptr, score_ptr):

@@ -134,25 +134,20 @@ float depth_for_side(const Face &f, const float *K, float target) {
 
 } // namespace
 
-// ---- frame batches (mc_match_adaptive_frames / _dev / _merged_dev) --------------------------------------------------------------
-// Where the nearest rows come from: one cascade pass over q_desc against the context's database (n_shards = 0), or the merge of
-// n_shards gathered packed blocks (device) against the context's tables.
-struct RowSource {
-	const float *q_desc;
-	const int32_t *packed_all;
-	int n_shards;
-};
-
+// ---- frame batches (mc_match_adaptive_frames / _dev / _merged_dev, and MATCH of mc_process_depth_queries*) ------------------------
 // Frames [frame_begin, frame_end) of the batch are processed (the cascade always takes the whole batch). `dev`: queries, planes and
 // the per-match / per-feature outputs are device pointers; otherwise host arrays, staged through the context's buffers. The planes
 // start with frame frame_begin; per-feature and per-match arrays use global feature ids; match_offsets and frame_info have one row per
 // frame of the range. frame_offsets, match_offsets and frame_info are host arrays either way. One synchronisation per call.
-static mc_status match_adaptive_frames(mc_ctx *ctx, bool dev, const char *who, const RowSource &src, const float *q_xy, const int32_t *q_image,
-                                       const int32_t *frame_offsets, int n_frames, int frame_begin, int frame_end, const float *depth,
-                                       const float *fill_distance, int width, int height, const mc_adaptive_model *models, int n_models,
-                                       float maximum_depth, float default_depth, float cauchy_scale, int32_t *match_offsets, int32_t *match_feature,
-                                       int32_t *match_image, float *match_xy, float *match_xyz, int32_t *nn_row, float *nn_dist, uint8_t *accepted,
-                                       int32_t *frame_info) {
+// q_world / q_fill (device, `dev` only, nullable): DEPTHPROP's per-feature depth data, gathered into match_world / match_fill by the
+// compaction. ev (nullable, 2 events): recorded on ctx->stream around the device work of MATCH (cascade or merge, finalize, compaction).
+mc_status match_adaptive_frames(mc_ctx *ctx, bool dev, const char *who, const RowSource &src, const float *q_xy, const int32_t *q_image,
+                                const int32_t *frame_offsets, int n_frames, int frame_begin, int frame_end, const float *depth,
+                                const float *fill_distance, int width, int height, const mc_adaptive_model *models, int n_models,
+                                float maximum_depth, float default_depth, float cauchy_scale, int32_t *match_offsets, int32_t *match_feature,
+                                int32_t *match_image, float *match_xy, float *match_xyz, int32_t *nn_row, float *nn_dist, uint8_t *accepted,
+                                int32_t *frame_info, const float *q_world, const float *q_fill, float *match_world, float *match_fill,
+                                cudaEvent_t *ev) {
 	if (!ctx) return MC_ERR_ARG;
 	auto fail = [&](mc_status st, const std::string &what) { ctx->err = std::string(who) + ": " + what; return st; };
 	const bool merge = src.n_shards > 0;
@@ -245,6 +240,7 @@ static mc_status match_adaptive_frames(mc_ctx *ctx, bool dev, const char *who, c
 	const dim3 grid((unsigned)((q_max + 255) / 256), (unsigned)n_range);
 	const mc_adaptive_model *d_curves = (const mc_adaptive_model *)(b + o_curves);
 	int32_t *d_moff = (int32_t *)(b + o_moff), *d_status = (int32_t *)(b + o_status), *d_bad = d_status + n_range;
+	if (ev) MC_CUDA(cudaEventRecord(ev[0], ctx->stream));
 	if (merge) {
 		MC_CUDA(cudaMemsetAsync(d_bad, 0, sizeof(int32_t) * (size_t)n_range, ctx->stream));
 		k_match_merge_adaptive<<<grid, 256, 0, ctx->stream>>>(src.packed_all, src.n_shards, Q, d_fo, d_xy, d_depth, d_fill, width, height,
@@ -258,7 +254,9 @@ static mc_status match_adaptive_frames(mc_ctx *ctx, bool dev, const char *who, c
 	}
 	MC_LAUNCH_CHECK();
 	MC_TRY(match_compact_frames_device(ctx, (const FrameDesc *)(b + o_fd), d_fo, n_range, n_models, (int32_t *)(b + o_acc_list), d_moff, d_feat,
-	                                   (int32_t *)(b + o_mrow), d_mimg, d_mxy, d_mxyz, d_status, (int32_t *)(b + o_nobj)));
+	                                   (int32_t *)(b + o_mrow), d_mimg, d_mxy, d_mxyz, d_status, (int32_t *)(b + o_nobj), q_world, q_fill,
+	                                   match_world, match_fill));
+	if (ev) MC_CUDA(cudaEventRecord(ev[1], ctx->stream));
 	// frame-local offsets and frame flags -> host; the host entry also takes the per-match and per-feature arrays
 	const size_t h_moff_bytes = sizeof(int32_t) * (size_t)stride * n_range, h_flag_bytes = sizeof(int32_t) * (merge ? 2 : 1) * (size_t)n_range;
 	MC_TRY(pinned(ctx, h_moff_bytes + h_flag_bytes));
@@ -370,7 +368,7 @@ mc_status mc_match_adaptive_frames(mc_ctx *ctx, const float *q_desc, const float
 	const RowSource src = {q_desc, nullptr, 0};
 	return match_adaptive_frames(ctx, false, "mc_match_adaptive_frames", src, q_xy, q_image, frame_offsets, n_frames, 0, n_frames, depth, fill_distance,
 	                             width, height, models, n_models, maximum_depth, default_depth, cauchy_scale, match_offsets, match_feature, match_image, match_xy,
-	                             match_xyz, nn_row, nn_dist, accepted, frame_info);
+	                             match_xyz, nn_row, nn_dist, accepted, frame_info, nullptr, nullptr, nullptr, nullptr, nullptr);
 }
 
 mc_status mc_match_adaptive_frames_dev(mc_ctx *ctx, const float *q_desc_dev, const float *q_xy_dev, const int32_t *q_image_dev, const int32_t *frame_offsets,
@@ -381,7 +379,8 @@ mc_status mc_match_adaptive_frames_dev(mc_ctx *ctx, const float *q_desc_dev, con
 	const RowSource src = {q_desc_dev, nullptr, 0};
 	return match_adaptive_frames(ctx, true, "mc_match_adaptive_frames_dev", src, q_xy_dev, q_image_dev, frame_offsets, n_frames, 0, n_frames, depth_dev,
 	                             fill_distance_dev, width, height, models, n_models, maximum_depth, default_depth, cauchy_scale, match_offsets,
-	                             match_feature_dev, match_image_dev, match_xy_dev, match_xyz_dev, nn_row_dev, nn_dist_dev, accepted_dev, frame_info);
+	                             match_feature_dev, match_image_dev, match_xy_dev, match_xyz_dev, nn_row_dev, nn_dist_dev, accepted_dev, frame_info, nullptr,
+	                             nullptr, nullptr, nullptr, nullptr);
 }
 
 mc_status mc_match_adaptive_frames_merged_dev(mc_ctx *ctx, const void *packed_all_dev, int n_shards, const float *q_xy_dev, const int32_t *q_image_dev,
@@ -395,7 +394,7 @@ mc_status mc_match_adaptive_frames_merged_dev(mc_ctx *ctx, const void *packed_al
 	return match_adaptive_frames(ctx, true, "mc_match_adaptive_frames_merged_dev", src, q_xy_dev, q_image_dev, frame_offsets, n_frames, frame_begin,
 	                             frame_end, depth_dev, fill_distance_dev, width, height, models, n_models, maximum_depth, default_depth, cauchy_scale,
 	                             match_offsets, match_feature_dev, match_image_dev, match_xy_dev, match_xyz_dev, nn_row_dev, nn_dist_dev, accepted_dev,
-	                             frame_info);
+	                             frame_info, nullptr, nullptr, nullptr, nullptr, nullptr);
 }
 
 } // extern "C"

@@ -211,8 +211,26 @@ mc_status copy_objects_device(mc_ctx *ctx, const int32_t *d_n, const int32_t *d_
                               int32_t *d_dst_model, float *d_dst_pose);
 mc_status match_compact_frames_device(mc_ctx *ctx, const FrameDesc *d_fd, const int32_t *d_out_base, int n_frames, int n_models, int32_t *d_acc_list,
                                       int32_t *d_match_offsets, int32_t *d_match_query, int32_t *d_match_row, int32_t *d_match_image,
-                                      float *d_match_xy, float *d_match_xyz, int32_t *d_status, int32_t *d_n_obj);
+                                      float *d_match_xy, float *d_match_xyz, int32_t *d_status, int32_t *d_n_obj,
+                                      const float *d_q_world = nullptr, const float *d_q_fill = nullptr, float *d_match_world = nullptr,
+                                      float *d_match_fill = nullptr);
 constexpr int kCompactCap = 8192;    // accepted matches per frame handled by the compaction (k_match_compact)
+
+// ---- moped3d's batched MATCH (adaptive.cu), shared by mc_match_adaptive_frames* and mc_process_depth_queries* ----
+// Where the nearest rows come from: one cascade pass over q_desc against the context's database (n_shards = 0), or the merge of
+// n_shards gathered packed blocks (device) against the context's tables.
+struct RowSource {
+	const float *q_desc;
+	const int32_t *packed_all;
+	int n_shards;
+};
+mc_status match_adaptive_frames(mc_ctx *ctx, bool dev, const char *who, const RowSource &src, const float *q_xy, const int32_t *q_image,
+                                const int32_t *frame_offsets, int n_frames, int frame_begin, int frame_end, const float *depth,
+                                const float *fill_distance, int width, int height, const mc_adaptive_model *models, int n_models,
+                                float maximum_depth, float default_depth, float cauchy_scale, int32_t *match_offsets, int32_t *match_feature,
+                                int32_t *match_image, float *match_xy, float *match_xyz, int32_t *nn_row, float *nn_dist, uint8_t *accepted,
+                                int32_t *frame_info, const float *q_world, const float *q_fill, float *match_world, float *match_fill,
+                                cudaEvent_t *ev);
 
 // ---- moped3d linkage clustering of all models of a frame at once (linkage.cu) ----
 struct LinkSlice {         // one model of a frame: matches lo .. lo+n of the frame, n x n matrix block at element sq of the arena

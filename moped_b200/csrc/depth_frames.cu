@@ -168,17 +168,25 @@ static mc_status depth_frame_enqueue(mc_ctx *lane, const DepthPlan &p, const cha
 	return MC_OK;
 }
 
-// Checks on the host, then plans every frame and lays out the metadata (per frame: local CSR, LinkSlices). Returns the number of
-// matches the per-match arrays must hold.
-static mc_status depth_plan(mc_ctx *ctx, const char *who, const int32_t *match_offsets, int n_frames, int n_models, int width, int height,
-                            const mc_depth_pipeline_params *P, int max_objects, std::vector<DepthPlan> &plans, std::vector<char> &meta, int *m_total) {
+static mc_status depth_params_check(mc_ctx *ctx, const char *who, const mc_depth_pipeline_params *P) {
 	auto fail = [&](mc_status st, const std::string &msg) { ctx->err = std::string(who) + ": " + msg; return st; };
-	if (!match_offsets || n_frames < 1 || n_models < 1 || width < 1 || height < 1 || max_objects <= 0) return fail(MC_ERR_ARG, "bad argument");
 	if (P->variant < 0 || P->variant > 1) return fail(MC_ERR_ARG, "variant must be 0 (back-projection) or 1 (reprojection)");
 	// with cutoff <= -1 the merge loop has no stopping point once a single cluster is left (the reference then spins on the host)
 	if (!(P->cluster_cutoff > -1.f)) return fail(MC_ERR_ARG, "cluster_cutoff must be > -1");
 	if (P->pose.n_pts_align < 1 || P->pose.n_pts_align > 8 || P->pose2.n_pts_align < 1 || P->pose2.n_pts_align > 8)
 		return fail(MC_ERR_ARG, "n_pts_align must be in 1..8");
+	return MC_OK;
+}
+
+// Checks on the host, then plans every frame and lays out the metadata (per frame: local CSR, LinkSlices). Returns the number of
+// matches the per-match arrays must hold. frame_status (nullable): a frame over the chain's limits (a model with more than 2048
+// matches, or more than 2^24 similarity entries) gets status 4 and an empty plan instead of failing the call.
+static mc_status depth_plan(mc_ctx *ctx, const char *who, const int32_t *match_offsets, int n_frames, int n_models, int width, int height,
+                            const mc_depth_pipeline_params *P, int max_objects, std::vector<DepthPlan> &plans, std::vector<char> &meta, int *m_total,
+                            int32_t *frame_status = nullptr) {
+	auto fail = [&](mc_status st, const std::string &msg) { ctx->err = std::string(who) + ": " + msg; return st; };
+	if (!match_offsets || n_frames < 1 || n_models < 1 || width < 1 || height < 1 || max_objects <= 0) return fail(MC_ERR_ARG, "bad argument");
+	MC_TRY(depth_params_check(ctx, who, P));
 	const int per_cl = P->cluster_min_pts + 1 > 1 ? P->cluster_min_pts + 1 : 1;     // a cluster has more than min_pts members
 	plans.assign((size_t)n_frames, DepthPlan());
 	meta.clear();
@@ -189,25 +197,37 @@ static mc_status depth_plan(mc_ctx *ctx, const char *who, const int32_t *match_o
 		if (row[0] < 0) return fail(MC_ERR_ARG, "match_offsets must be >= 0 (frame " + std::to_string(f) + ")");
 		p.base = row[0]; p.M = 0; p.n_slices = 0; p.n_max = 0; p.sq = 0; p.cl_cap = 0;
 		std::vector<LinkSlice> sl;
+		bool over = false;
 		for (int m = 0; m < n_models; m++) {
 			const int n = row[m + 1] - row[m];
 			if (n < 0) return fail(MC_ERR_ARG, "match_offsets must ascend (frame " + std::to_string(f) + ")");
-			if (n > kMaxModelMatches) return fail(MC_ERR_ARG, "a model has more than 2048 matches (frame " + std::to_string(f) + ")");
+			if (n > kMaxModelMatches) {
+				if (!frame_status) return fail(MC_ERR_ARG, "a model has more than 2048 matches (frame " + std::to_string(f) + ")");
+				over = true;
+			}
 			if (n == 0) continue;
 			sl.push_back(LinkSlice{ p.sq, row[m] - row[0], n, m, 0 });
 			p.sq += (int64_t)n * n;
 			p.n_max = std::max(p.n_max, n);
 			p.cl_cap += n / per_cl;
 		}
-		if (p.sq > kLinkArenaMax) return fail(MC_ERR_CAPACITY, "the models of frame " + std::to_string(f) + " need more than 2^24 similarity entries");
+		if (p.sq > kLinkArenaMax) {
+			if (!frame_status) return fail(MC_ERR_CAPACITY, "the models of frame " + std::to_string(f) + " need more than 2^24 similarity entries");
+			over = true;
+		}
 		p.M = row[n_models] - row[0];
+		if (over) {                                       // nothing of this frame runs
+			frame_status[f] = 4;
+			sl.clear();
+			p.M = 0; p.n_max = 0; p.sq = 0; p.cl_cap = 0;
+		}
 		p.n_slices = (int)sl.size();
 		mt = std::max(mt, (int)row[n_models]);
 		p.meta = meta.size();
 		const size_t slice_at = (((size_t)n_models + 1) * 4 + 15) & ~(size_t)15;
 		meta.resize(p.meta + ((slice_at + sizeof(LinkSlice) * sl.size() + 255) & ~(size_t)255));
 		int32_t *loc = (int32_t *)(meta.data() + p.meta);
-		for (int m = 0; m <= n_models; m++) loc[m] = row[m] - row[0];
+		for (int m = 0; m <= n_models; m++) loc[m] = over ? 0 : row[m] - row[0];
 		if (!sl.empty()) memcpy(meta.data() + p.meta + slice_at, sl.data(), sizeof(LinkSlice) * sl.size());
 	}
 	if (!ctx->d_cams) return fail(MC_ERR_STATE, "cameras not set (mc_set_cameras)");
@@ -215,9 +235,12 @@ static mc_status depth_plan(mc_ctx *ctx, const char *who, const int32_t *match_o
 	return MC_OK;
 }
 
+// span (nullable, 2 events): recorded on ctx->stream at the fork to the lanes and after their join; unlike stage_ms, it leaves the
+// frames dealt to the lanes
 static mc_status depth_frames_run(mc_ctx *ctx, const char *who, const std::vector<DepthPlan> &plans, const std::vector<char> &meta,
                                   const DepthInputs &in, int n_models, int W, int H, const mc_depth_pipeline_params *P, int max_objects,
-                                  int32_t *n_objects, int32_t *obj_model, float *obj_pose, float *obj_score, int32_t *frame_info, float *stage_ms) {
+                                  int32_t *n_objects, int32_t *obj_model, float *obj_pose, float *obj_score, int32_t *frame_info, float *stage_ms,
+                                  cudaEvent_t *span = nullptr) {
 	const int nf = (int)plans.size();
 	MC_TRY(reserve(ctx, ctx->scratch[23], meta.size() + 256));
 	char *d_meta = (char *)ctx->scratch[23].p;
@@ -239,6 +262,7 @@ static mc_status depth_frames_run(mc_ctx *ctx, const char *who, const std::vecto
 		ev.resize(6 * (size_t)nf);
 		for (auto &e : ev) MC_CUDA(cudaEventCreate(&e));
 	}
+	if (span) MC_CUDA(cudaEventRecord(span[0], ctx->stream));
 	MC_CUDA(cudaEventRecord(ctx->ev_fork, ctx->stream));
 	for (int l = 0; l < n_lanes; l++) MC_CUDA(cudaStreamWaitEvent(ctx->lanes[(size_t)l]->stream, ctx->ev_fork, 0));
 	if (n_lanes > ctx->lanes_pending) ctx->lanes_pending = n_lanes;
@@ -251,6 +275,7 @@ static mc_status depth_frames_run(mc_ctx *ctx, const char *who, const std::vecto
 	}
 	const mc_status sj = join_lanes(ctx);
 	if (st == MC_OK) st = sj;
+	if (st == MC_OK && span) MC_CUDA(cudaEventRecord(span[1], ctx->stream));
 	char *h = (char *)ctx->h_pinned;
 	if (st == MC_OK) {
 		MC_CUDA(cudaMemcpyAsync(h, d, bytes, cudaMemcpyDeviceToHost, ctx->stream));
@@ -283,6 +308,125 @@ static mc_status depth_frames_run(mc_ctx *ctx, const char *who, const std::vecto
 	if (bad_frame >= 0) { ctx->err = std::string(who) + ": a match of frame " + std::to_string(bad_frame) + " lies outside the depth map"; return MC_ERR_ARG; }
 	if (over_frame >= 0) { ctx->err = std::string(who) + ": frame " + std::to_string(over_frame) + " has more than max_objects objects"; return MC_ERR_CAPACITY; }
 	return MC_OK;
+}
+
+// ---- moped3d from features to objects (mc_process_depth_queries*) ----------------------------------------------------------------
+// MATCH (adaptive.cu) for frames [frame_begin, frame_end), its compaction also gathering DEPTHPROP's per-feature depth data per match,
+// into context scratch (global feature ids, as MATCH writes them); the one synchronisation of MATCH brings the offsets and the frame
+// flags to the host for the chain's plan; then the chain on the frame lanes. `dev` = false: the host inputs are uploaded first (the
+// range is then the whole batch). frame_info status: 1 a match outside the depth map, 2 a row outside the tables, 3 more than 8192
+// accepted matches, 4 over the chain's per-frame limits; such a frame gets no objects (with 2, 3 or 4 the chain does not run for it).
+static mc_status depth_queries(mc_ctx *ctx, bool dev, const char *who, const RowSource &src, const float *q_xy, const int32_t *q_image,
+                               const float *q_world, const float *q_fill, const int32_t *frame_offsets, int n_frames, int frame_begin,
+                               int frame_end, const float *depth, const float *fill_distance, int width, int height,
+                               const mc_adaptive_model *models, int n_models, float maximum_depth, float default_depth, float cauchy_scale,
+                               const mc_depth_pipeline_params *P, int max_objects, int32_t *n_objects, int32_t *obj_model, float *obj_pose,
+                               float *obj_score, int32_t *frame_info, float *stage_ms) {
+	if (!ctx) return MC_ERR_ARG;
+	auto fail = [&](mc_status st, const std::string &msg) { ctx->err = std::string(who) + ": " + msg; return st; };
+	if (!P || !n_objects || !obj_model || !obj_pose || !obj_score || max_objects <= 0 || !frame_offsets || n_frames < 1 || n_models < 1 ||
+	    width < 1 || height < 1 || !depth || !fill_distance)
+		return fail(MC_ERR_ARG, "bad argument");
+	if (frame_begin < 0 || frame_begin > frame_end || frame_end > n_frames) return fail(MC_ERR_ARG, "frame range outside 0..n_frames");
+	if (frame_offsets[0] != 0) return fail(MC_ERR_ARG, "frame_offsets[0] must be 0");
+	for (int f = 0; f < n_frames; f++)
+		if (frame_offsets[f + 1] < frame_offsets[f]) return fail(MC_ERR_ARG, "frame_offsets do not ascend");
+	const int Q = frame_offsets[n_frames], n_range = frame_end - frame_begin;
+	const bool any = frame_offsets[frame_end] > frame_offsets[frame_begin];
+	if (any && (!q_xy || !q_world || !q_fill || (!dev && !src.q_desc))) return fail(MC_ERR_ARG, "bad argument");
+	MC_TRY(depth_params_check(ctx, who, P));
+	if (!ctx->d_cams) return fail(MC_ERR_STATE, "cameras not set (mc_set_cameras)");
+	MC_CUDA(cudaSetDevice(ctx->device));
+	// per match (capacity Q, global ids): feature, image, xy, xyz, world, fill; the host entry's inputs behind them
+	const size_t planes = (size_t)width * height * n_range;
+	size_t off = 0;
+	auto take = [&](size_t bytes) { const size_t o = off; off += (bytes + 255) & ~(size_t)255; return o; };
+	const size_t o_feat = take(4ull * Q), o_img = take(4ull * Q), o_xy = take(8ull * Q), o_xyz = take(12ull * Q), o_w = take(12ull * Q), o_f = take(4ull * Q);
+	const size_t o_qw = dev ? 0 : take(12ull * Q), o_qf = dev ? 0 : take(4ull * Q), o_d = dev ? 0 : take(4 * planes), o_fd = dev ? 0 : take(4 * planes);
+	MC_TRY(reserve(ctx, ctx->scratch[16], off));
+	char *b = (char *)ctx->scratch[16].p;
+	RowSource rs = src;
+	const float *d_xy = q_xy, *d_qw = q_world, *d_qf = q_fill, *d_depth = depth, *d_fill = fill_distance;
+	const int32_t *d_img = q_image;
+	if (!dev) {
+		cudaStream_t s = ctx->stream;
+		if (Q > 0) {
+			MC_TRY(reserve(ctx, ctx->q_desc, sizeof(float) * (size_t)Q * ctx->D));
+			MC_TRY(reserve(ctx, ctx->q_xy, 8ull * Q));
+			MC_CUDA(cudaMemcpyAsync(ctx->q_desc.p, src.q_desc, sizeof(float) * (size_t)Q * ctx->D, cudaMemcpyHostToDevice, s));
+			MC_CUDA(cudaMemcpyAsync(ctx->q_xy.p, q_xy, 8ull * Q, cudaMemcpyHostToDevice, s));
+			MC_CUDA(cudaMemcpyAsync(b + o_qw, q_world, 12ull * Q, cudaMemcpyHostToDevice, s));
+			MC_CUDA(cudaMemcpyAsync(b + o_qf, q_fill, 4ull * Q, cudaMemcpyHostToDevice, s));
+			if (q_image) {
+				MC_TRY(reserve(ctx, ctx->q_image, 4ull * Q));
+				MC_CUDA(cudaMemcpyAsync(ctx->q_image.p, q_image, 4ull * Q, cudaMemcpyHostToDevice, s));
+				d_img = (const int32_t *)ctx->q_image.p;
+			}
+		}
+		MC_CUDA(cudaMemcpyAsync(b + o_d, depth, 4 * planes, cudaMemcpyHostToDevice, s));
+		MC_CUDA(cudaMemcpyAsync(b + o_fd, fill_distance, 4 * planes, cudaMemcpyHostToDevice, s));
+		rs.q_desc = (const float *)ctx->q_desc.p; d_xy = (const float *)ctx->q_xy.p;
+		d_qw = (const float *)(b + o_qw); d_qf = (const float *)(b + o_qf); d_depth = (const float *)(b + o_d); d_fill = (const float *)(b + o_fd);
+	}
+	DepthInputs in;
+	in.image = (const int32_t *)(b + o_img); in.xy = (const float *)(b + o_xy); in.xyz = (const float *)(b + o_xyz); in.world = (const float *)(b + o_w);
+	in.fill = (const float *)(b + o_f); in.depth = d_depth; in.distance = d_fill;
+	struct Events {                                     // MATCH start / end, chain fork / join (stage_ms)
+		cudaEvent_t e[4] = {nullptr, nullptr, nullptr, nullptr};
+		~Events() { for (cudaEvent_t x : e) if (x) cudaEventDestroy(x); }
+	} ev;
+	if (stage_ms) for (cudaEvent_t &x : ev.e) MC_CUDA(cudaEventCreate(&x));
+	const size_t stride = (size_t)n_models + 1;
+	// (at least one row each: MATCH takes a NULL array as an argument error, also for an empty range)
+	const size_t rows = n_range > 0 ? (size_t)n_range : 1;
+	std::vector<int32_t> moff(stride * rows), minfo(3 * rows, 0), status(rows, 0);
+	const mc_status sm = match_adaptive_frames(ctx, true, who, rs, d_xy, d_img, frame_offsets, n_frames, frame_begin, frame_end, d_depth, d_fill, width,
+	                                           height, models, n_models, maximum_depth, default_depth, cauchy_scale, moff.data(), (int32_t *)(b + o_feat),
+	                                           (int32_t *)in.image, (float *)in.xy, (float *)in.xyz, nullptr, nullptr, nullptr, minfo.data(), d_qw, d_qf,
+	                                           (float *)in.world, (float *)in.fill, stage_ms ? ev.e : nullptr);
+	bool match_failed = false;                          // frames MATCH left empty (its status 2, or 1 = over its cap)
+	for (int f = 0; f < n_range; f++)
+		if (minfo[3 * (size_t)f + 2]) { status[(size_t)f] = minfo[3 * (size_t)f + 2] == 2 ? 2 : 3; match_failed = true; }
+	if (sm != MC_OK && !match_failed) return sm;
+	if (n_range == 0) return MC_OK;
+	std::vector<DepthPlan> plans;
+	std::vector<char> meta;
+	std::vector<int32_t> plan_status((size_t)n_range, 0);
+	int M = 0;
+	MC_TRY(depth_plan(ctx, who, moff.data(), n_range, n_models, width, height, P, max_objects, plans, meta, &M, plan_status.data()));
+	std::vector<int32_t> info(4 * (size_t)n_range);
+	const mc_status sc = depth_frames_run(ctx, who, plans, meta, in, n_models, width, height, P, max_objects, n_objects, obj_model, obj_pose, obj_score,
+	                                      info.data(), nullptr, stage_ms ? ev.e + 2 : nullptr);
+	if (sc != MC_OK && sc != MC_ERR_ARG && sc != MC_ERR_CAPACITY) return sc;
+	int first_arg = -1, first_cap = -1;
+	for (int f = 0; f < n_range; f++) {
+		int32_t *fi = info.data() + 4 * (size_t)f;
+		if (plan_status[(size_t)f]) status[(size_t)f] = 4;
+		if (status[(size_t)f]) {                         // nothing ran after MATCH: no objects, no clusters
+			const int32_t *row = moff.data() + (size_t)f * stride;
+			fi[0] = 0; fi[1] = status[(size_t)f]; fi[2] = row[n_models] - row[0]; fi[3] = 0;
+		}
+		const int s = fi[1];
+		if ((s == 1 || s == 2) && first_arg < 0) first_arg = f;
+		if ((s == 3 || s == 4 || (s == 0 && fi[0] > max_objects)) && first_cap < 0) first_cap = f;
+	}
+	if (frame_info) memcpy(frame_info, info.data(), 16 * (size_t)n_range);
+	if (stage_ms) {
+		stage_ms[0] = stage_ms[1] = 0.f;
+		if (any) MC_CUDA(cudaEventElapsedTime(&stage_ms[0], ev.e[0], ev.e[1]));
+		if (sc == MC_OK || first_arg >= 0 || first_cap >= 0) MC_CUDA(cudaEventElapsedTime(&stage_ms[1], ev.e[2], ev.e[3]));
+	}
+	const std::string frame = "frame " + std::to_string(frame_begin + (first_arg >= 0 ? first_arg : first_cap));
+	if (first_arg >= 0)
+		return fail(MC_ERR_ARG, info[4 * (size_t)first_arg + 1] == 1 ? "a match of " + frame + " lies outside the depth map"
+		                                                             : frame + " has a nearest row outside the database tables");
+	if (first_cap >= 0) {
+		const int s = info[4 * (size_t)first_cap + 1];
+		return fail(MC_ERR_CAPACITY, frame + (s == 3   ? " has more than " + std::to_string(kCompactCap) + " accepted matches"
+		                                      : s == 4 ? " has a model with more than 2048 matches or needs more than 2^24 similarity entries"
+		                                               : " has more than max_objects objects"));
+	}
+	return sc;
 }
 
 } // namespace mc
@@ -375,6 +519,42 @@ mc_status mc_process_depth_frames_dev(mc_ctx *ctx, const int32_t *match_offsets,
 	in.depth = depth_dev; in.distance = fill_distance_dev;
 	return depth_frames_run(ctx, who, plans, meta, in, n_models, width, height, params, max_objects, n_objects, obj_model, obj_pose, obj_score,
 	                        frame_info, stage_ms);
+}
+
+mc_status mc_process_depth_queries(mc_ctx *ctx, const float *q_desc, const float *q_xy, const int32_t *q_image, const float *q_world, const float *q_fill,
+                                   const int32_t *frame_offsets, int n_frames, const float *depth, const float *fill_distance, int width, int height,
+                                   const mc_adaptive_model *models, int n_models, float maximum_depth, float default_depth, float cauchy_scale,
+                                   const mc_depth_pipeline_params *params, int max_objects, int32_t *n_objects, int32_t *obj_model, float *obj_pose,
+                                   float *obj_score, int32_t *frame_info, float *stage_ms) {
+	const RowSource src = {q_desc, nullptr, 0};
+	return depth_queries(ctx, false, "mc_process_depth_queries", src, q_xy, q_image, q_world, q_fill, frame_offsets, n_frames, 0, n_frames, depth,
+	                     fill_distance, width, height, models, n_models, maximum_depth, default_depth, cauchy_scale, params, max_objects, n_objects,
+	                     obj_model, obj_pose, obj_score, frame_info, stage_ms);
+}
+
+mc_status mc_process_depth_queries_dev(mc_ctx *ctx, const float *q_desc_dev, const float *q_xy_dev, const int32_t *q_image_dev,
+                                       const float *q_world_dev, const float *q_fill_dev, const int32_t *frame_offsets, int n_frames,
+                                       const float *depth_dev, const float *fill_distance_dev, int width, int height, const mc_adaptive_model *models,
+                                       int n_models, float maximum_depth, float default_depth, float cauchy_scale,
+                                       const mc_depth_pipeline_params *params, int max_objects, int32_t *n_objects, int32_t *obj_model,
+                                       float *obj_pose, float *obj_score, int32_t *frame_info, float *stage_ms) {
+	const RowSource src = {q_desc_dev, nullptr, 0};
+	return depth_queries(ctx, true, "mc_process_depth_queries_dev", src, q_xy_dev, q_image_dev, q_world_dev, q_fill_dev, frame_offsets, n_frames, 0,
+	                     n_frames, depth_dev, fill_distance_dev, width, height, models, n_models, maximum_depth, default_depth, cauchy_scale, params,
+	                     max_objects, n_objects, obj_model, obj_pose, obj_score, frame_info, stage_ms);
+}
+
+mc_status mc_process_depth_queries_merged_dev(mc_ctx *ctx, const void *packed_all_dev, int n_shards, const float *q_xy_dev, const int32_t *q_image_dev,
+                                              const float *q_world_dev, const float *q_fill_dev, const int32_t *frame_offsets, int n_frames,
+                                              int frame_begin, int frame_end, const float *depth_dev, const float *fill_distance_dev, int width,
+                                              int height, const mc_adaptive_model *models, int n_models, float maximum_depth, float default_depth,
+                                              float cauchy_scale, const mc_depth_pipeline_params *params, int max_objects, int32_t *n_objects,
+                                              int32_t *obj_model, float *obj_pose, float *obj_score, int32_t *frame_info, float *stage_ms) {
+	if (ctx && (!packed_all_dev || n_shards < 1)) { ctx->err = "mc_process_depth_queries_merged_dev: bad argument"; return MC_ERR_ARG; }
+	const RowSource src = {nullptr, (const int32_t *)packed_all_dev, n_shards};
+	return depth_queries(ctx, true, "mc_process_depth_queries_merged_dev", src, q_xy_dev, q_image_dev, q_world_dev, q_fill_dev, frame_offsets, n_frames,
+	                     frame_begin, frame_end, depth_dev, fill_distance_dev, width, height, models, n_models, maximum_depth, default_depth,
+	                     cauchy_scale, params, max_objects, n_objects, obj_model, obj_pose, obj_score, frame_info, stage_ms);
 }
 
 } // extern "C"

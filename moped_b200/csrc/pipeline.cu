@@ -32,18 +32,24 @@ mc_status filter_device(mc_ctx *ctx, const int32_t *d_match_offsets, const int32
 // acc_list from element out_base[f] on, match_query = out_base[f] + query index in the frame (with out_base = the frames'
 // first query ids: the batch-global query id); match_offsets row f (n_models + 1 entries, frame-local: 0 .. matches),
 // status[f] and n_obj[f]. A frame cannot write past its own queries' range (matches <= queries), so a batch needs no packing.
+// kDepthData (moped3d, mc_process_depth_queries*): DEPTHPROP's per-feature depthData.coord3D (q_world, 3 floats) and .fillDistance
+// (q_fill) are gathered into match_world / match_fill in the same pass; they are indexed by batch-global feature id, so out_base
+// must then hold the frames' first feature ids. The default instance has no such reads and is the one every other caller launches.
 __global__ void k_set_desc(FrameDesc *dst, FrameDesc v) { *dst = v; }
 
+template <bool kDepthData = false>
 __global__ void __launch_bounds__(1024)
 k_match_compact(const FrameDesc *__restrict__ fd, const int32_t *__restrict__ out_base, int64_t row_base,
                 const int32_t *__restrict__ model_of_row, const float *__restrict__ db_xyz, int n_models, int32_t *__restrict__ acc_list,
                 int32_t *__restrict__ match_offsets, int32_t *__restrict__ match_query, int32_t *__restrict__ match_row,
                 int32_t *__restrict__ match_image, float *__restrict__ match_xy, float *__restrict__ match_xyz,
-                int32_t *__restrict__ status, int32_t *__restrict__ n_obj) {
+                int32_t *__restrict__ status, int32_t *__restrict__ n_obj, const float *__restrict__ q_world = nullptr,
+                const float *__restrict__ q_fill = nullptr, float *__restrict__ match_world = nullptr, float *__restrict__ match_fill = nullptr) {
 	const int f = blockIdx.x;
 	fd += f;
 	const int base = out_base ? out_base[f] : 0;
 	acc_list += base; match_query += base; match_row += base; match_image += base; match_xy += 2 * (size_t)base; match_xyz += 3 * (size_t)base;
+	if (kDepthData) { match_world += 3 * (size_t)base; match_fill += base; }
 	match_offsets += (size_t)f * (n_models + 1);
 	status += f; n_obj += f;
 	const int32_t *__restrict__ nn_row = fd->nn_row;
@@ -101,6 +107,11 @@ k_match_compact(const FrameDesc *__restrict__ fd, const int32_t *__restrict__ ou
 		match_xy[2 * i] = q_xy[2 * q]; match_xy[2 * i + 1] = q_xy[2 * q + 1];
 		const int64_t lr = (int64_t)row - row_base;
 		match_xyz[3 * i] = db_xyz[3 * lr]; match_xyz[3 * i + 1] = db_xyz[3 * lr + 1]; match_xyz[3 * i + 2] = db_xyz[3 * lr + 2];
+		if (kDepthData) {
+			const size_t g = (size_t)base + q;
+			match_world[3 * i] = q_world[3 * g]; match_world[3 * i + 1] = q_world[3 * g + 1]; match_world[3 * i + 2] = q_world[3 * g + 2];
+			match_fill[i] = q_fill[g];
+		}
 		const int mprev = i > 0 ? (int)(keys[i - 1] >> 13) : -1;
 		for (int mm = mprev + 1; mm <= m; mm++) match_offsets[mm] = i;
 	}
@@ -282,13 +293,20 @@ mc_status gather_depth_points_device(mc_ctx *ctx, const int32_t *d_n, const int3
 	return MC_OK;
 }
 
-// for moped3d's batched MATCH (adaptive.cu): the compaction of n_frames frames in one launch
+// for moped3d's batched MATCH (adaptive.cu): the compaction of n_frames frames in one launch; with d_q_world given (then also d_q_fill,
+// d_match_world, d_match_fill, and d_out_base = the frames' first feature ids) it also gathers DEPTHPROP's per-feature depth data
 mc_status match_compact_frames_device(mc_ctx *ctx, const FrameDesc *d_fd, const int32_t *d_out_base, int n_frames, int n_models, int32_t *d_acc_list,
                                       int32_t *d_match_offsets, int32_t *d_match_query, int32_t *d_match_row, int32_t *d_match_image,
-                                      float *d_match_xy, float *d_match_xyz, int32_t *d_status, int32_t *d_n_obj) {
-	k_match_compact<<<n_frames, 1024, 0, ctx->stream>>>(d_fd, d_out_base, ctx->table_base, ctx->d_model_of_row, ctx->d_xyz, n_models, d_acc_list,
-	                                                   d_match_offsets, d_match_query, d_match_row, d_match_image, d_match_xy, d_match_xyz, d_status,
-	                                                   d_n_obj);
+                                      float *d_match_xy, float *d_match_xyz, int32_t *d_status, int32_t *d_n_obj, const float *d_q_world,
+                                      const float *d_q_fill, float *d_match_world, float *d_match_fill) {
+	if (d_q_world)
+		k_match_compact<true><<<n_frames, 1024, 0, ctx->stream>>>(d_fd, d_out_base, ctx->table_base, ctx->d_model_of_row, ctx->d_xyz, n_models, d_acc_list,
+		                                                         d_match_offsets, d_match_query, d_match_row, d_match_image, d_match_xy, d_match_xyz,
+		                                                         d_status, d_n_obj, d_q_world, d_q_fill, d_match_world, d_match_fill);
+	else
+		k_match_compact<<<n_frames, 1024, 0, ctx->stream>>>(d_fd, d_out_base, ctx->table_base, ctx->d_model_of_row, ctx->d_xyz, n_models, d_acc_list,
+		                                                   d_match_offsets, d_match_query, d_match_row, d_match_image, d_match_xy, d_match_xyz, d_status,
+		                                                   d_n_obj);
 	MC_LAUNCH_CHECK();
 	return MC_OK;
 }
