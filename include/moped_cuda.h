@@ -533,6 +533,28 @@ mc_status mc_process_depth_queries_merged_dev(mc_ctx *ctx, const void *packed_al
                                               const mc_depth_pipeline_params *params, int max_objects, int32_t *n_objects, int32_t *obj_model,
                                               float *obj_pose, float *obj_score, int32_t *frame_info, float *stage_ms);
 
+/* moped3d's FILTER_PROJECTION_DEPTH_CPU as FILTER and / or FILTER2 of the chain above (all five entries: mc_process_depth_frames*,
+ * mc_process_depth_queries*), for a pipeline that registers FILTER_PROJECTION_DEPTH_CUDA in place of FILTER_PROJECTION_CUDA. */
+typedef struct {
+	float plausible_sq_distance, depth_fraction, min_keypoint_fraction;  /* PlausibleSqDistance, DepthFraction, MinKeypointFraction */
+	float depth_K[4];                                                    /* the depth map's intrinsics (fx, fy, cx, cy) */
+	float depth_pose[7];                                                 /* the depth map's cameraPose (quat x y z w, t) */
+} mc_depth_filter_params;
+/* step 0 = FILTER, 1 = FILTER2 of the mc_process_depth_frames* / mc_process_depth_queries* chain. p != NULL: that step runs
+ * FILTER_PROJECTION_DEPTH with these parameters and these test points (test_offsets[n_models + 1] from 0, test_xyz model-major,
+ * copied to the device now). MinPoints / FeatureDistance / MinScore still come from mc_depth_pipeline_params. p == NULL: the step
+ * goes back to FILTER_PROJECTION (the default).
+ * Each step keeps its own table (each FILTER_PROJECTION_DEPTH_CPU instance draws its own TestSampleSize points), in device memory the
+ * context owns until the step is set again or mc_destroy: 12 bytes per test point, uploaded once and not per batch. A frame's depth
+ * and ".distance" planes are the ones the chain call takes; the depth camera's matrix is computed from depth_pose as
+ * mc_filter_projection_depth computes it, so every frame equals the stage-by-stage calls with mc_filter_projection_depth bit for bit.
+ * The penalty kernel adds one launch per depth-filtered step and frame; stage_ms counts it in FILTER / FILTER2.
+ * Errors (the previous setting stays): MC_ERR_ARG for a NULL ctx, a step outside 0..1, n_models < 1, test_offsets that do not start at 0
+ * or do not ascend, or a NULL test_xyz with points. A chain call whose n_models differs from a set table's returns MC_ERR_ARG before any
+ * launch; an object-sharded context (mc_process_depth_queries_merged_dev) takes global model ids, so every rank holds the whole table. */
+mc_status mc_set_depth_filter(mc_ctx *ctx, int step, const mc_depth_filter_params *p, const int32_t *test_offsets, const float *test_xyz,
+                              int n_models);
+
 /* Named integer options (scheduling / kernel-shape choices; unknown keys are an error):
  *   "pose_fit_thread_min"  mc_pose_hypotheses* calls with at least this many hypotheses and no inlier masks run one
  *                          THREAD per hypothesis instead of one 8-lane group (default 16384; 1 = always)

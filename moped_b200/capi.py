@@ -49,6 +49,17 @@ class DepthPipelineParams(C.Structure):
                 ("filter2_min_points", C.c_int32), ("filter2_feature_distance", C.c_float), ("filter2_min_score", C.c_float)]
 
 
+class DepthFilterParams(C.Structure):
+    """mc_depth_filter_params: FILTER_PROJECTION_DEPTH's own parameters and the depth camera, for one filter step of the moped3d chain."""
+    _fields_ = [("plausible_sq_distance", C.c_float), ("depth_fraction", C.c_float), ("min_keypoint_fraction", C.c_float),
+                ("depth_K", C.c_float * 4), ("depth_pose", C.c_float * 7)]
+
+    @classmethod
+    def of(cls, plausible_sq_distance, depth_fraction, min_keypoint_fraction, depth_K, depth_pose):
+        return cls(float(plausible_sq_distance), float(depth_fraction), float(min_keypoint_fraction), (C.c_float * 4)(*_f32(depth_K).reshape(4)),
+                   (C.c_float * 7)(*_f32(depth_pose).reshape(7)))
+
+
 # every symbol include/moped_cuda.h declares: name -> (restype, argtypes)
 SIGNATURES = {
     "mc_create": (C.c_int, [C.POINTER(C.c_void_p), C.c_int]),
@@ -154,6 +165,7 @@ SIGNATURES = {
     "mc_process_depth_queries_merged_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int] + [C.c_void_p] * 4 + [_i32p, C.c_int, C.c_int, C.c_int,
                                                       C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_float, C.c_float, C.c_float,
                                                       C.POINTER(DepthPipelineParams), C.c_int, _i32p, _i32p, _f32p, _f32p, _i32p, C.c_void_p]),
+    "mc_set_depth_filter": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(DepthFilterParams), C.c_void_p, C.c_void_p, C.c_int]),
 }
 
 MC_ERR_ARG = -2
@@ -769,6 +781,18 @@ class Context:
         arrays = [image_ptr, xy_ptr, xyz_ptr, world_ptr, fill_ptr, depth_ptr, fill_distance_ptr, int(width), int(height)]
         return self._depth_frames(self.L.mc_process_depth_frames_dev, "mc_process_depth_frames_dev", match_offsets, n_models, arrays, params,
                                   max_objects, times)
+
+    def set_depth_filter(self, step, params, test_offsets=None, test_xyz=None):
+        """mc_set_depth_filter: step 0 = FILTER, 1 = FILTER2 of the moped3d chain runs FILTER_PROJECTION_DEPTH with `params`
+        (DepthFilterParams) and the test points test_offsets [n_models + 1] / test_xyz [n, 3] (copied to the device now);
+        params=None puts the step back to FILTER_PROJECTION."""
+        if params is None:
+            self._check(self.L.mc_set_depth_filter(self.h, int(step), None, None, None, 0), "mc_set_depth_filter")
+            return
+        to = _i32(test_offsets).reshape(-1)
+        tx = _f32(test_xyz).reshape(-1) if test_xyz is not None else None
+        self._check(self.L.mc_set_depth_filter(self.h, int(step), C.byref(params), to.ctypes.data, tx.ctypes.data if tx is not None and tx.size else None,
+                                               len(to) - 1), "mc_set_depth_filter")
 
     def _depth_queries(self, fn, what, n_frames, n_models, args, params, max_objects, times, partial):
         p = params or self.default_depth_params()

@@ -143,6 +143,7 @@ void mc_destroy(mc_ctx *ctx) {
 	free_db(ctx);
 	sift_free(ctx);
 	cudaFree(ctx->d_cams);
+	for (DepthFilterTable &t : ctx->depth_filter) { cudaFree(t.d_offsets); cudaFree(t.d_xyz); }
 	free_scratch(ctx);
 	if (ctx->own_stream) cudaStreamDestroy(ctx->stream);
 	delete ctx;
@@ -319,11 +320,7 @@ mc_status mc_set_cameras(mc_ctx *ctx, const float *K, const float *cam_pose, int
 	std::vector<Camera> cams(n_images);
 	for (int i = 0; i < n_images; i++) {
 		for (int j = 0; j < 4; j++) cams[i].K[j] = K[4 * i + j];
-		const float *q = cam_pose + 7 * i, *t = q + 4;       // image->TM.init(cameraPose), moped.cpp:168-169
-		float *T = cams[i].TM;
-		T[0] = 1 - 2 * q[1] * q[1] - 2 * q[2] * q[2]; T[1] = 2 * q[0] * q[1] - 2 * q[3] * q[2]; T[2] = 2 * q[0] * q[2] + 2 * q[3] * q[1]; T[3] = t[0];
-		T[4] = 2 * q[0] * q[1] + 2 * q[3] * q[2]; T[5] = 1 - 2 * q[0] * q[0] - 2 * q[2] * q[2]; T[6] = 2 * q[1] * q[2] - 2 * q[3] * q[0]; T[7] = t[1];
-		T[8] = 2 * q[0] * q[2] - 2 * q[3] * q[1]; T[9] = 2 * q[1] * q[2] + 2 * q[3] * q[0]; T[10] = 1 - 2 * q[0] * q[0] - 2 * q[1] * q[1]; T[11] = t[2];
+		pose_tm(cam_pose + 7 * i, cams[i].TM);               // image->TM.init(cameraPose), moped.cpp:168-169
 	}
 	MC_CUDA(cudaStreamSynchronize(ctx->stream));
 	if (ctx->d_cams) { MC_CUDA(cudaFree(ctx->d_cams)); ctx->d_cams = nullptr; }
@@ -714,12 +711,7 @@ mc_status mc_filter_projection_depth(mc_ctx *ctx, const int32_t *match_offsets, 
 	MC_TRY(h2d(ctx, (float *)(b + o_d), depth, px));
 	MC_TRY(h2d(ctx, (float *)(b + o_f), fill_distance, px));
 	float TM[12];
-	{
-		const float *q = depth_pose, *t = q + 4;             // depthmap->TM.init(cameraPose), like mc_set_cameras
-		TM[0] = 1 - 2 * q[1] * q[1] - 2 * q[2] * q[2]; TM[1] = 2 * q[0] * q[1] - 2 * q[3] * q[2]; TM[2] = 2 * q[0] * q[2] + 2 * q[3] * q[1]; TM[3] = t[0];
-		TM[4] = 2 * q[0] * q[1] + 2 * q[3] * q[2]; TM[5] = 1 - 2 * q[0] * q[0] - 2 * q[2] * q[2]; TM[6] = 2 * q[1] * q[2] - 2 * q[3] * q[0]; TM[7] = t[1];
-		TM[8] = 2 * q[0] * q[2] - 2 * q[3] * q[1]; TM[9] = 2 * q[1] * q[2] + 2 * q[3] * q[0]; TM[10] = 1 - 2 * q[0] * q[0] - 2 * q[1] * q[1]; TM[11] = t[2];
-	}
+	pose_tm(depth_pose, TM);                                 // depthmap->TM.init(cameraPose)
 	MC_TRY(filter_depth_device(ctx, (int32_t *)(b + o_off), (int32_t *)(b + o_img), (float *)(b + o_xy), (float *)(b + o_xyz), n_models, M,
 	                           (int32_t *)(b + o_om), (float *)(b + o_op), nullptr, n_objects, min_points, feature_distance, min_score,
 	                           (int32_t *)(b + o_to), (float *)(b + o_tx), depth_K, TM, width, height, (float *)(b + o_d), (float *)(b + o_f),

@@ -46,6 +46,25 @@ struct DevBuf {            // grow-only device scratch
 	size_t cap = 0;
 };
 
+// TransformMatrix::init(cameraPose) on the host (moped.hpp:175-182): the 3x4 matrix of a pose (quaternion x y z w, translation).
+// One expression for every caller (mc_set_cameras, mc_filter_projection_depth, mc_set_depth_filter), so their bits agree.
+inline void pose_tm(const float *pose, float *T) {
+	const float *q = pose, *t = pose + 4;
+	T[0] = 1 - 2 * q[1] * q[1] - 2 * q[2] * q[2]; T[1] = 2 * q[0] * q[1] - 2 * q[3] * q[2]; T[2] = 2 * q[0] * q[2] + 2 * q[3] * q[1]; T[3] = t[0];
+	T[4] = 2 * q[0] * q[1] + 2 * q[3] * q[2]; T[5] = 1 - 2 * q[0] * q[0] - 2 * q[2] * q[2]; T[6] = 2 * q[1] * q[2] - 2 * q[3] * q[0]; T[7] = t[1];
+	T[8] = 2 * q[0] * q[2] - 2 * q[3] * q[1]; T[9] = 2 * q[1] * q[2] + 2 * q[3] * q[0]; T[10] = 1 - 2 * q[0] * q[0] - 2 * q[1] * q[1]; T[11] = t[2];
+}
+
+// FILTER_PROJECTION_DEPTH for one filter step of the moped3d chain (mc_set_depth_filter): the test points on the device, owned by the
+// context, and the step's parameters. d_offsets == nullptr: the step runs FILTER_PROJECTION.
+struct DepthFilterTable {
+	int32_t *d_offsets = nullptr;     // [n_models + 1], from 0
+	float *d_xyz = nullptr;           // test points, model-major (at least one point's room)
+	int n_models = 0;
+	float plausible_sq_distance = 0.f, depth_fraction = 0.f, min_keypoint_fraction = 0.f;
+	float K[4] = {0.f, 0.f, 0.f, 0.f}, TM[12] = {0.f};
+};
+
 } // namespace mc
 
 struct mc_ctx {
@@ -129,6 +148,7 @@ struct mc_ctx {
 	int lanes_pending = 0;            // lanes used since the last join
 	int batch_stats[4] = {0, 0, 0, 0};   // {frames, accepted matches, objects, lanes used} of the last batch
 	mc::DevBuf link_buf;                 // linkage clustering (linkage.cu): inputs, similarity matrices, agglomeration state
+	mc::DepthFilterTable depth_filter[2];   // FILTER / FILTER2 of mc_process_depth_frames* / _queries* (mc_set_depth_filter)
 	void *sift_state = nullptr;          // feature extraction (sift.cu): scale-space plan and buffers, created on first use
 };
 

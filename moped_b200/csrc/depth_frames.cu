@@ -8,7 +8,8 @@
 //            per model), then the clusters model-major (k_link_compact)
 //   POSE     k_gather_points with depthData.coord3D and the Cauchy weight of depthData.fillDistance, k_depth_ransac reading the
 //            cluster count from the device (grid and LM scratch sized by host upper bounds), k_pose_append
-//   FILTER   filter_device (moped3d's FILTER_PROJECTION_CPU is moped2's)
+//   FILTER   filter_device (moped3d's FILTER_PROJECTION_CPU is moped2's), or filter_depth_device (FILTER_PROJECTION_DEPTH) with the
+//            calling context's test points (mc_set_depth_filter) and the frame's own depth and ".distance" planes
 //   POSE2    the survivors stay in the object list (k_copy_objects), new objects from their rebuilt clusters are appended
 // No host synchronisation between the steps: counts stay on the device. The frames of a batch are dealt to the context's frame
 // lanes (pipeline.cu), each of which owns its buffers.
@@ -30,6 +31,13 @@ mc_status filter_device(mc_ctx *ctx, const int32_t *d_match_offsets, const int32
                         const int32_t *d_n_obj, int n_obj_cap, int min_points, float feat_dist, float min_score,
                         uint8_t *d_keep, float *d_score, int32_t *d_out_n, int32_t *d_cluster_model, int32_t *d_cluster_offsets,
                         int32_t *d_members, int32_t *d_surv_model, float *d_surv_pose, float *d_surv_score);
+mc_status filter_depth_device(mc_ctx *ctx, const int32_t *d_match_offsets, const int32_t *d_match_image, const float *d_match_xy,
+                              const float *d_match_xyz, int n_models, int max_matches, const int32_t *d_obj_model, const float *d_obj_pose,
+                              const int32_t *d_n_obj, int n_obj_cap, int min_points, float feat_dist, float min_score,
+                              const int32_t *d_test_offsets, const float *d_test_xyz, const float *depth_K4, const float *depth_TM12, int width,
+                              int height, const float *d_depth, const float *d_fill, float plausible_dist, float depth_fraction,
+                              float min_keypoint_fraction, uint8_t *d_keep, float *d_score, int32_t *d_out_n, int32_t *d_cluster_model,
+                              int32_t *d_cluster_offsets, int32_t *d_members, int32_t *d_surv_model, float *d_surv_pose, float *d_surv_score);
 
 // sum over a frame's models of n^2: the five similarity matrices and the merge lists of the linkage take 24 bytes per element,
 // so 2^24 elements are ~400 MB per lane (several models of the 2048-match limit of mc_cluster_linkage)
@@ -101,9 +109,10 @@ static mc_status depth_carve(mc_ctx *lane, int M, const DepthCaps &c, DepthBufs 
 }
 
 // Enqueue one frame on lane->stream; its objects go to the frame's output slots. `ev` (nullable, 6 events) brackets the five steps.
+// `df`: the FILTER / FILTER2 settings of the calling context (a lane is a context of its own and holds none).
 static mc_status depth_frame_enqueue(mc_ctx *lane, const DepthPlan &p, const char *d_meta, const DepthInputs &in, int f, int n_models, int W, int H,
-                                     const mc_depth_pipeline_params *P, int max_objects, int32_t *d_info, int32_t *d_model, float *d_pose,
-                                     float *d_score, cudaEvent_t *ev) {
+                                     const mc_depth_pipeline_params *P, const DepthFilterTable *df, int max_objects, int32_t *d_info,
+                                     int32_t *d_model, float *d_pose, float *d_score, cudaEvent_t *ev) {
 	mc_ctx *ctx = lane;
 	cudaStream_t s = lane->stream;
 	int32_t *o_info = d_info + 4 * (size_t)f;
@@ -128,6 +137,18 @@ static mc_status depth_frame_enqueue(mc_ctx *lane, const DepthPlan &p, const cha
 	link_carve(lane->link_buf.p, p.sq, p.M, p.n_slices, F);
 	const float scale = P->variant == 1 ? (float)25.0 : (float)0.100;
 	auto mark = [&](int i) { if (ev) cudaEventRecord(ev[i], s); };
+	// the FILTER step: FILTER_PROJECTION, or FILTER_PROJECTION_DEPTH with the step's test points and the frame's planes (the penalty kernel
+	// runs inside the step, so stage_ms counts it there)
+	auto filter = [&](const DepthFilterTable &t, int min_points, float feat_dist, float min_score) {
+		if (!t.d_offsets)
+			return filter_device(lane, d_off, image, xy, xyz, n_models, p.M, B.obj_model, B.obj_pose, B.st + 1, c.obj_cap, min_points, feat_dist,
+			                     min_score, B.keep, B.obj_score, B.st + 4, B.f_model, B.f_offsets, B.f_members, B.surv_model, B.surv_pose,
+			                     B.surv_score);
+		return filter_depth_device(lane, d_off, image, xy, xyz, n_models, p.M, B.obj_model, B.obj_pose, B.st + 1, c.obj_cap, min_points, feat_dist,
+		                           min_score, t.d_offsets, t.d_xyz, t.K, t.TM, W, H, F.depth, F.distance, t.plausible_sq_distance, t.depth_fraction,
+		                           t.min_keypoint_fraction, B.keep, B.obj_score, B.st + 4, B.f_model, B.f_offsets, B.f_members, B.surv_model,
+		                           B.surv_pose, B.surv_score);
+	};
 	MC_CUDA(cudaMemsetAsync(B.st, 0, 64, s));
 	mark(0);
 	// CLUSTER
@@ -144,9 +165,7 @@ static mc_status depth_frame_enqueue(mc_ctx *lane, const DepthPlan &p, const cha
 	                          B.obj_model, B.obj_pose));
 	mark(2);
 	// FILTER
-	MC_TRY(filter_device(lane, d_off, image, xy, xyz, n_models, p.M, B.obj_model, B.obj_pose, B.st + 1, c.obj_cap, P->filter_min_points,
-	                     P->filter_feature_distance, P->filter_min_score, B.keep, B.obj_score, B.st + 4, B.f_model, B.f_offsets, B.f_members,
-	                     B.surv_model, B.surv_pose, B.surv_score));
+	MC_TRY(filter(df[0], P->filter_min_points, P->filter_feature_distance, P->filter_min_score));
 	mark(3);
 	// POSE2: the surviving objects stay in the list, the objects found on their rebuilt clusters are appended
 	MC_TRY(copy_objects_device(lane, B.st + 4, B.surv_model, B.surv_pose, B.st + 1, B.obj_model, B.obj_pose));
@@ -158,9 +177,7 @@ static mc_status depth_frame_enqueue(mc_ctx *lane, const DepthPlan &p, const cha
 	                          B.obj_model, B.obj_pose));
 	mark(4);
 	// FILTER2
-	MC_TRY(filter_device(lane, d_off, image, xy, xyz, n_models, p.M, B.obj_model, B.obj_pose, B.st + 1, c.obj_cap, P->filter2_min_points,
-	                     P->filter2_feature_distance, P->filter2_min_score, B.keep, B.obj_score, B.st + 4, B.f_model, B.f_offsets, B.f_members,
-	                     B.surv_model, B.surv_pose, B.surv_score));
+	MC_TRY(filter(df[1], P->filter2_min_points, P->filter2_feature_distance, P->filter2_min_score));
 	mark(5);
 	k_depth_export<<<1, 128, 0, s>>>(B.st, p.M, B.surv_model, B.surv_pose, B.surv_score, max_objects, o_info, d_model + (size_t)f * max_objects,
 	                                 d_pose + 7 * (size_t)f * max_objects, d_score + (size_t)f * max_objects);
@@ -168,13 +185,19 @@ static mc_status depth_frame_enqueue(mc_ctx *lane, const DepthPlan &p, const cha
 	return MC_OK;
 }
 
-static mc_status depth_params_check(mc_ctx *ctx, const char *who, const mc_depth_pipeline_params *P) {
+static mc_status depth_params_check(mc_ctx *ctx, const char *who, const mc_depth_pipeline_params *P, int n_models) {
 	auto fail = [&](mc_status st, const std::string &msg) { ctx->err = std::string(who) + ": " + msg; return st; };
 	if (P->variant < 0 || P->variant > 1) return fail(MC_ERR_ARG, "variant must be 0 (back-projection) or 1 (reprojection)");
 	// with cutoff <= -1 the merge loop has no stopping point once a single cluster is left (the reference then spins on the host)
 	if (!(P->cluster_cutoff > -1.f)) return fail(MC_ERR_ARG, "cluster_cutoff must be > -1");
 	if (P->pose.n_pts_align < 1 || P->pose.n_pts_align > 8 || P->pose2.n_pts_align < 1 || P->pose2.n_pts_align > 8)
 		return fail(MC_ERR_ARG, "n_pts_align must be in 1..8");
+	for (int s = 0; s < 2; s++) {
+		const DepthFilterTable &t = ctx->depth_filter[s];
+		if (t.d_offsets && t.n_models != n_models)
+			return fail(MC_ERR_ARG, std::string(s ? "FILTER2" : "FILTER") + "'s depth-filter test points cover " + std::to_string(t.n_models) +
+			                            " models, the call has " + std::to_string(n_models) + " (mc_set_depth_filter)");
+	}
 	return MC_OK;
 }
 
@@ -186,7 +209,7 @@ static mc_status depth_plan(mc_ctx *ctx, const char *who, const int32_t *match_o
                             int32_t *frame_status = nullptr) {
 	auto fail = [&](mc_status st, const std::string &msg) { ctx->err = std::string(who) + ": " + msg; return st; };
 	if (!match_offsets || n_frames < 1 || n_models < 1 || width < 1 || height < 1 || max_objects <= 0) return fail(MC_ERR_ARG, "bad argument");
-	MC_TRY(depth_params_check(ctx, who, P));
+	MC_TRY(depth_params_check(ctx, who, P, n_models));
 	const int per_cl = P->cluster_min_pts + 1 > 1 ? P->cluster_min_pts + 1 : 1;     // a cluster has more than min_pts members
 	plans.assign((size_t)n_frames, DepthPlan());
 	meta.clear();
@@ -269,8 +292,8 @@ static mc_status depth_frames_run(mc_ctx *ctx, const char *who, const std::vecto
 	mc_status st = MC_OK;
 	for (int f = 0; f < nf && st == MC_OK; f++) {
 		mc_ctx *lane = ctx->lanes[(size_t)(f % n_lanes)];
-		st = depth_frame_enqueue(lane, plans[(size_t)f], d_meta, in, f, n_models, W, H, P, max_objects, d_info, d_model, d_pose, d_score,
-		                         stage_ms ? &ev[6 * (size_t)f] : nullptr);
+		st = depth_frame_enqueue(lane, plans[(size_t)f], d_meta, in, f, n_models, W, H, P, ctx->depth_filter, max_objects, d_info, d_model, d_pose,
+		                         d_score, stage_ms ? &ev[6 * (size_t)f] : nullptr);
 		if (st != MC_OK) ctx->err = lane->err;
 	}
 	const mc_status sj = join_lanes(ctx);
@@ -334,7 +357,7 @@ static mc_status depth_queries(mc_ctx *ctx, bool dev, const char *who, const Row
 	const int Q = frame_offsets[n_frames], n_range = frame_end - frame_begin;
 	const bool any = frame_offsets[frame_end] > frame_offsets[frame_begin];
 	if (any && (!q_xy || !q_world || !q_fill || (!dev && !src.q_desc))) return fail(MC_ERR_ARG, "bad argument");
-	MC_TRY(depth_params_check(ctx, who, P));
+	MC_TRY(depth_params_check(ctx, who, P, n_models));
 	if (!ctx->d_cams) return fail(MC_ERR_STATE, "cameras not set (mc_set_cameras)");
 	MC_CUDA(cudaSetDevice(ctx->device));
 	// per match (capacity Q, global ids): feature, image, xy, xyz, world, fill; the host entry's inputs behind them
@@ -445,6 +468,44 @@ void mc_depth_pipeline_default_params(mc_depth_pipeline_params *p) {
 	p->filter_min_points = 6; p->filter_feature_distance = 4096.f; p->filter_min_score = 2.f;     // FILTER(6, 4096, 2)
 	p->pose2 = mc_pose_params{ 64, 250, 4, 6, 8, 5.f, 2 }; p->pose2_alpha = 0.5f;          // POSE2(64, 250, 4, 6, 8, 5, 0.5)
 	p->filter2_min_points = 8; p->filter2_feature_distance = 8192.f; p->filter2_min_score = 1e-4f;  // FILTER2(8, 8192, 1e-4)
+}
+
+mc_status mc_set_depth_filter(mc_ctx *ctx, int step, const mc_depth_filter_params *p, const int32_t *test_offsets, const float *test_xyz,
+                              int n_models) {
+	if (!ctx) return MC_ERR_ARG;
+	auto fail = [&](const std::string &msg) { ctx->err = "mc_set_depth_filter: " + msg; return MC_ERR_ARG; };
+	if (step < 0 || step > 1) return fail("step must be 0 (FILTER) or 1 (FILTER2)");
+	if (p) {                                            // everything is checked before the current setting is touched
+		if (n_models < 1 || !test_offsets) return fail("bad argument");
+		if (test_offsets[0] != 0) return fail("test_offsets must start at 0");
+		for (int m = 0; m < n_models; m++)
+			if (test_offsets[m + 1] < test_offsets[m]) return fail("test_offsets must ascend");
+		if (test_offsets[n_models] > 0 && !test_xyz) return fail("test_xyz is NULL");
+	}
+	MC_CUDA(cudaSetDevice(ctx->device));
+	MC_CUDA(cudaStreamSynchronize(ctx->stream));       // the chain's last frames may still read the current table
+	DepthFilterTable t;
+	if (p) {                                            // copied once, into memory of its own (12 bytes per test point)
+		const size_t n_pts = (size_t)test_offsets[n_models];
+		cudaError_t e = cudaMalloc(&t.d_offsets, 4 * ((size_t)n_models + 1));
+		if (e == cudaSuccess) e = cudaMalloc(&t.d_xyz, 12 * std::max(n_pts, (size_t)1));
+		if (e == cudaSuccess) e = cudaMemcpyAsync(t.d_offsets, test_offsets, 4 * ((size_t)n_models + 1), cudaMemcpyHostToDevice, ctx->stream);
+		if (e == cudaSuccess && n_pts) e = cudaMemcpyAsync(t.d_xyz, test_xyz, 12 * n_pts, cudaMemcpyHostToDevice, ctx->stream);
+		if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+		if (e != cudaSuccess) {
+			cudaFree(t.d_offsets); cudaFree(t.d_xyz);
+			ctx->err = std::string("mc_set_depth_filter: ") + cudaGetErrorString(e);
+			return MC_ERR_CUDA;
+		}
+		t.n_models = n_models;
+		t.plausible_sq_distance = p->plausible_sq_distance; t.depth_fraction = p->depth_fraction; t.min_keypoint_fraction = p->min_keypoint_fraction;
+		for (int i = 0; i < 4; i++) t.K[i] = p->depth_K[i];
+		pose_tm(p->depth_pose, t.TM);                   // as mc_filter_projection_depth: the same bits
+	}
+	DepthFilterTable &cur = ctx->depth_filter[step];
+	cudaFree(cur.d_offsets); cudaFree(cur.d_xyz);
+	cur = t;
+	return MC_OK;
 }
 
 mc_status mc_process_depth_frames(mc_ctx *ctx, const int32_t *match_offsets, int n_frames, int n_models, const int32_t *match_image,

@@ -291,7 +291,8 @@ def make_depth_frame(seed: int = 1, n_models: int = 12, W: int = 640, H: int = 4
     to form a cluster) and the rest none. The depth map shows every instance as a patch at its depth over a slanted background; the
     fill-distance map has holes (> 0 = hallucinated depth). A model's matches come in random (query) order, instances interleaved.
     Returns dict(match_offsets[n_models+1], match_image, match_xy, match_xyz, match_world, match_fill, depth[H,W], fill_distance[H,W],
-    K, cam_pose, gt_model[V], gt_pose[V,7], junk_models)."""
+    K, cam_pose, gt_model[V], gt_pose[V,7], junk_models, model_offsets[n_models+1], model_xyz) — the last two are every model's keypoints
+    (model-major), where FILTER_PROJECTION_DEPTH draws its test points from."""
     rng = np.random.default_rng(BASE_SEED + 6151 * seed)
     K = K_DEPTH
     depth = (2.2 + 0.0006 * np.arange(W)[None, :] + 0.0004 * np.arange(H)[:, None]).astype(np.float32)
@@ -350,7 +351,8 @@ def make_depth_frame(seed: int = 1, n_models: int = 12, W: int = 640, H: int = 4
     return dict(match_offsets=np.array(offs, np.int32), match_image=np.zeros(M, np.int32), match_xy=cat(xy, 2), match_xyz=cat(xyz, 3),
                 match_world=cat(world, 3), match_fill=fill, depth=depth, fill_distance=fill_map, K=K.copy(), cam_pose=CAM_IDENTITY.copy(),
                 gt_model=np.array(gt_model, np.int32), gt_pose=np.stack(gt_pose) if gt_pose else np.zeros((0, 7), np.float32),
-                junk_models=np.sort(junk).astype(np.int32))
+                junk_models=np.sort(junk).astype(np.int32), model_offsets=(pts_per_model * np.arange(n_models + 1)).astype(np.int32),
+                model_xyz=np.concatenate(model_pts).astype(np.float32))
 
 
 def stack_depth_frames(frames):
