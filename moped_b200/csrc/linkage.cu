@@ -195,7 +195,8 @@ __global__ void __launch_bounds__(kLinkThreads) k_link_max(const LinkSlice *__re
 	__syncthreads();
 	if (threadIdx.x == 0) {
 		for (int w = 1; w < kLinkThreads / 32; w++) m = fmaxf(m, s_m[w]);
-		// values are >= 0 here (sums and products of exponentials): the int compare of the bit patterns orders them like floats
+		// m is never NaN: `v > m` and fmaxf skip the NaN of duplicate matches (get3DFilterK's 0/0). It is -1 (a negative int, which
+		// loses to the zeroed slot) or a sum / product of exponentials >= 0, whose int bit patterns order like the floats
 		atomicMax((int *)out_max, __float_as_int(m));
 	}
 }
@@ -264,7 +265,7 @@ __global__ void __launch_bounds__(kLinkThreads, 1) k_link_agglomerate(const Link
 	for (;;) {
 		const int nv = s_nv, r = s_r;      // r = position of the merged-away index in the list, or -1
 		// argmax over the pairs the reference's double loop visits: position a (not r, not r+1: erase-then-++ skips it) with every later
-		// position b; strict > keeps the first maximum in (a, b) order
+		// position b; strict > keeps the first maximum in (a, b) order and, like the reference's, never picks a NaN (duplicate matches)
 		float best = -1;
 		int ba = 0x7fffffff, bb = 0x7fffffff;
 		for (int a = tid; a < nv; a += blockDim.x) {

@@ -7,6 +7,8 @@
 //
 // Invariant per live list position a (list L of cluster ids, ascending; posOf = inverse):
 //     best[L[a]] = max over later positions b of D[L[a]][L[b]],  arg[L[a]] = the id at the SMALLEST such b   (strict > in scan order)
+// NaN similarities (duplicate matches) never win a strict >, so the max skips them like the reference's scan: best is never NaN
+// (-1 when a row has no finite entry left), and every repair below keeps it so.
 //
 // Written for a block of W threads as a sequence of phases (`blk.each(f)`: __syncthreads(); f(tid); __syncthreads(); on the
 // device, a loop over the threads on the host), so that tests/cpp/linkage_host.cpp can compile this very source with g++ and
@@ -158,7 +160,8 @@ LKX_FN void agglomerate_average(const Block<W> &blk, const State &s, const float
 				const int i = s.L[pos];
 				const float v = s.D[(size_t)i * n + p1];
 				if (s.arg[i] == p1) {
-					if (v < s.oldcol[i]) recompute_row(s, pos, nLn);
+					// NaN (0/0 of the 3-D filter at duplicate matches) never wins a compare: rescan instead of caching it
+					if (!(v >= s.oldcol[i])) recompute_row(s, pos, nLn);
 					else s.best[i] = v;
 				} else if (v > s.best[i] || (v == s.best[i] && s.arg[i] >= 0 && s.posOf[s.arg[i]] > pos1)) {
 					s.best[i] = v; s.arg[i] = p1;

@@ -230,6 +230,20 @@ def make_linkage_scene(seed: int = 1, n_per=(300, 200), n_out: int = 100, halluc
     return xy[perm], xyz[perm], world[perm], depth, dist
 
 
+def duplicate_matches(arrays, k: int, seed: int = 0):
+    """Per-match arrays (same length) with k of their rows overwritten by copies of k other rows: what SIFT's secondary orientation
+    peaks give, two matches of one model with the same pixel, model point and world point. Every copied pair makes get3DFilterK's
+    |dm - dw| / dm a 0/0, i.e. two NaN entries of the similarity matrix. Returns new arrays."""
+    n = len(arrays[0])
+    assert 2 * k <= n, (k, n)
+    perm = np.random.default_rng(BASE_SEED + 7919 * seed).permutation(n)
+    dst, src = perm[:k], perm[k:2 * k]
+    out = [np.array(a, copy=True) for a in arrays]
+    for a in out:
+        a[dst] = a[src]
+    return out
+
+
 def make_filter_depth_scene(seed: int = 1, n_models: int = 3, pts_per_model: int = 120, W: int = 320, H: int = 240, n_wrong: int = 2):
     """A frame state for moped3d's FILTER_PROJECTION_DEPTH step (inputs only): `n_models` box-like models (keypoints on a 12 cm cube), each
     seen once at a true pose in front of a Kinect-like camera, with a depth map that shows the objects as patches at their true depth over a
@@ -284,7 +298,8 @@ def make_filter_depth_scene(seed: int = 1, n_models: int = 3, pts_per_model: int
                 obj_model=np.array(obj_model, np.int32)[order], obj_pose=np.stack(obj_pose).astype(np.float32)[order])
 
 
-def make_depth_frame(seed: int = 1, n_models: int = 12, W: int = 640, H: int = 480, pts_per_model: int = 160, outlier_frac: float = 0.15):
+def make_depth_frame(seed: int = 1, n_models: int = 12, W: int = 640, H: int = 480, pts_per_model: int = 160, outlier_frac: float = 0.15,
+                     inst_matches=(40, 71), dup_frac: float = 0.0):
     """One 640x480 RGB-D frame of moped3d's recognition steps in the C-ABI layout of mc_process_depth_frames (FrameData after DEPTHPROP,
     identity camera, Kinect-like K): about a third of the `n_models` models are seen once or twice at planted poses (40-70 matched
     keypoints each, `outlier_frac` of them at random pixels with wrong depth), a few models get a handful of junk matches (3-6, too few
@@ -292,7 +307,9 @@ def make_depth_frame(seed: int = 1, n_models: int = 12, W: int = 640, H: int = 4
     fill-distance map has holes (> 0 = hallucinated depth). A model's matches come in random (query) order, instances interleaved.
     Returns dict(match_offsets[n_models+1], match_image, match_xy, match_xyz, match_world, match_fill, depth[H,W], fill_distance[H,W],
     K, cam_pose, gt_model[V], gt_pose[V,7], junk_models, model_offsets[n_models+1], model_xyz) — the last two are every model's keypoints
-    (model-major), where FILTER_PROJECTION_DEPTH draws its test points from."""
+    (model-major), where FILTER_PROJECTION_DEPTH draws its test points from.
+    `inst_matches` = [lo, hi) of the matched keypoints per instance (at most `pts_per_model`); with `dup_frac` > 0, that fraction of every
+    model's matches are copies of other matches of the model (duplicate_matches: same pixel, model point, world point and fill)."""
     rng = np.random.default_rng(BASE_SEED + 6151 * seed)
     K = K_DEPTH
     depth = (2.2 + 0.0006 * np.arange(W)[None, :] + 0.0004 * np.arange(H)[:, None]).astype(np.float32)
@@ -317,7 +334,7 @@ def make_depth_frame(seed: int = 1, n_models: int = 12, W: int = 640, H: int = 4
             t = np.array([(cx - K[2]) / K[0] * z, (cy - K[3]) / K[1] * z, z])
             q = rng.normal(size=4)
             q /= np.linalg.norm(q)
-            n = int(rng.integers(40, 71))
+            n = int(rng.integers(*inst_matches))
             X = model_pts[m][rng.choice(pts_per_model, n, replace=False)]
             cam3 = X @ quat_to_R(q).T + t
             uv = np.stack([cam3[:, 0] / cam3[:, 2] * K[0] + K[2], cam3[:, 1] / cam3[:, 2] * K[1] + K[3]], 1) + rng.normal(0, 0.4, (n, 2))
@@ -348,8 +365,16 @@ def make_depth_frame(seed: int = 1, n_models: int = 12, W: int = 640, H: int = 4
     M = offs[-1]
     cat = lambda a, k: (np.concatenate(a) if a else np.zeros((0, k))).astype(np.float32)
     fill = np.where(rng.random(M) < 0.7, 0.0, rng.uniform(0, 0.3, M)).astype(np.float32)
-    return dict(match_offsets=np.array(offs, np.int32), match_image=np.zeros(M, np.int32), match_xy=cat(xy, 2), match_xyz=cat(xyz, 3),
-                match_world=cat(world, 3), match_fill=fill, depth=depth, fill_distance=fill_map, K=K.copy(), cam_pose=CAM_IDENTITY.copy(),
+    xy, xyz, world = cat(xy, 2), cat(xyz, 3), cat(world, 3)
+    if dup_frac > 0:
+        for m in range(n_models):
+            lo, hi = offs[m], offs[m + 1]
+            k = int(round(dup_frac * (hi - lo)))
+            if k and 2 * k <= hi - lo:
+                xy[lo:hi], xyz[lo:hi], world[lo:hi], fill[lo:hi] = duplicate_matches((xy[lo:hi], xyz[lo:hi], world[lo:hi], fill[lo:hi]), k,
+                                                                                     seed=6151 * seed + m)
+    return dict(match_offsets=np.array(offs, np.int32), match_image=np.zeros(M, np.int32), match_xy=xy, match_xyz=xyz,
+                match_world=world, match_fill=fill, depth=depth, fill_distance=fill_map, K=K.copy(), cam_pose=CAM_IDENTITY.copy(),
                 gt_model=np.array(gt_model, np.int32), gt_pose=np.stack(gt_pose) if gt_pose else np.zeros((0, 7), np.float32),
                 junk_models=np.sort(junk).astype(np.int32), model_offsets=(pts_per_model * np.arange(n_models + 1)).astype(np.int32),
                 model_xyz=np.concatenate(model_pts).astype(np.float32))

@@ -67,11 +67,12 @@ def pose_step(fr, clusters, cams, params, alpha, seed, objects, variant=0):
             objects.append((m, p.copy()))
 
 
-def frame(fr, variant=0, seeds=(1, 2), cluster=CLUSTER, pose1=POSE1, pose2=POSE2, filter1=FILTER1, filter2=FILTER2):
-    """One make_depth_frame frame through the five steps -> dict(model, pose, score, clusters)."""
+def frame(fr, variant=0, seeds=(1, 2), cluster=CLUSTER, pose1=POSE1, pose2=POSE2, filter1=FILTER1, filter2=FILTER2, clusters=None):
+    """One make_depth_frame frame through the five steps -> dict(model, pose, score, clusters). `clusters` (optional, as cluster_step
+    returns them) replaces the CLUSTER step: POSE..FILTER2 alone."""
     cams = oracle.cameras(fr["K"], fr["cam_pose"])
     matches = dict(offsets=fr["match_offsets"], image=fr["match_image"], xy=fr["match_xy"], xyz=fr["match_xyz"])
-    cl = cluster_step(fr, cluster)
+    cl = cluster_step(fr, cluster) if clusters is None else clusters
     objects = []
     pose_step(fr, cl, cams, pose1, ALPHA, seeds[0], objects, variant)
     objects, cl2, _ = filter_step(matches, cams, objects, filter1)

@@ -240,10 +240,10 @@ def test_moped3d_chain_after_cluster_inside_its_own_pipeline(tmp_path):
 
 def test_cached_agglomeration_equals_default_kernel(gpu_ctx):
     """mc_set_option("linkage_cached", 1) (the default): the cached-row-maximum agglomeration (linkage_cached.cuh) gives the oracle's clusters —
-    and therefore the default kernel's — on the oracle's own similarity matrices, on tie-heavy quantised ones and on a 600-match
-    block-structured one (the host-emulated source already does: tests/test_linkage_cached_host.py)."""
+    and therefore the default kernel's — on the oracle's own similarity matrices, on tie-heavy quantised ones, on a 600-match
+    block-structured one and on matrices with NaN entries (the host-emulated source already does: tests/test_linkage_cached_host.py)."""
     from test_oracle3d_linkage import make_scene
-    from test_linkage_cached_host import random_similarity
+    from test_linkage_cached_host import duplicate_scene_similarity, nan_sprinkled, random_similarity
     rng = np.random.default_rng(2)
     mats = []
     for seed in range(3):
@@ -256,6 +256,13 @@ def test_cached_agglomeration_equals_default_kernel(gpu_ctx):
     K = np.where((g[:, None] == g[None, :]) & (g[:, None] < groups), 0.6 + 0.4 * rng.random((n, n)), 0.05 * rng.random((n, n))).astype(np.float32)
     K = np.maximum(K, K.T); np.fill_diagonal(K, 1.0)
     mats.append((K, 0.1, 7))
+    # NaN entries: the 600-match linkage scene with duplicated matches (get3DFilterK's 0/0), random matrices with NaN pairs
+    for seed, (n_dup, use3d) in enumerate(((30, 2), (60, 1), (5, 2))):
+        mats.append((duplicate_scene_similarity(seed, n_dup, use3d), 0.1, 7))
+    for case in range(6):
+        K = nan_sprinkled(rng, random_similarity(rng, int(rng.integers(200, 330)), case % 2 == 1), (0.001, 0.01, 0.1)[case % 3])
+        mats.append((K, float(rng.choice([0.2, 0.5, 0.75])), int(rng.integers(0, 4))))
+    assert all(np.isnan(m[0]).any() for m in mats[-9:])
     try:
         for cached in (1, 0):                       # 1 is the default since it was timed on B200 (profiles/linkage_bench_r2.jsonl); 0 = the O(n^2)-scan kernel
             gpu_ctx.set_option("linkage_cached", cached)

@@ -2,7 +2,8 @@
 mc_set_option("linkage_cached")) compiled by g++ with the 256 threads of its block emulated by a loop (tests/cpp/linkage_host.cpp),
 against the oracle's hierarchicalCluster (oracle/moped_linkage_oracle.c, bit-identical to the strict build of moped3d's
 CLUSTER_LINKAGE_CPU): identical clusters on tie-heavy quantised matrices (where the reference's scan-order tie rule and its
-erase-and-skip quirk decide) and on real-valued ones, threads of a phase visited in ascending and in descending order. The CUDA
+erase-and-skip quirk decide), on real-valued ones and on matrices with NaN entries (duplicate matches make get3DFilterK a 0/0; the
+reference's strict > never merges on a NaN), threads of a phase visited in ascending and in descending order. The CUDA
 kernel itself is checked on the device by tests/test_gpu_depth_pose.py::test_cached_agglomeration_equals_default_kernel."""
 import ctypes as C
 import os
@@ -53,6 +54,25 @@ def random_similarity(rng, n, quantised):
     return K
 
 
+def nan_sprinkled(rng, K, frac):
+    """K with a fraction `frac` of its off-diagonal pairs set to NaN on both sides"""
+    K = K.copy()
+    n = len(K)
+    i, j = np.triu_indices(n, 1)
+    pick = rng.random(len(i)) < frac
+    K[i[pick], j[pick]] = np.nan; K[j[pick], i[pick]] = np.nan
+    return K
+
+
+def duplicate_scene_similarity(seed, n_dup, use3d):
+    """the similarity matrix of make_linkage_scene(seed) with n_dup of its matches duplicated: 2 * n_dup NaN entries for
+    use3d 1 and 2"""
+    from moped_b200 import synth
+    xy, xyz, world, depth, dist = synth.make_linkage_scene(seed)
+    xy, xyz, world = synth.duplicate_matches((xy, xyz, world), n_dup, seed)
+    return oracle.linkage_similarity(xy, xyz, world, depth, dist, use3d_filter=use3d)
+
+
 def test_cached_agglomeration_equals_oracle(host_lib):
     rng = np.random.default_rng(0)
     merged = 0
@@ -67,6 +87,18 @@ def test_cached_agglomeration_equals_oracle(host_lib):
             assert np.array_equal(oo, co) and np.array_equal(om, cm), (case, n, cutoff, min_pts, order)
         merged += n - (len(oo) - 1)
     assert merged > 2000
+    # NaN similarities: the 600-match scene with duplicated matches, and random matrices with NaN pairs
+    nan_cases = [(duplicate_scene_similarity(seed, 5 + 11 * (seed % 6), 1 + seed % 2), 0.1, 7) for seed in range(8)]
+    for case in range(60):
+        n = int(rng.integers(2, 321))
+        K = nan_sprinkled(rng, random_similarity(rng, n, case % 2 == 1), float(rng.choice([0.001, 0.01, 0.03, 0.1])))
+        nan_cases.append((K, float(rng.choice([0.1, 0.2, 0.5, 0.75])), int(rng.integers(0, 4))))
+    assert sum(np.isnan(K).any() for K, _, _ in nan_cases) >= 50
+    for case, (K, cutoff, min_pts) in enumerate(nan_cases):
+        oo, om = oracle.linkage_agglomerate(K, cutoff, min_pts, 1)
+        for order in (0, 1):
+            co, cm = run_host(host_lib, K, cutoff, min_pts, order)
+            assert np.array_equal(oo, co) and np.array_equal(om, cm), ("nan", case, len(K), cutoff, min_pts, order)
 
 
 def test_cached_agglomeration_on_clustered_scenes(host_lib):
