@@ -183,19 +183,18 @@ mc_status match_adaptive_frames(mc_ctx *ctx, bool dev, const char *who, const Ro
 		return MC_OK;
 	}
 	MC_CUDA(cudaSetDevice(ctx->device));
-	const size_t planes = (size_t)width * height * n_range;
-	size_t off = 0;
-	auto take = [&](size_t bytes) { const size_t o = off; off += (bytes + 255) & ~(size_t)255; return o; };
-	const size_t o_depth = dev ? 0 : take(sizeof(float) * planes), o_fill = dev ? 0 : take(sizeof(float) * planes);
-	const size_t o_curves = take(sizeof(mc_adaptive_model) * (size_t)n_models), o_fo = take(sizeof(int32_t) * (n_range + 1ull));
-	const size_t o_fd = take(sizeof(FrameDesc) * (size_t)n_range), o_moff = take(sizeof(int32_t) * (size_t)stride * n_range);
-	// the compaction's overflow flags, then (merge) the flags of frames with a row outside the tables: one copy to the host
-	const size_t o_status = take(sizeof(int32_t) * 2 * (size_t)n_range), o_nobj = take(sizeof(int32_t) * (size_t)n_range);
-	const size_t o_acc_list = take(sizeof(int32_t) * (size_t)Q), o_mrow = take(sizeof(int32_t) * (size_t)Q);
-	const size_t o_mfeat = dev ? 0 : take(sizeof(int32_t) * (size_t)Q), o_mimg = dev ? 0 : take(sizeof(int32_t) * (size_t)Q);
-	const size_t o_mxy = dev ? 0 : take(sizeof(float) * 2 * (size_t)Q), o_mxyz = dev ? 0 : take(sizeof(float) * 3 * (size_t)Q);
-	MC_TRY(reserve(ctx, ctx->scratch[19], off));
-	char *b = (char *)ctx->scratch[19].p;
+	const size_t planes = (size_t)width * height * n_range, q = (size_t)Q, nr = (size_t)n_range;
+	mc_adaptive_model *d_curves; FrameDesc *d_fd;
+	int32_t *d_fo, *d_moff, *d_status, *d_nobj, *d_acc_list, *d_mrow, *up_feat = nullptr, *up_mimg = nullptr;
+	float *up_depth = nullptr, *up_fill = nullptr, *up_mxy = nullptr, *up_mxyz = nullptr;
+	MC_TRY(carve_scratch(ctx, ctx->scratch[kScrAdaptive], [&](Carve &c) {
+		if (!dev) { c.take(up_depth, planes); c.take(up_fill, planes); }
+		c.take(d_curves, n_models); c.take(d_fo, nr + 1); c.take(d_fd, nr); c.take(d_moff, (size_t)stride * nr);
+		// the compaction's overflow flags, then (merge) the flags of frames with a row outside the tables: one copy to the host
+		c.take(d_status, 2 * nr); c.take(d_nobj, nr);
+		c.take(d_acc_list, q); c.take(d_mrow, q);
+		if (!dev) { c.take(up_feat, q); c.take(up_mimg, q); c.take(up_mxy, 2 * q); c.take(up_mxyz, 3 * q); }
+	}));
 	const float *d_q = src.q_desc, *d_xy = q_xy, *d_depth = depth, *d_fill = fill_distance;
 	const int32_t *d_img = q_image;
 	int32_t *d_feat = match_feature, *d_mimg = match_image;
@@ -210,11 +209,11 @@ mc_status match_adaptive_frames(mc_ctx *ctx, bool dev, const char *who, const Ro
 			MC_CUDA(cudaMemcpyAsync(ctx->q_image.p, q_image, sizeof(int32_t) * (size_t)Q, cudaMemcpyHostToDevice, ctx->stream));
 			d_img = (const int32_t *)ctx->q_image.p;
 		}
-		MC_CUDA(cudaMemcpyAsync(b + o_depth, depth, sizeof(float) * planes, cudaMemcpyHostToDevice, ctx->stream));
-		MC_CUDA(cudaMemcpyAsync(b + o_fill, fill_distance, sizeof(float) * planes, cudaMemcpyHostToDevice, ctx->stream));
+		MC_CUDA(cudaMemcpyAsync(up_depth, depth, sizeof(float) * planes, cudaMemcpyHostToDevice, ctx->stream));
+		MC_CUDA(cudaMemcpyAsync(up_fill, fill_distance, sizeof(float) * planes, cudaMemcpyHostToDevice, ctx->stream));
 		d_q = (const float *)ctx->q_desc.p; d_xy = (const float *)ctx->q_xy.p;
-		d_depth = (const float *)(b + o_depth); d_fill = (const float *)(b + o_fill);
-		d_feat = (int32_t *)(b + o_mfeat); d_mimg = (int32_t *)(b + o_mimg); d_mxy = (float *)(b + o_mxy); d_mxyz = (float *)(b + o_mxyz);
+		d_depth = up_depth; d_fill = up_fill;
+		d_feat = up_feat; d_mimg = up_mimg; d_mxy = up_mxy; d_mxyz = up_mxyz;
 	}
 	// per-feature results: the caller's device arrays when given, the context's otherwise
 	int32_t *d_nn_row = dev ? nn_row : nullptr;
@@ -223,7 +222,6 @@ mc_status match_adaptive_frames(mc_ctx *ctx, bool dev, const char *who, const Ro
 	if (!d_nn_row) { MC_TRY(reserve(ctx, ctx->nn_row, sizeof(int32_t) * 2 * (size_t)Q)); d_nn_row = (int32_t *)ctx->nn_row.p; }
 	if (!d_nn_dist) { MC_TRY(reserve(ctx, ctx->nn_dist, sizeof(float) * 2 * (size_t)Q)); d_nn_dist = (float *)ctx->nn_dist.p; }
 	if (!d_acc) { MC_TRY(reserve(ctx, ctx->accepted, (size_t)Q)); d_acc = (uint8_t *)ctx->accepted.p; }
-	const int32_t *d_fo = (const int32_t *)(b + o_fo);
 	std::vector<FrameDesc> descs((size_t)n_range);
 	for (int f = 0; f < n_range; f++) {
 		FrameDesc &d = descs[(size_t)f];
@@ -232,14 +230,13 @@ mc_status match_adaptive_frames(mc_ctx *ctx, bool dev, const char *who, const Ro
 		d.nn_row = d_nn_row + 2 * (size_t)q0; d.accepted = d_acc + q0; d.q_xy = d_xy + 2 * (size_t)q0; d.q_image = d_img ? d_img + q0 : nullptr;
 		d.Q = range_offsets[f + 1] - q0;
 	}
-	MC_CUDA(cudaMemcpyAsync(b + o_curves, models, sizeof(mc_adaptive_model) * (size_t)n_models, cudaMemcpyHostToDevice, ctx->stream));
-	MC_CUDA(cudaMemcpyAsync(b + o_fo, range_offsets, sizeof(int32_t) * (n_range + 1ull), cudaMemcpyHostToDevice, ctx->stream));
-	MC_CUDA(cudaMemcpyAsync(b + o_fd, descs.data(), sizeof(FrameDesc) * (size_t)n_range, cudaMemcpyHostToDevice, ctx->stream));
+	MC_CUDA(cudaMemcpyAsync(d_curves, models, sizeof(mc_adaptive_model) * (size_t)n_models, cudaMemcpyHostToDevice, ctx->stream));
+	MC_CUDA(cudaMemcpyAsync(d_fo, range_offsets, sizeof(int32_t) * (n_range + 1ull), cudaMemcpyHostToDevice, ctx->stream));
+	MC_CUDA(cudaMemcpyAsync(d_fd, descs.data(), sizeof(FrameDesc) * (size_t)n_range, cudaMemcpyHostToDevice, ctx->stream));
 	AdaptiveParams P;
 	P.maximum_depth = maximum_depth; P.default_depth = default_depth; P.cauchy_scale = cauchy_scale;
 	const dim3 grid((unsigned)((q_max + 255) / 256), (unsigned)n_range);
-	const mc_adaptive_model *d_curves = (const mc_adaptive_model *)(b + o_curves);
-	int32_t *d_moff = (int32_t *)(b + o_moff), *d_status = (int32_t *)(b + o_status), *d_bad = d_status + n_range;
+	int32_t *d_bad = d_status + n_range;
 	if (ev) MC_CUDA(cudaEventRecord(ev[0], ctx->stream));
 	if (merge) {
 		MC_CUDA(cudaMemsetAsync(d_bad, 0, sizeof(int32_t) * (size_t)n_range, ctx->stream));
@@ -253,9 +250,8 @@ mc_status match_adaptive_frames(mc_ctx *ctx, bool dev, const char *who, const Ro
 		                                                       ctx->table_base, d_curves, n_models, P, d_acc);
 	}
 	MC_LAUNCH_CHECK();
-	MC_TRY(match_compact_frames_device(ctx, (const FrameDesc *)(b + o_fd), d_fo, n_range, n_models, (int32_t *)(b + o_acc_list), d_moff, d_feat,
-	                                   (int32_t *)(b + o_mrow), d_mimg, d_mxy, d_mxyz, d_status, (int32_t *)(b + o_nobj), q_world, q_fill,
-	                                   match_world, match_fill));
+	MC_TRY(match_compact_frames_device(ctx, d_fd, d_fo, n_range, n_models, d_acc_list, d_moff, d_feat, d_mrow, d_mimg, d_mxy, d_mxyz, d_status, d_nobj,
+	                                   q_world, q_fill, match_world, match_fill));
 	if (ev) MC_CUDA(cudaEventRecord(ev[1], ctx->stream));
 	// frame-local offsets and frame flags -> host; the host entry also takes the per-match and per-feature arrays
 	const size_t h_moff_bytes = sizeof(int32_t) * (size_t)stride * n_range, h_flag_bytes = sizeof(int32_t) * (merge ? 2 : 1) * (size_t)n_range;
@@ -336,21 +332,19 @@ mc_status mc_match_adaptive(mc_ctx *ctx, const float *q_desc, const float *q_xy,
 	MC_TRY(reserve(ctx, ctx->nn_dist, sizeof(float) * 2 * (size_t)Q));
 	MC_TRY(reserve(ctx, ctx->accepted, (size_t)Q));
 	MC_TRY(reserve(ctx, ctx->q_xy, sizeof(float) * 2 * (size_t)Q));
-	const size_t o_fill = (sizeof(float) * px + 255) & ~(size_t)255, o_curves = 2 * o_fill;
-	MC_TRY(reserve(ctx, ctx->scratch[19], o_curves + sizeof(mc_adaptive_model) * (size_t)n_models));
-	char *b = (char *)ctx->scratch[19].p;
+	float *d_depth, *d_fill; mc_adaptive_model *d_curves;
+	MC_TRY(carve_scratch(ctx, ctx->scratch[kScrAdaptive], [&](Carve &c) { c.take(d_depth, px); c.take(d_fill, px); c.take(d_curves, n_models); }));
 	MC_CUDA(cudaMemcpyAsync(ctx->q_desc.p, q_desc, sizeof(float) * (size_t)Q * ctx->D, cudaMemcpyHostToDevice, ctx->stream));
 	MC_CUDA(cudaMemcpyAsync(ctx->q_xy.p, q_xy, sizeof(float) * 2 * (size_t)Q, cudaMemcpyHostToDevice, ctx->stream));
-	MC_CUDA(cudaMemcpyAsync(b, depth, sizeof(float) * px, cudaMemcpyHostToDevice, ctx->stream));
-	MC_CUDA(cudaMemcpyAsync(b + o_fill, fill_distance, sizeof(float) * px, cudaMemcpyHostToDevice, ctx->stream));
-	MC_CUDA(cudaMemcpyAsync(b + o_curves, models, sizeof(mc_adaptive_model) * (size_t)n_models, cudaMemcpyHostToDevice, ctx->stream));
+	MC_CUDA(cudaMemcpyAsync(d_depth, depth, sizeof(float) * px, cudaMemcpyHostToDevice, ctx->stream));
+	MC_CUDA(cudaMemcpyAsync(d_fill, fill_distance, sizeof(float) * px, cudaMemcpyHostToDevice, ctx->stream));
+	MC_CUDA(cudaMemcpyAsync(d_curves, models, sizeof(mc_adaptive_model) * (size_t)n_models, cudaMemcpyHostToDevice, ctx->stream));
 	// the fixed-ratio flags of the plain matcher are overwritten by the adaptive kernel
 	MC_TRY(match_device(ctx, (const float *)ctx->q_desc.p, Q, 1.0f, MC_MATCH_TENSOR, (int32_t *)ctx->nn_row.p, (float *)ctx->nn_dist.p, (uint8_t *)ctx->accepted.p));
 	AdaptiveParams P;
 	P.maximum_depth = maximum_depth; P.default_depth = default_depth; P.cauchy_scale = cauchy_scale;
 	k_match_finalize_adaptive<<<(Q + 255) / 256, 256, 0, ctx->stream>>>((const int32_t *)ctx->nn_row.p, (const float *)ctx->nn_dist.p, Q, nullptr, (const float *)ctx->q_xy.p,
-	                                                                  (const float *)b, (const float *)(b + o_fill), width, height, ctx->d_model_of_row,
-	                                                                  ctx->table_base, (const mc_adaptive_model *)(b + o_curves), n_models, P,
+	                                                                  d_depth, d_fill, width, height, ctx->d_model_of_row, ctx->table_base, d_curves, n_models, P,
 	                                                                  (uint8_t *)ctx->accepted.p);
 	MC_LAUNCH_CHECK();
 	MC_CUDA(cudaMemcpyAsync(nn_row, ctx->nn_row.p, sizeof(int32_t) * 2 * (size_t)Q, cudaMemcpyDeviceToHost, ctx->stream));

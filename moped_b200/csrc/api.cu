@@ -53,13 +53,6 @@ mc_status process_frames_host(mc_ctx *ctx, const float *d_q, const float *d_qxy,
                               const mc_pipeline_params *P, int max_objects, int32_t *n_objects, int32_t *obj_model, float *obj_pose, float *obj_score,
                               int32_t *frame_info, float *stage_ms);
 
-// bump allocator over one grow-only device buffer, for the temporaries of a host-buffer call
-struct Arena {
-	mc_ctx *ctx; char *base = nullptr; size_t off = 0, cap = 0;
-	std::vector<size_t> sizes;
-	size_t plan(size_t bytes) { size_t o = off; off += (bytes + 255) & ~(size_t)255; return o; }
-};
-
 template <typename T> static mc_status h2d(mc_ctx *ctx, T *dst, const T *src, size_t n) {
 	if (n == 0) return MC_OK;
 	MC_CUDA(cudaMemcpyAsync(dst, src, n * sizeof(T), cudaMemcpyHostToDevice, ctx->stream));
@@ -388,23 +381,23 @@ mc_status mc_cluster_meanshift(mc_ctx *ctx, const int32_t *match_offsets, const 
 	}
 	MC_CUDA(cudaSetDevice(ctx->device));
 	const int M = match_offsets[n_models];
-	Arena A; A.ctx = ctx;
-	const size_t o_off = A.plan(4ull * (n_models + 1)), o_img = A.plan(4ull * (M + 1)), o_xy = A.plan(8ull * (M + 1));
-	const size_t o_n = A.plan(64), o_cm = A.plan(4ull * (M + 2)), o_co = A.plan(4ull * (M + 2)), o_mem = A.plan(4ull * (M + 2));
-	MC_TRY(reserve(ctx, ctx->scratch[11], A.off));
-	char *b = (char *)ctx->scratch[11].p;
-	MC_TRY(h2d(ctx, (int32_t *)(b + o_off), match_offsets, (size_t)n_models + 1));
-	MC_TRY(h2d(ctx, (int32_t *)(b + o_img), match_image, (size_t)M));
-	MC_TRY(h2d(ctx, (float *)(b + o_xy), match_xy, 2 * (size_t)M));
-	MC_TRY(cluster_device(ctx, (int32_t *)(b + o_off), (int32_t *)(b + o_img), (float *)(b + o_xy), n_models, n_images, M, radius, merge, min_pts,
-	                      max_iterations, (int32_t *)(b + o_n), (int32_t *)(b + o_cm), (int32_t *)(b + o_co), (int32_t *)(b + o_mem)));
+	const size_t m = (size_t)M;
+	int32_t *d_off, *d_img, *d_n, *d_cm, *d_co, *d_mem; float *d_xy;
+	MC_TRY(carve_scratch(ctx, ctx->scratch[kScrHostCluster], [&](Carve &c) {
+		c.take(d_off, (size_t)n_models + 1); c.take(d_img, m + 1); c.take(d_xy, 2 * (m + 1));
+		c.take(d_n, 16); c.take(d_cm, m + 2); c.take(d_co, m + 2); c.take(d_mem, m + 2);
+	}));
+	MC_TRY(h2d(ctx, d_off, match_offsets, (size_t)n_models + 1));
+	MC_TRY(h2d(ctx, d_img, match_image, m));
+	MC_TRY(h2d(ctx, d_xy, match_xy, 2 * m));
+	MC_TRY(cluster_device(ctx, d_off, d_img, d_xy, n_models, n_images, M, radius, merge, min_pts, max_iterations, d_n, d_cm, d_co, d_mem));
 	int32_t hn[2] = { 0, 0 };
-	MC_TRY(d2h(ctx, hn, (const int32_t *)(b + o_n), 2));
+	MC_TRY(d2h(ctx, hn, d_n, 2));
 	MC_CUDA(cudaStreamSynchronize(ctx->stream));
 	*n_clusters = hn[0];
-	MC_TRY(d2h(ctx, cluster_model, (const int32_t *)(b + o_cm), (size_t)hn[0]));
-	MC_TRY(d2h(ctx, cluster_offsets, (const int32_t *)(b + o_co), (size_t)hn[0] + 1));
-	MC_TRY(d2h(ctx, members, (const int32_t *)(b + o_mem), (size_t)hn[1]));
+	MC_TRY(d2h(ctx, cluster_model, d_cm, (size_t)hn[0]));
+	MC_TRY(d2h(ctx, cluster_offsets, d_co, (size_t)hn[0] + 1));
+	MC_TRY(d2h(ctx, members, d_mem, (size_t)hn[1]));
 	MC_CUDA(cudaStreamSynchronize(ctx->stream));
 	return MC_OK;
 }
@@ -435,37 +428,35 @@ mc_status mc_pose_hypotheses(mc_ctx *ctx, const int32_t *cluster_offsets, int n_
 		}
 		mask_off[h + 1] = mask_off[h] + n;
 	}
-	Arena A; A.ctx = ctx;
-	const size_t o_co = A.plan(4ull * (n_clusters + 1)), o_xy = A.plan(8ull * M), o_xyz = A.plan(12ull * M), o_im = A.plan(4ull * M);
-	const size_t o_hc = A.plan(4ull * n_hyp), o_sp = A.plan(4ull * n_hyp * na), o_iq = A.plan(16ull * n_hyp), o_mo = A.plan(8ull * (n_hyp + 1));
-	const size_t o_ni = A.plan(4ull * n_hyp), o_pl = A.plan(28ull * n_hyp), o_pr = A.plan(28ull * n_hyp), o_le = A.plan(8ull * n_hyp);
-	const size_t o_mask = A.plan(inlier_mask ? (size_t)mask_off[n_hyp] + 1 : 1);
-	MC_TRY(reserve(ctx, ctx->scratch[12], A.off));
-	char *b = (char *)ctx->scratch[12].p;
-	MC_TRY(h2d(ctx, (int32_t *)(b + o_co), cluster_offsets, (size_t)n_clusters + 1));
-	MC_TRY(h2d(ctx, (float *)(b + o_xy), pt_xy, 2 * (size_t)M));
-	MC_TRY(h2d(ctx, (float *)(b + o_xyz), pt_xyz, 3 * (size_t)M));
-	MC_TRY(h2d(ctx, (int32_t *)(b + o_im), pt_image, (size_t)M));
-	MC_TRY(h2d(ctx, (int32_t *)(b + o_hc), hyp_cluster, (size_t)n_hyp));
-	MC_TRY(h2d(ctx, (int32_t *)(b + o_sp), sample_pos, (size_t)n_hyp * na));
-	MC_TRY(h2d(ctx, (float *)(b + o_iq), init_quat, 4 * (size_t)n_hyp));
-	MC_TRY(h2d(ctx, (int64_t *)(b + o_mo), mask_off.data(), (size_t)n_hyp + 1));
+	const size_t m = (size_t)M, nh = (size_t)n_hyp;
+	int32_t *d_co, *d_im, *d_hc, *d_sp, *d_ni; float *d_xy, *d_xyz, *d_iq, *d_pl, *d_pr, *d_le; int64_t *d_mo; uint8_t *d_mask;
+	MC_TRY(carve_scratch(ctx, ctx->scratch[kScrHostPose], [&](Carve &c) {
+		c.take(d_co, (size_t)n_clusters + 1); c.take(d_xy, 2 * m); c.take(d_xyz, 3 * m); c.take(d_im, m);
+		c.take(d_hc, nh); c.take(d_sp, nh * na); c.take(d_iq, 4 * nh); c.take(d_mo, nh + 1);
+		c.take(d_ni, nh); c.take(d_pl, 7 * nh); c.take(d_pr, 7 * nh); c.take(d_le, 2 * nh);
+		c.take(d_mask, inlier_mask ? (size_t)mask_off[n_hyp] + 1 : 1);
+	}));
+	if (!inlier_mask) d_mask = nullptr;
+	MC_TRY(h2d(ctx, d_co, cluster_offsets, (size_t)n_clusters + 1));
+	MC_TRY(h2d(ctx, d_xy, pt_xy, 2 * m));
+	MC_TRY(h2d(ctx, d_xyz, pt_xyz, 3 * m));
+	MC_TRY(h2d(ctx, d_im, pt_image, m));
+	MC_TRY(h2d(ctx, d_hc, hyp_cluster, nh));
+	MC_TRY(h2d(ctx, d_sp, sample_pos, nh * na));
+	MC_TRY(h2d(ctx, d_iq, init_quat, 4 * nh));
+	MC_TRY(h2d(ctx, d_mo, mask_off.data(), nh + 1));
 	if (ctx->pose_exact_order) {
 		int n_max = 0;
 		for (int c = 0; c < n_clusters; c++) n_max = std::max(n_max, cluster_offsets[c + 1] - cluster_offsets[c]);
-		MC_TRY(pose_depth_hypotheses_device(ctx, 2, (int32_t *)(b + o_co), (float *)(b + o_xy), (float *)(b + o_xyz), nullptr, nullptr,
-		                                    (int32_t *)(b + o_im), (int32_t *)(b + o_hc), (int32_t *)(b + o_sp), (float *)(b + o_iq), n_hyp, n_max, params,
-		                                    0.f, (int64_t *)(b + o_mo), (int32_t *)(b + o_ni), (float *)(b + o_pl), (float *)(b + o_pr),
-		                                    (float *)(b + o_le), inlier_mask ? (uint8_t *)(b + o_mask) : nullptr));
+		MC_TRY(pose_depth_hypotheses_device(ctx, 2, d_co, d_xy, d_xyz, nullptr, nullptr, d_im, d_hc, d_sp, d_iq, n_hyp, n_max, params, 0.f, d_mo, d_ni,
+		                                    d_pl, d_pr, d_le, d_mask));
 	} else
-	MC_TRY(pose_hypotheses_device(ctx, (int32_t *)(b + o_co), (float *)(b + o_xy), (float *)(b + o_xyz), (int32_t *)(b + o_im), (int32_t *)(b + o_hc),
-	                              (int32_t *)(b + o_sp), (float *)(b + o_iq), n_hyp, params, (int64_t *)(b + o_mo), (int32_t *)(b + o_ni),
-	                              (float *)(b + o_pl), (float *)(b + o_pr), (float *)(b + o_le), inlier_mask ? (uint8_t *)(b + o_mask) : nullptr));
-	MC_TRY(d2h(ctx, n_inliers, (const int32_t *)(b + o_ni), (size_t)n_hyp));
-	MC_TRY(d2h(ctx, pose_lm, (const float *)(b + o_pl), 7 * (size_t)n_hyp));
-	MC_TRY(d2h(ctx, pose_refit, (const float *)(b + o_pr), 7 * (size_t)n_hyp));
-	MC_TRY(d2h(ctx, lm_err, (const float *)(b + o_le), 2 * (size_t)n_hyp));
-	if (inlier_mask) MC_TRY(d2h(ctx, inlier_mask, (const uint8_t *)(b + o_mask), (size_t)mask_off[n_hyp]));
+	MC_TRY(pose_hypotheses_device(ctx, d_co, d_xy, d_xyz, d_im, d_hc, d_sp, d_iq, n_hyp, params, d_mo, d_ni, d_pl, d_pr, d_le, d_mask));
+	MC_TRY(d2h(ctx, n_inliers, d_ni, nh));
+	MC_TRY(d2h(ctx, pose_lm, d_pl, 7 * nh));
+	MC_TRY(d2h(ctx, pose_refit, d_pr, 7 * nh));
+	MC_TRY(d2h(ctx, lm_err, d_le, 2 * nh));
+	if (inlier_mask) MC_TRY(d2h(ctx, inlier_mask, d_mask, (size_t)mask_off[n_hyp]));
 	MC_CUDA(cudaStreamSynchronize(ctx->stream));
 	return MC_OK;
 }
@@ -494,22 +485,22 @@ mc_status mc_pose_ransac(mc_ctx *ctx, const int32_t *cluster_offsets, int n_clus
 	MC_CUDA(cudaSetDevice(ctx->device));
 	const int M = cluster_offsets[n_clusters];
 	const int n_tasks = n_clusters * params->max_objects_per_cluster;
-	Arena A; A.ctx = ctx;
-	const size_t o_co = A.plan(4ull * (n_clusters + 1)), o_xy = A.plan(8ull * M), o_xyz = A.plan(12ull * M), o_im = A.plan(4ull * M);
-	const size_t o_f = A.plan(n_tasks), o_p = A.plan(28ull * n_tasks), o_nt = A.plan(4ull * n_tasks);
-	MC_TRY(reserve(ctx, ctx->scratch[13], A.off));
-	char *b = (char *)ctx->scratch[13].p;
-	MC_TRY(h2d(ctx, (int32_t *)(b + o_co), cluster_offsets, (size_t)n_clusters + 1));
-	MC_TRY(h2d(ctx, (float *)(b + o_xy), pt_xy, 2 * (size_t)M));
-	MC_TRY(h2d(ctx, (float *)(b + o_xyz), pt_xyz, 3 * (size_t)M));
-	MC_TRY(h2d(ctx, (int32_t *)(b + o_im), pt_image, (size_t)M));
-	MC_CUDA(cudaMemsetAsync(b + o_p, 0, 28ull * n_tasks, ctx->stream));
+	const size_t m = (size_t)M, nt = (size_t)n_tasks;
+	int32_t *d_co, *d_im, *d_nt; float *d_xy, *d_xyz, *d_p; uint8_t *d_f;
+	MC_TRY(carve_scratch(ctx, ctx->scratch[kScrHostRansac], [&](Carve &c) {
+		c.take(d_co, (size_t)n_clusters + 1); c.take(d_xy, 2 * m); c.take(d_xyz, 3 * m); c.take(d_im, m);
+		c.take(d_f, nt); c.take(d_p, 7 * nt); c.take(d_nt, nt);
+	}));
+	MC_TRY(h2d(ctx, d_co, cluster_offsets, (size_t)n_clusters + 1));
+	MC_TRY(h2d(ctx, d_xy, pt_xy, 2 * m));
+	MC_TRY(h2d(ctx, d_xyz, pt_xyz, 3 * m));
+	MC_TRY(h2d(ctx, d_im, pt_image, m));
+	MC_CUDA(cudaMemsetAsync(d_p, 0, 28 * nt, ctx->stream));
 	// exact-order mode (mc_set_option "pose_exact_order") is handled inside: the same staged driver with the order-preserving LM
-	MC_TRY(pose_ransac_device(ctx, (int32_t *)(b + o_co), nullptr, n_clusters, M, (float *)(b + o_xy), (float *)(b + o_xyz), (int32_t *)(b + o_im), nullptr,
-	                          params, (uint8_t *)(b + o_f), (float *)(b + o_p), (int32_t *)(b + o_nt)));
-	MC_TRY(d2h(ctx, found, (const uint8_t *)(b + o_f), (size_t)n_tasks));
-	MC_TRY(d2h(ctx, pose, (const float *)(b + o_p), 7 * (size_t)n_tasks));
-	MC_TRY(d2h(ctx, n_tests, (const int32_t *)(b + o_nt), (size_t)n_tasks));
+	MC_TRY(pose_ransac_device(ctx, d_co, nullptr, n_clusters, M, d_xy, d_xyz, d_im, nullptr, params, d_f, d_p, d_nt));
+	MC_TRY(d2h(ctx, found, d_f, nt));
+	MC_TRY(d2h(ctx, pose, d_p, 7 * nt));
+	MC_TRY(d2h(ctx, n_tests, d_nt, nt));
 	MC_CUDA(cudaStreamSynchronize(ctx->stream));
 	return MC_OK;
 }
@@ -546,34 +537,32 @@ mc_status mc_pose_depth_hypotheses(mc_ctx *ctx, int variant, const int32_t *clus
 		}
 		mask_off[h + 1] = mask_off[h] + n;
 	}
-	Arena A; A.ctx = ctx;
-	const size_t o_co = A.plan(4ull * (n_clusters + 1)), o_xy = A.plan(8ull * M), o_xyz = A.plan(12ull * M), o_w = A.plan(12ull * M),
-	             o_cw = A.plan(4ull * M), o_im = A.plan(4ull * M);
-	const size_t o_hc = A.plan(4ull * n_hyp), o_sp = A.plan(4ull * n_hyp * na), o_iq = A.plan(16ull * n_hyp), o_mo = A.plan(8ull * (n_hyp + 1));
-	const size_t o_ni = A.plan(4ull * n_hyp), o_pl = A.plan(28ull * n_hyp), o_pr = A.plan(28ull * n_hyp), o_le = A.plan(8ull * n_hyp);
-	const size_t o_mask = A.plan(inlier_mask ? (size_t)mask_off[n_hyp] + 1 : 1);
-	MC_TRY(reserve(ctx, ctx->scratch[18], A.off));
-	char *b = (char *)ctx->scratch[18].p;
-	MC_TRY(h2d(ctx, (int32_t *)(b + o_co), cluster_offsets, (size_t)n_clusters + 1));
-	MC_TRY(h2d(ctx, (float *)(b + o_xy), pt_xy, 2 * (size_t)M));
-	MC_TRY(h2d(ctx, (float *)(b + o_xyz), pt_xyz, 3 * (size_t)M));
-	MC_TRY(h2d(ctx, (float *)(b + o_w), pt_world, 3 * (size_t)M));
-	MC_TRY(h2d(ctx, (float *)(b + o_cw), pt_cauchy, (size_t)M));
-	MC_TRY(h2d(ctx, (int32_t *)(b + o_im), pt_image, (size_t)M));
-	MC_TRY(h2d(ctx, (int32_t *)(b + o_hc), hyp_cluster, (size_t)n_hyp));
-	MC_TRY(h2d(ctx, (int32_t *)(b + o_sp), sample_pos, (size_t)n_hyp * na));
-	MC_TRY(h2d(ctx, (float *)(b + o_iq), init_quat, 4 * (size_t)n_hyp));
-	MC_TRY(h2d(ctx, (int64_t *)(b + o_mo), mask_off.data(), (size_t)n_hyp + 1));
-	MC_TRY(pose_depth_hypotheses_device(ctx, variant, (int32_t *)(b + o_co), (float *)(b + o_xy), (float *)(b + o_xyz), (float *)(b + o_w),
-	                                    (float *)(b + o_cw), (int32_t *)(b + o_im), (int32_t *)(b + o_hc), (int32_t *)(b + o_sp), (float *)(b + o_iq),
-	                                    n_hyp, largest_cluster(cluster_offsets, n_clusters), params, alpha, (int64_t *)(b + o_mo),
-	                                    (int32_t *)(b + o_ni), (float *)(b + o_pl), (float *)(b + o_pr), (float *)(b + o_le),
-	                                    inlier_mask ? (uint8_t *)(b + o_mask) : nullptr));
-	MC_TRY(d2h(ctx, n_inliers, (const int32_t *)(b + o_ni), (size_t)n_hyp));
-	MC_TRY(d2h(ctx, pose_lm, (const float *)(b + o_pl), 7 * (size_t)n_hyp));
-	MC_TRY(d2h(ctx, pose_refit, (const float *)(b + o_pr), 7 * (size_t)n_hyp));
-	MC_TRY(d2h(ctx, lm_err, (const float *)(b + o_le), 2 * (size_t)n_hyp));
-	if (inlier_mask) MC_TRY(d2h(ctx, inlier_mask, (const uint8_t *)(b + o_mask), (size_t)mask_off[n_hyp]));
+	const size_t m = (size_t)M, nh = (size_t)n_hyp;
+	int32_t *d_co, *d_im, *d_hc, *d_sp, *d_ni; float *d_xy, *d_xyz, *d_w, *d_cw, *d_iq, *d_pl, *d_pr, *d_le; int64_t *d_mo; uint8_t *d_mask;
+	MC_TRY(carve_scratch(ctx, ctx->scratch[kScrHostPoseDepth], [&](Carve &c) {
+		c.take(d_co, (size_t)n_clusters + 1); c.take(d_xy, 2 * m); c.take(d_xyz, 3 * m); c.take(d_w, 3 * m); c.take(d_cw, m); c.take(d_im, m);
+		c.take(d_hc, nh); c.take(d_sp, nh * na); c.take(d_iq, 4 * nh); c.take(d_mo, nh + 1);
+		c.take(d_ni, nh); c.take(d_pl, 7 * nh); c.take(d_pr, 7 * nh); c.take(d_le, 2 * nh);
+		c.take(d_mask, inlier_mask ? (size_t)mask_off[n_hyp] + 1 : 1);
+	}));
+	if (!inlier_mask) d_mask = nullptr;
+	MC_TRY(h2d(ctx, d_co, cluster_offsets, (size_t)n_clusters + 1));
+	MC_TRY(h2d(ctx, d_xy, pt_xy, 2 * m));
+	MC_TRY(h2d(ctx, d_xyz, pt_xyz, 3 * m));
+	MC_TRY(h2d(ctx, d_w, pt_world, 3 * m));
+	MC_TRY(h2d(ctx, d_cw, pt_cauchy, m));
+	MC_TRY(h2d(ctx, d_im, pt_image, m));
+	MC_TRY(h2d(ctx, d_hc, hyp_cluster, nh));
+	MC_TRY(h2d(ctx, d_sp, sample_pos, nh * na));
+	MC_TRY(h2d(ctx, d_iq, init_quat, 4 * nh));
+	MC_TRY(h2d(ctx, d_mo, mask_off.data(), nh + 1));
+	MC_TRY(pose_depth_hypotheses_device(ctx, variant, d_co, d_xy, d_xyz, d_w, d_cw, d_im, d_hc, d_sp, d_iq, n_hyp, largest_cluster(cluster_offsets, n_clusters),
+	                                    params, alpha, d_mo, d_ni, d_pl, d_pr, d_le, d_mask));
+	MC_TRY(d2h(ctx, n_inliers, d_ni, nh));
+	MC_TRY(d2h(ctx, pose_lm, d_pl, 7 * nh));
+	MC_TRY(d2h(ctx, pose_refit, d_pr, 7 * nh));
+	MC_TRY(d2h(ctx, lm_err, d_le, 2 * nh));
+	if (inlier_mask) MC_TRY(d2h(ctx, inlier_mask, d_mask, (size_t)mask_off[n_hyp]));
 	MC_CUDA(cudaStreamSynchronize(ctx->stream));
 	return MC_OK;
 }
@@ -607,27 +596,26 @@ mc_status mc_pose_depth_ransac(mc_ctx *ctx, int variant, const int32_t *cluster_
 	const int M = cluster_offsets[n_clusters];
 	const int n_tasks = n_clusters * params->max_objects_per_cluster;
 	if (n_tasks <= 0) return MC_OK;
-	Arena A; A.ctx = ctx;
-	const size_t o_co = A.plan(4ull * (n_clusters + 1)), o_xy = A.plan(8ull * M), o_xyz = A.plan(12ull * M), o_w = A.plan(12ull * M),
-	             o_cw = A.plan(4ull * M), o_im = A.plan(4ull * M), o_tie = A.plan(4ull * M);
-	const size_t o_f = A.plan(n_tasks), o_p = A.plan(28ull * n_tasks), o_nt = A.plan(4ull * n_tasks);
-	MC_TRY(reserve(ctx, ctx->scratch[18], A.off));
-	char *b = (char *)ctx->scratch[18].p;
-	MC_TRY(h2d(ctx, (int32_t *)(b + o_co), cluster_offsets, (size_t)n_clusters + 1));
-	MC_TRY(h2d(ctx, (float *)(b + o_xy), pt_xy, 2 * (size_t)M));
-	MC_TRY(h2d(ctx, (float *)(b + o_xyz), pt_xyz, 3 * (size_t)M));
-	MC_TRY(h2d(ctx, (float *)(b + o_w), pt_world, 3 * (size_t)M));
-	MC_TRY(h2d(ctx, (float *)(b + o_cw), pt_cauchy, (size_t)M));
-	MC_TRY(h2d(ctx, (int32_t *)(b + o_im), pt_image, (size_t)M));
-	if (pt_tie) MC_TRY(h2d(ctx, (int32_t *)(b + o_tie), pt_tie, (size_t)M));
-	MC_CUDA(cudaMemsetAsync(b + o_p, 0, 28ull * n_tasks, ctx->stream));
-	MC_TRY(pose_depth_ransac_device(ctx, variant, (int32_t *)(b + o_co), n_clusters, largest_cluster(cluster_offsets, n_clusters), (float *)(b + o_xy),
-	                                (float *)(b + o_xyz), (float *)(b + o_w), (float *)(b + o_cw), (int32_t *)(b + o_im),
-	                                pt_tie ? (int32_t *)(b + o_tie) : nullptr, params, alpha, (uint8_t *)(b + o_f), (float *)(b + o_p),
-	                                (int32_t *)(b + o_nt), nullptr));
-	MC_TRY(d2h(ctx, found, (const uint8_t *)(b + o_f), (size_t)n_tasks));
-	MC_TRY(d2h(ctx, pose, (const float *)(b + o_p), 7 * (size_t)n_tasks));
-	MC_TRY(d2h(ctx, n_tests, (const int32_t *)(b + o_nt), (size_t)n_tasks));
+	const size_t m = (size_t)M, nt = (size_t)n_tasks;
+	int32_t *d_co, *d_im, *d_tie, *d_nt; float *d_xy, *d_xyz, *d_w, *d_cw, *d_p; uint8_t *d_f;
+	MC_TRY(carve_scratch(ctx, ctx->scratch[kScrHostPoseDepth], [&](Carve &c) {
+		c.take(d_co, (size_t)n_clusters + 1); c.take(d_xy, 2 * m); c.take(d_xyz, 3 * m); c.take(d_w, 3 * m); c.take(d_cw, m); c.take(d_im, m); c.take(d_tie, m);
+		c.take(d_f, nt); c.take(d_p, 7 * nt); c.take(d_nt, nt);
+	}));
+	if (!pt_tie) d_tie = nullptr;
+	MC_TRY(h2d(ctx, d_co, cluster_offsets, (size_t)n_clusters + 1));
+	MC_TRY(h2d(ctx, d_xy, pt_xy, 2 * m));
+	MC_TRY(h2d(ctx, d_xyz, pt_xyz, 3 * m));
+	MC_TRY(h2d(ctx, d_w, pt_world, 3 * m));
+	MC_TRY(h2d(ctx, d_cw, pt_cauchy, m));
+	MC_TRY(h2d(ctx, d_im, pt_image, m));
+	if (pt_tie) MC_TRY(h2d(ctx, d_tie, pt_tie, m));
+	MC_CUDA(cudaMemsetAsync(d_p, 0, 28 * nt, ctx->stream));
+	MC_TRY(pose_depth_ransac_device(ctx, variant, d_co, n_clusters, largest_cluster(cluster_offsets, n_clusters), d_xy, d_xyz, d_w, d_cw, d_im, d_tie,
+	                                params, alpha, d_f, d_p, d_nt, nullptr));
+	MC_TRY(d2h(ctx, found, d_f, nt));
+	MC_TRY(d2h(ctx, pose, d_p, 7 * nt));
+	MC_TRY(d2h(ctx, n_tests, d_nt, nt));
 	MC_CUDA(cudaStreamSynchronize(ctx->stream));
 	return MC_OK;
 }
@@ -643,32 +631,30 @@ mc_status mc_filter_projection(mc_ctx *ctx, const int32_t *match_offsets, const 
 	}
 	MC_CUDA(cudaSetDevice(ctx->device));
 	const int M = match_offsets[n_models];
-	const int no = n_objects > 0 ? n_objects : 1;
-	Arena A; A.ctx = ctx;
-	const size_t o_off = A.plan(4ull * (n_models + 1)), o_img = A.plan(4ull * (M + 1)), o_xy = A.plan(8ull * (M + 1)), o_xyz = A.plan(12ull * (M + 1));
-	const size_t o_om = A.plan(4ull * no), o_op = A.plan(28ull * no), o_keep = A.plan(no), o_sc = A.plan(4ull * no), o_n = A.plan(64);
-	const size_t o_cm = A.plan(4ull * (no + 2)), o_co = A.plan(4ull * (no + 2)), o_mem = A.plan(4ull * (M + 2));
-	const size_t o_sm = A.plan(4ull * no), o_sp = A.plan(28ull * no), o_ss = A.plan(4ull * no);
-	MC_TRY(reserve(ctx, ctx->scratch[14], A.off));
-	char *b = (char *)ctx->scratch[14].p;
-	MC_TRY(h2d(ctx, (int32_t *)(b + o_off), match_offsets, (size_t)n_models + 1));
-	MC_TRY(h2d(ctx, (int32_t *)(b + o_img), match_image, (size_t)M));
-	MC_TRY(h2d(ctx, (float *)(b + o_xy), match_xy, 2 * (size_t)M));
-	MC_TRY(h2d(ctx, (float *)(b + o_xyz), match_xyz, 3 * (size_t)M));
-	MC_TRY(h2d(ctx, (int32_t *)(b + o_om), obj_model, (size_t)n_objects));
-	MC_TRY(h2d(ctx, (float *)(b + o_op), obj_pose, 7 * (size_t)n_objects));
-	MC_TRY(filter_device(ctx, (int32_t *)(b + o_off), (int32_t *)(b + o_img), (float *)(b + o_xy), (float *)(b + o_xyz), n_models, M,
-	                     (int32_t *)(b + o_om), (float *)(b + o_op), nullptr, n_objects, min_points, feature_distance, min_score,
-	                     (uint8_t *)(b + o_keep), (float *)(b + o_sc), (int32_t *)(b + o_n), (int32_t *)(b + o_cm), (int32_t *)(b + o_co),
-	                     (int32_t *)(b + o_mem), (int32_t *)(b + o_sm), (float *)(b + o_sp), (float *)(b + o_ss)));
+	const size_t m = (size_t)M, no = n_objects > 0 ? (size_t)n_objects : 1;
+	int32_t *d_off, *d_img, *d_om, *d_n, *d_cm, *d_co, *d_mem, *d_sm; float *d_xy, *d_xyz, *d_op, *d_sc, *d_sp, *d_ss; uint8_t *d_keep;
+	MC_TRY(carve_scratch(ctx, ctx->scratch[kScrHostFilter], [&](Carve &c) {
+		c.take(d_off, (size_t)n_models + 1); c.take(d_img, m + 1); c.take(d_xy, 2 * (m + 1)); c.take(d_xyz, 3 * (m + 1));
+		c.take(d_om, no); c.take(d_op, 7 * no); c.take(d_keep, no); c.take(d_sc, no); c.take(d_n, 16);
+		c.take(d_cm, no + 2); c.take(d_co, no + 2); c.take(d_mem, m + 2);
+		c.take(d_sm, no); c.take(d_sp, 7 * no); c.take(d_ss, no);
+	}));
+	MC_TRY(h2d(ctx, d_off, match_offsets, (size_t)n_models + 1));
+	MC_TRY(h2d(ctx, d_img, match_image, m));
+	MC_TRY(h2d(ctx, d_xy, match_xy, 2 * m));
+	MC_TRY(h2d(ctx, d_xyz, match_xyz, 3 * m));
+	MC_TRY(h2d(ctx, d_om, obj_model, (size_t)n_objects));
+	MC_TRY(h2d(ctx, d_op, obj_pose, 7 * (size_t)n_objects));
+	MC_TRY(filter_device(ctx, d_off, d_img, d_xy, d_xyz, n_models, M, d_om, d_op, nullptr, n_objects, min_points, feature_distance, min_score, d_keep,
+	                     d_sc, d_n, d_cm, d_co, d_mem, d_sm, d_sp, d_ss));
 	int32_t hn[2] = { 0, 0 };
-	MC_TRY(d2h(ctx, hn, (const int32_t *)(b + o_n), 2));
-	MC_TRY(d2h(ctx, keep, (const uint8_t *)(b + o_keep), (size_t)n_objects));
-	MC_TRY(d2h(ctx, score, (const float *)(b + o_sc), (size_t)n_objects));
+	MC_TRY(d2h(ctx, hn, d_n, 2));
+	MC_TRY(d2h(ctx, keep, d_keep, (size_t)n_objects));
+	MC_TRY(d2h(ctx, score, d_sc, (size_t)n_objects));
 	MC_CUDA(cudaStreamSynchronize(ctx->stream));
 	*n_survivors = hn[0];
-	MC_TRY(d2h(ctx, cluster_offsets, (const int32_t *)(b + o_co), (size_t)hn[0] + 1));
-	MC_TRY(d2h(ctx, members, (const int32_t *)(b + o_mem), (size_t)hn[1]));
+	MC_TRY(d2h(ctx, cluster_offsets, d_co, (size_t)hn[0] + 1));
+	MC_TRY(d2h(ctx, members, d_mem, (size_t)hn[1]));
 	MC_CUDA(cudaStreamSynchronize(ctx->stream));
 	return MC_OK;
 }
@@ -691,41 +677,39 @@ mc_status mc_filter_projection_depth(mc_ctx *ctx, const int32_t *match_offsets, 
 	const int M = match_offsets[n_models];
 	const int NT = test_offsets[n_models];
 	const size_t px = (size_t)width * height;
-	const int no = n_objects > 0 ? n_objects : 1;
-	Arena A; A.ctx = ctx;
-	const size_t o_off = A.plan(4ull * (n_models + 1)), o_img = A.plan(4ull * (M + 1)), o_xy = A.plan(8ull * (M + 1)), o_xyz = A.plan(12ull * (M + 1));
-	const size_t o_om = A.plan(4ull * no), o_op = A.plan(28ull * no), o_keep = A.plan(no), o_sc = A.plan(4ull * no), o_n = A.plan(64);
-	const size_t o_cm = A.plan(4ull * (no + 2)), o_co = A.plan(4ull * (no + 2)), o_mem = A.plan(4ull * (M + 2));
-	const size_t o_sm = A.plan(4ull * no), o_sp = A.plan(28ull * no), o_ss = A.plan(4ull * no);
-	const size_t o_to = A.plan(4ull * (n_models + 1)), o_tx = A.plan(12ull * (NT + 1)), o_d = A.plan(4ull * px), o_f = A.plan(4ull * px);
-	MC_TRY(reserve(ctx, ctx->scratch[14], A.off));
-	char *b = (char *)ctx->scratch[14].p;
-	MC_TRY(h2d(ctx, (int32_t *)(b + o_off), match_offsets, (size_t)n_models + 1));
-	MC_TRY(h2d(ctx, (int32_t *)(b + o_img), match_image, (size_t)M));
-	MC_TRY(h2d(ctx, (float *)(b + o_xy), match_xy, 2 * (size_t)M));
-	MC_TRY(h2d(ctx, (float *)(b + o_xyz), match_xyz, 3 * (size_t)M));
-	MC_TRY(h2d(ctx, (int32_t *)(b + o_om), obj_model, (size_t)n_objects));
-	MC_TRY(h2d(ctx, (float *)(b + o_op), obj_pose, 7 * (size_t)n_objects));
-	MC_TRY(h2d(ctx, (int32_t *)(b + o_to), test_offsets, (size_t)n_models + 1));
-	MC_TRY(h2d(ctx, (float *)(b + o_tx), test_xyz, 3 * (size_t)NT));
-	MC_TRY(h2d(ctx, (float *)(b + o_d), depth, px));
-	MC_TRY(h2d(ctx, (float *)(b + o_f), fill_distance, px));
+	const size_t m = (size_t)M, no = n_objects > 0 ? (size_t)n_objects : 1;
+	int32_t *d_off, *d_img, *d_om, *d_n, *d_cm, *d_co, *d_mem, *d_sm, *d_to; float *d_xy, *d_xyz, *d_op, *d_sc, *d_sp, *d_ss, *d_tx, *d_d, *d_f;
+	uint8_t *d_keep;
+	MC_TRY(carve_scratch(ctx, ctx->scratch[kScrHostFilter], [&](Carve &c) {
+		c.take(d_off, (size_t)n_models + 1); c.take(d_img, m + 1); c.take(d_xy, 2 * (m + 1)); c.take(d_xyz, 3 * (m + 1));
+		c.take(d_om, no); c.take(d_op, 7 * no); c.take(d_keep, no); c.take(d_sc, no); c.take(d_n, 16);
+		c.take(d_cm, no + 2); c.take(d_co, no + 2); c.take(d_mem, m + 2);
+		c.take(d_sm, no); c.take(d_sp, 7 * no); c.take(d_ss, no);
+		c.take(d_to, (size_t)n_models + 1); c.take(d_tx, 3 * ((size_t)NT + 1)); c.take(d_d, px); c.take(d_f, px);
+	}));
+	MC_TRY(h2d(ctx, d_off, match_offsets, (size_t)n_models + 1));
+	MC_TRY(h2d(ctx, d_img, match_image, m));
+	MC_TRY(h2d(ctx, d_xy, match_xy, 2 * m));
+	MC_TRY(h2d(ctx, d_xyz, match_xyz, 3 * m));
+	MC_TRY(h2d(ctx, d_om, obj_model, (size_t)n_objects));
+	MC_TRY(h2d(ctx, d_op, obj_pose, 7 * (size_t)n_objects));
+	MC_TRY(h2d(ctx, d_to, test_offsets, (size_t)n_models + 1));
+	MC_TRY(h2d(ctx, d_tx, test_xyz, 3 * (size_t)NT));
+	MC_TRY(h2d(ctx, d_d, depth, px));
+	MC_TRY(h2d(ctx, d_f, fill_distance, px));
 	float TM[12];
 	pose_tm(depth_pose, TM);                                 // depthmap->TM.init(cameraPose)
-	MC_TRY(filter_depth_device(ctx, (int32_t *)(b + o_off), (int32_t *)(b + o_img), (float *)(b + o_xy), (float *)(b + o_xyz), n_models, M,
-	                           (int32_t *)(b + o_om), (float *)(b + o_op), nullptr, n_objects, min_points, feature_distance, min_score,
-	                           (int32_t *)(b + o_to), (float *)(b + o_tx), depth_K, TM, width, height, (float *)(b + o_d), (float *)(b + o_f),
-	                           plausible_sq_distance, depth_fraction, min_keypoint_fraction,
-	                           (uint8_t *)(b + o_keep), (float *)(b + o_sc), (int32_t *)(b + o_n), (int32_t *)(b + o_cm), (int32_t *)(b + o_co),
-	                           (int32_t *)(b + o_mem), (int32_t *)(b + o_sm), (float *)(b + o_sp), (float *)(b + o_ss)));
+	MC_TRY(filter_depth_device(ctx, d_off, d_img, d_xy, d_xyz, n_models, M, d_om, d_op, nullptr, n_objects, min_points, feature_distance, min_score, d_to,
+	                           d_tx, depth_K, TM, width, height, d_d, d_f, plausible_sq_distance, depth_fraction, min_keypoint_fraction, d_keep, d_sc,
+	                           d_n, d_cm, d_co, d_mem, d_sm, d_sp, d_ss));
 	int32_t hn[2] = { 0, 0 };
-	MC_TRY(d2h(ctx, hn, (const int32_t *)(b + o_n), 2));
-	MC_TRY(d2h(ctx, keep, (const uint8_t *)(b + o_keep), (size_t)n_objects));
-	MC_TRY(d2h(ctx, score, (const float *)(b + o_sc), (size_t)n_objects));
+	MC_TRY(d2h(ctx, hn, d_n, 2));
+	MC_TRY(d2h(ctx, keep, d_keep, (size_t)n_objects));
+	MC_TRY(d2h(ctx, score, d_sc, (size_t)n_objects));
 	MC_CUDA(cudaStreamSynchronize(ctx->stream));
 	*n_survivors = hn[0];
-	MC_TRY(d2h(ctx, cluster_offsets, (const int32_t *)(b + o_co), (size_t)hn[0] + 1));
-	MC_TRY(d2h(ctx, members, (const int32_t *)(b + o_mem), (size_t)hn[1]));
+	MC_TRY(d2h(ctx, cluster_offsets, d_co, (size_t)hn[0] + 1));
+	MC_TRY(d2h(ctx, members, d_mem, (size_t)hn[1]));
 	MC_CUDA(cudaStreamSynchronize(ctx->stream));
 	return MC_OK;
 }

@@ -300,14 +300,15 @@ mc_status cluster_device(mc_ctx *ctx, const int32_t *d_match_offsets, const int3
                          int n_models, int n_images, int max_matches, float radius, float merge, int min_pts, int max_iter,
                          int32_t *d_out_n, int32_t *d_cluster_model, int32_t *d_cluster_offsets, int32_t *d_members) {
 	if (n_models <= 0) return MC_OK;
-	DevBuf &b_count = ctx->scratch[0], &b_sizes = ctx->scratch[1], &b_members = ctx->scratch[2], &b_f = ctx->scratch[3], &b_i = ctx->scratch[4];
+	DevBuf &b_count = ctx->scratch[kScrClusterCount], &b_sizes = ctx->scratch[kScrClusterSizes], &b_members = ctx->scratch[kScrClusterMembers],
+	       &b_f = ctx->scratch[kScrClusterF], &b_i = ctx->scratch[kScrClusterI], &b_list = ctx->scratch[kScrClusterList];
 	MC_TRY(reserve(ctx, b_count, sizeof(int32_t) * (n_models + 1)));
 	MC_TRY(reserve(ctx, b_sizes, sizeof(int32_t) * (max_matches + 1)));
 	MC_TRY(reserve(ctx, b_members, sizeof(int32_t) * (max_matches + 1)));
 	MC_TRY(reserve(ctx, b_f, sizeof(float) * 4 * (size_t)(max_matches + 1)));
 	MC_TRY(reserve(ctx, b_i, sizeof(int32_t) * 7 * (size_t)(max_matches + 1)));
-	MC_TRY(reserve(ctx, ctx->scratch[8], sizeof(int32_t) * (size_t)(n_models + 16)));
-	int32_t *d_list = (int32_t *)ctx->scratch[8].p + 16, *d_n_list = (int32_t *)ctx->scratch[8].p;
+	MC_TRY(reserve(ctx, b_list, sizeof(int32_t) * (size_t)(n_models + 16)));
+	int32_t *d_list = (int32_t *)b_list.p + 16, *d_n_list = (int32_t *)b_list.p;
 	k_cluster_nonempty<<<1, 1024, 0, ctx->stream>>>(d_match_offsets, n_models, min_pts, (int32_t *)b_count.p, d_list, d_n_list);
 	MC_LAUNCH_CHECK();
 	k_meanshift<<<n_models < 64 ? n_models : 64, kClusterThreads, kClusterSmem, ctx->stream>>>(d_match_offsets, d_match_image, d_match_xy, n_models, n_images,

@@ -46,6 +46,49 @@ struct DevBuf {            // grow-only device scratch
 	size_t cap = 0;
 };
 
+// mc_ctx::scratch: one grow-only buffer per owner. The frame graphs (pipeline.cu) key on the address of every slot.
+enum ScratchSlot : int {
+	kScrClusterCount,         // cluster_device: per-model cluster counts
+	kScrClusterSizes,         // cluster_device: cluster sizes
+	kScrClusterMembers,       // cluster_device: cluster members
+	kScrClusterF,             // cluster_device: per-match float state
+	kScrClusterI,             // cluster_device: per-match int state
+	kScrClusterList,          // cluster_device: the models to cluster and their count
+	kScrFilterIn,             // filter_device: object x match inlier flags
+	kScrFilterOwner,          // filter_device: owner of each match
+	kScrFilterOwned,          // filter_device: matches owned per object
+	kScrFilterRaw,            // filter_device, depth variant: scores before the depth penalty
+	kScrFitStream,            // pose_hypotheses_device: counters of the persistent fit kernel
+	kScrRefitLists,           // pose_hypotheses_device: refit buckets
+	kScrRansac,               // ransac_staged_launch: RansacState
+	kScrDepthLm,              // pose_depth.cu: per-warp LM work arrays
+	kScrAdaptive,             // adaptive.cu: uploads and per-frame state of mc_match_adaptive and match_adaptive_frames
+	kScrFrame,                // pipeline.cu carve: a frame's chain (FrameBufs)
+	kScrDepthFrame,           // depth_frames.cu depth_carve: a frame's chain (DepthBufs)
+	kScrDepthMeta,            // depth_frames_run: per-frame model CSR and LinkSlices
+	kScrDepthFramesIn,        // mc_process_depth_frames: uploaded per-match arrays and depth maps
+	kScrDepthQueries,         // depth_queries: per-match arrays of mc_process_depth_queries*
+	kScrHostCluster,          // mc_cluster_meanshift
+	kScrHostPose,             // mc_pose_hypotheses
+	kScrHostRansac,           // mc_pose_ransac
+	// the two entries of each pair below share one buffer: they never run at the same time on a context, and a caller that
+	// alternates them reuses the larger allocation
+	kScrHostPoseDepth,        // mc_pose_depth_hypotheses, mc_pose_depth_ransac
+	kScrHostFilter,           // mc_filter_projection, mc_filter_projection_depth
+	kScratchSlots
+};
+
+// Consecutive arrays in one buffer, each on a 256-byte boundary. A layout is a callable that takes every array once, in order:
+// run with base == nullptr it only sizes the buffer (the pointers it sets are null), run with a base it points each array into it.
+struct Carve {
+	char *base = nullptr;
+	size_t off = 0;
+	template <class T> void take(T *&p, size_t n) {
+		p = base ? (T *)(base + off) : nullptr;
+		off += (n * sizeof(T) + 255) & ~(size_t)255;
+	}
+};
+
 // TransformMatrix::init(cameraPose) on the host (moped.hpp:175-182): the 3x4 matrix of a pose (quaternion x y z w, translation).
 // One expression for every caller (mc_set_cameras, mc_filter_projection_depth, mc_set_depth_filter), so their bits agree.
 inline void pose_tm(const float *pose, float *T) {
@@ -106,7 +149,7 @@ struct mc_ctx {
 	int match_stagger = 1;            // mc_set_option "match_stagger": CTAs of one DB split start at different tiles
 	int match_reserve_sms = 0;        // mc_set_option "match_reserve_sms": SMs the persistent matching kernel leaves to concurrent work
 	mc::DevBuf nn_row, nn_dist, accepted, q_xy, q_image;
-	mc::DevBuf scratch[24];
+	mc::DevBuf scratch[mc::kScratchSlots];
 	void *h_pinned = nullptr; size_t h_pinned_cap = 0;
 	int last_stats[4] = {0, 0, 0, 0};
 	int last_match_q = 0, last_match_tensor = 0;   // queries / mode of the last match_device pass (mc_match_last_stats)
@@ -189,6 +232,17 @@ inline mc_status reserve(mc_ctx *ctx, DevBuf &b, size_t bytes) {
 	return MC_OK;
 }
 
+// Sizes `layout` (a Carve layout), grows b to fit it and points its arrays into b. Inside a graph capture a buffer that has to
+// grow fails with MC_ERR_STATE (reserve) and no pointer is set.
+template <class Layout> inline mc_status carve_scratch(mc_ctx *ctx, DevBuf &b, Layout &&layout) {
+	Carve c;
+	layout(c);
+	MC_TRY(reserve(ctx, b, c.off));
+	c = Carve{(char *)b.p};
+	layout(c);
+	return MC_OK;
+}
+
 inline mc_status pinned(mc_ctx *ctx, size_t bytes) {
 	if (bytes <= ctx->h_pinned_cap) return MC_OK;
 	if (ctx->h_pinned) { MC_CUDA(cudaFreeHost(ctx->h_pinned)); ctx->h_pinned = nullptr; ctx->h_pinned_cap = 0; }
@@ -235,6 +289,20 @@ mc_status match_compact_frames_device(mc_ctx *ctx, const FrameDesc *d_fd, const 
                                       const float *d_q_world = nullptr, const float *d_q_fill = nullptr, float *d_match_world = nullptr,
                                       float *d_match_fill = nullptr);
 constexpr int kCompactCap = 8192;    // accepted matches per frame handled by the compaction (k_match_compact)
+
+// The result slots of a frame batch, on the device (ctx->batch_out) and in its pinned host copy: per frame info[4] = {objects,
+// status, accepted matches, clusters}, model[max_objects], pose[7 * max_objects] and score[max_objects], each field frame-major.
+struct BatchSlots { int32_t *info, *model; float *pose, *score; };
+inline size_t batch_slots_bytes(int n_frames, int max_objects) { return (16 + 36 * (size_t)max_objects) * (size_t)n_frames; }
+inline BatchSlots batch_slots(void *base, int n_frames, int max_objects) {
+	char *b = (char *)base;
+	const size_t nf = (size_t)n_frames, mo = (size_t)max_objects;
+	return { (int32_t *)b, (int32_t *)(b + 16 * nf), (float *)(b + (16 + 4 * mo) * nf), (float *)(b + (16 + 32 * mo) * nf) };
+}
+// Host copy of the slots -> the caller's arrays: frame_info (nullable) and n_objects of every frame, the objects of a frame whose
+// status is 0 and whose objects fit. first_bad / first_over: the first frame with a non-zero status / more than max_objects objects, or -1.
+void unpack_batch(const BatchSlots &h, int n_frames, int max_objects, int32_t *n_objects, int32_t *obj_model, float *obj_pose, float *obj_score,
+                  int32_t *frame_info, int &first_bad, int &first_over);
 
 // ---- moped3d's batched MATCH (adaptive.cu), shared by mc_match_adaptive_frames* and mc_process_depth_queries* ----
 // Where the nearest rows come from: one cascade pass over q_desc against the context's database (n_shards = 0), or the merge of

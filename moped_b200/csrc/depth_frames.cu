@@ -87,35 +87,25 @@ struct DepthBufs {
 	int32_t *f_model, *f_offsets, *f_members, *surv_model; float *surv_pose, *surv_score;
 };
 
-static mc_status depth_carve(mc_ctx *lane, int M, const DepthCaps &c, DepthBufs &B) {
-	size_t off = 0;
-	auto take = [&](size_t bytes) { size_t o = off; off += (bytes + 255) & ~(size_t)255; return o; };
-	const size_t m1 = (size_t)M + 2, c2 = (size_t)c.cl_cap + 2, o2 = (size_t)c.obj_cap + 2, t1 = (size_t)c.task_cap + 1;
-	const size_t o_st = take(64), o_clm = take(4 * c2), o_clo = take(4 * c2), o_clmem = take(4 * m1);
-	const size_t o_pxy = take(8 * m1), o_pxyz = take(12 * m1), o_pw = take(12 * m1), o_pc = take(4 * m1), o_pim = take(4 * m1), o_ptie = take(4 * m1);
-	const size_t o_found = take(t1), o_tpose = take(28 * t1), o_nt = take(4 * t1);
-	const size_t o_om = take(4 * o2), o_op = take(28 * o2), o_os = take(4 * o2), o_keep = take(o2);
-	const size_t o_fm = take(4 * o2), o_fo = take(4 * o2), o_fmem = take(4 * m1), o_sm = take(4 * o2), o_sp = take(28 * o2), o_ss = take(4 * o2);
-	MC_TRY(reserve(lane, lane->scratch[9], off));
-	char *b = (char *)lane->scratch[9].p;
-	B.st = (int32_t *)(b + o_st); B.cl_model = (int32_t *)(b + o_clm); B.cl_offsets = (int32_t *)(b + o_clo); B.cl_members = (int32_t *)(b + o_clmem);
-	B.pt_xy = (float *)(b + o_pxy); B.pt_xyz = (float *)(b + o_pxyz); B.pt_world = (float *)(b + o_pw); B.pt_cauchy = (float *)(b + o_pc);
-	B.pt_image = (int32_t *)(b + o_pim); B.pt_tie = (int32_t *)(b + o_ptie);
-	B.found = (uint8_t *)(b + o_found); B.task_pose = (float *)(b + o_tpose); B.n_tests = (int32_t *)(b + o_nt);
-	B.obj_model = (int32_t *)(b + o_om); B.obj_pose = (float *)(b + o_op); B.obj_score = (float *)(b + o_os); B.keep = (uint8_t *)(b + o_keep);
-	B.f_model = (int32_t *)(b + o_fm); B.f_offsets = (int32_t *)(b + o_fo); B.f_members = (int32_t *)(b + o_fmem);
-	B.surv_model = (int32_t *)(b + o_sm); B.surv_pose = (float *)(b + o_sp); B.surv_score = (float *)(b + o_ss);
-	return MC_OK;
+static mc_status depth_carve(mc_ctx *lane, int M, const DepthCaps &caps, DepthBufs &B) {
+	const size_t m1 = (size_t)M + 2, c2 = (size_t)caps.cl_cap + 2, o2 = (size_t)caps.obj_cap + 2, t1 = (size_t)caps.task_cap + 1;
+	return carve_scratch(lane, lane->scratch[kScrDepthFrame], [&](Carve &c) {
+		c.take(B.st, 16); c.take(B.cl_model, c2); c.take(B.cl_offsets, c2); c.take(B.cl_members, m1);
+		c.take(B.pt_xy, 2 * m1); c.take(B.pt_xyz, 3 * m1); c.take(B.pt_world, 3 * m1); c.take(B.pt_cauchy, m1); c.take(B.pt_image, m1); c.take(B.pt_tie, m1);
+		c.take(B.found, t1); c.take(B.task_pose, 7 * t1); c.take(B.n_tests, t1);
+		c.take(B.obj_model, o2); c.take(B.obj_pose, 7 * o2); c.take(B.obj_score, o2); c.take(B.keep, o2);
+		c.take(B.f_model, o2); c.take(B.f_offsets, o2); c.take(B.f_members, m1); c.take(B.surv_model, o2); c.take(B.surv_pose, 7 * o2); c.take(B.surv_score, o2);
+	});
 }
 
 // Enqueue one frame on lane->stream; its objects go to the frame's output slots. `ev` (nullable, 6 events) brackets the five steps.
 // `df`: the FILTER / FILTER2 settings of the calling context (a lane is a context of its own and holds none).
 static mc_status depth_frame_enqueue(mc_ctx *lane, const DepthPlan &p, const char *d_meta, const DepthInputs &in, int f, int n_models, int W, int H,
-                                     const mc_depth_pipeline_params *P, const DepthFilterTable *df, int max_objects, int32_t *d_info,
-                                     int32_t *d_model, float *d_pose, float *d_score, cudaEvent_t *ev) {
+                                     const mc_depth_pipeline_params *P, const DepthFilterTable *df, int max_objects, const BatchSlots &out,
+                                     cudaEvent_t *ev) {
 	mc_ctx *ctx = lane;
 	cudaStream_t s = lane->stream;
-	int32_t *o_info = d_info + 4 * (size_t)f;
+	int32_t *o_info = out.info + 4 * (size_t)f;
 	if (p.M == 0) {                                     // nothing to cluster: no objects
 		MC_CUDA(cudaMemsetAsync(o_info, 0, 16, s));
 		if (ev) for (int i = 0; i < 6; i++) MC_CUDA(cudaEventRecord(ev[i], s));
@@ -179,8 +169,8 @@ static mc_status depth_frame_enqueue(mc_ctx *lane, const DepthPlan &p, const cha
 	// FILTER2
 	MC_TRY(filter(df[1], P->filter2_min_points, P->filter2_feature_distance, P->filter2_min_score));
 	mark(5);
-	k_depth_export<<<1, 128, 0, s>>>(B.st, p.M, B.surv_model, B.surv_pose, B.surv_score, max_objects, o_info, d_model + (size_t)f * max_objects,
-	                                 d_pose + 7 * (size_t)f * max_objects, d_score + (size_t)f * max_objects);
+	k_depth_export<<<1, 128, 0, s>>>(B.st, p.M, B.surv_model, B.surv_pose, B.surv_score, max_objects, o_info, out.model + (size_t)f * max_objects,
+	                                 out.pose + 7 * (size_t)f * max_objects, out.score + (size_t)f * max_objects);
 	MC_LAUNCH_CHECK();
 	return MC_OK;
 }
@@ -265,18 +255,13 @@ static mc_status depth_frames_run(mc_ctx *ctx, const char *who, const std::vecto
                                   int32_t *n_objects, int32_t *obj_model, float *obj_pose, float *obj_score, int32_t *frame_info, float *stage_ms,
                                   cudaEvent_t *span = nullptr) {
 	const int nf = (int)plans.size();
-	MC_TRY(reserve(ctx, ctx->scratch[23], meta.size() + 256));
-	char *d_meta = (char *)ctx->scratch[23].p;
+	MC_TRY(reserve(ctx, ctx->scratch[kScrDepthMeta], meta.size() + 256));
+	char *d_meta = (char *)ctx->scratch[kScrDepthMeta].p;
 	MC_CUDA(cudaMemcpyAsync(d_meta, meta.data(), meta.size(), cudaMemcpyHostToDevice, ctx->stream));
-	const size_t per = 16 + (size_t)max_objects * 36;
-	const size_t bytes = per * (size_t)nf;
+	const size_t bytes = batch_slots_bytes(nf, max_objects);
 	MC_TRY(reserve(ctx, ctx->batch_out, bytes + 256));
 	MC_TRY(pinned(ctx, bytes + 256));
-	char *d = (char *)ctx->batch_out.p;
-	int32_t *d_info = (int32_t *)d;
-	int32_t *d_model = (int32_t *)(d + 16ull * nf);
-	float *d_pose = (float *)(d + (16ull + 4ull * max_objects) * nf);
-	float *d_score = (float *)(d + (16ull + 32ull * max_objects) * nf);
+	const BatchSlots d = batch_slots(ctx->batch_out.p, nf, max_objects);
 	int n_lanes = stage_ms ? 1 : std::min(std::max(ctx->n_lanes_wanted, 1), nf);
 	MC_TRY(ensure_lanes(ctx, n_lanes));
 	for (int l = 0; l < n_lanes; l++) { ctx->lanes[(size_t)l]->linkage_cached = ctx->linkage_cached; ctx->lanes[(size_t)l]->lm_finite_check = ctx->lm_finite_check; }
@@ -292,16 +277,15 @@ static mc_status depth_frames_run(mc_ctx *ctx, const char *who, const std::vecto
 	mc_status st = MC_OK;
 	for (int f = 0; f < nf && st == MC_OK; f++) {
 		mc_ctx *lane = ctx->lanes[(size_t)(f % n_lanes)];
-		st = depth_frame_enqueue(lane, plans[(size_t)f], d_meta, in, f, n_models, W, H, P, ctx->depth_filter, max_objects, d_info, d_model, d_pose,
-		                         d_score, stage_ms ? &ev[6 * (size_t)f] : nullptr);
+		st = depth_frame_enqueue(lane, plans[(size_t)f], d_meta, in, f, n_models, W, H, P, ctx->depth_filter, max_objects, d,
+		                         stage_ms ? &ev[6 * (size_t)f] : nullptr);
 		if (st != MC_OK) ctx->err = lane->err;
 	}
 	const mc_status sj = join_lanes(ctx);
 	if (st == MC_OK) st = sj;
 	if (st == MC_OK && span) MC_CUDA(cudaEventRecord(span[1], ctx->stream));
-	char *h = (char *)ctx->h_pinned;
 	if (st == MC_OK) {
-		MC_CUDA(cudaMemcpyAsync(h, d, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+		MC_CUDA(cudaMemcpyAsync(ctx->h_pinned, ctx->batch_out.p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
 		MC_CUDA(cudaStreamSynchronize(ctx->stream));
 	}
 	if (stage_ms) {
@@ -313,21 +297,9 @@ static mc_status depth_frames_run(mc_ctx *ctx, const char *who, const std::vecto
 		for (auto &e : ev) cudaEventDestroy(e);
 	}
 	if (st != MC_OK) return st;
-	const int32_t *h_info = (const int32_t *)h;
-	const int32_t *h_model = (const int32_t *)(h + 16ull * nf);
-	const float *h_pose = (const float *)(h + (16ull + 4ull * max_objects) * nf);
-	const float *h_score = (const float *)(h + (16ull + 32ull * max_objects) * nf);
-	int bad_frame = -1, over_frame = -1;
-	for (int f = 0; f < nf; f++) {
-		const int n = h_info[4 * f];
-		if (frame_info) memcpy(frame_info + 4 * f, h_info + 4 * f, 16);
-		n_objects[f] = n;
-		if (h_info[4 * f + 1]) { if (bad_frame < 0) bad_frame = f; continue; }
-		if (n > max_objects) { if (over_frame < 0) over_frame = f; continue; }
-		memcpy(obj_model + (size_t)f * max_objects, h_model + (size_t)f * max_objects, 4ull * n);
-		memcpy(obj_pose + 7 * (size_t)f * max_objects, h_pose + 7 * (size_t)f * max_objects, 28ull * n);
-		memcpy(obj_score + (size_t)f * max_objects, h_score + (size_t)f * max_objects, 4ull * n);
-	}
+	int bad_frame, over_frame;
+	unpack_batch(batch_slots(ctx->h_pinned, nf, max_objects), nf, max_objects, n_objects, obj_model, obj_pose, obj_score, frame_info, bad_frame,
+	             over_frame);
 	if (bad_frame >= 0) { ctx->err = std::string(who) + ": a match of frame " + std::to_string(bad_frame) + " lies outside the depth map"; return MC_ERR_ARG; }
 	if (over_frame >= 0) { ctx->err = std::string(who) + ": frame " + std::to_string(over_frame) + " has more than max_objects objects"; return MC_ERR_CAPACITY; }
 	return MC_OK;
@@ -361,13 +333,12 @@ static mc_status depth_queries(mc_ctx *ctx, bool dev, const char *who, const Row
 	if (!ctx->d_cams) return fail(MC_ERR_STATE, "cameras not set (mc_set_cameras)");
 	MC_CUDA(cudaSetDevice(ctx->device));
 	// per match (capacity Q, global ids): feature, image, xy, xyz, world, fill; the host entry's inputs behind them
-	const size_t planes = (size_t)width * height * n_range;
-	size_t off = 0;
-	auto take = [&](size_t bytes) { const size_t o = off; off += (bytes + 255) & ~(size_t)255; return o; };
-	const size_t o_feat = take(4ull * Q), o_img = take(4ull * Q), o_xy = take(8ull * Q), o_xyz = take(12ull * Q), o_w = take(12ull * Q), o_f = take(4ull * Q);
-	const size_t o_qw = dev ? 0 : take(12ull * Q), o_qf = dev ? 0 : take(4ull * Q), o_d = dev ? 0 : take(4 * planes), o_fd = dev ? 0 : take(4 * planes);
-	MC_TRY(reserve(ctx, ctx->scratch[16], off));
-	char *b = (char *)ctx->scratch[16].p;
+	const size_t planes = (size_t)width * height * n_range, q = (size_t)Q;
+	int32_t *m_feat, *m_img; float *m_xy, *m_xyz, *m_world, *m_fill, *up_qw = nullptr, *up_qf = nullptr, *up_depth = nullptr, *up_fill = nullptr;
+	MC_TRY(carve_scratch(ctx, ctx->scratch[kScrDepthQueries], [&](Carve &c) {
+		c.take(m_feat, q); c.take(m_img, q); c.take(m_xy, 2 * q); c.take(m_xyz, 3 * q); c.take(m_world, 3 * q); c.take(m_fill, q);
+		if (!dev) { c.take(up_qw, 3 * q); c.take(up_qf, q); c.take(up_depth, planes); c.take(up_fill, planes); }
+	}));
 	RowSource rs = src;
 	const float *d_xy = q_xy, *d_qw = q_world, *d_qf = q_fill, *d_depth = depth, *d_fill = fill_distance;
 	const int32_t *d_img = q_image;
@@ -378,22 +349,21 @@ static mc_status depth_queries(mc_ctx *ctx, bool dev, const char *who, const Row
 			MC_TRY(reserve(ctx, ctx->q_xy, 8ull * Q));
 			MC_CUDA(cudaMemcpyAsync(ctx->q_desc.p, src.q_desc, sizeof(float) * (size_t)Q * ctx->D, cudaMemcpyHostToDevice, s));
 			MC_CUDA(cudaMemcpyAsync(ctx->q_xy.p, q_xy, 8ull * Q, cudaMemcpyHostToDevice, s));
-			MC_CUDA(cudaMemcpyAsync(b + o_qw, q_world, 12ull * Q, cudaMemcpyHostToDevice, s));
-			MC_CUDA(cudaMemcpyAsync(b + o_qf, q_fill, 4ull * Q, cudaMemcpyHostToDevice, s));
+			MC_CUDA(cudaMemcpyAsync(up_qw, q_world, 12ull * Q, cudaMemcpyHostToDevice, s));
+			MC_CUDA(cudaMemcpyAsync(up_qf, q_fill, 4ull * Q, cudaMemcpyHostToDevice, s));
 			if (q_image) {
 				MC_TRY(reserve(ctx, ctx->q_image, 4ull * Q));
 				MC_CUDA(cudaMemcpyAsync(ctx->q_image.p, q_image, 4ull * Q, cudaMemcpyHostToDevice, s));
 				d_img = (const int32_t *)ctx->q_image.p;
 			}
 		}
-		MC_CUDA(cudaMemcpyAsync(b + o_d, depth, 4 * planes, cudaMemcpyHostToDevice, s));
-		MC_CUDA(cudaMemcpyAsync(b + o_fd, fill_distance, 4 * planes, cudaMemcpyHostToDevice, s));
+		MC_CUDA(cudaMemcpyAsync(up_depth, depth, 4 * planes, cudaMemcpyHostToDevice, s));
+		MC_CUDA(cudaMemcpyAsync(up_fill, fill_distance, 4 * planes, cudaMemcpyHostToDevice, s));
 		rs.q_desc = (const float *)ctx->q_desc.p; d_xy = (const float *)ctx->q_xy.p;
-		d_qw = (const float *)(b + o_qw); d_qf = (const float *)(b + o_qf); d_depth = (const float *)(b + o_d); d_fill = (const float *)(b + o_fd);
+		d_qw = up_qw; d_qf = up_qf; d_depth = up_depth; d_fill = up_fill;
 	}
 	DepthInputs in;
-	in.image = (const int32_t *)(b + o_img); in.xy = (const float *)(b + o_xy); in.xyz = (const float *)(b + o_xyz); in.world = (const float *)(b + o_w);
-	in.fill = (const float *)(b + o_f); in.depth = d_depth; in.distance = d_fill;
+	in.image = m_img; in.xy = m_xy; in.xyz = m_xyz; in.world = m_world; in.fill = m_fill; in.depth = d_depth; in.distance = d_fill;
 	struct Events {                                     // MATCH start / end, chain fork / join (stage_ms)
 		cudaEvent_t e[4] = {nullptr, nullptr, nullptr, nullptr};
 		~Events() { for (cudaEvent_t x : e) if (x) cudaEventDestroy(x); }
@@ -404,9 +374,8 @@ static mc_status depth_queries(mc_ctx *ctx, bool dev, const char *who, const Row
 	const size_t rows = n_range > 0 ? (size_t)n_range : 1;
 	std::vector<int32_t> moff(stride * rows), minfo(3 * rows, 0), status(rows, 0);
 	const mc_status sm = match_adaptive_frames(ctx, true, who, rs, d_xy, d_img, frame_offsets, n_frames, frame_begin, frame_end, d_depth, d_fill, width,
-	                                           height, models, n_models, maximum_depth, default_depth, cauchy_scale, moff.data(), (int32_t *)(b + o_feat),
-	                                           (int32_t *)in.image, (float *)in.xy, (float *)in.xyz, nullptr, nullptr, nullptr, minfo.data(), d_qw, d_qf,
-	                                           (float *)in.world, (float *)in.fill, stage_ms ? ev.e : nullptr);
+	                                           height, models, n_models, maximum_depth, default_depth, cauchy_scale, moff.data(), m_feat, m_img, m_xy,
+	                                           m_xyz, nullptr, nullptr, nullptr, minfo.data(), d_qw, d_qf, m_world, m_fill, stage_ms ? ev.e : nullptr);
 	bool match_failed = false;                          // frames MATCH left empty (its status 2, or 1 = over its cap)
 	for (int f = 0; f < n_range; f++)
 		if (minfo[3 * (size_t)f + 2]) { status[(size_t)f] = minfo[3 * (size_t)f + 2] == 2 ? 2 : 3; match_failed = true; }
@@ -535,25 +504,22 @@ mc_status mc_process_depth_frames(mc_ctx *ctx, const int32_t *match_offsets, int
 	}
 	MC_CUDA(cudaSetDevice(ctx->device));
 	const size_t px = (size_t)width * height, Ms = (size_t)M + 1;
-	size_t off = 0;
-	auto take = [&](size_t b) { size_t o = off; off += (b + 255) & ~(size_t)255; return o; };
-	const size_t o_im = take(4 * Ms), o_xy = take(8 * Ms), o_xyz = take(12 * Ms), o_w = take(12 * Ms), o_f = take(4 * Ms);
-	const size_t o_d = take(4 * px * n_frames), o_fd = take(4 * px * n_frames);
-	MC_TRY(reserve(ctx, ctx->scratch[15], off));
-	char *b = (char *)ctx->scratch[15].p;
+	int32_t *d_im; float *d_xy, *d_xyz, *d_w, *d_f, *d_d, *d_fd;
+	MC_TRY(carve_scratch(ctx, ctx->scratch[kScrDepthFramesIn], [&](Carve &c) {
+		c.take(d_im, Ms); c.take(d_xy, 2 * Ms); c.take(d_xyz, 3 * Ms); c.take(d_w, 3 * Ms); c.take(d_f, Ms);
+		c.take(d_d, px * n_frames); c.take(d_fd, px * n_frames);
+	}));
 	cudaStream_t s = ctx->stream;
 	if (M > 0) {
-		MC_CUDA(cudaMemcpyAsync(b + o_im, match_image, 4ull * M, cudaMemcpyHostToDevice, s));
-		MC_CUDA(cudaMemcpyAsync(b + o_xy, match_xy, 8ull * M, cudaMemcpyHostToDevice, s));
-		MC_CUDA(cudaMemcpyAsync(b + o_xyz, match_xyz, 12ull * M, cudaMemcpyHostToDevice, s));
-		MC_CUDA(cudaMemcpyAsync(b + o_w, match_world, 12ull * M, cudaMemcpyHostToDevice, s));
-		MC_CUDA(cudaMemcpyAsync(b + o_f, match_fill, 4ull * M, cudaMemcpyHostToDevice, s));
+		MC_CUDA(cudaMemcpyAsync(d_im, match_image, 4ull * M, cudaMemcpyHostToDevice, s));
+		MC_CUDA(cudaMemcpyAsync(d_xy, match_xy, 8ull * M, cudaMemcpyHostToDevice, s));
+		MC_CUDA(cudaMemcpyAsync(d_xyz, match_xyz, 12ull * M, cudaMemcpyHostToDevice, s));
+		MC_CUDA(cudaMemcpyAsync(d_w, match_world, 12ull * M, cudaMemcpyHostToDevice, s));
+		MC_CUDA(cudaMemcpyAsync(d_f, match_fill, 4ull * M, cudaMemcpyHostToDevice, s));
 	}
-	MC_CUDA(cudaMemcpyAsync(b + o_d, depth, 4 * px * n_frames, cudaMemcpyHostToDevice, s));
-	MC_CUDA(cudaMemcpyAsync(b + o_fd, fill_distance, 4 * px * n_frames, cudaMemcpyHostToDevice, s));
-	DepthInputs in;
-	in.image = (const int32_t *)(b + o_im); in.xy = (const float *)(b + o_xy); in.xyz = (const float *)(b + o_xyz); in.world = (const float *)(b + o_w);
-	in.fill = (const float *)(b + o_f); in.depth = (const float *)(b + o_d); in.distance = (const float *)(b + o_fd);
+	MC_CUDA(cudaMemcpyAsync(d_d, depth, 4 * px * n_frames, cudaMemcpyHostToDevice, s));
+	MC_CUDA(cudaMemcpyAsync(d_fd, fill_distance, 4 * px * n_frames, cudaMemcpyHostToDevice, s));
+	const DepthInputs in = { d_im, d_xy, d_xyz, d_w, d_f, d_d, d_fd };
 	return depth_frames_run(ctx, who, plans, meta, in, n_models, width, height, params, max_objects, n_objects, obj_model, obj_pose, obj_score,
 	                        frame_info, stage_ms);
 }

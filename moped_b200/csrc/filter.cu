@@ -318,7 +318,7 @@ static mc_status filter_device_impl(mc_ctx *ctx, const int32_t *d_match_offsets,
                         uint8_t *d_keep, float *d_score, int32_t *d_out_n, int32_t *d_cluster_model, int32_t *d_cluster_offsets,
                         int32_t *d_members, int32_t *d_surv_model, float *d_surv_pose, float *d_surv_score) {
 	if (!ctx->d_cams) { ctx->err = "filter: cameras not set (mc_set_cameras)"; return MC_ERR_STATE; }
-	DevBuf &b_in = ctx->scratch[5], &b_owner = ctx->scratch[6], &b_owned = ctx->scratch[7];
+	DevBuf &b_in = ctx->scratch[kScrFilterIn], &b_owner = ctx->scratch[kScrFilterOwner], &b_owned = ctx->scratch[kScrFilterOwned];
 	const int stride = max_matches > 0 ? max_matches : 1;
 	const int cap = n_obj_cap > 0 ? n_obj_cap : 1;
 	MC_TRY(reserve(ctx, b_in, (size_t)cap * stride));
@@ -326,7 +326,7 @@ static mc_status filter_device_impl(mc_ctx *ctx, const int32_t *d_match_offsets,
 	MC_TRY(reserve(ctx, b_owned, sizeof(int32_t) * (size_t)(cap + 1)));
 	// depth variant: ownership is decided by the projection score (d_raw), pruning and output use the penalised one (d_score)
 	float *d_raw = d_score;
-	if (D) { MC_TRY(reserve(ctx, ctx->scratch[22], sizeof(float) * (size_t)(cap + 1))); d_raw = (float *)ctx->scratch[22].p; }
+	if (D) { MC_TRY(reserve(ctx, ctx->scratch[kScrFilterRaw], sizeof(float) * (size_t)(cap + 1))); d_raw = (float *)ctx->scratch[kScrFilterRaw].p; }
 	if (n_obj_cap > 0) {
 		const int score_grid = (n_obj_cap * 32 + 127) / 128 < ctx->num_sms ? (n_obj_cap * 32 + 127) / 128 : ctx->num_sms;
 		k_filter_score<<<score_grid, 128, 0, ctx->stream>>>(d_match_offsets, d_match_image, d_match_xy, d_match_xyz, ctx->d_cams, d_obj_model,

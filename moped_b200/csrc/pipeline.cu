@@ -186,31 +186,18 @@ struct FrameBufs {
 };
 
 static mc_status carve(mc_ctx *ctx, FrameBufs &B, int Q, int n_models, int cl_cap, int task_cap, int obj_cap) {
-	size_t off = 0;
-	auto take = [&](size_t bytes) { size_t o = off; off += (bytes + 255) & ~(size_t)255; return o; };
-	const size_t o_nn_row = take(8ull * Q), o_nn_dist = take(8ull * Q), o_acc = take(Q);
-	const size_t o_acc_list = take(4ull * Q), o_moff = take(4ull * (n_models + 2)), o_mq = take(4ull * Q), o_mr = take(4ull * Q),
-	             o_mi = take(4ull * Q), o_mxy = take(8ull * Q), o_mxyz = take(12ull * Q);
-	const size_t o_status = take(64), o_cln = take(64), o_clm = take(4ull * (Q + 2)), o_clo = take(4ull * (Q + 2)), o_clmem = take(4ull * (Q + 2));
-	const size_t o_pxy = take(8ull * Q), o_pxyz = take(12ull * Q), o_pim = take(4ull * Q), o_ptie = take(4ull * Q);
-	const size_t o_found = take(task_cap), o_tpose = take(28ull * task_cap), o_ntests = take(4ull * task_cap);
-	const size_t o_nobj = take(64), o_om = take(4ull * obj_cap), o_op = take(28ull * obj_cap), o_os = take(4ull * obj_cap), o_keep = take(obj_cap);
-	const size_t o_fn = take(64), o_fm = take(4ull * (obj_cap + 2)), o_fo = take(4ull * (obj_cap + 2)), o_fmem = take(4ull * (Q + 2)),
-	             o_sm = take(4ull * obj_cap), o_sp = take(28ull * obj_cap), o_ss = take(4ull * obj_cap);
-	MC_TRY(reserve(ctx, ctx->scratch[10], off));
-	char *b = (char *)ctx->scratch[10].p;
-	B.nn_row = (int32_t *)(b + o_nn_row); B.nn_dist = (float *)(b + o_nn_dist); B.accepted = (uint8_t *)(b + o_acc);
-	B.acc_list = (int32_t *)(b + o_acc_list); B.match_offsets = (int32_t *)(b + o_moff); B.match_query = (int32_t *)(b + o_mq);
-	B.match_row = (int32_t *)(b + o_mr); B.match_image = (int32_t *)(b + o_mi); B.match_xy = (float *)(b + o_mxy); B.match_xyz = (float *)(b + o_mxyz);
-	B.status = (int32_t *)(b + o_status); B.cl_n = (int32_t *)(b + o_cln); B.cl_model = (int32_t *)(b + o_clm); B.cl_offsets = (int32_t *)(b + o_clo);
-	B.cl_members = (int32_t *)(b + o_clmem);
-	B.pt_xy = (float *)(b + o_pxy); B.pt_xyz = (float *)(b + o_pxyz); B.pt_image = (int32_t *)(b + o_pim); B.pt_tie = (int32_t *)(b + o_ptie);
-	B.found = (uint8_t *)(b + o_found); B.task_pose = (float *)(b + o_tpose); B.n_tests = (int32_t *)(b + o_ntests);
-	B.n_obj = (int32_t *)(b + o_nobj); B.obj_model = (int32_t *)(b + o_om); B.obj_pose = (float *)(b + o_op); B.obj_score = (float *)(b + o_os);
-	B.keep = (uint8_t *)(b + o_keep);
-	B.f_n = (int32_t *)(b + o_fn); B.f_model = (int32_t *)(b + o_fm); B.f_offsets = (int32_t *)(b + o_fo); B.f_members = (int32_t *)(b + o_fmem);
-	B.surv_model = (int32_t *)(b + o_sm); B.surv_pose = (float *)(b + o_sp); B.surv_score = (float *)(b + o_ss);
-	return MC_OK;
+	const size_t q = (size_t)Q, q2 = q + 2, o2 = (size_t)obj_cap + 2;
+	return carve_scratch(ctx, ctx->scratch[kScrFrame], [&](Carve &c) {
+		c.take(B.nn_row, 2 * q); c.take(B.nn_dist, 2 * q); c.take(B.accepted, q);
+		c.take(B.acc_list, q); c.take(B.match_offsets, (size_t)n_models + 2); c.take(B.match_query, q); c.take(B.match_row, q);
+		c.take(B.match_image, q); c.take(B.match_xy, 2 * q); c.take(B.match_xyz, 3 * q);
+		c.take(B.status, 16); c.take(B.cl_n, 16); c.take(B.cl_model, q2); c.take(B.cl_offsets, q2); c.take(B.cl_members, q2);
+		c.take(B.pt_xy, 2 * q); c.take(B.pt_xyz, 3 * q); c.take(B.pt_image, q); c.take(B.pt_tie, q);
+		c.take(B.found, task_cap); c.take(B.task_pose, 7 * (size_t)task_cap); c.take(B.n_tests, task_cap);
+		c.take(B.n_obj, 16); c.take(B.obj_model, obj_cap); c.take(B.obj_pose, 7 * (size_t)obj_cap); c.take(B.obj_score, obj_cap); c.take(B.keep, obj_cap);
+		c.take(B.f_n, 16); c.take(B.f_model, o2); c.take(B.f_offsets, o2); c.take(B.f_members, q2);
+		c.take(B.surv_model, obj_cap); c.take(B.surv_pose, 7 * (size_t)obj_cap); c.take(B.surv_score, obj_cap);
+	});
 }
 
 struct FrameCaps { int cl_cap, obj_cap, task_cap; };
@@ -463,17 +450,16 @@ mc_status process_frame_device(mc_ctx *ctx, const float *d_q, const float *d_qxy
 //   phase 1  (gathered records) objects, FILTER, POSE2 tasks     -> record in slot `rank`
 //   phase 2  (gathered records) objects, FILTER2, export
 // Record of a phase: found[task_cap] (bytes) | pose[task_cap][7] | n_tests[task_cap], each part 256-byte aligned.
-struct ShardSlot { uint8_t *found; float *pose; int32_t *n_tests; };
+struct ShardSlot { uint8_t *found; float *pose; int32_t *n_tests; size_t bytes; };
 
-static size_t shard_slot_bytes(int task_cap) {
-	auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
-	return up((size_t)task_cap) + up(28ull * task_cap) + up(4ull * task_cap);
-}
+// record `slot` of `exchange`; exchange == nullptr: the record's size only
 static ShardSlot shard_slot(void *exchange, int slot, int task_cap) {
-	auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
-	char *b = (char *)exchange + (size_t)slot * shard_slot_bytes(task_cap);
 	ShardSlot s;
-	s.found = (uint8_t *)b; s.pose = (float *)(b + up((size_t)task_cap)); s.n_tests = (int32_t *)(b + up((size_t)task_cap) + up(28ull * task_cap));
+	auto layout = [&](Carve &c) { c.take(s.found, task_cap); c.take(s.pose, 7 * (size_t)task_cap); c.take(s.n_tests, task_cap); };
+	Carve c;
+	layout(c);
+	s.bytes = c.off;
+	if (exchange) { c = Carve{(char *)exchange + (size_t)slot * s.bytes}; layout(c); }
 	return s;
 }
 
@@ -490,7 +476,7 @@ __global__ void k_shard_select(const uint8_t *__restrict__ exchange, size_t slot
 	n_tests[t] = ((const int32_t *)(b + o_tests))[t];
 }
 
-size_t frame_shard_slot_bytes(int Q, const mc_pipeline_params *P) { return shard_slot_bytes(frame_caps(Q, P).task_cap); }
+size_t frame_shard_slot_bytes(int Q, const mc_pipeline_params *P) { return shard_slot(nullptr, 0, frame_caps(Q, P).task_cap).bytes; }
 
 mc_status process_frame_sharded_device(mc_ctx *ctx, int phase, const int32_t *d_nn_row, const uint8_t *d_accepted, const float *d_qxy,
                                        const int32_t *d_qimg, int Q, const mc_pipeline_params *P, int shard_rank, int shard_world, void *d_exchange,
@@ -502,11 +488,10 @@ mc_status process_frame_sharded_device(mc_ctx *ctx, int phase, const int32_t *d_
 	FrameBufs B;
 	MC_TRY(carve(ctx, B, Q, ctx->n_models, caps.cl_cap, caps.task_cap, caps.obj_cap));
 	const FrameDesc *fd = (const FrameDesc *)ctx->frame_desc.p;
-	const size_t slot_bytes = shard_slot_bytes(caps.task_cap);
 	const ShardSlot mine = shard_slot(d_exchange, shard_rank, caps.task_cap), base = shard_slot(d_exchange, 0, caps.task_cap);
 	const size_t o_pose = (size_t)((char *)base.pose - (char *)base.found), o_tests = (size_t)((char *)base.n_tests - (char *)base.found);
 	auto select = [&](int n_tasks, int max_obj) -> mc_status {
-		k_shard_select<<<(n_tasks + 255) / 256, 256, 0, ctx->stream>>>((const uint8_t *)d_exchange, slot_bytes, o_pose, o_tests, shard_world, n_tasks, max_obj,
+		k_shard_select<<<(n_tasks + 255) / 256, 256, 0, ctx->stream>>>((const uint8_t *)d_exchange, base.bytes, o_pose, o_tests, shard_world, n_tasks, max_obj,
 		                                                              B.found, B.task_pose, B.n_tests);
 		MC_LAUNCH_CHECK();
 		return MC_OK;
@@ -846,46 +831,46 @@ mc_status process_frames_device(mc_ctx *ctx, const float *d_q, const float *d_qx
 mc_status process_frames_host(mc_ctx *ctx, const float *d_q, const float *d_qxy, const int32_t *d_qimg, const int32_t *frame_offsets, int n_frames,
                               const mc_pipeline_params *P, int max_objects, int32_t *n_objects, int32_t *obj_model, float *obj_pose, float *obj_score,
                               int32_t *frame_info, float *stage_ms) {
-	const size_t per = 16 + (size_t)max_objects * 36;
-	const size_t bytes = per * (size_t)n_frames;
+	const size_t bytes = batch_slots_bytes(n_frames, max_objects);
 	MC_TRY(reserve(ctx, ctx->batch_out, bytes + 256));
 	MC_TRY(pinned(ctx, bytes + 256));
-	char *d = (char *)ctx->batch_out.p;
-	int32_t *d_info = (int32_t *)d;
-	int32_t *d_model = (int32_t *)(d + 16ull * n_frames);
-	float *d_pose = (float *)(d + (16ull + 4ull * max_objects) * n_frames);
-	float *d_score = (float *)(d + (16ull + 32ull * max_objects) * n_frames);
+	const BatchSlots d = batch_slots(ctx->batch_out.p, n_frames, max_objects);
 	cudaEvent_t ev[3];
 	if (stage_ms) for (int i = 0; i < 3; i++) MC_CUDA(cudaEventCreate(&ev[i]));
-	MC_TRY(process_frames_device(ctx, d_q, d_qxy, d_qimg, frame_offsets, 0, n_frames, P, max_objects, nullptr, nullptr, d_info, d_model, d_pose, d_score,
+	MC_TRY(process_frames_device(ctx, d_q, d_qxy, d_qimg, frame_offsets, 0, n_frames, P, max_objects, nullptr, nullptr, d.info, d.model, d.pose, d.score,
 	                             stage_ms ? ev : nullptr));
-	char *h = (char *)ctx->h_pinned;
-	MC_CUDA(cudaMemcpyAsync(h, d, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+	MC_CUDA(cudaMemcpyAsync(ctx->h_pinned, ctx->batch_out.p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
 	MC_CUDA(cudaStreamSynchronize(ctx->stream));
 	if (stage_ms) {
 		cudaEventElapsedTime(&stage_ms[0], ev[0], ev[1]);
 		cudaEventElapsedTime(&stage_ms[1], ev[1], ev[2]);
 		for (int i = 0; i < 3; i++) cudaEventDestroy(ev[i]);
 	}
-	const int32_t *h_info = (const int32_t *)h;
-	const int32_t *h_model = (const int32_t *)(h + 16ull * n_frames);
-	const float *h_pose = (const float *)(h + (16ull + 4ull * max_objects) * n_frames);
-	const float *h_score = (const float *)(h + (16ull + 32ull * max_objects) * n_frames);
-	mc_status st = MC_OK;
+	const BatchSlots h = batch_slots(ctx->h_pinned, n_frames, max_objects);
 	int tot_m = 0, tot_o = 0;
-	for (int f = 0; f < n_frames; f++) {
-		const int n = h_info[4 * f];
-		if (frame_info) memcpy(frame_info + 4 * f, h_info + 4 * f, 16);
-		n_objects[f] = n;
-		tot_m += h_info[4 * f + 2]; tot_o += n;
-		if (h_info[4 * f + 1]) { ctx->err = "process_frames: more than 8192 accepted matches in one frame"; st = MC_ERR_CAPACITY; continue; }
-		if (n > max_objects) { ctx->err = "process_frames: object buffer too small"; st = MC_ERR_CAPACITY; continue; }
-		memcpy(obj_model + (size_t)f * max_objects, h_model + (size_t)f * max_objects, 4ull * n);
-		memcpy(obj_pose + 7 * (size_t)f * max_objects, h_pose + 7 * (size_t)f * max_objects, 28ull * n);
-		memcpy(obj_score + (size_t)f * max_objects, h_score + (size_t)f * max_objects, 4ull * n);
-	}
+	for (int f = 0; f < n_frames; f++) { tot_m += h.info[4 * f + 2]; tot_o += h.info[4 * f]; }
 	ctx->batch_stats[1] = tot_m; ctx->batch_stats[2] = tot_o;
-	return st;
+	int first_bad, first_over;
+	unpack_batch(h, n_frames, max_objects, n_objects, obj_model, obj_pose, obj_score, frame_info, first_bad, first_over);
+	if (first_bad >= 0) { ctx->err = "process_frames: more than 8192 accepted matches in one frame"; return MC_ERR_CAPACITY; }
+	if (first_over >= 0) { ctx->err = "process_frames: object buffer too small"; return MC_ERR_CAPACITY; }
+	return MC_OK;
+}
+
+void unpack_batch(const BatchSlots &h, int n_frames, int max_objects, int32_t *n_objects, int32_t *obj_model, float *obj_pose, float *obj_score,
+                  int32_t *frame_info, int &first_bad, int &first_over) {
+	first_bad = first_over = -1;
+	for (int f = 0; f < n_frames; f++) {
+		const int n = h.info[4 * f];
+		if (frame_info) memcpy(frame_info + 4 * f, h.info + 4 * f, 16);
+		n_objects[f] = n;
+		if (h.info[4 * f + 1]) { if (first_bad < 0) first_bad = f; continue; }
+		if (n > max_objects) { if (first_over < 0) first_over = f; continue; }
+		const size_t at = (size_t)f * max_objects;
+		memcpy(obj_model + at, h.model + at, 4ull * n);
+		memcpy(obj_pose + 7 * at, h.pose + 7 * at, 28ull * n);
+		memcpy(obj_score + at, h.score + at, 4ull * n);
+	}
 }
 
 } // namespace mc

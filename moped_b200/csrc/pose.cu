@@ -1059,8 +1059,9 @@ mc_status pose_hypotheses_device(mc_ctx *ctx, const int32_t *d_cluster_offsets, 
 	// many hypotheses and no inlier masks wanted: one thread per hypothesis; otherwise one 8-lane group per hypothesis
 	if (!d_mask && n_hyp >= ctx->fit_thread_min && ctx->fit_stream) {
 		// persistent phase-synchronous kernel + scoring kernel (the default throughput shape)
-		MC_TRY(reserve(ctx, ctx->scratch[20], 256));
-		MC_CUDA(cudaMemsetAsync(ctx->scratch[20].p, 0, 256, ctx->stream));
+		DevBuf &b_fit = ctx->scratch[kScrFitStream];
+		MC_TRY(reserve(ctx, b_fit, 256));
+		MC_CUDA(cudaMemsetAsync(b_fit.p, 0, 256, ctx->stream));
 #define MC_FIT_STREAM(S, MINB)                                                                                                               \
 		do {                                                                                                                                 \
 			const size_t smem = (size_t)(S) * kStreamFloats * kStreamThreads * sizeof(float);                                                           \
@@ -1071,7 +1072,7 @@ mc_status pose_hypotheses_device(mc_ctx *ctx, const int32_t *d_cluster_offsets, 
 			const int64_t want = ((int64_t)n_hyp + kStreamThreads - 1) / kStreamThreads, cap = (int64_t)per_sm * ctx->num_sms;                \
 			k_pose_fit_stream<S, MINB><<<(unsigned)(want < cap ? want : cap), kStreamThreads, smem, ctx->stream>>>(                          \
 			    d_cluster_offsets, d_xy, d_xyz, d_image, ctx->d_cams, d_hyp_cluster, d_sample_pos, d_init_quat, n_hyp, pp->n_pts_align,      \
-			    pp->max_lm_tests, (uint32_t *)ctx->scratch[20].p, d_n_inliers, d_pose_lm, d_lm_err);                                         \
+			    pp->max_lm_tests, (uint32_t *)b_fit.p, d_n_inliers, d_pose_lm, d_lm_err);                                                    \
 		} while (0)
 		if (pp->n_pts_align <= 5) MC_FIT_STREAM(5, 3);       // (4 CTAs per SM at 128 registers: measured, no gain — 5.00 vs 4.95 ms per 131072 hypotheses)
 		else if (pp->n_pts_align == 6) MC_FIT_STREAM(6, 3);
@@ -1082,8 +1083,8 @@ mc_status pose_hypotheses_device(mc_ctx *ctx, const int32_t *d_cluster_offsets, 
 		                                                        pp->error_threshold, d_n_inliers, d_pose_lm);
 		MC_LAUNCH_CHECK();
 		// refit of the accepted ones from per-size lists
-		MC_TRY(reserve(ctx, ctx->scratch[21], 256 + sizeof(int32_t) * (size_t)kRefitBuckets * n_hyp));
-		int32_t *counts = (int32_t *)ctx->scratch[21].p, *lists = counts + 64;
+		MC_TRY(reserve(ctx, ctx->scratch[kScrRefitLists], 256 + sizeof(int32_t) * (size_t)kRefitBuckets * n_hyp));
+		int32_t *counts = (int32_t *)ctx->scratch[kScrRefitLists].p, *lists = counts + 64;
 		MC_CUDA(cudaMemsetAsync(counts, 0, 256, ctx->stream));
 		k_refit_buckets<<<(n_hyp + 255) / 256, 256, 0, ctx->stream>>>(n_hyp, pp->min_npts_object, d_n_inliers, d_pose_lm, d_pose_refit, counts, lists);
 		MC_LAUNCH_CHECK();

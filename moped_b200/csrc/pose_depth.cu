@@ -141,8 +141,8 @@ k_depth_ransac(const int32_t *__restrict__ cluster_offsets, int n_clusters_cap, 
 static mc_status depth_scratch(mc_ctx *ctx, size_t warps, size_t slice, float **out) {
 	const size_t bytes = warps * slice * sizeof(float);
 	if (bytes > (size_t)8 << 30) { ctx->err = "pose (depth): cluster too large for the per-warp LM scratch"; return MC_ERR_ARG; }
-	MC_TRY(reserve(ctx, ctx->scratch[17], bytes));
-	*out = (float *)ctx->scratch[17].p;
+	MC_TRY(reserve(ctx, ctx->scratch[kScrDepthLm], bytes));
+	*out = (float *)ctx->scratch[kScrDepthLm].p;
 	return MC_OK;
 }
 

@@ -251,19 +251,14 @@ mc_status ransac_staged_launch(mc_ctx *ctx, const int32_t *d_cluster_offsets, co
 		L.slot_base[l] = L.slots;
 		L.slots += (L.h_begin[l + 1] - L.h_begin[l] + L.hpi[l] - 1) / L.hpi[l];
 	}
-	size_t off = 0;
-	auto take = [&](size_t bytes) { size_t o = off; off += (bytes + 255) & ~(size_t)255; return o; };
-	const size_t o_first = take(4ull * n_tasks), o_done = take(4ull * n_tasks), o_qpos = take(4ull * n_tasks), o_queue = take(4ull * n_tasks),
-	             o_cnt = take(64), o_fail = take(n_tasks), o_fit = take(28ull * n_tasks * HA),
-	             o_chunk = take(28ull * n_tasks * (L.slots > 0 ? L.slots : 1));
 	const size_t refit_floats = ((size_t)P::kRefitFloatsPerPoint * n_points_cap + (size_t)P::kRefitFloatsPerTask * n_clusters_cap) * pp->max_objects_per_cluster;
-	const size_t o_refit = take(4ull * refit_floats);
-	MC_TRY(reserve(ctx, ctx->scratch[16], off));
-	char *b = (char *)ctx->scratch[16].p;
+	const size_t nt = (size_t)n_tasks;
 	RansacState S;
-	S.first = (int32_t *)(b + o_first); S.done = (int32_t *)(b + o_done); S.qpos = (int32_t *)(b + o_qpos); S.queue = (int32_t *)(b + o_queue);
-	S.counters = (int32_t *)(b + o_cnt); S.fail = (uint8_t *)(b + o_fail); S.fit_pose = (float *)(b + o_fit); S.chunk_pose = (float *)(b + o_chunk);
-	S.refit_scratch = refit_floats ? (float *)(b + o_refit) : nullptr;
+	MC_TRY(carve_scratch(ctx, ctx->scratch[kScrRansac], [&](Carve &c) {
+		c.take(S.first, nt); c.take(S.done, nt); c.take(S.qpos, nt); c.take(S.queue, nt); c.take(S.counters, 16); c.take(S.fail, nt);
+		c.take(S.fit_pose, 7 * nt * HA); c.take(S.chunk_pose, 7 * nt * (L.slots > 0 ? L.slots : 1)); c.take(S.refit_scratch, refit_floats);
+	}));
+	if (!refit_floats) S.refit_scratch = nullptr;
 	S.shard_rank = ctx->ransac_shard_rank; S.shard_world = ctx->ransac_shard_world;
 	k_ransac_init<<<(n_tasks + 255) / 256, 256, 0, ctx->stream>>>(S, n_tasks);
 	MC_LAUNCH_CHECK();
