@@ -409,11 +409,32 @@ mc_status mc_sift_extract(mc_ctx *ctx, const uint8_t *gray, int n_images, int he
  * mc_process_frames_dev without leaving HBM. counts_dev may exceed max_keypoints (see above). */
 mc_status mc_sift_extract_dev(mc_ctx *ctx, const uint8_t *gray_dev, int n_images, int height, int width, int double_size,
                               int max_keypoints, float *xy_dev, float *scale_ori_dev, float *desc_dev, int32_t *counts_dev);
+/* ---- UNDISTORTED_IMAGE (UTIL_UNDISTORT), the step both pipelines register before SIFT (pipeline3d_cuda.hpp:2) ---------------- */
+/* UNDISTORTED_IMAGE (UTIL_UNDISTORT: cvInitUndistortMap + cvRemap, bilinear, constant border 0) for images of camera `camera`:
+ * K = (fx, fy, cx, cy) as given to mc_set_cameras, kc = OpenCV's (k1, k2, p1, p2[, k3]), n_kc 4 or 5; kc == NULL clears.
+ * The remap table of a height x width image is built on the host once per call, in double precision in the order of OpenCV's
+ * scalar loop, and kept in device memory the context owns (8 bytes per pixel: 2.4 MB for 640x480) until the camera is set again,
+ * cleared, or mc_destroy. Images undistorted with it equal cv2.initUndistortRectifyMap(K, kc, None, K, (width, height), CV_32FC1)
+ * followed by cv2.remap(INTER_LINEAR, BORDER_CONSTANT, 0) bit for bit (K and kc rounded to float as here).
+ * Errors (the previous table stays): MC_ERR_ARG for camera outside 0..15, n_kc other than 4 or 5, a non-finite K or kc, fx or fy
+ * equal to 0, height or width outside 8..32767. */
+mc_status mc_set_undistortion(mc_ctx *ctx, int camera, const float *K, const float *kc, int n_kc, int height, int width);
+/* n_images images of camera `camera` (height x width bytes each) -> out, same layout; one kernel launch for the batch.
+ * Errors: MC_ERR_STATE when the camera has no table; MC_ERR_ARG for a NULL pointer, n_images outside 1..65535, a camera outside
+ * 0..15 or a size other than the table's. */
+mc_status mc_undistort(mc_ctx *ctx, int camera, const uint8_t *gray, int n_images, int height, int width, uint8_t *out);
+/* Same with device pointers, asynchronous on the context's stream (gray_dev and out_dev must not overlap): composes with
+ * mc_sift_extract_dev for camera rigs. */
+mc_status mc_undistort_dev(mc_ctx *ctx, int camera, const uint8_t *gray_dev, int n_images, int height, int width, uint8_t *out_dev);
+
 /* Images in, objects out: FEAT chained to MATCH..FILTER2 for a batch of n_frames single-camera frames of one size (each
  * frame is what Moped::processImages gets with one image, moped2/libmoped/src/moped.cpp:166-194; camera 0 of
- * mc_set_cameras applies to every frame). Descriptors stay in HBM between the steps, normalised on the device with the
+ * mc_set_cameras applies to every frame). When camera 0 has an undistortion table (mc_set_undistortion), the uploaded batch is
+ * undistorted on the device first (one more launch), as UNDISTORTED_IMAGE runs before SIFT in the reference's pipeline; a size
+ * other than the table's returns MC_ERR_ARG before any launch. Without a table the images go to SIFT as given.
+ * Descriptors stay in HBM between the steps, normalised on the device with the
  * MATCH stage's expression. Outputs like mc_process_frames; n_features (optional) = keypoints per frame;
- * stage_ms (optional, 3 floats) = device time of FEAT (incl. the image upload), MATCH, CLUSTER..FILTER2. */
+ * stage_ms (optional, 3 floats) = device time of FEAT (incl. the image upload and undistortion), MATCH, CLUSTER..FILTER2. */
 mc_status mc_process_images(mc_ctx *ctx, const uint8_t *gray, int n_frames, int height, int width, int double_size, int max_keypoints,
                             const mc_pipeline_params *params, int max_objects, int32_t *n_objects, int32_t *obj_model, float *obj_pose,
                             float *obj_score, int32_t *n_features, int32_t *frame_info, float *stage_ms);

@@ -15,7 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "libmoped_cuda.so")
-SOURCES = ["api.cu", "match.cu", "adaptive.cu", "cluster.cu", "pose.cu", "pose_exact.cu", "pose_depth.cu", "filter.cu", "pipeline.cu", "depth_frames.cu", "sift.cu", "linkage.cu", "sm_partition.cu", "model_db.cpp"]
+SOURCES = ["api.cu", "match.cu", "adaptive.cu", "cluster.cu", "pose.cu", "pose_exact.cu", "pose_depth.cu", "filter.cu", "pipeline.cu", "depth_frames.cu", "sift.cu", "undistort.cu", "linkage.cu", "sm_partition.cu", "model_db.cpp"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 COMMON = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC", "-Xcompiler", "-Wall"] + os.environ.get("MOPED_NVCC_FLAGS", "").split()
 LIB = os.environ.get("MOPED_LIB", LIB)
@@ -23,7 +23,8 @@ LIB = os.environ.get("MOPED_LIB", LIB)
 # sift.cu keeps multiply and add separate so that its sums round like the reference's scalar code; filter.cu likewise (its
 # reprojections and scores then equal the oracle's bit for bit: ownership and pruning decisions can never differ by a rounding)
 PER_FILE = {"pose.cu": ["-ftz=true"], "pose_depth.cu": ["-ftz=true", "-fmad=false"], "pose_exact.cu": ["-ftz=true", "-fmad=false"], "sift.cu": ["-fmad=false"], "filter.cu": ["-fmad=false"], "linkage.cu": ["-fmad=false"],
-            "adaptive.cu": ["-Xcompiler", "-ffp-contract=off"]}   # its host arithmetic (ratio curves) rounds like a strict-IEEE build
+            "adaptive.cu": ["-Xcompiler", "-ffp-contract=off"],   # its host arithmetic (ratio curves) rounds like a strict-IEEE build
+            "undistort.cu": ["-Xcompiler", "-ffp-contract=off"]}  # likewise its host remap tables (OpenCV's scalar loop in double)
 
 
 def nvcc() -> str:

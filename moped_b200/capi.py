@@ -166,6 +166,9 @@ SIGNATURES = {
                                                       C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_float, C.c_float, C.c_float,
                                                       C.POINTER(DepthPipelineParams), C.c_int, _i32p, _i32p, _f32p, _f32p, _i32p, C.c_void_p]),
     "mc_set_depth_filter": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(DepthFilterParams), C.c_void_p, C.c_void_p, C.c_int]),
+    "mc_set_undistortion": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int]),
+    "mc_undistort": (C.c_int, [C.c_void_p, C.c_int, _u8p, C.c_int, C.c_int, C.c_int, _u8p]),
+    "mc_undistort_dev": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
 }
 
 MC_ERR_ARG = -2
@@ -639,6 +642,27 @@ class Context:
         if want_times:
             out[0]["stage_ms"] = ms
         return out
+
+    def set_undistortion(self, camera, K, kc, height, width):
+        """mc_set_undistortion: UNDISTORTED_IMAGE for camera `camera` (K = (fx, fy, cx, cy), kc = (k1, k2, p1, p2[, k3])) on
+        height x width images; kc=None clears the camera's table."""
+        if kc is None:
+            self._check(self.L.mc_set_undistortion(self.h, int(camera), None, None, 0, int(height), int(width)), "mc_set_undistortion")
+            return
+        Kf, kf = _f32(K).reshape(-1), _f32(kc).reshape(-1)
+        self._check(self.L.mc_set_undistortion(self.h, int(camera), Kf.ctypes.data, kf.ctypes.data, len(kf), int(height), int(width)),
+                    "mc_set_undistortion")
+
+    def undistort(self, gray, camera=0):
+        """mc_undistort: a batch [B,H,W] (or one [H,W]) of uint8 images of `camera` -> the undistorted images, same shape"""
+        g = np.ascontiguousarray(gray, dtype=np.uint8)
+        b = g.reshape((-1,) + g.shape[-2:])
+        out = np.empty_like(b)
+        self._check(self.L.mc_undistort(self.h, int(camera), b.reshape(-1), b.shape[0], b.shape[1], b.shape[2], out.reshape(-1)), "mc_undistort")
+        return out.reshape(g.shape)
+
+    def undistort_dev(self, gray_ptr, B, H, W, out_ptr, camera=0):
+        self._check(self.L.mc_undistort_dev(self.h, int(camera), gray_ptr, B, H, W, out_ptr), "mc_undistort_dev")
 
     def sift_dev(self, gray_ptr, B, H, W, double_size, max_keypoints, xy_ptr, so_ptr, desc_ptr, counts_ptr):
         self._check(self.L.mc_sift_extract_dev(self.h, gray_ptr, B, H, W, 1 if double_size else 0, max_keypoints, xy_ptr, so_ptr, desc_ptr,

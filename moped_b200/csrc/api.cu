@@ -137,6 +137,7 @@ void mc_destroy(mc_ctx *ctx) {
 	sift_free(ctx);
 	cudaFree(ctx->d_cams);
 	for (DepthFilterTable &t : ctx->depth_filter) { cudaFree(t.d_offsets); cudaFree(t.d_xyz); }
+	for (UndistortTable &t : ctx->undistort) cudaFree(t.d_map);
 	free_scratch(ctx);
 	if (ctx->own_stream) cudaStreamDestroy(ctx->stream);
 	delete ctx;

@@ -75,6 +75,7 @@ enum ScratchSlot : int {
 	// alternates them reuses the larger allocation
 	kScrHostPoseDepth,        // mc_pose_depth_hypotheses, mc_pose_depth_ransac
 	kScrHostFilter,           // mc_filter_projection, mc_filter_projection_depth
+	kScrUndistort,            // mc_undistort: the uploaded images and their undistorted copies
 	kScratchSlots
 };
 
@@ -106,6 +107,14 @@ struct DepthFilterTable {
 	int n_models = 0;
 	float plausible_sq_distance = 0.f, depth_fraction = 0.f, min_keypoint_fraction = 0.f;
 	float K[4] = {0.f, 0.f, 0.f, 0.f}, TM[12] = {0.f};
+};
+
+// UNDISTORTED_IMAGE of one camera (mc_set_undistortion): a RemapEntry per pixel, then the 32 x 32 RemapWeights (undistort.cuh), in
+// one device allocation the context owns. d_map == nullptr: no table.
+constexpr int kUndistortCameras = 16;
+struct UndistortTable {
+	void *d_map = nullptr;
+	int height = 0, width = 0;
 };
 
 } // namespace mc
@@ -193,6 +202,7 @@ struct mc_ctx {
 	mc::DevBuf link_buf;                 // linkage clustering (linkage.cu): inputs, similarity matrices, agglomeration state
 	mc::DepthFilterTable depth_filter[2];   // FILTER / FILTER2 of mc_process_depth_frames* / _queries* (mc_set_depth_filter)
 	void *sift_state = nullptr;          // feature extraction (sift.cu): scale-space plan and buffers, created on first use
+	mc::UndistortTable undistort[mc::kUndistortCameras];   // per camera (mc_set_undistortion); camera 0 serves mc_process_images
 };
 
 namespace mc {
@@ -271,6 +281,7 @@ size_t frame_shard_slot_bytes(int Q, const mc_pipeline_params *P);
 mc_status process_frame_sharded_device(mc_ctx *ctx, int phase, const int32_t *d_nn_row, const uint8_t *d_accepted, const float *d_qxy,
                                        const int32_t *d_qimg, int Q, const mc_pipeline_params *P, int shard_rank, int shard_world, void *d_exchange,
                                        int max_objects, int32_t *d_out_info, int32_t *d_out_model, float *d_out_pose, float *d_out_score);
+mc_status undistort_device(mc_ctx *ctx, int camera, const uint8_t *d_in, int B, int H, int W, uint8_t *d_out);
 mc_status match_device(mc_ctx *ctx, const float *d_q, int Q, float ratio, int mode,
                        int32_t *d_nn_row, float *d_nn_dist, uint8_t *d_accepted);
 

@@ -1100,21 +1100,39 @@ extern "C" mc_status mc_process_images(mc_ctx *ctx, const uint8_t *gray, int n_f
 	}
 	if (!ctx->d_db) { ctx->err = "mc_process_images: no database uploaded"; return MC_ERR_STATE; }
 	if (ctx->D != 128) { ctx->err = "mc_process_images: the database does not hold 128-d descriptors"; return MC_ERR_STATE; }
+	// UNDISTORTED_IMAGE before SIFT when camera 0 has a table (mc_set_undistortion); its size is checked before anything is queued
+	const UndistortTable &und = ctx->undistort[0];
+	if (und.d_map && (und.height != height || und.width != width)) {
+		ctx->err = "mc_process_images: images are " + std::to_string(width) + "x" + std::to_string(height) + ", camera 0's undistortion table is " +
+		           std::to_string(und.width) + "x" + std::to_string(und.height);
+		return MC_ERR_ARG;
+	}
 	MC_CUDA(cudaSetDevice(ctx->device));
 	SiftState *s = state(ctx);
 	const size_t npx = (size_t)n_frames * height * width, nk = (size_t)n_frames * max_keypoints;
-	MC_TRY(reserve(ctx, s->gray, ((npx + 255) & ~(size_t)255) + nk * (2 + 128 + 1) * sizeof(float) + (size_t)(2 * n_frames + 2) * sizeof(int32_t) + 1024));
-	uint8_t *d_gray = (uint8_t *)s->gray.p;
-	float *d_xy = (float *)(d_gray + ((npx + 255) & ~(size_t)255));
-	float *d_desc = d_xy + nk * 2;
-	int32_t *d_qimg = (int32_t *)(d_desc + nk * 128);
-	int32_t *d_counts = d_qimg + nk, *d_offsets = d_counts + n_frames;
+	uint8_t *d_gray = nullptr, *d_undist = nullptr;
+	float *d_xy = nullptr, *d_desc = nullptr;
+	int32_t *d_qimg = nullptr, *d_counts = nullptr;
+	MC_TRY(carve_scratch(ctx, s->gray, [&](Carve &c) {
+		c.take(d_gray, npx);
+		c.take(d_undist, und.d_map ? npx : 0);
+		c.take(d_xy, nk * 2);
+		c.take(d_desc, nk * 128);
+		c.take(d_qimg, nk);
+		c.take(d_counts, (size_t)2 * n_frames + 2);       // counts[n_frames], then offsets[n_frames + 1]
+	}));
+	int32_t *d_offsets = d_counts + n_frames;
 	MC_TRY(pinned(ctx, (size_t)(2 * n_frames + 2) * sizeof(int32_t)));
 	cudaEvent_t ev[2];
 	if (stage_ms) { MC_CUDA(cudaEventCreate(&ev[0])); MC_CUDA(cudaEventCreate(&ev[1])); MC_CUDA(cudaEventRecord(ev[0], ctx->stream)); }
 	MC_CUDA(cudaMemcpyAsync(d_gray, gray, npx, cudaMemcpyHostToDevice, ctx->stream));
 	MC_CUDA(cudaMemsetAsync(d_qimg, 0, nk * sizeof(int32_t), ctx->stream));           // one camera per frame: imageIdx = 0
-	MC_TRY(sift_extract_device(ctx, d_gray, n_frames, height, width, double_size, max_keypoints, d_xy, nullptr, d_desc, d_counts, d_offsets, 1));
+	const uint8_t *d_feat_in = d_gray;
+	if (und.d_map) {
+		MC_TRY(undistort_device(ctx, 0, d_gray, n_frames, height, width, d_undist));
+		d_feat_in = d_undist;
+	}
+	MC_TRY(sift_extract_device(ctx, d_feat_in, n_frames, height, width, double_size, max_keypoints, d_xy, nullptr, d_desc, d_counts, d_offsets, 1));
 	int32_t *h = (int32_t *)ctx->h_pinned;
 	MC_CUDA(cudaMemcpyAsync(h, d_counts, (size_t)(2 * n_frames + 1) * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
 	if (stage_ms) MC_CUDA(cudaEventRecord(ev[1], ctx->stream));
