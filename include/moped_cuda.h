@@ -438,6 +438,21 @@ mc_status mc_undistort_dev(mc_ctx *ctx, int camera, const uint8_t *gray_dev, int
 mc_status mc_process_images(mc_ctx *ctx, const uint8_t *gray, int n_frames, int height, int width, int double_size, int max_keypoints,
                             const mc_pipeline_params *params, int max_objects, int32_t *n_objects, int32_t *obj_model, float *obj_pose,
                             float *obj_score, int32_t *n_features, int32_t *frame_info, float *stage_ms);
+/* Images in, objects out for camera rigs: n_frames frames of n_cameras images each, gray = [n_frames][n_cameras][height][width]
+ * bytes, all of one size. Frame f is what Moped::processImages gets with n_cameras images: image c of every frame belongs to camera c,
+ * whose intrinsics and pose are entry c of mc_set_cameras and whose undistortion table, if it has one, is camera c's of
+ * mc_set_undistortion (an image of a camera without a table goes to SIFT as given; one remap launch serves the whole batch, none
+ * when no camera of the rig has a table). The frame's query list is the keypoints of camera 0, then camera 1, ..., each in
+ * FEAT_SIFT_CPU's order with imageIdx = camera, as FEAT_SIFT_CUDA::process appends them; MATCH..FILTER2 run as in
+ * mc_process_frames. Outputs as mc_process_images, except n_features (optional) = n_frames x n_cameras keypoint counts, one per
+ * image, in input order. n_cameras = 1 is mc_process_images (same outputs, same launches) with the camera check below.
+ * Errors, all before any launch: MC_ERR_ARG for n_cameras outside 1..16, n_frames x n_cameras above 65535, or a camera of the rig
+ * whose table is not height x width; MC_ERR_STATE when mc_set_cameras set fewer than n_cameras cameras, and as mc_process_images.
+ * An image with more than max_keypoints keypoints returns MC_ERR_CAPACITY; n_features still holds the numbers found. */
+mc_status mc_process_rig_images(mc_ctx *ctx, const uint8_t *gray, int n_frames, int n_cameras, int height, int width,
+                                int double_size, int max_keypoints, const mc_pipeline_params *params, int max_objects,
+                                int32_t *n_objects, int32_t *obj_model, float *obj_pose, float *obj_score,
+                                int32_t *n_features, int32_t *frame_info, float *stage_ms);
 /* test/bench introspection: one plane of the scale-space left by the last extraction (stack 0 Gaussian 0..5, 1 DoG 0..4,
  * 2 gradient magnitude 0..2, 3 orientation 0..2); out may be NULL to query the octave's size. */
 mc_status mc_sift_read_plane(mc_ctx *ctx, int frame, int octave, int stack, int index, float *out, int32_t *rows, int32_t *cols);

@@ -119,6 +119,8 @@ SIGNATURES = {
     "mc_sift_extract_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "mc_process_images": (C.c_int, [C.c_void_p, _u8p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(PipelineParams), C.c_int, _i32p, _i32p,
                                     _f32p, _f32p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "mc_process_rig_images": (C.c_int, [C.c_void_p, _u8p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(PipelineParams), C.c_int,
+                                        _i32p, _i32p, _f32p, _f32p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "mc_sift_profile_read": (C.c_int, [C.c_void_p, C.POINTER(C.c_float), C.POINTER(C.c_double)]),
     "mc_sift_read_plane": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "mc_set_option": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int64]),
@@ -638,6 +640,28 @@ class Context:
                                              om.reshape(-1), op.reshape(-1), os_.reshape(-1), nf.ctypes.data, info.ctypes.data,
                                              ms.ctypes.data if want_times else None), "mc_process_images")
         out = [dict(model=om[f, :n[f]].copy(), pose=op[f, :n[f]].copy(), score=os_[f, :n[f]].copy(), n_features=int(nf[f]), info=info[f].copy())
+               for f in range(B)]
+        if want_times:
+            out[0]["stage_ms"] = ms
+        return out
+
+    def process_rig_images(self, gray, double_size=True, max_keypoints=4096, params=None, max_objects=64, want_times=False):
+        """FEAT..FILTER2 for a batch of camera-rig frames [B,C,H,W] uint8, image c of a frame from camera c -> list of dicts (model,
+        pose, score, n_features = keypoints per camera, info)."""
+        g = np.ascontiguousarray(gray, dtype=np.uint8)
+        B, Cn, H, W = g.shape
+        p = params or self.default_params()
+        n = np.zeros(B, np.int32)
+        om = np.zeros((B, max_objects), np.int32)
+        op = np.zeros((B, max_objects, 7), np.float32)
+        os_ = np.zeros((B, max_objects), np.float32)
+        nf = np.zeros((B, Cn), np.int32)
+        info = np.zeros((B, 4), np.int32)
+        ms = np.zeros(3, np.float32)
+        self._check(self.L.mc_process_rig_images(self.h, g.reshape(-1), B, Cn, H, W, 1 if double_size else 0, max_keypoints, C.byref(p),
+                                                 max_objects, n, om.reshape(-1), op.reshape(-1), os_.reshape(-1), nf.ctypes.data, info.ctypes.data,
+                                                 ms.ctypes.data if want_times else None), "mc_process_rig_images")
+        out = [dict(model=om[f, :n[f]].copy(), pose=op[f, :n[f]].copy(), score=os_[f, :n[f]].copy(), n_features=nf[f].copy(), info=info[f].copy())
                for f in range(B)]
         if want_times:
             out[0]["stage_ms"] = ms

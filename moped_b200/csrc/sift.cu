@@ -1087,66 +1087,106 @@ extern "C" mc_status mc_sift_extract(mc_ctx *ctx, const uint8_t *gray, int n_ima
 	return rc;
 }
 
+namespace mc {
+
+// Rig frames: image b of the batch belongs to camera b % n_cameras, so its keypoints, entries [offs[b], offs[b+1]) of the compacted
+// list, get imageIdx = that camera. One CTA per image.
+__global__ void k_rig_image_index(const int32_t *__restrict__ offs, int n_cameras, int32_t *__restrict__ q_image) {
+	const int b = blockIdx.x, c = b % n_cameras, hi = offs[b + 1];
+	for (int i = offs[b] + threadIdx.x; i < hi; i += blockDim.x) q_image[i] = c;
+}
+
 /* Images in, objects out (SURVEY.md 8f rows 1+3 chained): FEAT -> MATCH -> CLUSTER -> POSE -> FILTER -> POSE2 -> FILTER2 for a
- * batch of single-camera frames. The descriptors never leave HBM: the describe kernel writes them compacted and already
- * normalised the way MATCH normalises its queries; only the per-frame keypoint counts (4 B each) come back to the host
- * before MATCH is launched, because the frame partition of the query list is host-side state of the batch driver. */
-extern "C" mc_status mc_process_images(mc_ctx *ctx, const uint8_t *gray, int n_frames, int height, int width, int double_size, int max_keypoints,
-                                       const mc_pipeline_params *params, int max_objects, int32_t *n_objects, int32_t *obj_model, float *obj_pose,
-                                       float *obj_score, int32_t *n_features, int32_t *frame_info, float *stage_ms) {
-	if (!ctx) return MC_ERR_ARG;
+ * batch of n_frames frames of n_cameras images each, image c of a frame from camera c. The descriptors never leave HBM: the describe
+ * kernel writes them compacted (image-major, so a frame's images follow each other in camera order) and already normalised the way
+ * MATCH normalises its queries; only the per-image keypoint counts and offsets (4 B each) come back to the host before MATCH is
+ * launched, because the frame partition of the query list is host-side state of the batch driver. */
+static mc_status process_images(mc_ctx *ctx, const char *who, const uint8_t *gray, int n_frames, int n_cameras, int height, int width,
+                                int double_size, int max_keypoints, const mc_pipeline_params *params, int max_objects, int32_t *n_objects,
+                                int32_t *obj_model, float *obj_pose, float *obj_score, int32_t *n_features, int32_t *frame_info, float *stage_ms) {
+	const std::string name(who);
 	if (!gray || !params || !n_objects || !obj_model || !obj_pose || !obj_score || n_frames < 1 || max_keypoints < 1 || max_objects < 1) {
-		ctx->err = "mc_process_images: bad argument"; return MC_ERR_ARG;
+		ctx->err = name + ": bad argument"; return MC_ERR_ARG;
 	}
-	if (!ctx->d_db) { ctx->err = "mc_process_images: no database uploaded"; return MC_ERR_STATE; }
-	if (ctx->D != 128) { ctx->err = "mc_process_images: the database does not hold 128-d descriptors"; return MC_ERR_STATE; }
-	// UNDISTORTED_IMAGE before SIFT when camera 0 has a table (mc_set_undistortion); its size is checked before anything is queued
-	const UndistortTable &und = ctx->undistort[0];
-	if (und.d_map && (und.height != height || und.width != width)) {
-		ctx->err = "mc_process_images: images are " + std::to_string(width) + "x" + std::to_string(height) + ", camera 0's undistortion table is " +
-		           std::to_string(und.width) + "x" + std::to_string(und.height);
-		return MC_ERR_ARG;
-	}
+	if (!ctx->d_db) { ctx->err = name + ": no database uploaded"; return MC_ERR_STATE; }
+	if (ctx->D != 128) { ctx->err = name + ": the database does not hold 128-d descriptors"; return MC_ERR_STATE; }
+	// UNDISTORTED_IMAGE before SIFT for the cameras with a table (mc_set_undistortion); their sizes are checked before anything is queued
+	bool undistort = false;
+	MC_TRY(undistort_check_rig(ctx, who, n_cameras, height, width, &undistort));
 	MC_CUDA(cudaSetDevice(ctx->device));
 	SiftState *s = state(ctx);
-	const size_t npx = (size_t)n_frames * height * width, nk = (size_t)n_frames * max_keypoints;
+	const int n_img = n_frames * n_cameras;
+	const size_t npx = (size_t)n_img * height * width, nk = (size_t)n_img * max_keypoints;
 	uint8_t *d_gray = nullptr, *d_undist = nullptr;
 	float *d_xy = nullptr, *d_desc = nullptr;
 	int32_t *d_qimg = nullptr, *d_counts = nullptr;
 	MC_TRY(carve_scratch(ctx, s->gray, [&](Carve &c) {
 		c.take(d_gray, npx);
-		c.take(d_undist, und.d_map ? npx : 0);
+		c.take(d_undist, undistort ? npx : 0);
 		c.take(d_xy, nk * 2);
 		c.take(d_desc, nk * 128);
 		c.take(d_qimg, nk);
-		c.take(d_counts, (size_t)2 * n_frames + 2);       // counts[n_frames], then offsets[n_frames + 1]
+		c.take(d_counts, (size_t)2 * n_img + 2);          // counts[n_img], then offsets[n_img + 1]
 	}));
-	int32_t *d_offsets = d_counts + n_frames;
-	MC_TRY(pinned(ctx, (size_t)(2 * n_frames + 2) * sizeof(int32_t)));
+	int32_t *d_offsets = d_counts + n_img;
+	MC_TRY(pinned(ctx, (size_t)(2 * n_img + 2) * sizeof(int32_t)));
 	cudaEvent_t ev[2];
 	if (stage_ms) { MC_CUDA(cudaEventCreate(&ev[0])); MC_CUDA(cudaEventCreate(&ev[1])); MC_CUDA(cudaEventRecord(ev[0], ctx->stream)); }
 	MC_CUDA(cudaMemcpyAsync(d_gray, gray, npx, cudaMemcpyHostToDevice, ctx->stream));
-	MC_CUDA(cudaMemsetAsync(d_qimg, 0, nk * sizeof(int32_t), ctx->stream));           // one camera per frame: imageIdx = 0
+	if (n_cameras == 1) MC_CUDA(cudaMemsetAsync(d_qimg, 0, nk * sizeof(int32_t), ctx->stream));     // one camera per frame: imageIdx = 0
 	const uint8_t *d_feat_in = d_gray;
-	if (und.d_map) {
-		MC_TRY(undistort_device(ctx, 0, d_gray, n_frames, height, width, d_undist));
+	if (undistort) {
+		MC_TRY(undistort_rig_device(ctx, n_cameras, d_gray, n_img, height, width, d_undist));
 		d_feat_in = d_undist;
 	}
-	MC_TRY(sift_extract_device(ctx, d_feat_in, n_frames, height, width, double_size, max_keypoints, d_xy, nullptr, d_desc, d_counts, d_offsets, 1));
+	MC_TRY(sift_extract_device(ctx, d_feat_in, n_img, height, width, double_size, max_keypoints, d_xy, nullptr, d_desc, d_counts, d_offsets, 1));
+	if (n_cameras > 1) {
+		k_rig_image_index<<<n_img, 128, 0, ctx->stream>>>(d_offsets, n_cameras, d_qimg);
+		MC_LAUNCH_CHECK();
+	}
 	int32_t *h = (int32_t *)ctx->h_pinned;
-	MC_CUDA(cudaMemcpyAsync(h, d_counts, (size_t)(2 * n_frames + 1) * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
+	MC_CUDA(cudaMemcpyAsync(h, d_counts, (size_t)(2 * n_img + 1) * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
 	if (stage_ms) MC_CUDA(cudaEventRecord(ev[1], ctx->stream));
 	MC_CUDA(cudaStreamSynchronize(ctx->stream));
 	if (stage_ms) { cudaEventElapsedTime(&stage_ms[0], ev[0], ev[1]); cudaEventDestroy(ev[0]); cudaEventDestroy(ev[1]); }
-	std::vector<int32_t> offsets(h + n_frames, h + 2 * n_frames + 1);
+	std::vector<int32_t> offsets(n_frames + 1);       // frame f = images [f * n_cameras, (f + 1) * n_cameras)
+	for (int f = 0; f <= n_frames; ++f) offsets[f] = h[n_img + f * n_cameras];
 	bool overflow = false;
-	for (int f = 0; f < n_frames; ++f) {
-		if (n_features) n_features[f] = h[f];
-		overflow |= h[f] > max_keypoints;
+	for (int i = 0; i < n_img; ++i) {
+		if (n_features) n_features[i] = h[i];
+		overflow |= h[i] > max_keypoints;
 	}
-	if (overflow) { ctx->err = "mc_process_images: more keypoints than max_keypoints in a frame (n_features[] holds the numbers found)"; return MC_ERR_CAPACITY; }
+	if (overflow) { ctx->err = name + ": more keypoints than max_keypoints in a frame (n_features[] holds the numbers found)"; return MC_ERR_CAPACITY; }
 	return process_frames_host(ctx, d_desc, d_xy, d_qimg, offsets.data(), n_frames, params, max_objects, n_objects, obj_model, obj_pose, obj_score,
 	                           frame_info, stage_ms ? stage_ms + 1 : nullptr);
+}
+
+} // namespace mc
+
+extern "C" mc_status mc_process_images(mc_ctx *ctx, const uint8_t *gray, int n_frames, int height, int width, int double_size, int max_keypoints,
+                                       const mc_pipeline_params *params, int max_objects, int32_t *n_objects, int32_t *obj_model, float *obj_pose,
+                                       float *obj_score, int32_t *n_features, int32_t *frame_info, float *stage_ms) {
+	if (!ctx) return MC_ERR_ARG;
+	return process_images(ctx, "mc_process_images", gray, n_frames, 1, height, width, double_size, max_keypoints, params, max_objects, n_objects,
+	                      obj_model, obj_pose, obj_score, n_features, frame_info, stage_ms);
+}
+
+extern "C" mc_status mc_process_rig_images(mc_ctx *ctx, const uint8_t *gray, int n_frames, int n_cameras, int height, int width, int double_size,
+                                           int max_keypoints, const mc_pipeline_params *params, int max_objects, int32_t *n_objects,
+                                           int32_t *obj_model, float *obj_pose, float *obj_score, int32_t *n_features, int32_t *frame_info,
+                                           float *stage_ms) {
+	if (!ctx) return MC_ERR_ARG;
+	if (n_cameras < 1 || n_cameras > kUndistortCameras) {
+		ctx->err = "mc_process_rig_images: n_cameras must be in 1.." + std::to_string(kUndistortCameras); return MC_ERR_ARG;
+	}
+	if ((int64_t)n_frames * n_cameras > 65535) { ctx->err = "mc_process_rig_images: more than 65535 images in a batch"; return MC_ERR_ARG; }
+	if (ctx->n_images < n_cameras) {
+		ctx->err = "mc_process_rig_images: " + std::to_string(n_cameras) + " cameras in the rig, " + std::to_string(ctx->n_images) +
+		           " set with mc_set_cameras";
+		return MC_ERR_STATE;
+	}
+	return process_images(ctx, "mc_process_rig_images", gray, n_frames, n_cameras, height, width, double_size, max_keypoints, params, max_objects,
+	                      n_objects, obj_model, obj_pose, obj_score, n_features, frame_info, stage_ms);
 }
 
 /* With mc_set_profiling on: device time (ms, summed) of the five octave-0 Gaussian+DoG launches of the last extraction and

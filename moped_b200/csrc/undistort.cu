@@ -12,9 +12,14 @@ namespace mc {
 
 constexpr int kUndBlockX = 32, kUndBlockY = 8, kUndPix = 4;     // a thread writes 4 consecutive pixels of one row
 
-// grid (columns / 128, rows / 8, images); the weight table is copied to shared memory by every block
+// Image z of a batch belongs to camera z % n_cameras; a camera without a table (null map) has its images copied through.
+struct UndistortMaps {
+	const RemapEntry *map[kUndistortCameras];
+};
+
+// grid (columns / 128, rows / 8, images); the weight table (the same for every camera) is copied to shared memory by every block
 __global__ void __launch_bounds__(kUndBlockX * kUndBlockY) k_undistort(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst,
-                                                                       const RemapEntry *__restrict__ map,
+                                                                       const __grid_constant__ UndistortMaps maps, int n_cameras,
                                                                        const RemapWeights *__restrict__ wtab, int H, int W, int vec4) {
 	__shared__ RemapWeights w[kInterTab * kInterTab];
 	const int tid = threadIdx.y * kUndBlockX + threadIdx.x;
@@ -25,15 +30,23 @@ __global__ void __launch_bounds__(kUndBlockX * kUndBlockY) k_undistort(const uin
 	const size_t plane = (size_t)H * W;
 	const uint8_t *img = src + blockIdx.z * plane;
 	uint8_t *out = dst + blockIdx.z * plane + (size_t)y * W + x0;
-	const RemapEntry *m = map + (size_t)y * W + x0;
+	const RemapEntry *map = maps.map[blockIdx.z % n_cameras];
 	const int n = min(kUndPix, W - x0);
 	uint8_t px[kUndPix];
+	if (map) {
+		const RemapEntry *m = map + (size_t)y * W + x0;
 #pragma unroll
-	for (int k = 0; k < kUndPix; k++) {
-		if (k < n) {
-			const RemapEntry e = m[k];
-			px[k] = remap_pixel(img, H, W, e, w[e.frac]);
+		for (int k = 0; k < kUndPix; k++) {
+			if (k < n) {
+				const RemapEntry e = m[k];
+				px[k] = remap_pixel(img, H, W, e, w[e.frac]);
+			}
 		}
+	} else {
+		const uint8_t *in = img + (size_t)y * W + x0;
+#pragma unroll
+		for (int k = 0; k < kUndPix; k++)
+			if (k < n) px[k] = und_load(in + k);
 	}
 	if (vec4 && n == kUndPix) {
 		*(uint32_t *)out = (uint32_t)px[0] | (uint32_t)px[1] << 8 | (uint32_t)px[2] << 16 | (uint32_t)px[3] << 24;
@@ -65,21 +78,52 @@ static mc_status camera_table(mc_ctx *ctx, const char *who, int camera, int H, i
 	return MC_OK;
 }
 
-static mc_status launch_undistort(mc_ctx *ctx, const UndistortTable &t, const uint8_t *d_in, int B, uint8_t *d_out) {
-	const int H = t.height, W = t.width;
+// One launch for a batch of n_cameras-camera frames; wtab is the weight table of any camera's allocation.
+static mc_status launch_undistort(mc_ctx *ctx, const UndistortMaps &maps, int n_cameras, const RemapWeights *wtab, const uint8_t *d_in, int B,
+                                  int H, int W, uint8_t *d_out) {
 	const dim3 block(kUndBlockX, kUndBlockY);
 	const dim3 grid((W + kUndBlockX * kUndPix - 1) / (kUndBlockX * kUndPix), (H + kUndBlockY - 1) / kUndBlockY, B);
 	const int vec4 = W % 4 == 0 && (uintptr_t)d_out % 4 == 0;
-	const RemapEntry *map = (const RemapEntry *)t.d_map;
-	k_undistort<<<grid, block, 0, ctx->stream>>>(d_in, d_out, map, (const RemapWeights *)(map + (size_t)H * W), H, W, vec4);
+	k_undistort<<<grid, block, 0, ctx->stream>>>(d_in, d_out, maps, n_cameras, wtab, H, W, vec4);
 	MC_LAUNCH_CHECK();
 	return MC_OK;
 }
 
-mc_status undistort_device(mc_ctx *ctx, int camera, const uint8_t *d_in, int B, int H, int W, uint8_t *d_out) {
-	const UndistortTable *t = nullptr;
-	MC_TRY(camera_table(ctx, "undistort", camera, H, W, &t));
-	return launch_undistort(ctx, *t, d_in, B, d_out);
+static const RemapEntry *table_map(const UndistortTable &t) { return (const RemapEntry *)t.d_map; }
+static const RemapWeights *table_weights(const UndistortTable &t) { return (const RemapWeights *)(table_map(t) + (size_t)t.height * t.width); }
+
+static mc_status launch_camera(mc_ctx *ctx, const UndistortTable &t, const uint8_t *d_in, int B, uint8_t *d_out) {
+	UndistortMaps maps = {};
+	maps.map[0] = table_map(t);
+	return launch_undistort(ctx, maps, 1, table_weights(t), d_in, B, t.height, t.width, d_out);
+}
+
+mc_status undistort_check_rig(mc_ctx *ctx, const char *who, int n_cameras, int H, int W, bool *any) {
+	*any = false;
+	for (int c = 0; c < n_cameras; c++) {
+		const UndistortTable &t = ctx->undistort[c];
+		if (!t.d_map) continue;
+		if (t.height != H || t.width != W) {
+			ctx->err = std::string(who) + ": images are " + std::to_string(W) + "x" + std::to_string(H) + ", camera " + std::to_string(c) +
+			           "'s undistortion table is " + std::to_string(t.width) + "x" + std::to_string(t.height);
+			return MC_ERR_ARG;
+		}
+		*any = true;
+	}
+	return MC_OK;
+}
+
+mc_status undistort_rig_device(mc_ctx *ctx, int n_cameras, const uint8_t *d_in, int B, int H, int W, uint8_t *d_out) {
+	UndistortMaps maps = {};
+	const RemapWeights *wtab = nullptr;
+	for (int c = 0; c < n_cameras; c++) {
+		const UndistortTable &t = ctx->undistort[c];
+		if (!t.d_map) continue;
+		maps.map[c] = table_map(t);
+		wtab = table_weights(t);
+	}
+	if (!wtab) { ctx->err = "undistort: no camera of the rig has an undistortion table"; return MC_ERR_STATE; }
+	return launch_undistort(ctx, maps, n_cameras, wtab, d_in, B, H, W, d_out);
 }
 
 } // namespace mc
@@ -126,7 +170,7 @@ extern "C" mc_status mc_undistort_dev(mc_ctx *ctx, int camera, const uint8_t *gr
 	MC_CUDA(cudaSetDevice(ctx->device));
 	const UndistortTable *t = nullptr;
 	MC_TRY(camera_table(ctx, "mc_undistort_dev", camera, height, width, &t));
-	return launch_undistort(ctx, *t, gray_dev, n_images, out_dev);
+	return launch_camera(ctx, *t, gray_dev, n_images, out_dev);
 }
 
 extern "C" mc_status mc_undistort(mc_ctx *ctx, int camera, const uint8_t *gray, int n_images, int height, int width, uint8_t *out) {
@@ -139,7 +183,7 @@ extern "C" mc_status mc_undistort(mc_ctx *ctx, int camera, const uint8_t *gray, 
 	uint8_t *d_in = nullptr, *d_out = nullptr;
 	MC_TRY(carve_scratch(ctx, ctx->scratch[kScrUndistort], [&](Carve &c) { c.take(d_in, n); c.take(d_out, n); }));
 	MC_CUDA(cudaMemcpyAsync(d_in, gray, n, cudaMemcpyHostToDevice, ctx->stream));
-	MC_TRY(launch_undistort(ctx, *t, d_in, n_images, d_out));
+	MC_TRY(launch_camera(ctx, *t, d_in, n_images, d_out));
 	MC_CUDA(cudaMemcpyAsync(out, d_out, n, cudaMemcpyDeviceToHost, ctx->stream));
 	MC_CUDA(cudaStreamSynchronize(ctx->stream));
 	return MC_OK;
