@@ -453,8 +453,40 @@ mc_status mc_process_rig_images(mc_ctx *ctx, const uint8_t *gray, int n_frames, 
                                 int double_size, int max_keypoints, const mc_pipeline_params *params, int max_objects,
                                 int32_t *n_objects, int32_t *obj_model, float *obj_pose, float *obj_score,
                                 int32_t *n_features, int32_t *frame_info, float *stage_ms);
+/* One camera of a rig as mc_process_rig_cameras reads it: the camera's image of frame f is height x width bytes at
+ * gray + f * frame_stride. Per-camera buffers [n_frames][height][width] have frame_stride = height * width; camera c of one
+ * [n_frames][C][H][W] buffer is gray = base + c * H * W with frame_stride = C * H * W. */
+typedef struct {
+	const uint8_t *gray;      /* camera c's image of frame 0 */
+	int64_t frame_stride;     /* bytes between frames, >= height * width */
+	int32_t height, width;    /* this camera's image size, 8..32767 each */
+} mc_rig_camera;
+/* mc_process_rig_images for rigs whose cameras may differ in image size and whose images may sit in separate buffers: camera c's
+ * images are described by cameras[c]. Its intrinsics and pose are entry c of mc_set_cameras; its undistortion table, if it has one,
+ * is camera c's of mc_set_undistortion and must be that camera's own size. Cameras of one size form a group and share one SIFT batch
+ * (and one remap launch when a camera of the group has a table); the groups' keypoints are then merged on the device so that frame f's
+ * query list is camera 0's keypoints, then camera 1's, ..., each in FEAT_SIFT_CPU's order with imageIdx = camera, exactly as
+ * mc_process_rig_images orders them. When every camera has one size the call issues mc_process_rig_images' launches. Outputs as
+ * mc_process_rig_images: n_features (optional) = n_frames x n_cameras counts, frame-major; stage_ms (optional, 3 floats) with FEAT
+ * including the merge. Errors, all before any copy or launch: MC_ERR_ARG for n_cameras outside 1..16, a NULL pointer, n_frames,
+ * max_keypoints or max_objects below 1, a size outside 8..32767, frame_stride < height * width, a table whose size is not its
+ * camera's, more than 65535 images, or more than 7281 images of one size (SIFT's batch limit); MC_ERR_STATE when mc_set_cameras set
+ * fewer than n_cameras cameras, no database is uploaded or its descriptors are not 128-d. An image with more than max_keypoints
+ * keypoints returns MC_ERR_CAPACITY; n_features still holds the numbers found. */
+mc_status mc_process_rig_cameras(mc_ctx *ctx, const mc_rig_camera *cameras, int n_cameras, int n_frames, int double_size,
+                                 int max_keypoints, const mc_pipeline_params *params, int max_objects, int32_t *n_objects,
+                                 int32_t *obj_model, float *obj_pose, float *obj_score, int32_t *n_features, int32_t *frame_info,
+                                 float *stage_ms);
+/* The same with every cameras[c].gray a device pointer (the array `cameras` itself on the host); results on the host, like
+ * mc_process_frames_dev. A group whose cameras already lie [frame][camera-in-group] in one buffer is read in place; other
+ * groups are gathered with device-to-device copies. The images are not modified. */
+mc_status mc_process_rig_cameras_dev(mc_ctx *ctx, const mc_rig_camera *cameras, int n_cameras, int n_frames, int double_size,
+                                     int max_keypoints, const mc_pipeline_params *params, int max_objects, int32_t *n_objects,
+                                     int32_t *obj_model, float *obj_pose, float *obj_score, int32_t *n_features,
+                                     int32_t *frame_info, float *stage_ms);
 /* test/bench introspection: one plane of the scale-space left by the last extraction (stack 0 Gaussian 0..5, 1 DoG 0..4,
- * 2 gradient magnitude 0..2, 3 orientation 0..2); out may be NULL to query the octave's size. */
+ * 2 gradient magnitude 0..2, 3 orientation 0..2); out may be NULL to query the octave's size. After a mc_process_rig_cameras*
+ * call with cameras of several sizes it is the scale-space of the last size group's batch. */
 mc_status mc_sift_read_plane(mc_ctx *ctx, int frame, int octave, int stack, int index, float *out, int32_t *rows, int32_t *cols);
 
 /* ---- moped3d clustering (SURVEY.md 8f row 4): replaces CLUSTER_LINKAGE_CPU::process for the matches of ONE model,

@@ -38,6 +38,11 @@ class PipelineParams(C.Structure):
                 ("pose2", PoseParams), ("filter2_min_points", C.c_int32), ("filter2_feature_distance", C.c_float), ("filter2_min_score", C.c_float)]
 
 
+class RigCamera(C.Structure):
+    """mc_rig_camera: camera c's image of frame f is height x width bytes at gray + f * frame_stride."""
+    _fields_ = [("gray", C.c_void_p), ("frame_stride", C.c_int64), ("height", C.c_int32), ("width", C.c_int32)]
+
+
 class DepthPipelineParams(C.Structure):
     """mc_depth_pipeline_params: moped3d's CLUSTER_LINKAGE -> POSE -> FILTER -> POSE2 -> FILTER2."""
     _fields_ = [("variant", C.c_int32),
@@ -121,6 +126,10 @@ SIGNATURES = {
                                     _f32p, _f32p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "mc_process_rig_images": (C.c_int, [C.c_void_p, _u8p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(PipelineParams), C.c_int,
                                         _i32p, _i32p, _f32p, _f32p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "mc_process_rig_cameras": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(PipelineParams), C.c_int, _i32p, _i32p,
+                                         _f32p, _f32p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "mc_process_rig_cameras_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(PipelineParams), C.c_int, _i32p,
+                                             _i32p, _f32p, _f32p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "mc_sift_profile_read": (C.c_int, [C.c_void_p, C.POINTER(C.c_float), C.POINTER(C.c_double)]),
     "mc_sift_read_plane": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "mc_set_option": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int64]),
@@ -661,6 +670,39 @@ class Context:
         self._check(self.L.mc_process_rig_images(self.h, g.reshape(-1), B, Cn, H, W, 1 if double_size else 0, max_keypoints, C.byref(p),
                                                  max_objects, n, om.reshape(-1), op.reshape(-1), os_.reshape(-1), nf.ctypes.data, info.ctypes.data,
                                                  ms.ctypes.data if want_times else None), "mc_process_rig_images")
+        out = [dict(model=om[f, :n[f]].copy(), pose=op[f, :n[f]].copy(), score=os_[f, :n[f]].copy(), n_features=nf[f].copy(), info=info[f].copy())
+               for f in range(B)]
+        if want_times:
+            out[0]["stage_ms"] = ms
+        return out
+
+    def process_rig_cameras(self, images, double_size=True, max_keypoints=4096, params=None, max_objects=64, want_times=False):
+        """mc_process_rig_cameras: FEAT..FILTER2 for camera-rig frames whose cameras may differ in size; images = one uint8 array
+        (n_frames, H_c, W_c) per camera c -> the per-frame dicts of process_rig_images."""
+        ims = [np.ascontiguousarray(g, dtype=np.uint8) for g in images]
+        cams = (RigCamera * len(ims))(*[RigCamera(g.ctypes.data, g.shape[1] * g.shape[2], g.shape[1], g.shape[2]) for g in ims])
+        return self._rig_cameras("mc_process_rig_cameras", cams, len(ims[0]), double_size, max_keypoints, params, max_objects, want_times)
+
+    def process_rig_cameras_dev(self, ptrs, strides, sizes, n_frames, double_size=True, max_keypoints=4096, params=None, max_objects=64,
+                                want_times=False):
+        """mc_process_rig_cameras_dev: camera c's image of frame f is sizes[c] = (H, W) bytes at device address ptrs[c] + f * strides[c]
+        -> the per-frame dicts of process_rig_images."""
+        cams = (RigCamera * len(ptrs))(*[RigCamera(int(p), int(st), int(h), int(w)) for p, st, (h, w) in zip(ptrs, strides, sizes)])
+        return self._rig_cameras("mc_process_rig_cameras_dev", cams, n_frames, double_size, max_keypoints, params, max_objects, want_times)
+
+    def _rig_cameras(self, fn, cams, B, double_size, max_keypoints, params, max_objects, want_times):
+        Cn = len(cams)
+        p = params or self.default_params()
+        n = np.zeros(B, np.int32)
+        om = np.zeros((B, max_objects), np.int32)
+        op = np.zeros((B, max_objects, 7), np.float32)
+        os_ = np.zeros((B, max_objects), np.float32)
+        nf = np.zeros((B, Cn), np.int32)
+        info = np.zeros((B, 4), np.int32)
+        ms = np.zeros(3, np.float32)
+        self._check(getattr(self.L, fn)(self.h, C.cast(cams, C.c_void_p), Cn, B, 1 if double_size else 0, max_keypoints, C.byref(p), max_objects,
+                                        n, om.reshape(-1), op.reshape(-1), os_.reshape(-1), nf.ctypes.data, info.ctypes.data,
+                                        ms.ctypes.data if want_times else None), fn)
         out = [dict(model=om[f, :n[f]].copy(), pose=op[f, :n[f]].copy(), score=os_[f, :n[f]].copy(), n_features=nf[f].copy(), info=info[f].copy())
                for f in range(B)]
         if want_times:

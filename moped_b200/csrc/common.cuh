@@ -281,10 +281,11 @@ size_t frame_shard_slot_bytes(int Q, const mc_pipeline_params *P);
 mc_status process_frame_sharded_device(mc_ctx *ctx, int phase, const int32_t *d_nn_row, const uint8_t *d_accepted, const float *d_qxy,
                                        const int32_t *d_qimg, int Q, const mc_pipeline_params *P, int shard_rank, int shard_world, void *d_exchange,
                                        int max_objects, int32_t *d_out_info, int32_t *d_out_model, float *d_out_pose, float *d_out_score);
-// Camera rigs (undistort.cu): image b of a batch belongs to camera b % n_cameras. undistort_check_rig: MC_ERR_ARG when one of the rig's
-// tables is not H x W; *any = some camera of the rig has a table. undistort_rig_device: one launch for the batch (at least one table).
-mc_status undistort_check_rig(mc_ctx *ctx, const char *who, int n_cameras, int H, int W, bool *any);
-mc_status undistort_rig_device(mc_ctx *ctx, int n_cameras, const uint8_t *d_in, int B, int H, int W, uint8_t *d_out);
+// Camera rigs (undistort.cu). undistort_check_rig: has[c] = camera c has a table; MC_ERR_ARG when that table is not H[c] x W[c].
+// undistort_rig_device: one launch for a batch of H x W images whose image b belongs to camera cameras[b % n_cameras] (at least one
+// of them with a table).
+mc_status undistort_check_rig(mc_ctx *ctx, const char *who, int n_cameras, const int *H, const int *W, bool *has);
+mc_status undistort_rig_device(mc_ctx *ctx, const int *cameras, int n_cameras, const uint8_t *d_in, int B, int H, int W, uint8_t *d_out);
 mc_status match_device(mc_ctx *ctx, const float *d_q, int Q, float ratio, int mode,
                        int32_t *d_nn_row, float *d_nn_dist, uint8_t *d_accepted);
 

@@ -22,6 +22,7 @@
 // orientation peak descending.
 #include "common.cuh"
 
+#include <algorithm>
 #include <math.h>
 #include <string.h>
 
@@ -891,23 +892,52 @@ void sift_free(mc_ctx *ctx) {
 	ctx->sift_state = nullptr;
 }
 
+// Device bytes of sift_plan's buffers for a batch shape
+struct SiftBytes {
+	size_t pyr, tmp, cand, kp, counters;
+	int cap_cand;
+};
+
+static SiftBytes sift_bytes(int B, int H, int W, int dbl, int max_kp) {
+	const int rows = dbl ? 2 * H - 2 : H, cols = dbl ? 2 * W - 2 : W;
+	const int per_px = (kSiftScales + 3) + (kSiftScales + 2) + 2 * kSiftScales + 1;   // gauss, dog, grad, ori, claim
+	size_t total = 0;
+	for (int r = rows, c = cols, n = 0; r > 12 && c > 12 && n < kSiftMaxOct; r >>= 1, c >>= 1, n++) total += (size_t)r * c * per_px * B;
+	SiftBytes b;
+	b.pyr = total * sizeof(float) + 256;
+	b.tmp = (size_t)rows * cols * B * sizeof(float) + 256;
+	b.cap_cand = B * (max_kp > 8192 ? max_kp : 8192) * 2;
+	b.cand = (size_t)b.cap_cand * sizeof(SiftCand);
+	b.kp = (size_t)B * max_kp * sizeof(SiftKp);
+	b.counters = (size_t)(B + 1) * sizeof(int);
+	return b;
+}
+
+static mc_status sift_reserve(mc_ctx *ctx, SiftState *s, const SiftBytes &b) {
+	if (!s->pyr.p || b.pyr > s->pyr.cap) s->B = 0;     // the pyramid moves: the plan's octave pointers go stale, the next sift_plan replans
+	MC_TRY(reserve(ctx, s->pyr, b.pyr));
+	MC_TRY(reserve(ctx, s->tmp, b.tmp));
+	MC_TRY(reserve(ctx, s->tmp2, b.tmp));
+	MC_TRY(reserve(ctx, s->cand, b.cand));
+	MC_TRY(reserve(ctx, s->kp, b.kp));
+	MC_TRY(reserve(ctx, s->counters, b.counters));
+	MC_TRY(reserve(ctx, s->offs, b.counters));
+	return MC_OK;
+}
+
 // (re)plans the scale-space for a batch shape: octave sizes like GetKeypoints' loop (libsiftfast.cpp:344-348)
 static mc_status sift_plan(mc_ctx *ctx, SiftState *s, int B, int H, int W, int dbl, int max_kp) {
 	if (s->B == B && s->H == H && s->W == W && s->dbl == dbl && s->max_kp == max_kp) return MC_OK;
-	int rows = dbl ? 2 * H - 2 : H, cols = dbl ? 2 * W - 2 : W;
+	const int rows = dbl ? 2 * H - 2 : H, cols = dbl ? 2 * W - 2 : W;
 	int n = 0;
-	size_t total = 0;
-	const int per_px = (kSiftScales + 3) + (kSiftScales + 2) + 2 * kSiftScales + 1;   // gauss, dog, grad, ori, claim
 	int r = rows, c = cols;
 	while (r > 12 && c > 12 && n < kSiftMaxOct) {
 		s->oct[n].rows = r; s->oct[n].cols = c; s->oct[n].plane = (size_t)r * c;
-		total += (size_t)r * c * per_px * B;
 		r >>= 1; c >>= 1; n++;
 	}
 	s->n_oct = n;
-	MC_TRY(reserve(ctx, s->pyr, total * sizeof(float) + 256));
-	MC_TRY(reserve(ctx, s->tmp, (size_t)rows * cols * B * sizeof(float) + 256));
-	MC_TRY(reserve(ctx, s->tmp2, (size_t)rows * cols * B * sizeof(float) + 256));
+	const SiftBytes bytes = sift_bytes(B, H, W, dbl, max_kp);
+	MC_TRY(sift_reserve(ctx, s, bytes));
 	float *p = (float *)s->pyr.p;
 	for (int o = 0; o < n; ++o) {
 		SiftOct &q = s->oct[o];
@@ -918,11 +948,7 @@ static mc_status sift_plan(mc_ctx *ctx, SiftState *s, int B, int H, int W, int d
 		q.ori = p; p += pl * kSiftScales;
 		q.claim = (int32_t *)p; p += pl;
 	}
-	s->cap_cand = B * (max_kp > 8192 ? max_kp : 8192) * 2;
-	MC_TRY(reserve(ctx, s->cand, (size_t)s->cap_cand * sizeof(SiftCand)));
-	MC_TRY(reserve(ctx, s->kp, (size_t)B * max_kp * sizeof(SiftKp)));
-	MC_TRY(reserve(ctx, s->counters, (size_t)(B + 1) * sizeof(int)));
-	MC_TRY(reserve(ctx, s->offs, (size_t)(B + 1) * sizeof(int32_t)));
+	s->cap_cand = bytes.cap_cand;
 	if (!s->lut.p) {
 		MC_TRY(reserve(ctx, s->lut, 256 * sizeof(float)));
 		float lut[256];
@@ -1096,51 +1122,230 @@ __global__ void k_rig_image_index(const int32_t *__restrict__ offs, int n_camera
 	for (int i = offs[b] + threadIdx.x; i < hi; i += blockDim.x) q_image[i] = c;
 }
 
+// Rigs with cameras of several sizes: each size group ran its own SIFT batch, images [frame][camera-in-group], into its own compacted
+// list. Camera c's image of frame f is image f * k[c] of its group's batch: its count found is counts[c][f * k[c]] and its keypoints
+// are entries [offs[c][f * k[c]], offs[c][f * k[c] + 1]) of xy[c] / desc[c] (the pointers already advanced to the camera's slot).
+struct RigMerge {
+	const int32_t *counts[kUndistortCameras], *offs[kUndistortCameras];
+	const float *xy[kUndistortCameras], *desc[kUndistortCameras];
+	int k[kUndistortCameras];
+};
+
+constexpr int kMergeScanThreads = 1024, kMergeThreads = 256, kMergeSplit = 8;
+
+// One CTA: frame-major image i = f * n_cameras + c gets counts[i] = the count found and offs[i] = where its keypoints go in the merged
+// list, so offs[f * n_cameras] is frame f's query offset and offs[n_img] the total. The destinations use the numbers SIFT wrote
+// (offset differences), which a count found above max_keypoints exceeds.
+__global__ void __launch_bounds__(kMergeScanThreads) k_rig_merge_scan(const __grid_constant__ RigMerge m, int n_cameras, int n_img,
+                                                                      int32_t *__restrict__ counts, int32_t *__restrict__ offs) {
+	__shared__ int warp_sum[kMergeScanThreads / 32];
+	const int per = (n_img + kMergeScanThreads - 1) / kMergeScanThreads;
+	const int lo = min((int)threadIdx.x * per, n_img), hi = min(lo + per, n_img);
+	int sum = 0;
+	for (int i = lo; i < hi; ++i) {
+		const int c = i % n_cameras;
+		const int32_t *o = m.offs[c] + (i / n_cameras) * m.k[c];
+		sum += o[1] - o[0];
+	}
+	const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+	int incl = sum;
+#pragma unroll
+	for (int d = 1; d < 32; d <<= 1) {
+		const int v = __shfl_up_sync(0xffffffffu, incl, d);
+		if (lane >= d) incl += v;
+	}
+	if (lane == 31) warp_sum[warp] = incl;
+	__syncthreads();
+	if (warp == 0) {
+		int w = warp_sum[lane];
+#pragma unroll
+		for (int d = 1; d < 32; d <<= 1) {
+			const int v = __shfl_up_sync(0xffffffffu, w, d);
+			if (lane >= d) w += v;
+		}
+		warp_sum[lane] = w;
+	}
+	__syncthreads();
+	int run = incl - sum + (warp ? warp_sum[warp - 1] : 0);
+	for (int i = lo; i < hi; ++i) {
+		const int c = i % n_cameras, b = (i / n_cameras) * m.k[c];
+		const int32_t *o = m.offs[c] + b;
+		counts[i] = m.counts[c][b];
+		offs[i] = run;
+		run += o[1] - o[0];
+	}
+	if (threadIdx.x == kMergeScanThreads - 1) offs[n_img] = run;
+}
+
+// grid (n_img, kMergeSplit): frame-major image i's descriptors (128 floats, as float4) and xy move from its group's list to offs[i] of
+// the merged list, and its keypoints get imageIdx = camera.
+__global__ void __launch_bounds__(kMergeThreads) k_rig_merge_interleave(const __grid_constant__ RigMerge m, int n_cameras,
+                                                                        const int32_t *__restrict__ offs, float *__restrict__ xy,
+                                                                        float *__restrict__ desc, int32_t *__restrict__ q_image) {
+	const int i = blockIdx.x, c = i % n_cameras;
+	const int32_t *so = m.offs[c] + (i / n_cameras) * m.k[c];
+	const int src = so[0], dst = offs[i], n = offs[i + 1] - dst;
+	const int t0 = blockIdx.y * kMergeThreads + threadIdx.x, step = gridDim.y * kMergeThreads;
+	const float4 *s4 = (const float4 *)(m.desc[c] + (size_t)src * 128);
+	float4 *d4 = (float4 *)(desc + (size_t)dst * 128);
+#pragma unroll 4
+	for (int t = t0; t < n * 32; t += step) d4[t] = __ldg(s4 + t);
+	const float2 *s2 = (const float2 *)(m.xy[c] + (size_t)src * 2);
+	float2 *d2 = (float2 *)(xy + (size_t)dst * 2);
+	for (int t = t0; t < n; t += step) {
+		d2[t] = __ldg(s2 + t);
+		q_image[dst + t] = c;
+	}
+}
+
+// Checks of the rig entries before anything is read or queued
+static mc_status rig_check(mc_ctx *ctx, const char *who, int n_frames, int n_cameras) {
+	const std::string name(who);
+	if (n_cameras < 1 || n_cameras > kUndistortCameras) {
+		ctx->err = name + ": n_cameras must be in 1.." + std::to_string(kUndistortCameras); return MC_ERR_ARG;
+	}
+	if ((int64_t)n_frames * n_cameras > 65535) { ctx->err = name + ": more than 65535 images in a batch"; return MC_ERR_ARG; }
+	if (ctx->n_images < n_cameras) {
+		ctx->err = name + ": " + std::to_string(n_cameras) + " cameras in the rig, " + std::to_string(ctx->n_images) + " set with mc_set_cameras";
+		return MC_ERR_STATE;
+	}
+	return MC_OK;
+}
+
+// Cameras of one image size, in camera order. Their images form one SIFT batch laid out [frame][camera-in-group].
+struct RigGroup {
+	int H = 0, W = 0, k = 0;
+	int cams[kUndistortCameras];
+	bool table = false;               // a camera of the group has an undistortion table: one remap launch
+	bool packed = false;              // the cameras' images already lie in the batch layout, in one buffer
+	size_t n = 0, npx = 0;            // images, bytes of the batch
+	uint8_t *d_gray = nullptr, *d_undist = nullptr;
+	float *d_xy = nullptr, *d_desc = nullptr;
+	int32_t *d_counts = nullptr;      // counts[n], then offsets[n + 1]
+};
+
 /* Images in, objects out (SURVEY.md 8f rows 1+3 chained): FEAT -> MATCH -> CLUSTER -> POSE -> FILTER -> POSE2 -> FILTER2 for a
- * batch of n_frames frames of n_cameras images each, image c of a frame from camera c. The descriptors never leave HBM: the describe
- * kernel writes them compacted (image-major, so a frame's images follow each other in camera order) and already normalised the way
- * MATCH normalises its queries; only the per-image keypoint counts and offsets (4 B each) come back to the host before MATCH is
- * launched, because the frame partition of the query list is host-side state of the batch driver. */
-static mc_status process_images(mc_ctx *ctx, const char *who, const uint8_t *gray, int n_frames, int n_cameras, int height, int width,
+ * batch of n_frames frames of n_cameras images each, camera c's images as cams[c] describes them, in host (dev = false) or device
+ * memory. Cameras of one size run as one SIFT batch. The descriptors never leave HBM: the describe kernel writes them compacted
+ * (image-major) and already normalised the way MATCH normalises its queries. With one size group, a frame's images follow each other
+ * in camera order already; with several, two merge kernels interleave the groups' lists into that order. Only the per-image keypoint
+ * counts and offsets (4 B each) come back to the host before MATCH is launched, because the frame partition of the query list is
+ * host-side state of the batch driver. */
+static mc_status process_images(mc_ctx *ctx, const char *who, const mc_rig_camera *cams, int n_cameras, int n_frames, bool dev,
                                 int double_size, int max_keypoints, const mc_pipeline_params *params, int max_objects, int32_t *n_objects,
                                 int32_t *obj_model, float *obj_pose, float *obj_score, int32_t *n_features, int32_t *frame_info, float *stage_ms) {
 	const std::string name(who);
-	if (!gray || !params || !n_objects || !obj_model || !obj_pose || !obj_score || n_frames < 1 || max_keypoints < 1 || max_objects < 1) {
+	if (!cams || !params || !n_objects || !obj_model || !obj_pose || !obj_score || n_frames < 1 || max_keypoints < 1 || max_objects < 1) {
 		ctx->err = name + ": bad argument"; return MC_ERR_ARG;
 	}
 	if (!ctx->d_db) { ctx->err = name + ": no database uploaded"; return MC_ERR_STATE; }
 	if (ctx->D != 128) { ctx->err = name + ": the database does not hold 128-d descriptors"; return MC_ERR_STATE; }
+	int H[kUndistortCameras], W[kUndistortCameras];
+	std::vector<RigGroup> groups;
+	for (int c = 0; c < n_cameras; ++c) {
+		const mc_rig_camera &cam = cams[c];
+		if (!cam.gray) { ctx->err = name + ": camera " + std::to_string(c) + " has no images"; return MC_ERR_ARG; }
+		if (cam.height < 8 || cam.height > 32767 || cam.width < 8 || cam.width > 32767) {
+			ctx->err = name + ": camera " + std::to_string(c) + "'s images are " + std::to_string(cam.width) + "x" + std::to_string(cam.height) +
+			           "; sizes must be in 8..32767";
+			return MC_ERR_ARG;
+		}
+		if (cam.frame_stride < (int64_t)cam.height * cam.width) {
+			ctx->err = name + ": camera " + std::to_string(c) + "'s frame_stride is below height x width"; return MC_ERR_ARG;
+		}
+		H[c] = cam.height; W[c] = cam.width;
+		size_t g = 0;
+		while (g < groups.size() && (groups[g].H != H[c] || groups[g].W != W[c])) ++g;
+		if (g == groups.size()) { groups.emplace_back(); groups[g].H = H[c]; groups[g].W = W[c]; }
+		groups[g].cams[groups[g].k++] = c;
+	}
+	for (const RigGroup &g : groups)
+		if ((int64_t)n_frames * g.k * 3 * kSiftScales > 65535) {
+			ctx->err = name + ": more than " + std::to_string(65535 / (3 * kSiftScales)) + " images of one size in a batch"; return MC_ERR_ARG;
+		}
 	// UNDISTORTED_IMAGE before SIFT for the cameras with a table (mc_set_undistortion); their sizes are checked before anything is queued
-	bool undistort = false;
-	MC_TRY(undistort_check_rig(ctx, who, n_cameras, height, width, &undistort));
+	bool has_table[kUndistortCameras];
+	MC_TRY(undistort_check_rig(ctx, who, n_cameras, H, W, has_table));
 	MC_CUDA(cudaSetDevice(ctx->device));
 	SiftState *s = state(ctx);
+	const bool merge = groups.size() > 1;
+	SiftBytes need = {};                  // every group's batch fits the scale-space buffers: nothing is reallocated between groups
+	for (RigGroup &g : groups) {
+		const size_t plane = (size_t)g.H * g.W;
+		g.n = (size_t)n_frames * g.k;
+		g.npx = g.n * plane;
+		const mc_rig_camera &c0 = cams[g.cams[0]];
+		g.packed = c0.frame_stride == (int64_t)(g.k * plane);
+		for (int j = 0; j < g.k; ++j) {
+			g.table |= has_table[g.cams[j]];
+			g.packed &= cams[g.cams[j]].gray == c0.gray + j * plane && cams[g.cams[j]].frame_stride == c0.frame_stride;
+		}
+		const SiftBytes b = sift_bytes((int)g.n, g.H, g.W, double_size ? 1 : 0, max_keypoints);
+		need.pyr = std::max(need.pyr, b.pyr); need.tmp = std::max(need.tmp, b.tmp); need.cand = std::max(need.cand, b.cand);
+		need.kp = std::max(need.kp, b.kp); need.counters = std::max(need.counters, b.counters);
+	}
+	MC_TRY(sift_reserve(ctx, s, need));
 	const int n_img = n_frames * n_cameras;
-	const size_t npx = (size_t)n_img * height * width, nk = (size_t)n_img * max_keypoints;
-	uint8_t *d_gray = nullptr, *d_undist = nullptr;
+	const size_t nk = (size_t)n_img * max_keypoints;
 	float *d_xy = nullptr, *d_desc = nullptr;
 	int32_t *d_qimg = nullptr, *d_counts = nullptr;
 	MC_TRY(carve_scratch(ctx, s->gray, [&](Carve &c) {
-		c.take(d_gray, npx);
-		c.take(d_undist, undistort ? npx : 0);
+		for (RigGroup &g : groups) {
+			c.take(g.d_gray, dev && g.packed ? 0 : g.npx);     // device images in the batch layout are read where they are
+			c.take(g.d_undist, g.table ? g.npx : 0);
+		}
 		c.take(d_xy, nk * 2);
 		c.take(d_desc, nk * 128);
 		c.take(d_qimg, nk);
-		c.take(d_counts, (size_t)2 * n_img + 2);          // counts[n_img], then offsets[n_img + 1]
+		c.take(d_counts, (size_t)2 * n_img + 2);          // counts[n_img], then offsets[n_img + 1], frame-major
+		for (RigGroup &g : groups) {                      // with several groups each has its own list, merged into the arrays above
+			const size_t gk = merge ? g.n * max_keypoints : 0;
+			c.take(g.d_xy, gk * 2);
+			c.take(g.d_desc, gk * 128);
+			c.take(g.d_counts, merge ? 2 * g.n + 2 : 0);
+		}
 	}));
 	int32_t *d_offsets = d_counts + n_img;
+	if (!merge) { groups[0].d_xy = d_xy; groups[0].d_desc = d_desc; groups[0].d_counts = d_counts; }
 	MC_TRY(pinned(ctx, (size_t)(2 * n_img + 2) * sizeof(int32_t)));
 	cudaEvent_t ev[2];
 	if (stage_ms) { MC_CUDA(cudaEventCreate(&ev[0])); MC_CUDA(cudaEventCreate(&ev[1])); MC_CUDA(cudaEventRecord(ev[0], ctx->stream)); }
-	MC_CUDA(cudaMemcpyAsync(d_gray, gray, npx, cudaMemcpyHostToDevice, ctx->stream));
-	if (n_cameras == 1) MC_CUDA(cudaMemsetAsync(d_qimg, 0, nk * sizeof(int32_t), ctx->stream));     // one camera per frame: imageIdx = 0
-	const uint8_t *d_feat_in = d_gray;
-	if (undistort) {
-		MC_TRY(undistort_rig_device(ctx, n_cameras, d_gray, n_img, height, width, d_undist));
-		d_feat_in = d_undist;
+	const cudaMemcpyKind kind = dev ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
+	for (RigGroup &g : groups) {                          // each group's batch: one copy when it is packed, else one per camera
+		const size_t plane = (size_t)g.H * g.W;
+		if (dev && g.packed) continue;
+		if (g.packed) { MC_CUDA(cudaMemcpyAsync(g.d_gray, cams[g.cams[0]].gray, g.npx, kind, ctx->stream)); continue; }
+		for (int j = 0; j < g.k; ++j) {
+			const mc_rig_camera &cam = cams[g.cams[j]];
+			MC_CUDA(cudaMemcpy2DAsync(g.d_gray + j * plane, g.k * plane, cam.gray, (size_t)cam.frame_stride, plane, n_frames, kind, ctx->stream));
+		}
 	}
-	MC_TRY(sift_extract_device(ctx, d_feat_in, n_img, height, width, double_size, max_keypoints, d_xy, nullptr, d_desc, d_counts, d_offsets, 1));
-	if (n_cameras > 1) {
+	if (n_cameras == 1) MC_CUDA(cudaMemsetAsync(d_qimg, 0, nk * sizeof(int32_t), ctx->stream));     // one camera per frame: imageIdx = 0
+	for (RigGroup &g : groups) {
+		const uint8_t *d_feat_in = dev && g.packed ? cams[g.cams[0]].gray : g.d_gray;
+		if (g.table) {
+			MC_TRY(undistort_rig_device(ctx, g.cams, g.k, d_feat_in, (int)g.n, g.H, g.W, g.d_undist));
+			d_feat_in = g.d_undist;
+		}
+		MC_TRY(sift_extract_device(ctx, d_feat_in, (int)g.n, g.H, g.W, double_size, max_keypoints, g.d_xy, nullptr, g.d_desc, g.d_counts,
+		                           g.d_counts + g.n, 1));
+	}
+	if (merge) {
+		RigMerge m = {};
+		for (const RigGroup &g : groups)
+			for (int j = 0; j < g.k; ++j) {
+				const int c = g.cams[j];
+				m.counts[c] = g.d_counts + j;
+				m.offs[c] = g.d_counts + g.n + j;
+				m.xy[c] = g.d_xy;
+				m.desc[c] = g.d_desc;
+				m.k[c] = g.k;
+			}
+		k_rig_merge_scan<<<1, kMergeScanThreads, 0, ctx->stream>>>(m, n_cameras, n_img, d_counts, d_offsets);
+		MC_LAUNCH_CHECK();
+		k_rig_merge_interleave<<<dim3(n_img, kMergeSplit), kMergeThreads, 0, ctx->stream>>>(m, n_cameras, d_offsets, d_xy, d_desc, d_qimg);
+		MC_LAUNCH_CHECK();
+	} else if (n_cameras > 1) {
 		k_rig_image_index<<<n_img, 128, 0, ctx->stream>>>(d_offsets, n_cameras, d_qimg);
 		MC_LAUNCH_CHECK();
 	}
@@ -1167,7 +1372,9 @@ extern "C" mc_status mc_process_images(mc_ctx *ctx, const uint8_t *gray, int n_f
                                        const mc_pipeline_params *params, int max_objects, int32_t *n_objects, int32_t *obj_model, float *obj_pose,
                                        float *obj_score, int32_t *n_features, int32_t *frame_info, float *stage_ms) {
 	if (!ctx) return MC_ERR_ARG;
-	return process_images(ctx, "mc_process_images", gray, n_frames, 1, height, width, double_size, max_keypoints, params, max_objects, n_objects,
+	if (!gray) { ctx->err = "mc_process_images: bad argument"; return MC_ERR_ARG; }
+	const mc_rig_camera cam = { gray, (int64_t)height * width, height, width };
+	return process_images(ctx, "mc_process_images", &cam, 1, n_frames, false, double_size, max_keypoints, params, max_objects, n_objects,
 	                      obj_model, obj_pose, obj_score, n_features, frame_info, stage_ms);
 }
 
@@ -1176,16 +1383,32 @@ extern "C" mc_status mc_process_rig_images(mc_ctx *ctx, const uint8_t *gray, int
                                            int32_t *obj_model, float *obj_pose, float *obj_score, int32_t *n_features, int32_t *frame_info,
                                            float *stage_ms) {
 	if (!ctx) return MC_ERR_ARG;
-	if (n_cameras < 1 || n_cameras > kUndistortCameras) {
-		ctx->err = "mc_process_rig_images: n_cameras must be in 1.." + std::to_string(kUndistortCameras); return MC_ERR_ARG;
-	}
-	if ((int64_t)n_frames * n_cameras > 65535) { ctx->err = "mc_process_rig_images: more than 65535 images in a batch"; return MC_ERR_ARG; }
-	if (ctx->n_images < n_cameras) {
-		ctx->err = "mc_process_rig_images: " + std::to_string(n_cameras) + " cameras in the rig, " + std::to_string(ctx->n_images) +
-		           " set with mc_set_cameras";
-		return MC_ERR_STATE;
-	}
-	return process_images(ctx, "mc_process_rig_images", gray, n_frames, n_cameras, height, width, double_size, max_keypoints, params, max_objects,
+	MC_TRY(rig_check(ctx, "mc_process_rig_images", n_frames, n_cameras));
+	if (!gray) { ctx->err = "mc_process_rig_images: bad argument"; return MC_ERR_ARG; }
+	mc_rig_camera cams[kUndistortCameras];          // camera c of one [n_frames][n_cameras][height][width] buffer
+	const int64_t plane = (int64_t)height * width;
+	for (int c = 0; c < n_cameras; ++c) cams[c] = { gray + c * plane, n_cameras * plane, height, width };
+	return process_images(ctx, "mc_process_rig_images", cams, n_cameras, n_frames, false, double_size, max_keypoints, params, max_objects,
+	                      n_objects, obj_model, obj_pose, obj_score, n_features, frame_info, stage_ms);
+}
+
+extern "C" mc_status mc_process_rig_cameras(mc_ctx *ctx, const mc_rig_camera *cameras, int n_cameras, int n_frames, int double_size,
+                                            int max_keypoints, const mc_pipeline_params *params, int max_objects, int32_t *n_objects,
+                                            int32_t *obj_model, float *obj_pose, float *obj_score, int32_t *n_features, int32_t *frame_info,
+                                            float *stage_ms) {
+	if (!ctx) return MC_ERR_ARG;
+	MC_TRY(rig_check(ctx, "mc_process_rig_cameras", n_frames, n_cameras));
+	return process_images(ctx, "mc_process_rig_cameras", cameras, n_cameras, n_frames, false, double_size, max_keypoints, params, max_objects,
+	                      n_objects, obj_model, obj_pose, obj_score, n_features, frame_info, stage_ms);
+}
+
+extern "C" mc_status mc_process_rig_cameras_dev(mc_ctx *ctx, const mc_rig_camera *cameras, int n_cameras, int n_frames, int double_size,
+                                                int max_keypoints, const mc_pipeline_params *params, int max_objects, int32_t *n_objects,
+                                                int32_t *obj_model, float *obj_pose, float *obj_score, int32_t *n_features,
+                                                int32_t *frame_info, float *stage_ms) {
+	if (!ctx) return MC_ERR_ARG;
+	MC_TRY(rig_check(ctx, "mc_process_rig_cameras_dev", n_frames, n_cameras));
+	return process_images(ctx, "mc_process_rig_cameras_dev", cameras, n_cameras, n_frames, true, double_size, max_keypoints, params, max_objects,
 	                      n_objects, obj_model, obj_pose, obj_score, n_features, frame_info, stage_ms);
 }
 

@@ -98,28 +98,27 @@ static mc_status launch_camera(mc_ctx *ctx, const UndistortTable &t, const uint8
 	return launch_undistort(ctx, maps, 1, table_weights(t), d_in, B, t.height, t.width, d_out);
 }
 
-mc_status undistort_check_rig(mc_ctx *ctx, const char *who, int n_cameras, int H, int W, bool *any) {
-	*any = false;
+mc_status undistort_check_rig(mc_ctx *ctx, const char *who, int n_cameras, const int *H, const int *W, bool *has) {
 	for (int c = 0; c < n_cameras; c++) {
 		const UndistortTable &t = ctx->undistort[c];
-		if (!t.d_map) continue;
-		if (t.height != H || t.width != W) {
-			ctx->err = std::string(who) + ": images are " + std::to_string(W) + "x" + std::to_string(H) + ", camera " + std::to_string(c) +
+		has[c] = t.d_map != nullptr;
+		if (!has[c]) continue;
+		if (t.height != H[c] || t.width != W[c]) {
+			ctx->err = std::string(who) + ": images are " + std::to_string(W[c]) + "x" + std::to_string(H[c]) + ", camera " + std::to_string(c) +
 			           "'s undistortion table is " + std::to_string(t.width) + "x" + std::to_string(t.height);
 			return MC_ERR_ARG;
 		}
-		*any = true;
 	}
 	return MC_OK;
 }
 
-mc_status undistort_rig_device(mc_ctx *ctx, int n_cameras, const uint8_t *d_in, int B, int H, int W, uint8_t *d_out) {
+mc_status undistort_rig_device(mc_ctx *ctx, const int *cameras, int n_cameras, const uint8_t *d_in, int B, int H, int W, uint8_t *d_out) {
 	UndistortMaps maps = {};
 	const RemapWeights *wtab = nullptr;
-	for (int c = 0; c < n_cameras; c++) {
-		const UndistortTable &t = ctx->undistort[c];
+	for (int j = 0; j < n_cameras; j++) {
+		const UndistortTable &t = ctx->undistort[cameras[j]];
 		if (!t.d_map) continue;
-		maps.map[c] = table_map(t);
+		maps.map[j] = table_map(t);
 		wtab = table_weights(t);
 	}
 	if (!wtab) { ctx->err = "undistort: no camera of the rig has an undistortion table"; return MC_ERR_STATE; }
