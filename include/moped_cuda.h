@@ -484,6 +484,31 @@ mc_status mc_process_rig_cameras_dev(mc_ctx *ctx, const mc_rig_camera *cameras, 
                                      int max_keypoints, const mc_pipeline_params *params, int max_objects, int32_t *n_objects,
                                      int32_t *obj_model, float *obj_pose, float *obj_score, int32_t *n_features,
                                      int32_t *frame_info, float *stage_ms);
+/* FEAT alone for the frames mc_process_rig_cameras takes: the front half of that call (the upload or in-place read, the remap of each
+ * size group with a table, SIFT per size group and the merge into frame-major order), with the query arrays left in the caller's device
+ * buffers instead of going on to MATCH. No database is needed. For hosts that run MATCH themselves (an object-sharded database, see
+ * INTEGRATION.md §4c) or a step of their own between FEAT and MATCH (moped3d's DEPTHPROP before mc_process_depth_queries_dev).
+ *   q_desc_dev   n_frames x n_cameras x max_keypoints rows of 128 floats, 16-byte aligned: the descriptors, normalised with MATCH's
+ *                expression (the kernels store them as float4)
+ *   q_xy_dev     the same number of rows of 2 floats, 8-byte aligned (coord2D); q_image_dev the same number of ints (imageIdx = camera)
+ *                The call cannot see the buffers' sizes: each must hold all those rows, since SIFT writes up to max_keypoints per image
+ *                before the counts are known.
+ *   frame_offsets  host, n_frames + 1 ints: frame f owns rows [frame_offsets[f], frame_offsets[f+1]); rows from frame_offsets[n_frames]
+ *                on are unspecified
+ *   n_features   optional host, n_frames x n_cameras keypoint counts, frame-major; feat_ms optional host, 1 float: device time of FEAT
+ * The arrays are exactly what mc_process_rig_cameras hands to MATCH: mc_process_frames_dev on them returns what mc_process_rig_cameras
+ * returns, and the call issues that call's launches and copies before MATCH. The call synchronises the context's stream once, to read
+ * the offsets. Errors, all before any copy or launch: those of mc_process_rig_cameras except the database's and max_objects, plus
+ * MC_ERR_ARG for a NULL or misaligned q_desc_dev, q_xy_dev or q_image_dev and a NULL frame_offsets. An image with more than max_keypoints
+ * keypoints returns
+ * MC_ERR_CAPACITY; n_features still holds the numbers found. */
+mc_status mc_extract_rig_cameras(mc_ctx *ctx, const mc_rig_camera *cameras, int n_cameras, int n_frames, int double_size, int max_keypoints,
+                                 float *q_desc_dev, float *q_xy_dev, int32_t *q_image_dev, int32_t *frame_offsets, int32_t *n_features,
+                                 float *feat_ms);
+/* The same with every cameras[c].gray a device pointer, as mc_process_rig_cameras_dev reads them. */
+mc_status mc_extract_rig_cameras_dev(mc_ctx *ctx, const mc_rig_camera *cameras, int n_cameras, int n_frames, int double_size, int max_keypoints,
+                                     float *q_desc_dev, float *q_xy_dev, int32_t *q_image_dev, int32_t *frame_offsets, int32_t *n_features,
+                                     float *feat_ms);
 /* test/bench introspection: one plane of the scale-space left by the last extraction (stack 0 Gaussian 0..5, 1 DoG 0..4,
  * 2 gradient magnitude 0..2, 3 orientation 0..2); out may be NULL to query the octave's size. After a mc_process_rig_cameras*
  * call with cameras of several sizes it is the scale-space of the last size group's batch. */

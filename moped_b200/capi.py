@@ -130,6 +130,10 @@ SIGNATURES = {
                                          _f32p, _f32p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "mc_process_rig_cameras_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(PipelineParams), C.c_int, _i32p,
                                              _i32p, _f32p, _f32p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "mc_extract_rig_cameras": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int] + [C.c_void_p] * 3 + [_i32p, C.c_void_p,
+                                                                                                                    C.c_void_p]),
+    "mc_extract_rig_cameras_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int] + [C.c_void_p] * 3 + [_i32p, C.c_void_p,
+                                                                                                                        C.c_void_p]),
     "mc_sift_profile_read": (C.c_int, [C.c_void_p, C.POINTER(C.c_float), C.POINTER(C.c_double)]),
     "mc_sift_read_plane": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "mc_set_option": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int64]),
@@ -708,6 +712,45 @@ class Context:
         if want_times:
             out[0]["stage_ms"] = ms
         return out
+
+    def extract_rig_cameras(self, images, desc, xy, image, double_size=True, max_keypoints=4096, want_times=False, partial=False):
+        """mc_extract_rig_cameras: FEAT of process_rig_cameras alone; images = one uint8 array (n_frames, H_c, W_c) per camera c. The query
+        arrays go to the contiguous CUDA tensors desc (float32, rows of 128), xy (float32, rows of 2) and image (int32), each with room for
+        n_frames x n_cameras x max_keypoints rows. Returns (frame_offsets [n_frames + 1], n_features [n_frames, n_cameras], feat_ms or
+        None); partial=True appends the status and returns it for any failure of the call instead of raising."""
+        ims = [np.ascontiguousarray(g, dtype=np.uint8) for g in images]
+        cams = (RigCamera * len(ims))(*[RigCamera(g.ctypes.data, g.shape[1] * g.shape[2], g.shape[1], g.shape[2]) for g in ims])
+        return self._extract_rig("mc_extract_rig_cameras", cams, len(ims[0]), desc, xy, image, double_size, max_keypoints, want_times, partial)
+
+    def extract_rig_cameras_dev(self, ptrs, strides, sizes, n_frames, desc, xy, image, double_size=True, max_keypoints=4096,
+                                want_times=False, partial=False):
+        """mc_extract_rig_cameras_dev: the images as process_rig_cameras_dev takes them, the outputs as extract_rig_cameras."""
+        cams = (RigCamera * len(ptrs))(*[RigCamera(int(p), int(st), int(h), int(w)) for p, st, (h, w) in zip(ptrs, strides, sizes)])
+        return self._extract_rig("mc_extract_rig_cameras_dev", cams, n_frames, desc, xy, image, double_size, max_keypoints, want_times, partial)
+
+    @staticmethod
+    def _check_outputs(fn, rows, desc, xy, image):
+        """the output tensors hold rows rows of their kind on the device; the kernels store desc rows as float4 (16-byte aligned)"""
+        import torch
+        for name, t, dtype, width in (("desc", desc, torch.float32, 128), ("xy", xy, torch.float32, 2), ("image", image, torch.int32, 1)):
+            if not isinstance(t, torch.Tensor) or not t.is_cuda or t.dtype != dtype or not t.is_contiguous():
+                raise ValueError(f"{fn}: {name} must be a contiguous CUDA tensor of {dtype}")
+            if t.numel() < rows * width:
+                raise ValueError(f"{fn}: {name} holds {t.numel() // width} rows, {rows} needed (n_frames x n_cameras x max_keypoints)")
+        if desc.data_ptr() % 16 or xy.data_ptr() % 8:
+            raise ValueError(f"{fn}: desc must be 16-byte and xy 8-byte aligned")
+
+    def _extract_rig(self, fn, cams, B, desc, xy, image, double_size, max_keypoints, want_times, partial):
+        self._check_outputs(fn, max(B, 0) * len(cams) * max(max_keypoints, 0), desc, xy, image)
+        fo = np.zeros(max(B, 0) + 1, np.int32)
+        nf = np.zeros((max(B, 1), len(cams)), np.int32)
+        ms = np.zeros(1, np.float32)
+        st = getattr(self.L, fn)(self.h, C.cast(cams, C.c_void_p), len(cams), B, 1 if double_size else 0, max_keypoints, desc.data_ptr(),
+                                 xy.data_ptr(), image.data_ptr(), fo, nf.ctypes.data, ms.ctypes.data if want_times else None)
+        if st != 0 and not partial:
+            self._check(st, fn)
+        out = (fo, nf[:B], float(ms[0]) if want_times else None)
+        return out + (int(st),) if partial else out
 
     def set_undistortion(self, camera, K, kc, height, width):
         """mc_set_undistortion: UNDISTORTED_IMAGE for camera `camera` (K = (fx, fy, cx, cy), kc = (k1, k2, p1, p2[, k3])) on

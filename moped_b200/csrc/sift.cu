@@ -1224,22 +1224,19 @@ struct RigGroup {
 	int32_t *d_counts = nullptr;      // counts[n], then offsets[n + 1]
 };
 
-/* Images in, objects out (SURVEY.md 8f rows 1+3 chained): FEAT -> MATCH -> CLUSTER -> POSE -> FILTER -> POSE2 -> FILTER2 for a
- * batch of n_frames frames of n_cameras images each, camera c's images as cams[c] describes them, in host (dev = false) or device
- * memory. Cameras of one size run as one SIFT batch. The descriptors never leave HBM: the describe kernel writes them compacted
- * (image-major) and already normalised the way MATCH normalises its queries. With one size group, a frame's images follow each other
- * in camera order already; with several, two merge kernels interleave the groups' lists into that order. Only the per-image keypoint
- * counts and offsets (4 B each) come back to the host before MATCH is launched, because the frame partition of the query list is
- * host-side state of the batch driver. */
-static mc_status process_images(mc_ctx *ctx, const char *who, const mc_rig_camera *cams, int n_cameras, int n_frames, bool dev,
-                                int double_size, int max_keypoints, const mc_pipeline_params *params, int max_objects, int32_t *n_objects,
-                                int32_t *obj_model, float *obj_pose, float *obj_score, int32_t *n_features, int32_t *frame_info, float *stage_ms) {
+/* FEAT for a batch of n_frames frames of n_cameras images each, camera c's images as cams[c] describes them, in host (dev = false)
+ * or device memory: UNDISTORTED_IMAGE and SIFT per size group, then the frame-major query arrays (SURVEY.md 8f row 3). Cameras of one
+ * size run as one SIFT batch. The describe kernel writes the descriptors compacted (image-major) and already normalised the way MATCH
+ * normalises its queries. With one size group, a frame's images follow each other in camera order already; with several, two merge
+ * kernels interleave the groups' lists into that order. d_desc / d_xy / d_qimg are the caller's arrays of n_frames x n_cameras x
+ * max_keypoints rows, or NULL for arrays carved from the context's SIFT scratch (returned through the references). Only the per-image
+ * keypoint counts and offsets (4 B each) come back to the host, in the call's one synchronisation: frame_offsets[n_frames + 1] is the
+ * frame partition of the query list, host-side state of the batch driver. Every check is made before any copy or launch. */
+static mc_status extract_rig(mc_ctx *ctx, const char *who, const mc_rig_camera *cams, int n_cameras, int n_frames, bool dev, int double_size,
+                             int max_keypoints, float *&d_desc, float *&d_xy, int32_t *&d_qimg, int32_t *frame_offsets, int32_t *n_features,
+                             float *feat_ms) {
 	const std::string name(who);
-	if (!cams || !params || !n_objects || !obj_model || !obj_pose || !obj_score || n_frames < 1 || max_keypoints < 1 || max_objects < 1) {
-		ctx->err = name + ": bad argument"; return MC_ERR_ARG;
-	}
-	if (!ctx->d_db) { ctx->err = name + ": no database uploaded"; return MC_ERR_STATE; }
-	if (ctx->D != 128) { ctx->err = name + ": the database does not hold 128-d descriptors"; return MC_ERR_STATE; }
+	if (!cams || n_frames < 1 || max_keypoints < 1) { ctx->err = name + ": bad argument"; return MC_ERR_ARG; }
 	int H[kUndistortCameras], W[kUndistortCameras];
 	std::vector<RigGroup> groups;
 	for (int c = 0; c < n_cameras; ++c) {
@@ -1287,16 +1284,18 @@ static mc_status process_images(mc_ctx *ctx, const char *who, const mc_rig_camer
 	MC_TRY(sift_reserve(ctx, s, need));
 	const int n_img = n_frames * n_cameras;
 	const size_t nk = (size_t)n_img * max_keypoints;
-	float *d_xy = nullptr, *d_desc = nullptr;
-	int32_t *d_qimg = nullptr, *d_counts = nullptr;
+	const bool own = !d_desc;                           // the query arrays live in the context's scratch
+	int32_t *d_counts = nullptr;
 	MC_TRY(carve_scratch(ctx, s->gray, [&](Carve &c) {
 		for (RigGroup &g : groups) {
 			c.take(g.d_gray, dev && g.packed ? 0 : g.npx);     // device images in the batch layout are read where they are
 			c.take(g.d_undist, g.table ? g.npx : 0);
 		}
-		c.take(d_xy, nk * 2);
-		c.take(d_desc, nk * 128);
-		c.take(d_qimg, nk);
+		if (own) {
+			c.take(d_xy, nk * 2);
+			c.take(d_desc, nk * 128);
+			c.take(d_qimg, nk);
+		}
 		c.take(d_counts, (size_t)2 * n_img + 2);          // counts[n_img], then offsets[n_img + 1], frame-major
 		for (RigGroup &g : groups) {                      // with several groups each has its own list, merged into the arrays above
 			const size_t gk = merge ? g.n * max_keypoints : 0;
@@ -1309,7 +1308,7 @@ static mc_status process_images(mc_ctx *ctx, const char *who, const mc_rig_camer
 	if (!merge) { groups[0].d_xy = d_xy; groups[0].d_desc = d_desc; groups[0].d_counts = d_counts; }
 	MC_TRY(pinned(ctx, (size_t)(2 * n_img + 2) * sizeof(int32_t)));
 	cudaEvent_t ev[2];
-	if (stage_ms) { MC_CUDA(cudaEventCreate(&ev[0])); MC_CUDA(cudaEventCreate(&ev[1])); MC_CUDA(cudaEventRecord(ev[0], ctx->stream)); }
+	if (feat_ms) { MC_CUDA(cudaEventCreate(&ev[0])); MC_CUDA(cudaEventCreate(&ev[1])); MC_CUDA(cudaEventRecord(ev[0], ctx->stream)); }
 	const cudaMemcpyKind kind = dev ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
 	for (RigGroup &g : groups) {                          // each group's batch: one copy when it is packed, else one per camera
 		const size_t plane = (size_t)g.H * g.W;
@@ -1351,17 +1350,35 @@ static mc_status process_images(mc_ctx *ctx, const char *who, const mc_rig_camer
 	}
 	int32_t *h = (int32_t *)ctx->h_pinned;
 	MC_CUDA(cudaMemcpyAsync(h, d_counts, (size_t)(2 * n_img + 1) * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
-	if (stage_ms) MC_CUDA(cudaEventRecord(ev[1], ctx->stream));
+	if (feat_ms) MC_CUDA(cudaEventRecord(ev[1], ctx->stream));
 	MC_CUDA(cudaStreamSynchronize(ctx->stream));
-	if (stage_ms) { cudaEventElapsedTime(&stage_ms[0], ev[0], ev[1]); cudaEventDestroy(ev[0]); cudaEventDestroy(ev[1]); }
-	std::vector<int32_t> offsets(n_frames + 1);       // frame f = images [f * n_cameras, (f + 1) * n_cameras)
-	for (int f = 0; f <= n_frames; ++f) offsets[f] = h[n_img + f * n_cameras];
+	if (feat_ms) { cudaEventElapsedTime(feat_ms, ev[0], ev[1]); cudaEventDestroy(ev[0]); cudaEventDestroy(ev[1]); }
+	for (int f = 0; f <= n_frames; ++f) frame_offsets[f] = h[n_img + f * n_cameras];     // frame f = images [f * n_cameras, (f + 1) * n_cameras)
 	bool overflow = false;
 	for (int i = 0; i < n_img; ++i) {
 		if (n_features) n_features[i] = h[i];
 		overflow |= h[i] > max_keypoints;
 	}
 	if (overflow) { ctx->err = name + ": more keypoints than max_keypoints in a frame (n_features[] holds the numbers found)"; return MC_ERR_CAPACITY; }
+	return MC_OK;
+}
+
+/* Images in, objects out (SURVEY.md 8f rows 1+3 chained): extract_rig into the context's scratch, then MATCH -> CLUSTER -> POSE ->
+ * FILTER -> POSE2 -> FILTER2. The descriptors never leave HBM. */
+static mc_status process_images(mc_ctx *ctx, const char *who, const mc_rig_camera *cams, int n_cameras, int n_frames, bool dev,
+                                int double_size, int max_keypoints, const mc_pipeline_params *params, int max_objects, int32_t *n_objects,
+                                int32_t *obj_model, float *obj_pose, float *obj_score, int32_t *n_features, int32_t *frame_info, float *stage_ms) {
+	const std::string name(who);
+	if (!cams || !params || !n_objects || !obj_model || !obj_pose || !obj_score || n_frames < 1 || max_keypoints < 1 || max_objects < 1) {
+		ctx->err = name + ": bad argument"; return MC_ERR_ARG;
+	}
+	if (!ctx->d_db) { ctx->err = name + ": no database uploaded"; return MC_ERR_STATE; }
+	if (ctx->D != 128) { ctx->err = name + ": the database does not hold 128-d descriptors"; return MC_ERR_STATE; }
+	float *d_desc = nullptr, *d_xy = nullptr;
+	int32_t *d_qimg = nullptr;
+	std::vector<int32_t> offsets(n_frames + 1);
+	MC_TRY(extract_rig(ctx, who, cams, n_cameras, n_frames, dev, double_size, max_keypoints, d_desc, d_xy, d_qimg, offsets.data(), n_features,
+	                   stage_ms));
 	return process_frames_host(ctx, d_desc, d_xy, d_qimg, offsets.data(), n_frames, params, max_objects, n_objects, obj_model, obj_pose, obj_score,
 	                           frame_info, stage_ms ? stage_ms + 1 : nullptr);
 }
@@ -1410,6 +1427,33 @@ extern "C" mc_status mc_process_rig_cameras_dev(mc_ctx *ctx, const mc_rig_camera
 	MC_TRY(rig_check(ctx, "mc_process_rig_cameras_dev", n_frames, n_cameras));
 	return process_images(ctx, "mc_process_rig_cameras_dev", cameras, n_cameras, n_frames, true, double_size, max_keypoints, params, max_objects,
 	                      n_objects, obj_model, obj_pose, obj_score, n_features, frame_info, stage_ms);
+}
+
+static mc_status extract_rig_cameras(mc_ctx *ctx, const char *who, const mc_rig_camera *cameras, int n_cameras, int n_frames, bool dev,
+                                     int double_size, int max_keypoints, float *q_desc_dev, float *q_xy_dev, int32_t *q_image_dev,
+                                     int32_t *frame_offsets, int32_t *n_features, float *feat_ms) {
+	if (!ctx) return MC_ERR_ARG;
+	MC_TRY(rig_check(ctx, who, n_frames, n_cameras));
+	if (!q_desc_dev || !q_xy_dev || !q_image_dev || !frame_offsets) { ctx->err = std::string(who) + ": bad argument"; return MC_ERR_ARG; }
+	if ((uintptr_t)q_desc_dev % 16 || (uintptr_t)q_xy_dev % 8 || (uintptr_t)q_image_dev % 4) {     // float4 / float2 / int stores
+		ctx->err = std::string(who) + ": q_desc_dev must be 16-byte, q_xy_dev 8-byte and q_image_dev 4-byte aligned"; return MC_ERR_ARG;
+	}
+	return extract_rig(ctx, who, cameras, n_cameras, n_frames, dev, double_size, max_keypoints, q_desc_dev, q_xy_dev, q_image_dev, frame_offsets,
+	                   n_features, feat_ms);
+}
+
+extern "C" mc_status mc_extract_rig_cameras(mc_ctx *ctx, const mc_rig_camera *cameras, int n_cameras, int n_frames, int double_size,
+                                            int max_keypoints, float *q_desc_dev, float *q_xy_dev, int32_t *q_image_dev, int32_t *frame_offsets,
+                                            int32_t *n_features, float *feat_ms) {
+	return extract_rig_cameras(ctx, "mc_extract_rig_cameras", cameras, n_cameras, n_frames, false, double_size, max_keypoints, q_desc_dev, q_xy_dev,
+	                           q_image_dev, frame_offsets, n_features, feat_ms);
+}
+
+extern "C" mc_status mc_extract_rig_cameras_dev(mc_ctx *ctx, const mc_rig_camera *cameras, int n_cameras, int n_frames, int double_size,
+                                                int max_keypoints, float *q_desc_dev, float *q_xy_dev, int32_t *q_image_dev, int32_t *frame_offsets,
+                                                int32_t *n_features, float *feat_ms) {
+	return extract_rig_cameras(ctx, "mc_extract_rig_cameras_dev", cameras, n_cameras, n_frames, true, double_size, max_keypoints, q_desc_dev, q_xy_dev,
+	                           q_image_dev, frame_offsets, n_features, feat_ms);
 }
 
 /* With mc_set_profiling on: device time (ms, summed) of the five octave-0 Gaussian+DoG launches of the last extraction and
